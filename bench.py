@@ -2,6 +2,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # this repo's CUDA path
     python bench.py --impl reference --steps K --warmup W    # the reference's own CPU modules (oracle/_ref)
+    python bench.py ... --dump-outputs DIR                   # also writes the last timed step's outputs as DIR/*.npy
 
 Prints ONE JSON line (rank 0).  A "step" is one pass of the hot path over one batch of synthetic
 tracks: BASELINE.json configs[1] (15,000 tracks x 10 frames vs 15,000 shop items, k=20) at N=1.
@@ -250,7 +251,7 @@ class Workload:
         if world > 1 and G_total > 0 and self.peer is None:
             self.retr = pkg.ShardedRetriever(eng, self.gallery, self.glo)
         self.graph = None
-        self.graph_out = None
+        self.last_out = None             # what the last step returned (the graph's static outputs when replayed)
         self.stamps = None
 
     # one pass of the hot path, inputs resident in HBM
@@ -259,7 +260,7 @@ class Workload:
         if self.G == 0:                                               # aggregation only (cfg 4)
             return eng.aggregate(self.seq, self.mask)
         if self.world == 1:
-            return eng.search(self.seq, self.mask, self.gallery, self.k)[1:]     # one library call (seam_search)
+            return eng.search(self.seq, self.mask, self.gallery, self.k)     # one library call (seam_search)
         if self.peer is not None:
             return self.retr.search_peer(self.seq, self.mask, self.peer)
         return self.retr.search(self.seq, self.mask, self.k)        # NCCL all-gather fallback (eager)
@@ -290,15 +291,16 @@ class Workload:
                 self.stamps = torch.zeros(2, dtype=torch.int64, device=dev)
                 self.peer.device_barrier()
                 self.eng.device_stamp(self.stamps, 0)
-            self.graph_out = self.hot_path()
+            self.last_out = self.hot_path()
             if self.world > 1:
                 self.eng.device_stamp(self.stamps, 1)
 
     def step(self):
         if self.graph is not None:
             self.graph.replay()
-            return self.graph_out
-        return self.hot_path()
+        else:
+            self.last_out = self.hot_path()
+        return self.last_out
 
     def launch_note(self):
         if self.graph is not None:
@@ -306,8 +308,21 @@ class Workload:
         return "eager launches" + (" + NCCL all-gathers" if self.world > 1 else "")
 
     def free(self):
-        self.graph = self.graph_out = self.peer = self.retr = self.gallery = self.gal = self.seq = None
+        self.graph = self.last_out = self.peer = self.retr = self.gallery = self.gal = self.seq = None
         torch.cuda.empty_cache()
+
+
+def dump_outputs(out_dir, outputs):
+    """<out_dir>/<name>.npy for each array the timed step returned to its caller: on one GPU seam_search's
+    descriptors (Q,256) and the (Q,k) scores, margins and gallery indices (about 20 MB); sharded, the (Q,k) three.
+    Indices are stored as float64, which holds every int32 exactly.  The inputs come from fixed seeds, so two builds
+    run with the same arguments can be compared output for output."""
+    import numpy as np
+    names = ("descriptors", "scores", "margins", "indices")[-len(outputs):]
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in zip(names, outputs):
+        a = t.cpu().numpy().astype(np.float64 if name == "indices" else np.float32)
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def stage_record(wl, kern, ms, peaks):
@@ -416,6 +431,8 @@ def run_ours(args):
     sampler = ClockSampler(local)                             # samples through the device-timed AND the e2e timed regions
     sampler.start()
     ms = timed(wl.step, args.steps, warmup, wl.stamps if wl.graph is not None else None)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, wl.last_out)
     rank_alignment = ("the replayed graph is [cross-rank barrier kernel, device time stamp, step, device time stamp]: the GPUs "
                       "enter the step together and the step is timed between the stamps (host launch skew is not step time)"
                       if (wl.graph is not None and wl.stamps is not None) else None)
@@ -626,7 +643,7 @@ def parity_check(pkg, eng, wl, res, e2e_idx, weights, world, rank, dev):
     single-GPU search of the whole gallery; (iii) the end-to-end leg returned the same indices.  Rank 0 does the
     checking; the other ranks only contribute their gallery shards."""
     import torch.distributed as dist
-    sc, mg, ix = res
+    sc, mg, ix = res[-3:]
     launch = wl.launch_note()
     par = "single GPU"
     if world > 1:
@@ -679,7 +696,13 @@ def main():
     ap.add_argument("--steps", type=int, default=30)
     ap.add_argument("--warmup", type=int, default=5)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step returned as DIR/<name>.npy (CUDA path)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to the CUDA path (--impl ours)")
     if args.impl == "reference":
         run_reference(args)
     else:
