@@ -30,4 +30,4 @@ if G:
     extra = (f" | P={plan['ctas_per_query_tile']} cap={plan['list_capacity']} sublist max={int(cn.max())} "
              f"row total mean={cn.sum(1).mean():.0f} max={int(cn.sum(1).max())} fallback_rows={int(st[0])} "
              f"ws={plan['bytes'] / 2**20:.0f} MiB")
-print(f"Q={Q} T={T} G={G} nseed={os.environ.get('SEAM_SCORE_NSEED','-')} mode={os.environ.get('SEAM_DEBUG_SCORE_MODE','0')}: " + ", ".join(f"{k}={v[0]/v[1]*1e3:.1f}us" for k, v in pr.items() if v[1]) + extra)
+print(f"Q={Q} T={T} G={G}: " + ", ".join(f"{k}={v[0]/v[1]*1e3:.1f}us" for k, v in pr.items() if v[1]) + extra)

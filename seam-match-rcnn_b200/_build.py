@@ -17,10 +17,6 @@ SOURCES = ["seam_b200.cu"]
 HEADERS = sorted(f for f in os.listdir(CSRC) if f.endswith(".cuh"))   # every header goes into the content hash
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
               "-shared", "-Xcompiler", "-fPIC"]
-# SEAM_BUILD_DIAGNOSTICS=1 also compiles the scorer's measurement variants (partial epilogues, selected at
-# run time with SEAM_DEBUG_SCORE_MODE=1..5; they return wrong results and are not part of a product build)
-if os.environ.get("SEAM_BUILD_DIAGNOSTICS", "0") == "1":
-    NVCC_FLAGS = NVCC_FLAGS + ["-DSEAM_DIAGNOSTIC_VARIANTS"]
 
 
 def _nvcc() -> str:
@@ -48,17 +44,6 @@ def is_stale() -> bool:
         return True
     with open(INFO_PATH) as f:
         return f.read().strip() != source_hash()
-
-
-def build_variant(name: str, defines) -> str:
-    """Developer A/B builds: the library compiled with extra -D flags into libseam_b200.<name>.so (selected at
-    run time with SEAM_B200_LIB=<path>).  Never used by the product path."""
-    out = os.path.join(HERE, f"libseam_b200.{name}.so")
-    cmd = [_nvcc()] + NVCC_FLAGS + [f"-D{d}" for d in defines] + ["-o", out] + [os.path.join(CSRC, s) for s in SOURCES]
-    proc = subprocess.run(cmd, capture_output=True, text=True)
-    if proc.returncode != 0:
-        raise RuntimeError("nvcc failed:\n" + " ".join(cmd) + "\n" + proc.stdout + proc.stderr)
-    return out
 
 
 def build(force: bool = False, verbose: bool = False) -> str:

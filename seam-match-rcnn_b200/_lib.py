@@ -167,9 +167,6 @@ def load(build_if_missing: bool = True) -> C.CDLL:
     if _lib is not None:
         return _lib
     path = _build.LIB_PATH
-    override = os.environ.get("SEAM_B200_LIB")          # developer A/B builds (scripts/build_variants.py)
-    if override:
-        path, build_if_missing = override, False
     if build_if_missing:
         try:
             _build.build()

@@ -97,39 +97,6 @@ __device__ __forceinline__ float* local_out(const Params& p, uint32_t xstep) {
 
 using ptx::treduce;
 
-// developer diagnostic (SEAM_AGG_TIMELINE builds only; the attention output is sacrificed): per-CTA
-// globaltimer stamps at slots 0..7 of an 8 x u64 record in the att buffer
-#ifdef SEAM_AGG_TIMELINE
-#define SEAM_TL(p, slot) do { if ((p).att && lane == 0) reinterpret_cast<unsigned long long*>((p).att)[blockIdx.x * 8 + (slot)] = ptx::globaltimer_ns(); } while (0)
-#else
-#define SEAM_TL(p, slot) do { } while (0)
-#endif
-#ifdef SEAM_AGG_TIMELINE3
-#define SEAM_TL3(p, slot) do { if ((p).att && lane == 0) reinterpret_cast<unsigned long long*>((p).att)[blockIdx.x * 8 + (slot)] = ptx::globaltimer_ns(); } while (0)
-#else
-#define SEAM_TL3(p, slot) do { } while (0)
-#endif
-#ifdef SEAM_AGG_TIMELINE2
-#define SEAM_TL2(p, slot) do { if ((p).att && lane == 0) reinterpret_cast<unsigned long long*>((p).att)[blockIdx.x * 8 + (slot)] = ptx::globaltimer_ns(); } while (0)
-#else
-#define SEAM_TL2(p, slot) do { } while (0)
-#endif
-
-// developer diagnostic (SEAM_AGG_PHASES builds; the attention output is sacrificed): clock64 deltas of producer warp 0
-// per phase of the long-track kernel's iteration, summed over its iterations, 16 x i64 per CTA in the att buffer
-#ifdef SEAM_AGG_PHASES
-#define SEAM_PH(i) do { if (warp == 0 && lane == 0) { const long long t_ = clock64(); s.phase[i] += t_ - ph_prev; ph_prev = t_; } } while (0)
-#else
-#define SEAM_PH(i) do { } while (0)
-#endif
-
-// the same for the short-track kernel at TR = 10 (the counters live in the unused tail of warp 0's scalar block)
-#ifdef SEAM_AGG_PHASES
-#define SEAM_WPH(i) do { if (TR == 10 && warp == 0 && lane == 0) { const long long t_ = clock64(); reinterpret_cast<long long*>(scal + 40)[i] += t_ - ph_prev; ph_prev = t_; } } while (0)
-#else
-#define SEAM_WPH(i) do { } while (0)
-#endif
-
 // ---- packed fp32 pairs (FFMA2 / FMUL2): the streaming pass is bound by instruction issue
 typedef unsigned long long u64;
 __device__ __forceinline__ u64 pk(float lo, float hi) {
@@ -244,11 +211,6 @@ __device__ __forceinline__ void store_r2(uint8_t* rt, int pos, int c, float r0, 
 // to the NWARPS / 4 warps that share it, two chunks (32 coalesced loads per thread) in flight at a time.
 // A serial load by the four helper warps alone took 22 dependent round trips (~17 us, the floor of the
 // kernel at small Q); producers do their share while their first frames are in flight.
-#ifdef SEAM_AGG_HELPER_INIT      // developer A/B: the helper warps alone load M
-#define SEAM_AGG_INIT_WARPS(all) HELPER_WARPS
-#else
-#define SEAM_AGG_INIT_WARPS(all) (all)
-#endif
 template <int NWARPS, int INFLIGHT>
 __device__ __forceinline__ void load_m_tmem(const Params& p, Meta* meta, int warp, int lane) {
   constexpr int NPART = NWARPS / 4, NCHUNK = 16 + 2 * (KT / 32);
@@ -323,11 +285,7 @@ __device__ __forceinline__ void helper_role(const Params& p, uint8_t* fz, int hw
     const long long f = first0 + u;
     if (f < p.Q) n_cta += (p.Q - f + stride - 1) / stride;
   }
-#if defined(SEAM_AGG_DIAG_NO_PUBLISH) || defined(SEAM_AGG_GDIAG)    // developer diagnostic (wrong results): streaming pass alone
-  const int nbatch = 0;
-#else
   const int nbatch = (int)((n_cta + NB - 1) / NB);
-#endif
   const float ms_inv = p.fold[Fold::CONSTS + 9];        // 1 / S
   const bool mc = p.x_on && p.x.world > 1 && p.x.q_all_mc != nullptr;
   const uint32_t rt_addr = ptx::smem_u32(fz + OFF_RT), tail_addr = ptx::smem_u32(fz + OFF_TAIL);
@@ -344,9 +302,6 @@ __device__ __forceinline__ void helper_role(const Params& p, uint8_t* fz, int hw
       if constexpr (POOL_SMEM) ptx::mbar_wait(&meta->tile_full[buf], (uint32_t)(b >> 1) & 1u, 102);   // short tracks: a batch every few us
       else ptx::mbar_wait_idle(&meta->tile_full[buf], (uint32_t)(b >> 1) & 1u, IDLE_NS, 102);          // long tracks: tens of us away
       if (b == 0) ptx::mbar_wait(&meta->m_ready, 0u, 108);
-      if (b == 0) SEAM_TL(p, 3);
-      if (b == 3) SEAM_TL3(p, 0);
-      if (b == 4) SEAM_TL3(p, 5);
       ptx::tc_fence_after();
       if (ptx::elect_one()) {
         const uint32_t r1 = rt_addr + buf * RT_BYTES, r2 = r1 + RT_TERM_BYTES;
@@ -354,11 +309,7 @@ __device__ __forceinline__ void helper_role(const Params& p, uint8_t* fz, int hw
         for (int h = 0; h < 2; ++h) {
           const uint32_t d = tmem + COL_D + h * NB;
 #pragma unroll
-#ifdef SEAM_AGG_DIAG_NO_MMA      // developer diagnostic (wrong results): one MMA per half instead of 48
-          for (int ks = 0; ks < 1; ++ks) {
-#else
           for (int ks = 0; ks < 16; ++ks) {               // k-steps of 16
-#endif
             const uint32_t boff = (uint32_t)(ks >> 2) * (NB * 128) + (uint32_t)(ks & 3) * 32;
             const uint64_t b1 = ptx::umma_desc_k_sw128(r1 + boff), b2 = ptx::umma_desc_k_sw128(r2 + boff);
             const uint32_t a1 = tmem + COL_M1 + h * 128 + ks * 8;
@@ -373,27 +324,17 @@ __device__ __forceinline__ void helper_role(const Params& p, uint8_t* fz, int hw
           }
         }
         ptx::umma_commit(&meta->acc_full);
-        if (b == 0) SEAM_TL(p, 4);
-        if (b == nbatch - 1) SEAM_TL(p, 5);
       }
-      if (b == 3) SEAM_TL3(p, 1);
       __syncwarp();
     }
     // ---------------------------------------------------- read-back: thread = channel, register = track
     // Only warp 0 polls (the batch above, then its own MMAs: a few hundred ns); the other three helper warps wait at a
     // hardware barrier, which costs no issue slots (four polling warps executed ~10 % of the kernel's instructions).
     // The barrier also hands on what warp 0 acquired from the producers (slot_track, fscale, pooled').
-#ifdef SEAM_AGG_POLL      // developer A/B: every helper warp polls
-    ptx::mbar_wait(&meta->acc_full, (uint32_t)b & 1u, 103);
-    ptx::mbar_wait(&meta->tile_full[buf], (uint32_t)(b >> 1) & 1u, 104);
-    ptx::tc_fence_after();
-#else
     if (hw == 0) ptx::mbar_wait(&meta->acc_full, (uint32_t)b & 1u, 103);
-    if (hw == 0 && b == 3) SEAM_TL3(p, 2);
     ptx::tc_fence_before();
     ptx::named_bar_sync(6, HELPER_WARPS * 32);
     ptx::tc_fence_after();
-#endif
     uint32_t d0[16], d1[16];
     ptx::tmem_ld_x16(lane_base + COL_D, d0);
     ptx::tmem_ld_x16(lane_base + COL_D + NB, d1);
@@ -401,7 +342,6 @@ __device__ __forceinline__ void helper_role(const Params& p, uint8_t* fz, int hw
     ptx::tmem_ld_wait_x16(d1);
     ptx::tc_fence_before();
     ptx::named_bar_sync(1, HELPER_WARPS * 32);           // the accumulator may be overwritten by the next batch
-    if (hw == 0 && b == 3) SEAM_TL3(p, 3);
     const int ch = hw * 32 + lane;
     const float* pool = reinterpret_cast<const float*>(fz + OFF_POOL + buf * POOL_BYTES);
 #pragma unroll
@@ -464,8 +404,6 @@ __device__ __forceinline__ void helper_role(const Params& p, uint8_t* fz, int hw
     }
     __syncwarp();
     if (lane == 0) ptx::mbar_arrive(&meta->buf_free[buf]);
-    if (hw == 0 && b == nbatch - 1) SEAM_TL(p, 6);
-    if (hw == 0 && b == 3) SEAM_TL3(p, 4);
   }
   if constexpr (POOL_SMEM) {
     if (p.x_on && p.x.world > 1 && !mc) {                // this thread's remote rows are written before the CTA is counted
@@ -485,7 +423,7 @@ __device__ __forceinline__ void fused_setup(uint8_t* fz, int warp, int helper0, 
       ptx::mbar_init(&meta->buf_free[i], HELPER_WARPS);
     }
     ptx::mbar_init(&meta->acc_full, 1);
-    ptx::mbar_init(&meta->m_ready, SEAM_AGG_INIT_WARPS(m_warps));
+    ptx::mbar_init(&meta->m_ready, m_warps);
     meta->next_slot = 0u;
     ptx::fence_mbar_init();
   }
@@ -525,9 +463,6 @@ struct Cfg<10> { static constexpr int NW = 11, SLOTS = 1, LOADER = 1, REGS_P = 1
 template <>
 struct Cfg<16> { static constexpr int NW = 8, SLOTS = 1, LOADER = 0, REGS_P = 224, REGS_H = 56; };
 
-#ifndef SEAM_AGG_M_INFLIGHT
-#define SEAM_AGG_M_INFLIGHT 4
-#endif
 template <int TR>
 constexpr size_t warp_smem_bytes() {
   return 1024 + fused_bytes<true>() + (size_t)Cfg<TR>::NW * Cfg<TR>::SLOTS * TR * D * 4   // track buffers
@@ -545,7 +480,7 @@ aggregate_fused_warp_kernel(const __grid_constant__ CUtensorMap tmSeq, const Par
   constexpr int NW = Cfg<TR>::NW, SLOTS = Cfg<TR>::SLOTS;
   constexpr bool LOADER = Cfg<TR>::LOADER != 0;
   static_assert(!LOADER || SLOTS == 1, "the loader warp serves single-buffer producers");
-  constexpr int M_INFLIGHT = TR >= 10 ? SEAM_AGG_M_INFLIGHT : 2;     // chunks of M a producer warp has in flight at start
+  constexpr int M_INFLIGHT = TR >= 10 ? 4 : 2;     // chunks of M a producer warp has in flight at start
   extern __shared__ uint8_t smem_raw[];
   const uint32_t raw_addr = ptx::smem_u32(smem_raw);
   uint8_t* fz = smem_raw + (((raw_addr + 1023u) & ~1023u) - raw_addr);        // fused area (1 KB aligned), then producers
@@ -575,8 +510,6 @@ aggregate_fused_warp_kernel(const __grid_constant__ CUtensorMap tmSeq, const Par
     ptx::mbar_init(&empty_all[warp], 1);
     ptx::fence_mbar_init();
   }
-  if (warp == 0) SEAM_TL(p, 0);
-  if (warp == 0) SEAM_TL2(p, 0);
   __syncwarp();
   const int Tmax = p.Tmax;
   const long long first = first0 + warp;
@@ -618,11 +551,7 @@ aggregate_fused_warp_kernel(const __grid_constant__ CUtensorMap tmSeq, const Par
       __syncwarp();
     } else if (lane < len) {
       const float* src = p.seq + (long long)(lane + 1) * p.frame_stride + track * p.track_stride;
-#ifdef SEAM_AGG_NO_HINT
-      ptx::bulk_load_1d(xbuf + ((size_t)slot * TR + lane) * D, src, D * 4, &bars[slot]);
-#else
       ptx::bulk_load_1d_hint(xbuf + ((size_t)slot * TR + lane) * D, src, D * 4, &bars[slot], pol);
-#endif
     }
   };
 
@@ -636,7 +565,6 @@ aggregate_fused_warp_kernel(const __grid_constant__ CUtensorMap tmSeq, const Par
     raw_next = peek(first + (long long)AHEAD * stride);
   }
   fused_setup<1>(fz, warp, NW, NW + HELPER_WARPS + Cfg<TR>::LOADER);
-  if (warp == 0) SEAM_TL2(p, 1);
 
   if (LOADER && warp == NW + HELPER_WARPS) {
     // ------------------------------------------------------------------------------ loader warp: lane w serves producer w
@@ -697,13 +625,7 @@ aggregate_fused_warp_kernel(const __grid_constant__ CUtensorMap tmSeq, const Par
     helper_role<1, true>(p, fz, warp & 3, lane, NW, first0, stride, out_local, xstep);
   } else {
     ptx::reg_inc<Cfg<TR>::REGS_P>();
-    if (warp == 0) SEAM_TL2(p, 2);
-    if (warp == 0) SEAM_TL2(p, 3);
-#ifndef SEAM_AGG_HELPER_INIT
     load_m_tmem<NW + HELPER_WARPS + Cfg<TR>::LOADER, M_INFLIGHT>(p, meta, warp, lane);   // while the first frames are in flight
-    if (warp == 0) SEAM_TL(p, 1);
-    if (warp == 0) SEAM_TL2(p, 4);
-#endif
 
     const float* fold = p.fold;
     const Vec8 ut = load_vec8(fold + Fold::U_THETA, lane);
@@ -717,14 +639,8 @@ aggregate_fused_warp_kernel(const __grid_constant__ CUtensorMap tmSeq, const Par
                          : comp == 3 ? fold[Fold::CONSTS + 2] : 0.f;
 
     int it = 0;
-#ifdef SEAM_AGG_PHASES
-    long long ph_prev = clock64();
-    if (TR == 10 && warp == 0 && lane < 24) scal[40 + lane] = 0.f;
-    __syncwarp();
-#endif
 #pragma unroll 1
     for (long long track = first; track < p.Q; track += stride, ++it) {
-      SEAM_WPH(0);
       const int slot = it % SLOTS;
       const uint32_t phase = (uint32_t)(it / SLOTS) & 1u;
       if constexpr (SLOTS > 1) {
@@ -733,11 +649,6 @@ aggregate_fused_warp_kernel(const __grid_constant__ CUtensorMap tmSeq, const Par
         raw_next = peek(track + (long long)SLOTS * stride);
       }
       ptx::mbar_wait(&bars[slot], phase, 105);
-      SEAM_WPH(1);
-      if (warp == 0 && it == 0) SEAM_TL(p, 2);
-      if (warp == 0 && it == 0) SEAM_TL2(p, 5);
-      if (warp == 0 && it == 1) SEAM_TL2(p, 6);
-      if (warp == 0 && it == 2) SEAM_TL2(p, 7);
       const int len = slot_len[slot];
       const float* xs = xbuf + (size_t)slot * TR * D;
 
@@ -750,9 +661,7 @@ aggregate_fused_warp_kernel(const __grid_constant__ CUtensorMap tmSeq, const Par
         // the track's slot in the batch under construction: the shared-memory atomic's round trip (~200 cycles) is
         // started here and used after the weighted sums
         unsigned ticket = 0u;
-#ifndef SEAM_AGG_DIAG_NO_PUBLISH
         if (lane == 0) ticket = atomicAdd(&meta->next_slot, 1u);
-#endif
         Vec8 x[TR];
 #pragma unroll
         for (int t0 = 0; t0 < TR; t0 += 8) {            // 8 frames = 32 totals per butterfly: the 5 dependent shuffle rounds
@@ -788,7 +697,6 @@ aggregate_fused_warp_kernel(const __grid_constant__ CUtensorMap tmSeq, const Par
           }
           if (lane < 4 * nf) scal[4 * t0 + lane] = tot + my_const;
         }
-        SEAM_WPH(2);
         if constexpr (SLOTS == 1) {
           __syncwarp();                                // all lanes hold their frames in registers:
           if constexpr (LOADER) {
@@ -799,7 +707,6 @@ aggregate_fused_warp_kernel(const __grid_constant__ CUtensorMap tmSeq, const Par
           }
         }
         __syncwarp();
-        SEAM_WPH(3);
 
         // ---- attention over the track's frames (lane = frame)
         const int L = FULL ? TR : len;
@@ -822,7 +729,6 @@ aggregate_fused_warp_kernel(const __grid_constant__ CUtensorMap tmSeq, const Par
         __syncwarp();                                    // all lanes have read b, c, d
         if (lane < TR) scal[4 * lane + 1] = e_t;         // d -> e
         __syncwarp();
-        SEAM_WPH(4);
         // One loop gives the softmax denominator (every lane sums the e_t itself: no reduction) and the second
         // interaction q_j = sum_t p_t relu(a_t + b_j) / T, p_t = e_t / z.
         float z = 0.f, q_j = 0.f;
@@ -837,12 +743,9 @@ aggregate_fused_warp_kernel(const __grid_constant__ CUtensorMap tmSeq, const Par
         q_j = (many && valid) ? q_j * inv_len * inv_z : 0.f;
         __syncwarp();                                    // all lanes have read the a_t, e_t
         if (lane < TR) *reinterpret_cast<float4*>(scal + 4 * lane) = make_float4(p_t, p_t, q_j, q_j);
-#if !defined(SEAM_AGG_TIMELINE) && !defined(SEAM_AGG_TIMELINE2) && !defined(SEAM_AGG_TIMELINE3) && !defined(SEAM_AGG_PHASES)
         if (p.att && lane < Tmax) p.att[(size_t)track * Tmax + lane] = p_t;
-#endif
         __syncwarp();
 
-        SEAM_WPH(5);
         // ---- weighted sums over frames, 8 channels per lane; sum_j q_j on the way (every lane adds the broadcast q)
         Vec8 pov = zero_vec8(), rv = zero_vec8();
         float qsum = 0.f;
@@ -878,15 +781,7 @@ aggregate_fused_warp_kernel(const __grid_constant__ CUtensorMap tmSeq, const Par
         mx = ptx::warp_max(mx);
         float inv;
         const float s = track_scale(mx, &inv);
-#ifdef SEAM_AGG_DIAG_NO_PUBLISH
-        if (mx == 123.456f) p.out[track] = s + po0.x + po1.y + r0.x + r1.w;
-        return;
-#endif
-        SEAM_WPH(6);
-        if (warp == 0 && it == 5) SEAM_TL3(p, 6);
         const Slot sl = wait_slot(meta, __shfl_sync(ptx::FULL_MASK, ticket, 0));
-        SEAM_WPH(7);
-        if (warp == 0 && it == 5) SEAM_TL3(p, 7);
         uint8_t* rt = fz + OFF_RT + sl.buf * RT_BYTES;
         store_r4(rt, sl.pos, 4 * lane, r0, s);
         store_r4(rt, sl.pos, 128 + 4 * lane, r1, s);
@@ -900,20 +795,13 @@ aggregate_fused_warp_kernel(const __grid_constant__ CUtensorMap tmSeq, const Par
         ptx::fence_proxy_async_smem();                   // the r rows are read by the tensor core (async proxy)
         __syncwarp();
         if (lane == 0) ptx::mbar_arrive(&meta->tile_full[sl.buf]);
-        SEAM_WPH(8);
       };
       if (len == TR) process(std::true_type{});
       else process(std::false_type{});
     }
-#ifdef SEAM_AGG_PHASES
-    __syncwarp();
-    if (TR == 10 && warp == 0 && lane < 16 && p.att)
-      reinterpret_cast<long long*>(p.att)[blockIdx.x * 16 + lane] = lane == 15 ? (long long)it : lane < 12 ? reinterpret_cast<long long*>(scal + 40)[lane] : 0ll;
-#endif
   }
   fused_teardown(fz, warp, NW);
   if (p.x_on && p.x_last) xchg::signal_all(p.x, xchg::KIND_Q, xstep);
-  if (warp == 0) SEAM_TL(p, 7);
 }
 
 
@@ -947,9 +835,6 @@ struct GSmem {
   float x[GWARPS][FB][D];              // 8 x 16 KB
   GroupSmem<GW> g[GWARPS / GW];
   uint64_t bar[GWARPS];
-#ifdef SEAM_AGG_PHASES
-  long long phase[16];                 // developer diagnostic: cycles warp 0 spent in each phase of its iterations
-#endif
 };
 template <int GW>
 constexpr size_t group_smem_bytes() { return 1024 + fused_bytes<false>() + sizeof(GSmem<GW>); }
@@ -1041,11 +926,7 @@ aggregate_fused_group_kernel(const __grid_constant__ CUtensorMap tmSeq, const Pa
       __syncwarp();
     } else if (lane < nw) {
       const float* src = p.seq + (long long)(FB * wg + lane + 1) * p.frame_stride + track * p.track_stride;
-#ifdef SEAM_AGG_NO_HINT
-      ptx::bulk_load_1d(xs + (size_t)lane * D, src, D * 4, bar);
-#else
       ptx::bulk_load_1d_hint(xs + (size_t)lane * D, src, D * 4, bar, pol);
-#endif
     }
   };
   // the first track is requested before the CTA-wide set-up
@@ -1058,7 +939,7 @@ aggregate_fused_group_kernel(const __grid_constant__ CUtensorMap tmSeq, const Pa
 
   if (warp >= GWARPS) {
     ptx::reg_dec<GREGS_H>();
-    load_m_tmem<SEAM_AGG_INIT_WARPS(GWARPS + HELPER_WARPS), 2>(p, meta, SEAM_AGG_INIT_WARPS(GWARPS + HELPER_WARPS) == HELPER_WARPS ? warp - GWARPS : warp, lane);
+    load_m_tmem<GWARPS + HELPER_WARPS, 2>(p, meta, warp, lane);
     helper_role<GW, false>(p, fz, warp - GWARPS, lane, GROUPS_PER_CTA, first0, stride, out_local, xstep);
   } else {
     ptx::reg_inc<GREGS_P>();
@@ -1075,20 +956,11 @@ aggregate_fused_group_kernel(const __grid_constant__ CUtensorMap tmSeq, const Pa
     const int SF0 = FB * wg + (lane >> 2);
     float* const sc_dst = (comp < 2 ? &gs.ad[0][0] : &gs.bc[0][0]) + (SF0 >> 1) * 4 + ((comp & 1) << 1) + (SF0 & 1);
 
-#ifndef SEAM_AGG_HELPER_INIT
     load_m_tmem<GWARPS + HELPER_WARPS, 2>(p, meta, warp, lane);   // while the first frames are in flight
-#endif
     int it = 0;
-#ifdef SEAM_AGG_PHASES
-    long long ph_prev = clock64();
-    if (warp == 0 && lane < 16) s.phase[lane] = 0;
-    __syncwarp();
-#endif
 #pragma unroll 1
     for (long long track = first; track < p.Q; track += stride, ++it) {
-      SEAM_PH(0);
       ptx::mbar_wait(bar, (uint32_t)it & 1u, 106);
-      SEAM_PH(1);
       const int nw = max(0, min(len - FB * wg, FB));
 
       // ---- my 16 frames -> registers (zeros past the block's end), four dots per frame, the 32 totals of 8 frames per
@@ -1111,24 +983,14 @@ aggregate_fused_group_kernel(const __grid_constant__ CUtensorMap tmSeq, const Pa
         // frame F = FB wg + t0 + (lane >> 2): a, d -> ad[F / 2][F % 2 (+ 2)], b, c -> bc[...], zero past the track's end
         sc_dst[2 * t0] = (comp < 2 || SF0 + t0 < len) ? tot + my_const : 0.f;
       }
-      SEAM_PH(2);
       // the buffer is free again: fetch this warp's block of the group's next track
       const int len_next = decode(track + stride, raw_next);
       __syncwarp();
       issue(track + stride, len_next);
-      SEAM_PH(3);
-#if defined(SEAM_AGG_GDIAG) && SEAM_AGG_GDIAG == 1      // developer diagnostic (wrong results): frames -> registers + dots only
-      if (len == -5) p.out[track] = x[3].a + x[15].d;
-      len = len_next;
-      continue;
-#endif
       ptx::named_bar_sync(bar_id, GW * 32);                       // #1 all scalars of the track are visible
-      SEAM_PH(4);
-#ifndef SEAM_AGG_DIAG_NO_PUBLISH
       // the track's slot in the batch under construction is claimed now, its (~200 cycle) round trip used much later
       unsigned my_slot = 0u;
       if (wg == 0 && lane == 0) my_slot = atomicAdd(&meta->next_slot, 1u);
-#endif
 
       // ---- attention over the track's frames: lane = (frame f of my block, half of the j / t range).  The loops
       // take two frames per step ({b_e, b_o, c_e, c_o}: one 16-byte load, one packed add, one packed fma) and run over
@@ -1175,9 +1037,7 @@ aggregate_fused_group_kernel(const __grid_constant__ CUtensorMap tmSeq, const Pa
       const float e_t = valid ? expf(s_t - m_w) : 0.f;
       if (half == 0) gs.ad[F >> 1][2 + (F & 1)] = e_t;            // d (read above by both lanes of the frame) -> e
       if (lane == 0) gs.red_max[wg] = m_w;
-      SEAM_PH(5);
       ptx::named_bar_sync(bar_id, GW * 32);                       // #2 e and m_w of the whole track are visible
-      SEAM_PH(6);
       float m = gs.red_max[0];
 #pragma unroll
       for (int w = 1; w < GW; ++w) m = fmaxf(m, gs.red_max[w]);
@@ -1187,7 +1047,6 @@ aggregate_fused_group_kernel(const __grid_constant__ CUtensorMap tmSeq, const Pa
         const float mw = gs.red_max[w];
         scale[w] = mw > -INFINITY ? expf(mw - m) : 0.f;            // a warp without frames of this track: -inf
       }
-      SEAM_PH(7);
       float q_j = 0.f, z = 0.f;                                    // q_j = sum_t relu(b_j + a_t) p_t / T
       {
         const u64 b2 = pk(b_f, b_f);
@@ -1205,20 +1064,12 @@ aggregate_fused_group_kernel(const __grid_constant__ CUtensorMap tmSeq, const Pa
       const float inv_z = z > 0.f ? 1.f / z : 0.f;
       const float p_t = e_t * scale[wg] * inv_z;
       q_j = len > 1 ? q_j * inv_len * inv_z : 0.f;
-#if !defined(SEAM_AGG_TIMELINE) && !defined(SEAM_AGG_TIMELINE2) && !defined(SEAM_AGG_TIMELINE3) && !defined(SEAM_AGG_PHASES)
       if (p.att && half == 0 && F < Tmax) p.att[(size_t)track * Tmax + F] = p_t;
-#endif
       if (!valid) q_j = 0.f;
       const float qsum_w = ptx::warp_sum(half == 0 ? q_j : 0.f);
       if (half == 0) *reinterpret_cast<float4*>(&gs.pq[F][0]) = make_float4(p_t, p_t, q_j, q_j);
       __syncwarp();
 
-#if defined(SEAM_AGG_GDIAG) && SEAM_AGG_GDIAG == 2      // developer diagnostic (wrong results): ... + attention, no weighted sums
-      if (len == -5) p.out[track] = x[3].a + x[15].d;
-      len = len_next;
-      continue;
-#endif
-      SEAM_PH(8);
       // ---- partial weighted sums over my frames, 8 channels per lane.  {p, p}, {q, q} come from shared memory (one
       // broadcast load per frame, four in flight); frames past the block's end are zero in registers and need no guard.
       Vec8 pov = zero_vec8(), rv = zero_vec8();
@@ -1249,19 +1100,10 @@ aggregate_fused_group_kernel(const __grid_constant__ CUtensorMap tmSeq, const Pa
         if (lane == 0) {
           gs.red_q[wg] = qsum_w;
           gs.red_rmax[wg] = pm;
-#ifndef SEAM_AGG_DIAG_NO_PUBLISH
           if (wg == 0) gs.slot = my_slot;
-#endif
         }
       }
-      SEAM_PH(9);
       ptx::named_bar_sync(bar_id, GW * 32);                       // #5 partial sums, maxima and the slot are visible
-      SEAM_PH(10);
-#ifdef SEAM_AGG_DIAG_NO_PUBLISH
-      if (gs.red_rmax[0] == 123.456f) p.out[track] = gs.part[0][lane];
-      len = len_next;
-      continue;
-#endif
 
       // ---- warp w finishes channels [CW w, CW (w+1)), CW = 256 / GW, and publishes them
       {
@@ -1273,10 +1115,7 @@ aggregate_fused_group_kernel(const __grid_constant__ CUtensorMap tmSeq, const Pa
         for (int w = 1; w < GW; ++w) rb += gs.red_rmax[w];
         float inv;
         const float scale = track_scale(rb, &inv);
-        if (warp == 0 && it == 40) SEAM_TL3(p, 6);
         ptx::mbar_wait(&meta->buf_free[buf], ((batch >> 1) & 1u) ^ 1u, 107);
-        SEAM_PH(11);
-        if (warp == 0 && it == 40) SEAM_TL3(p, 7);
         uint8_t* rt = fz + OFF_RT + buf * RT_BYTES;
         constexpr int CW = D / GW;
 #pragma unroll
@@ -1312,13 +1151,8 @@ aggregate_fused_group_kernel(const __grid_constant__ CUtensorMap tmSeq, const Pa
         __syncwarp();
         if (lane == 0) ptx::mbar_arrive(&meta->tile_full[buf]);
       }
-      SEAM_PH(12);
       len = len_next;
     }
-#ifdef SEAM_AGG_PHASES
-    __syncwarp();
-    if (warp == 0 && lane < 16 && p.att) reinterpret_cast<long long*>(p.att)[blockIdx.x * 16 + lane] = lane == 15 ? (long long)it : s.phase[lane];
-#endif
   }
   fused_teardown(fz, warp, GWARPS);
   if (p.x_on && p.x_last) xchg::signal_all(p.x, xchg::KIND_Q, xstep);

@@ -76,14 +76,12 @@ struct Params {
   int P;                      // sub-list slots per row: max CTAs sharing one query tile's sweep
   int CAP;                    // entries per sub-list
   int nseed;                  // threshold-only sample tiles at the start of a segment
-  int mode;                   // 0 = normal; 1 = accumulators are drained unread (MMA-only ceiling)
   const float* cg;            // (G)
   uint32_t* thr_global;       // (Q) ordered-uint image of the per-row lower bound
   uint32_t* rowcnt;           // (Q, P, 4) quad records in each sub-list
   uint32_t* rowflag;          // (Q) nonzero: the row lost candidates, must be ranked exhaustively
   uint2* rowbuf;              // (Q, P, 4, CAP x 8 bytes) = CAP/2 quad records {w0,w1,w2,w3} per sub-list
   float* gmax;                // (Q, P, 4, 16) final group maxima of each thread (disjoint column groups)
-  unsigned long long* cta_ns; // (grid, 2) optional: {duration in ns, segments} per CTA (developer diagnostics)
   int tb[MAX_GRID + 1];       // CTA b sweeps the linearised tiles [tb[b], tb[b+1]) (cost-balanced on the host)
   // rank-of-target variant (VAR_RANK): per-row band (lo, hi] around the target's value and, per sub-list,
   // the number of elements certainly above it
@@ -121,6 +119,7 @@ struct Segment {
 // whose head is the first thing the previous CTA sweeps -- by the time this CTA gets to the tail the
 // row's bound has long been published in thr_global (after the sample sweep, then every 8 tiles), and
 // the tail starts warm without samples.  Every row is thus sampled once, not once per piece.
+constexpr int NSEED = 4;               // sample tiles of a sampled segment (the rank variant takes none)
 __device__ __forceinline__ Segment segment_before(const Params& p, long long t_begin, long long t_hi, long long t_end,
                                                   long long& next_hi) {
   Segment s;
@@ -218,27 +217,20 @@ __device__ __forceinline__ float tagged_reg(uint32_t acc, float cg, uint32_t kee
 }
 // Only the low address word advances: a sub-list never straddles a 4 GiB boundary (power-of-two size,
 // aligned to it).
-template <int VAR>
 __device__ __forceinline__ void append_quad(uint64_t& wp, float m, float cmp, float w0, float w1, float w2, float w3) {
-  if constexpr (VAR == 0 || VAR == 5) {
-    asm volatile(
-        "{\n"
-        ".reg .pred p;\n"
-        ".reg .b32 lo, hi;\n"
-        "setp.gt.f32 p, %1, %2;\n"
-        "@p st.global.v4.f32 [%0], {%3, %4, %5, %6};\n"
-        "mov.b64 {lo, hi}, %0;\n"
-        "@p add.u32 lo, lo, 16;\n"
-        "mov.b64 %0, {lo, hi};\n"
-        "}\n"
-        : "+l"(wp)
-        : "f"(m), "f"(cmp), "f"(w0), "f"(w1), "f"(w2), "f"(w3)
-        : "memory");
-  } else if constexpr (VAR == 2) {   // diagnostics: no store
-    asm volatile("{\n.reg .pred p;\n.reg .b32 lo, hi;\nsetp.gt.f32 p, %1, %2;\nmov.b64 {lo, hi}, %0;\n"
-                 "@p add.u32 lo, lo, 16;\nmov.b64 %0, {lo, hi};\n}\n"
-                 : "+l"(wp) : "f"(m), "f"(cmp) : "memory");
-  }
+  asm volatile(
+      "{\n"
+      ".reg .pred p;\n"
+      ".reg .b32 lo, hi;\n"
+      "setp.gt.f32 p, %1, %2;\n"
+      "@p st.global.v4.f32 [%0], {%3, %4, %5, %6};\n"
+      "mov.b64 {lo, hi}, %0;\n"
+      "@p add.u32 lo, lo, 16;\n"
+      "mov.b64 %0, {lo, hi};\n"
+      "}\n"
+      : "+l"(wp)
+      : "f"(m), "f"(cmp), "f"(w0), "f"(w1), "f"(w2), "f"(w3)
+      : "memory");
 }
 
 // ties the destination registers of an in-flight tcgen05.ld to the wait so the compiler
@@ -260,16 +252,12 @@ __device__ __forceinline__ void tmem_ld_wait_x32(uint32_t (&a)[32]) {
 struct TileTags {
   uint32_t t1, t2, t3;   // bits [0,6), [6,12), [12,18) of the gallery tile index
 };
-template <int VAR, int GOFF, int Q0>
+template <int GOFF, int Q0>
 __device__ __forceinline__ void filter16(const uint32_t (&r)[16], const float* cgp, float (&gm)[GROUPS], uint64_t& wp,
                                          float cmp, uint32_t keep, const TileTags& tg) {
   float cgv[16];
 #pragma unroll
   for (int c4 = 0; c4 < 4; ++c4) {
-    if constexpr (VAR == 5) {   // diagnostics: no column term
-      cgv[c4 * 4 + 0] = cgv[c4 * 4 + 1] = cgv[c4 * 4 + 2] = cgv[c4 * 4 + 3] = -0.f;
-      continue;
-    }
     const float4 g4 = *reinterpret_cast<const float4*>(cgp + c4 * 4);
     cgv[c4 * 4 + 0] = g4.x;
     cgv[c4 * 4 + 1] = g4.y;
@@ -303,7 +291,7 @@ __device__ __forceinline__ void filter16(const uint32_t (&r)[16], const float* c
   for (int q = 0; q < 4; ++q) {
     const float m = fmaxf(max3(w[4 * q], w[4 * q + 1], w[4 * q + 2]), w[4 * q + 3]);
     gm[GOFF + q] = fmaxf(gm[GOFF + q], m);
-    append_quad<VAR>(wp, m, cmp, w[4 * q], w[4 * q + 1], w[4 * q + 2], w[4 * q + 3]);
+    append_quad(wp, m, cmp, w[4 * q], w[4 * q + 1], w[4 * q + 2], w[4 * q + 3]);
   }
 }
 
@@ -341,11 +329,11 @@ __device__ __forceinline__ void filter16_rank(const uint32_t (&r)[16], const flo
           : "+r"(above), "=f"(t[e])
           : "f"(w[e]), "f"(hi));
     const float m = fmaxf(max3(t[0], t[1], t[2]), t[3]);
-    append_quad<0>(wp, m, lo_or_inf, w[0], w[1], w[2], w[3]);
+    append_quad(wp, m, lo_or_inf, w[0], w[1], w[2], w[3]);
   }
 }
 
-template <int VAR>   // 0 = product; 2..4 = developer diagnostics (partial epilogues, wrong results)
+template <int VAR>   // 0 = top-k candidate filter; VAR_RANK = rank of one designated gallery item per query
 __global__ void __launch_bounds__(THREADS, 1)
 score_topk_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB, const Params p) {
   extern __shared__ uint8_t smem_raw[];
@@ -400,7 +388,6 @@ score_topk_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant
   long long t_begin, t_end;
   t_begin = p.tb[blockIdx.x];
   t_end = p.tb[blockIdx.x + 1];
-  const uint64_t dbg_t0 = p.cta_ns ? ptx::globaltimer_ns() : 0;
 
   if (warp == 0) {
     // ================================================================= TMA producer
@@ -572,58 +559,50 @@ score_topk_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant
       }
       ptx::mbar_wait(&t_full[acc], aphase);
       ptx::tc_fence_after();
-      if (p.mode == 1) {
-        ptx::tc_fence_before();
-        __syncwarp();
-        if (lane == 0) {
-          ptx::mbar_arrive(&t_empty[acc]);
-          ptx::mbar_arrive(&cg_empty[acc]);
-        }
+      // four chunks of 16 columns; the first load is issued before anything else is derived
+      const uint32_t taddr = tmem_base + (uint32_t(lq * 32) << 16) + acc * BN + cq * QCOLS;
+      uint32_t ra[16], rb[16];
+      ptx::tmem_ld_x16(taddr, ra);
+      const bool seed = (cmd.y & CMD_SEED) != 0;
+      if (!seed && !(st & ST_CLOSED) && (uint32_t)wp - wlo_begin > room)   // no room for another tile:
+        st |= ST_CLOSED | ST_LOSSY;                                         // the row goes to the exhaustive path
+      const float cmp = (seed || (st & ST_CLOSED)) ? INFINITY : thr;
+      const float* cgp = cg_s + acc * BN + cq * QCOLS;
+      TileTags tg;
+      tg.t1 = (uint32_t)cmd.x & TAG_MASK;
+      tg.t2 = ((uint32_t)cmd.x >> TAG_BITS) & TAG_MASK;
+      tg.t3 = ((uint32_t)cmd.x >> (2 * TAG_BITS)) & TAG_MASK;
+      ptx::tmem_ld_wait_x16(ra);
+      ptx::tmem_ld_x16(taddr + 16, rb);
+      if constexpr (VAR == VAR_RANK) filter16_rank(ra, cgp, wp, above, cmp, rank_hi, keep, tg, 0);
+      else filter16<0, 0>(ra, cgp, gm, wp, cmp, keep, tg);
+      ptx::tmem_ld_wait_x16(rb);
+      ptx::tmem_ld_x16(taddr + 32, ra);
+      if constexpr (VAR == VAR_RANK) filter16_rank(rb, cgp + 16, wp, above, cmp, rank_hi, keep, tg, 4);
+      else filter16<4, 4>(rb, cgp + 16, gm, wp, cmp, keep, tg);
+      ptx::tmem_ld_wait_x16(ra);
+      ptx::tmem_ld_x16(taddr + 48, rb);
+      // The MMA of the tile after next cannot start before the slowest of the 16 warps has read its
+      // columns, so the last load is waited for right away (half-way through the tile's work, the
+      // scheduler's other warps fill the gap) and the slot handed back before the remaining two chunks.
+      ptx::tmem_ld_wait_x16(rb);
+      ptx::tc_fence_before();
+      __syncwarp();
+      if (lane == 0) ptx::mbar_arrive(&t_empty[acc]);
+      if constexpr (VAR == VAR_RANK) {
+        filter16_rank(ra, cgp + 32, wp, above, cmp, rank_hi, keep, tg, 8);
+        filter16_rank(rb, cgp + 48, wp, above, cmp, rank_hi, keep, tg, 12);
       } else {
-        // four chunks of 16 columns; the first load is issued before anything else is derived
-        const uint32_t taddr = tmem_base + (uint32_t(lq * 32) << 16) + acc * BN + cq * QCOLS;
-        uint32_t ra[16], rb[16];
-        ptx::tmem_ld_x16(taddr, ra);
-        const bool seed = (cmd.y & CMD_SEED) != 0;
-        if (!seed && !(st & ST_CLOSED) && (uint32_t)wp - wlo_begin > room)   // no room for another tile:
-          st |= ST_CLOSED | ST_LOSSY;                                         // the row goes to the exhaustive path
-        const float cmp = (seed || (st & ST_CLOSED)) ? INFINITY : thr;
-        const float* cgp = cg_s + acc * BN + cq * QCOLS;
-        TileTags tg;
-        tg.t1 = (uint32_t)cmd.x & TAG_MASK;
-        tg.t2 = ((uint32_t)cmd.x >> TAG_BITS) & TAG_MASK;
-        tg.t3 = ((uint32_t)cmd.x >> (2 * TAG_BITS)) & TAG_MASK;
-        ptx::tmem_ld_wait_x16(ra);
-        ptx::tmem_ld_x16(taddr + 16, rb);
-        if constexpr (VAR == VAR_RANK) filter16_rank(ra, cgp, wp, above, cmp, rank_hi, keep, tg, 0);
-        else filter16<VAR, 0, 0>(ra, cgp, gm, wp, cmp, keep, tg);
-        ptx::tmem_ld_wait_x16(rb);
-        ptx::tmem_ld_x16(taddr + 32, ra);
-        if constexpr (VAR == VAR_RANK) filter16_rank(rb, cgp + 16, wp, above, cmp, rank_hi, keep, tg, 4);
-        else filter16<VAR, 4, 4>(rb, cgp + 16, gm, wp, cmp, keep, tg);
-        ptx::tmem_ld_wait_x16(ra);
-        ptx::tmem_ld_x16(taddr + 48, rb);
-        // The MMA of the tile after next cannot start before the slowest of the 16 warps has read its
-        // columns, so the last load is waited for right away (half-way through the tile's work, the
-        // scheduler's other warps fill the gap) and the slot handed back before the remaining two chunks.
-        ptx::tmem_ld_wait_x16(rb);
-        ptx::tc_fence_before();
-        __syncwarp();
-        if (lane == 0) ptx::mbar_arrive(&t_empty[acc]);
-        if constexpr (VAR == VAR_RANK) {
-          filter16_rank(ra, cgp + 32, wp, above, cmp, rank_hi, keep, tg, 8);
-          filter16_rank(rb, cgp + 48, wp, above, cmp, rank_hi, keep, tg, 12);
-        } else {
-          filter16<VAR, 8, 8>(ra, cgp + 32, gm, wp, cmp, keep, tg);
-          filter16<VAR, 12, 12>(rb, cgp + 48, gm, wp, cmp, keep, tg);
-        }
-        __syncwarp();
-        if (lane == 0) ptx::mbar_arrive(&cg_empty[acc]);
-        // share the bound: each of the row's 4 threads vouches for 8 distinct items at or above the
-        // 8th largest of its 16 group maxima (re-derived every other tile), the smallest of the four
-        // values therefore for 32
-        const bool seed_end = (cmd.y & CMD_SEED_END) != 0;
-        if constexpr (VAR != VAR_RANK) {
+        filter16<8, 8>(ra, cgp + 32, gm, wp, cmp, keep, tg);
+        filter16<12, 12>(rb, cgp + 48, gm, wp, cmp, keep, tg);
+      }
+      __syncwarp();
+      if (lane == 0) ptx::mbar_arrive(&cg_empty[acc]);
+      // share the bound: each of the row's 4 threads vouches for 8 distinct items at or above the
+      // 8th largest of its 16 group maxima (re-derived every other tile), the smallest of the four
+      // values therefore for 32
+      const bool seed_end = (cmd.y & CMD_SEED_END) != 0;
+      if constexpr (VAR != VAR_RANK) {
         if ((itile & 1) || seed_end) {
           thr_x[R * NQ + cq] = eighth_largest_of_16(gm);
           // After the sample sweep the four warps of a row meet once, so that the first appended
@@ -636,26 +615,25 @@ score_topk_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant
           const uint32_t old = atomicMax(p.thr_global + grow, ptx::float_to_ordered(thr));
           thr = fmaxf(thr, ptx::ordered_to_float(old));
         }
-        }
-        ++itile;
-        // ---- segment end: publish the list length, the bound and the loss flag
-        if ((cmd.y & CMD_SEG_END) && (st & ST_ROW)) {
-          if (st & ST_SLOT) {
-            const size_t li = ((size_t)grow * p.P + (st >> 8)) * NQ + cq;
-            p.rowcnt[li] = ((uint32_t)wp - wlo_begin) >> 4;   // quads
-            if constexpr (VAR == VAR_RANK) {
-              p.rank_above[li] = (int32_t)above;
-            } else {
-              float4* gd = reinterpret_cast<float4*>(p.gmax + li * GROUPS);
-              gd[0] = make_float4(gm[0], gm[1], gm[2], gm[3]);
-              gd[1] = make_float4(gm[4], gm[5], gm[6], gm[7]);
-              gd[2] = make_float4(gm[8], gm[9], gm[10], gm[11]);
-              gd[3] = make_float4(gm[12], gm[13], gm[14], gm[15]);
-            }
+      }
+      ++itile;
+      // ---- segment end: publish the list length, the bound and the loss flag
+      if ((cmd.y & CMD_SEG_END) && (st & ST_ROW)) {
+        if (st & ST_SLOT) {
+          const size_t li = ((size_t)grow * p.P + (st >> 8)) * NQ + cq;
+          p.rowcnt[li] = ((uint32_t)wp - wlo_begin) >> 4;   // quads
+          if constexpr (VAR == VAR_RANK) {
+            p.rank_above[li] = (int32_t)above;
+          } else {
+            float4* gd = reinterpret_cast<float4*>(p.gmax + li * GROUPS);
+            gd[0] = make_float4(gm[0], gm[1], gm[2], gm[3]);
+            gd[1] = make_float4(gm[4], gm[5], gm[6], gm[7]);
+            gd[2] = make_float4(gm[8], gm[9], gm[10], gm[11]);
+            gd[3] = make_float4(gm[12], gm[13], gm[14], gm[15]);
           }
-          if (st & ST_LOSSY) atomicOr(p.rowflag + grow, 1u);
-          if constexpr (VAR != VAR_RANK) atomicMax(p.thr_global + grow, ptx::float_to_ordered(thr));
         }
+        if (st & ST_LOSSY) atomicOr(p.rowflag + grow, 1u);
+        if constexpr (VAR != VAR_RANK) atomicMax(p.thr_global + grow, ptx::float_to_ordered(thr));
       }
       if (++acc == 2) {
         acc = 0;
@@ -666,10 +644,6 @@ score_topk_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant
 
   ptx::tc_fence_before();
   __syncthreads();
-  if (p.cta_ns && tid == 0) {
-    p.cta_ns[2 * blockIdx.x] = ptx::globaltimer_ns() - dbg_t0;
-    p.cta_ns[2 * blockIdx.x + 1] = (unsigned long long)(t_end / p.ntiles_n - t_begin / p.ntiles_n + 1);
-  }
   if (warp == 2) ptx::tmem_dealloc(tmem_base, 512);
 }
 

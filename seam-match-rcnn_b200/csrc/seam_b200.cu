@@ -42,8 +42,6 @@ struct seam_handle {
   __half* tw_conv[4] = {nullptr, nullptr, nullptr, nullptr};
   float* tw_misc = nullptr;           // bias0..3 (256,256,256,1024) | lin_wt (1024*256) | lin_b | bn_scale | bn_shift
   bool have_tower = false;
-  // developer overrides, read once at seam_create (never consulted on the hot path)
-  int dbg_score_grid = 0, dbg_agg_grid = 0, dbg_cta_ns = 0, dbg_no_tm = 0, score_nseed = 4;
   struct Span { int kernel; cudaEvent_t a, b; };
   std::vector<Span> spans;            // recorded while profiling
   std::vector<cudaEvent_t> free_events;
@@ -80,11 +78,6 @@ static_assert(exact::PLAN_MAX_GRID == score::MAX_GRID, "the re-score kernels car
 static thread_local char g_create_err[256] = "";
 
 static unsigned int* g_watchdog_host[64] = {};
-
-static int env_int(const char* name, int dflt) {
-  const char* v = getenv(name);
-  return v && *v ? atoi(v) : dflt;
-}
 
 static int fail(seam_handle* h, int code, const char* fmt, ...) {
   va_list ap;
@@ -130,7 +123,6 @@ static inline bool aligned16(const void* p) { return (reinterpret_cast<uintptr_t
 // (1+Tmax, Q, 256) with the caller's strides.  Returns whether the map is usable.
 static int encode_seq_map(seam_handle* h, const aggf::Params& p, int box_frames, CUtensorMap* tm) {
   memset(tm, 0, sizeof(*tm));
-  if (h->dbg_no_tm) return 0;
   if (!p.seq || p.Q <= 0 || (p.track_stride * 4) % 16 != 0 || (p.frame_stride * 4) % 16 != 0 || p.track_stride < 256 ||
       p.frame_stride < 256 || box_frames > p.Tmax)
     return 0;
@@ -144,19 +136,19 @@ static int encode_seq_map(seam_handle* h, const aggf::Params& p, int box_frames,
 }
 
 template <int TR>
-static void launch_aggregate_warp(seam_handle* h, aggf::Params& p, int num_sms, cudaStream_t stream) {   // num_sms = CTA cap
+static void launch_aggregate_warp(seam_handle* h, aggf::Params& p, cudaStream_t stream) {
   constexpr int NW = aggf::Cfg<TR>::NW;
   const int want = (p.Q + NW - 1) / NW;
-  const int grid = want < num_sms ? want : num_sms;
+  const int grid = want < h->num_sms ? want : h->num_sms;
   CUtensorMap tm;
   p.use_tm = p.Tmax == TR ? encode_seq_map(h, p, TR, &tm) : (memset(&tm, 0, sizeof(tm)), 0);
   aggf::aggregate_fused_warp_kernel<TR><<<grid, aggf::warp_threads<TR>(), aggf::warp_smem_bytes<TR>(), stream>>>(tm, p);
 }
 template <int GW>
-static void launch_aggregate_group(seam_handle* h, aggf::Params& p, int num_sms, cudaStream_t stream) {
+static void launch_aggregate_group(seam_handle* h, aggf::Params& p, cudaStream_t stream) {
   constexpr int GPC = aggf::GWARPS / GW;
   const int want = (p.Q + GPC - 1) / GPC;
-  const int grid = want < num_sms ? want : num_sms;
+  const int grid = want < h->num_sms ? want : h->num_sms;
   CUtensorMap tm;
   p.use_tm = encode_seq_map(h, p, aggf::FB, &tm);
   aggf::aggregate_fused_group_kernel<GW><<<grid, aggf::GTHREADS, aggf::group_smem_bytes<GW>(), stream>>>(tm, p);
@@ -245,11 +237,6 @@ int seam_create(seam_handle** out, int device) {
     return fail(nullptr, SEAM_ERR_CUDA, "cuTensorMapEncodeTiled not available from the driver");
   }
   h->encode = reinterpret_cast<PFN_encodeTiled>(fn);
-  h->dbg_score_grid = env_int("SEAM_DEBUG_SCORE_GRID", 0);
-  h->dbg_agg_grid = env_int("SEAM_DEBUG_AGG_GRID", 0);
-  h->dbg_cta_ns = env_int("SEAM_DEBUG_CTA_NS", 0);
-  h->dbg_no_tm = env_int("SEAM_DEBUG_AGG_NO_TM", 0);      // developer A/B: per-frame bulk copies instead of one tensor-map box
-  h->score_nseed = env_int("SEAM_SCORE_NSEED", 4);
   // watchdog records live in host-mapped memory so that they survive a trapped launch: one buffer per
   // device for the life of the process (the device-side pointer must never dangle)
   if (device < 64) {
@@ -269,12 +256,6 @@ int seam_create(seam_handle** out, int device) {
   // opt in to large dynamic shared memory once
   cudaFuncSetAttribute(score::score_topk_kernel<0>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                        (int)score::SMEM_BYTES);
-#ifdef SEAM_DIAGNOSTIC_VARIANTS   // partial epilogues for measurements (wrong results): never in a product build
-  cudaFuncSetAttribute(score::score_topk_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)score::SMEM_BYTES);
-  cudaFuncSetAttribute(score::score_topk_kernel<3>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)score::SMEM_BYTES);
-  cudaFuncSetAttribute(score::score_topk_kernel<4>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)score::SMEM_BYTES);
-  cudaFuncSetAttribute(score::score_topk_kernel<5>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)score::SMEM_BYTES);
-#endif
   cudaFuncSetAttribute(score::score_topk_kernel<score::VAR_RANK>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                        (int)score::SMEM_BYTES);
   cudaFuncSetAttribute(aggf::aggregate_fused_warp_kernel<4>, cudaFuncAttributeMaxDynamicSharedMemorySize,
@@ -437,7 +418,6 @@ static int aggregate_impl(seam_handle* h, const xchg::Exchange* x, int row0, int
     // protocol: one CTA, zero tracks / zero-length tracks, descriptors = 0
     if (Tmax == 0) { p.Tmax = 1; p.lens = nullptr; p.mask = nullptr; p.seq = nullptr; p.Q = -Q; }
   }
-  const int cap = h->dbg_agg_grid > 0 && h->dbg_agg_grid < h->num_sms ? h->dbg_agg_grid : h->num_sms;
   if (p.Q < 0) return fail(h, SEAM_ERR_UNSUPPORTED, "%s: Tmax == 0 in the sharded search", who);
   if (p.Q == 0) {
     // nothing to aggregate on this rank: only the signal is needed
@@ -447,11 +427,11 @@ static int aggregate_impl(seam_handle* h, const xchg::Exchange* x, int row0, int
     }
     return SEAM_OK;
   }
-  if (Tmax <= 4) launch_aggregate_warp<4>(h, p, cap, stream);
-  else if (Tmax <= 10) launch_aggregate_warp<10>(h, p, cap, stream);
-  else if (Tmax <= 16) launch_aggregate_warp<16>(h, p, cap, stream);
-  else if (Tmax <= 32) launch_aggregate_group<2>(h, p, cap, stream);   // two warps per track
-  else launch_aggregate_group<4>(h, p, cap, stream);                   // 33..64 frames: four warps per track
+  if (Tmax <= 4) launch_aggregate_warp<4>(h, p, stream);
+  else if (Tmax <= 10) launch_aggregate_warp<10>(h, p, stream);
+  else if (Tmax <= 16) launch_aggregate_warp<16>(h, p, stream);
+  else if (Tmax <= 32) launch_aggregate_group<2>(h, p, stream);   // two warps per track
+  else launch_aggregate_group<4>(h, p, stream);                   // 33..64 frames: four warps per track
   SEAM_LAUNCHED(h, "aggregate kernel");
   return SEAM_OK;
 }
@@ -553,7 +533,7 @@ struct ScorePlan {
 // range per CTA (score_tc.cuh).  A query tile's gallery sweep is therefore shared by at most P
 // CTAs ("pieces"); each piece owns 4 candidate sub-lists per row (one per epilogue thread of
 // the row) of CAP entries, CAP >= 3 times the expected number of appends.
-static ScorePlan plan_score(int num_sms, int Q, int G, int nseed_override = -1, int nseed_default = 4, int cap_grid = 0) {
+static ScorePlan plan_score(int num_sms, int Q, int G, bool rank) {
   ScorePlan s;
   s.num_mtiles = (Q + score::BM - 1) / score::BM;
   s.ntiles_n = (G + score::BN - 1) / score::BN;
@@ -561,9 +541,8 @@ static ScorePlan plan_score(int num_sms, int Q, int G, int nseed_override = -1, 
   if (s.ntiles_n < 1) s.ntiles_n = 1;
   s.total_tiles = (long long)s.num_mtiles * s.ntiles_n;
   s.grid = s.total_tiles < num_sms ? (int)s.total_tiles : num_sms;
-  if (cap_grid > 0 && cap_grid < s.grid) s.grid = cap_grid;   // developer diagnostics only (seam_create reads the override)
   if (s.grid > score::MAX_GRID) s.grid = score::MAX_GRID;
-  s.nseed = nseed_override >= 0 ? nseed_override : nseed_default;
+  s.nseed = rank ? 0 : score::NSEED;
   // Cost-balanced contiguous ranges.  A tile costs 1; a segment start costs SEG_COST (query tile load,
   // epilogue hand-over); a segment that holds its row's first gallery tile -- or is all a CTA has --
   // also sweeps min(nseed, length) threshold-only sample tiles (score_tc.cuh, segment_before).  walk()
@@ -650,7 +629,7 @@ static ScorePlan plan_score(int num_sms, int Q, int G, int nseed_override = -1, 
     need = 16.0 * 3.0 * (64.0 + 32.0 * log(T));
   }
   if (need > T * tile_bytes) need = T * tile_bytes;          // a thread cannot append more than it sees
-  if (nseed_override == 0) {
+  if (rank) {
     // rank-of-target variant: a thread appends the quads holding an element inside the band around the
     // target's value -- about 1-2 % of its columns for a target in the bulk of the ranking; budget 6 %
     const double band = 0.06 * T * score::QCOLS * 16.0;
@@ -683,12 +662,12 @@ static ScorePlan plan_score(int num_sms, int Q, int G, int nseed_override = -1, 
 size_t seam_score_workspace_bytes(const seam_handle* h, int Q, int G, int k) {
   (void)k;
   if (!h || Q <= 0 || G <= 0) return 256;
-  return plan_score(h->num_sms, Q, G, -1, h->score_nseed, h->dbg_score_grid).total;
+  return plan_score(h->num_sms, Q, G, false).total;
 }
 
 int seam_score_plan(const seam_handle* h, int Q, int G, int64_t* out) {
   if (!h || !out || Q <= 0 || G <= 0) return SEAM_ERR_BAD_ARG;
-  const ScorePlan s = plan_score(h->num_sms, Q, G, -1, h->score_nseed, h->dbg_score_grid);
+  const ScorePlan s = plan_score(h->num_sms, Q, G, false);
   const int64_t v[14] = {s.num_mtiles, s.ntiles_n, s.grid, s.P, s.CAP, (int64_t)s.off_a16,
                          (int64_t)s.off_rq, (int64_t)s.off_anorm, (int64_t)s.off_thr, (int64_t)s.off_rowcnt,
                          (int64_t)s.off_rowbuf, (int64_t)s.off_cnt, (int64_t)s.off_rows, (int64_t)s.total};
@@ -699,7 +678,7 @@ int seam_score_plan(const seam_handle* h, int Q, int G, int64_t* out) {
 // Pure host logic (no handle, no device): the tile ranges of the scorer's persistent CTAs.
 int seam_score_partition(int num_sms, int Q, int G, int rank_variant, int32_t* bounds, int bounds_len, int32_t* out6) {
   if (num_sms < 1 || Q <= 0 || G <= 0 || !bounds || !out6) return SEAM_ERR_BAD_ARG;
-  const ScorePlan s = plan_score(num_sms, Q, G, rank_variant ? 0 : -1);
+  const ScorePlan s = plan_score(num_sms, Q, G, rank_variant != 0);
   if (bounds_len < s.grid + 1) return SEAM_ERR_BAD_ARG;
   for (int b = 0; b <= s.grid; ++b) bounds[b] = s.tb[b];
   out6[0] = s.num_mtiles;
@@ -760,7 +739,7 @@ static int score_topk_impl(seam_handle* h, const xchg::Exchange* x, const float*
   if (!q || !g || !g16 || !cg || !gstat || !workspace) return fail(h, SEAM_ERR_BAD_ARG, "seam_score_topk: null pointer");
   if (!aligned16(q) || !aligned16(g) || !aligned16(g16) || (reinterpret_cast<uintptr_t>(workspace) & 255u))
     return fail(h, SEAM_ERR_UNSUPPORTED, "seam_score_topk: q/g/g16 need 16-byte, workspace 256-byte alignment");
-  const ScorePlan s = plan_score(h->num_sms, Q, G, -1, h->score_nseed, h->dbg_score_grid);
+  const ScorePlan s = plan_score(h->num_sms, Q, G, false);
   if (s.ntiles_n > (1 << 18))
     return fail(h, SEAM_ERR_UNSUPPORTED, "seam_score_topk: G=%d exceeds the 2^26 gallery rows one shard may hold", G);
   if (workspace_bytes < s.total)
@@ -803,11 +782,6 @@ static int score_topk_impl(seam_handle* h, const xchg::Exchange* x, const float*
   sp.CAP = s.CAP;
   sp.nseed = s.nseed;
   for (int b = 0; b <= s.grid; ++b) sp.tb[b] = s.tb[b];
-#ifdef SEAM_DIAGNOSTIC_VARIANTS
-  sp.mode = env_int("SEAM_DEBUG_SCORE_MODE", 0);   // developer diagnostics only (SEAM_BUILD_DIAGNOSTICS=1 builds)
-#else
-  sp.mode = 0;
-#endif
   sp.cg = cg;
   sp.thr_global = thr;
   sp.rowcnt = rowcnt;
@@ -817,19 +791,8 @@ static int score_topk_impl(seam_handle* h, const xchg::Exchange* x, const float*
   sp.rank_lo = nullptr;
   sp.rank_hi = nullptr;
   sp.rank_above = nullptr;
-  // developer diagnostics: SEAM_DEBUG_CTA_NS=1 records per-CTA durations at the tail of the fallback-row list
-  sp.cta_ns = (h->dbg_cta_ns && (size_t)Q * 4 >= 8192)
-                  ? reinterpret_cast<unsigned long long*>(ws + s.off_rows + (((size_t)Q * 4 - 4096) & ~(size_t)7))
-                  : nullptr;
   {
     ProfileScope prof(h, SEAM_KERNEL_SCORE, stream);
-#ifdef SEAM_DIAGNOSTIC_VARIANTS
-    if (sp.mode == 2) score::score_topk_kernel<2><<<s.grid, score::THREADS, score::SMEM_BYTES, stream>>>(tmA, tmB, sp);
-    else if (sp.mode == 3) score::score_topk_kernel<3><<<s.grid, score::THREADS, score::SMEM_BYTES, stream>>>(tmA, tmB, sp);
-    else if (sp.mode == 4) score::score_topk_kernel<4><<<s.grid, score::THREADS, score::SMEM_BYTES, stream>>>(tmA, tmB, sp);
-    else if (sp.mode == 5) score::score_topk_kernel<5><<<s.grid, score::THREADS, score::SMEM_BYTES, stream>>>(tmA, tmB, sp);
-    else
-#endif
     score::score_topk_kernel<0><<<s.grid, score::THREADS, score::SMEM_BYTES, stream>>>(tmA, tmB, sp);
     SEAM_LAUNCHED(h, "score_topk_kernel");
   }
@@ -1021,7 +984,7 @@ int seam_rank_of_target(seam_handle* h, const float* q, int Q, const float* g, i
 
 size_t seam_rank_workspace_bytes(const seam_handle* h, int Q, int G) {
   if (!h || Q <= 0 || G <= 0) return 256;
-  return plan_score(h->num_sms, Q, G, 0, h->score_nseed, h->dbg_score_grid).total;
+  return plan_score(h->num_sms, Q, G, true).total;
 }
 
 // Tensor-core path: prepare queries -> exact target margins + bands -> score_topk_kernel<VAR_RANK> (counts
@@ -1043,7 +1006,7 @@ int seam_rank_of_target_prepared(seam_handle* h, const float* q, int Q, const fl
     return fail(h, SEAM_ERR_BAD_ARG, "seam_rank_of_target_prepared: null pointer");
   if (!aligned16(q) || !aligned16(g) || !aligned16(g16) || (reinterpret_cast<uintptr_t>(workspace) & 255u))
     return fail(h, SEAM_ERR_UNSUPPORTED, "seam_rank_of_target_prepared: q/g/g16 need 16-byte, workspace 256-byte alignment");
-  const ScorePlan s = plan_score(h->num_sms, Q, G, 0, h->score_nseed, h->dbg_score_grid);
+  const ScorePlan s = plan_score(h->num_sms, Q, G, true);
   if (s.ntiles_n > (1 << 18))
     return fail(h, SEAM_ERR_UNSUPPORTED, "seam_rank_of_target_prepared: G=%d exceeds the 2^26 gallery rows one shard may hold", G);
   if (workspace_bytes < s.total)
@@ -1087,7 +1050,6 @@ int seam_rank_of_target_prepared(seam_handle* h, const float* q, int Q, const fl
   sp.P = s.P;
   sp.CAP = s.CAP;
   sp.nseed = 0;
-  sp.mode = score::VAR_RANK;
   for (int b = 0; b <= s.grid; ++b) sp.tb[b] = s.tb[b];
   sp.cg = cg;
   sp.thr_global = thr;
@@ -1095,7 +1057,6 @@ int seam_rank_of_target_prepared(seam_handle* h, const float* q, int Q, const fl
   sp.rowflag = rowflag;
   sp.rowbuf = rowbuf;
   sp.gmax = gmax;
-  sp.cta_ns = nullptr;
   sp.rank_lo = lo;
   sp.rank_hi = hi;
   sp.rank_above = above;

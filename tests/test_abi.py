@@ -84,3 +84,17 @@ def test_ctypes_bindings_match_the_header():
         assert len(fn.argtypes) == n, f"{name}: header has {n} parameters, binding {len(fn.argtypes)}"
         seen += 1
     assert seen == len(pkg.declared_symbols())
+
+
+def test_library_has_one_build_and_reads_no_environment():
+    """The CUDA sources compile one way only: no preprocessor switch, no -D flag, and no environment variable
+    that changes at run time what the library computes or how it partitions the work."""
+    import re
+    from seam_match_rcnn_b200 import _build
+    assert not [f for f in _build.NVCC_FLAGS if f.startswith("-D")]
+    for f in sorted(os.listdir(_build.CSRC)):
+        if f.endswith((".cu", ".cuh")):
+            with open(os.path.join(_build.CSRC, f)) as fh:
+                text = fh.read()
+            assert not re.search(r"^\s*#\s*(if|ifdef|ifndef)\b", text, flags=re.M), f"{f}: conditional compilation"
+            assert "getenv" not in text, f"{f}: reads the environment"

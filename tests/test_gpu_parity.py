@@ -74,13 +74,14 @@ def test_aggregate_every_kernel_variant(Q, T, ragged, weights, engine):
         assert torch.equal(out.cpu()[single], seq[1][single])
 
 
-@pytest.mark.parametrize("Q,T,ragged", [(7500, 4, (1, 4)), (5000, 10, None), (5200, 9, (0, 9)), (3700, 16, None),
-                                        (3600, 14, (2, 14)), (1900, 32, None), (1850, 27, (17, 27)), (950, 64, None),
-                                        (930, 50, (33, 50))])
+@pytest.mark.parametrize("Q,T,ragged", [(7500, 4, (1, 4)), (7200, 10, None), (7300, 9, (0, 9)), (7150, 16, None),
+                                        (7250, 14, (2, 14)), (7400, 32, None), (7350, 27, (17, 27)), (7104, 64, None),
+                                        (7200, 50, (33, 50))])
 def test_aggregate_many_tracks_per_warp(Q, T, ragged, weights, engine):
     """Every kernel variant with MORE tracks than producers (three or more iterations per producer warp: buffers are
-    refilled -- by the loader warp at T <= 10, by the producers themselves otherwise -- batches are recycled), against
-    the oracle on a sample of tracks; lens and mask paths agree bit for bit."""
+    refilled -- by the loader warp at T <= 10, by the producers themselves otherwise) and at least three tensor-core
+    batches of 16 tracks per CTA (Q >= 3 x 16 x 148 SMs of a B200: the two batch buffers are reused from the third
+    batch on), against the oracle on a sample of tracks; lens and mask paths agree bit for bit."""
     seq, mask, lens = so.synth_tracks(Q, T, seed=3 * Q + T, ragged=ragged)
     out = engine.aggregate(seq.to(DEV), mask.to(DEV))
     out2 = engine.aggregate(seq.to(DEV), None, lens=torch.as_tensor(lens))
