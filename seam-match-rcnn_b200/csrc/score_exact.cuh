@@ -12,6 +12,7 @@
 #include <cuda_fp16.h>
 #include "exchange.cuh"
 #include "fold.cuh"
+#include "score_tc.cuh"
 #include "sm100_ptx.cuh"
 #include "warp_sort.cuh"
 
@@ -23,29 +24,6 @@ constexpr float FP16_MAX = 65504.f;
 // two operand roundings (2^-11 each) + fp32 accumulation slack.
 constexpr float EPS_COEFF = 9.9e-4f;   // 2^-10 = 9.77e-4, plus accumulation slack
 constexpr float TAG_REL_ERR = 8e-6f;   // > 2^-17 = 7.63e-6: 6 mantissa bits replaced by a column tag
-
-// The scorer's work decomposition as the re-score / resolve kernels need it: CTA b of the tensor-core pass swept the
-// linearised tiles [tb[b], tb[b+1]); a query tile's sweep was shared by `pieces` consecutive CTAs, each of which wrote
-// 4 sub-lists per row (count + group maxima, every call).  Slots beyond a row's pieces hold stale data from other
-// problem shapes and are never looked at -- so nothing has to be reset between calls.
-constexpr int PLAN_MAX_GRID = 160;
-struct PiecePlan {
-  int ntiles_n, nb;
-  int tb[PLAN_MAX_GRID + 1];
-};
-__device__ __forceinline__ int plan_cta_of_tile(const PiecePlan& pl, long long t) {
-  int lo = 0, hi = pl.nb - 1;
-  while (lo < hi) {
-    const int mid = (lo + hi + 1) >> 1;
-    if ((long long)pl.tb[mid] <= t) lo = mid;
-    else hi = mid - 1;
-  }
-  return lo;
-}
-__device__ __forceinline__ int plan_pieces_of_row(const PiecePlan& pl, int qi) {
-  const long long r0 = (long long)(qi >> 7) * pl.ntiles_n;            // query tiles of 128 rows (score::BM)
-  return plan_cta_of_tile(pl, r0 + pl.ntiles_n - 1) - plan_cta_of_tile(pl, r0) + 1;
-}
 
 __device__ __forceinline__ float softmax1(float l0, float l1) {
   const float m = fmaxf(l0, l1);
@@ -212,7 +190,7 @@ struct RescoreParams {
   int32_t* fallback_rows; // (Q)
   int x_on;               // sharded search: queries from the exchange's q_all, lists to the queries' owners
   xchg::Exchange x;
-  PiecePlan plan;         // which of the row's nlists slots the tensor-core pass wrote
+  score::TilePlan plan;   // which of the row's nlists slots the tensor-core pass wrote
 };
 
 // Where a query's top-k row goes.  Single GPU: row qi of the caller's (Q,k) outputs.  Sharded search: slot
@@ -291,7 +269,7 @@ __global__ void __launch_bounds__(256) rescore_kernel(const RescoreParams p) {
   const bool overflow = p.counters[1] != 0 || p.gstat[1] != 0.f;
   bool certified = !overflow && p.rowflag[qi] == 0;
   const float tau = ptx::ordered_to_float(p.thr_global[qi]);
-  const int nl_valid = min(p.nlists, 4 * plan_pieces_of_row(p.plan, qi));   // the sub-lists written for this row
+  const int nl_valid = min(p.nlists, 4 * score::pieces_of_row(p.plan, qi));   // the sub-lists written for this row
   float cv = -INFINITY;
   uint32_t cidx = 0xffffffffu;
   uint2* wb = wbuf[warp];
@@ -349,11 +327,10 @@ __global__ void __launch_bounds__(256) rescore_kernel(const RescoreParams p) {
     if (nval <= 128) start_cut(std::integral_constant<int, 4>{});
     else if (nval <= 256) start_cut(std::integral_constant<int, 8>{});
   }
-  // A record is a quad {w0,w1,w2,w3} of adjacent gallery rows (score_tc.cuh): the 6 low mantissa bits of
-  // w0 hold the quad's position inside its 64-column quarter, those of w1..w3 the gallery tile index;
-  // the quarter is the sub-list's index mod 4.  Two levels: quads whose maximum passes the cut are
-  // compacted into qb (one ballot per 32 quads); every 32 of those are expanded into elements, which
-  // are compacted into wb and merged into the best 32 as before.
+  // A record is a quad {w0,w1,w2,w3} of adjacent gallery rows whose tags name them (score_tc.cuh,
+  // quad_first_col).  Two levels: quads whose maximum passes the cut are compacted into qb (one ballot
+  // per 32 quads); every 32 of those are expanded into elements, which are compacted into wb and merged
+  // into the best 32 as before.
   const int capq = p.CAP / 2;
   const uint4* rowq = reinterpret_cast<const uint4*>(p.rowbuf) + (size_t)qi * p.nlists * capq;
   uint4* qb = qbuf[warp];
@@ -423,10 +400,9 @@ __global__ void __launch_bounds__(256) rescore_kernel(const RescoreParams p) {
           const uint32_t mask = __ballot_sync(ptx::FULL_MASK, pass);
           if (mask == 0u) continue;                  // warp-uniform
           if (pass) {
-            const uint32_t tile = (e[u].y & 63u) | ((e[u].z & 63u) << 6) | ((e[u].w & 63u) << 12);
             const int pos = qfill + __popc(mask & ((1u << lane) - 1u));
             qb[pos] = e[u];
-            qc[pos] = tile * 256u + (uint32_t)((j0 + u) & 3) * 64u + (e[u].x & 63u) * 4u;
+            qc[pos] = score::quad_first_col(e[u], l0 + j0 + u);
           }
           qfill += __popc(mask);
           if (qfill >= 32) {
@@ -911,7 +887,7 @@ struct RankResolveParams {
   const float* gstat;
   const int32_t* target;
   int Q, G, nlists, CAP;
-  PiecePlan plan;
+  score::TilePlan plan;
   int32_t* out_rank;
   float* out_margin;         // optional
   int32_t* counters;         // [0] rows for the exhaustive kernel, [1] query overflow flag
@@ -971,7 +947,7 @@ __global__ void __launch_bounds__(256) rank_resolve_kernel(const RankResolvePara
     fill = 0;
     __syncwarp();
   };
-  const int nl_valid = min(p.nlists, 4 * plan_pieces_of_row(p.plan, qi));
+  const int nl_valid = min(p.nlists, 4 * score::pieces_of_row(p.plan, qi));
   for (int l0 = 0; l0 < nl_valid && ok; l0 += 32) {
     const int my_l = l0 + lane;
     const uint32_t my_n = my_l < nl_valid ? p.rowcnt[(size_t)qi * p.nlists + my_l] : 0u;
@@ -985,8 +961,7 @@ __global__ void __launch_bounds__(256) rank_resolve_kernel(const RankResolvePara
         const bool have = base + lane < n;
         const uint4 rec = have ? __ldcs(lp + base + lane) : make_uint4(0u, 0u, 0u, 0u);
         const uint32_t wv[4] = {rec.x, rec.y, rec.z, rec.w};
-        const uint32_t tile = (rec.y & 63u) | ((rec.z & 63u) << 6) | ((rec.w & 63u) << 12);
-        const uint32_t col = tile * 256u + (uint32_t)(j & 3) * 64u + (rec.x & 63u) * 4u;
+        const uint32_t col = score::quad_first_col(rec, l0 + j);
 #pragma unroll
         for (int el = 0; el < 4; ++el) {
           const float ev = __uint_as_float(wv[el]);

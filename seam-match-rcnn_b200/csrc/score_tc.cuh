@@ -70,9 +70,34 @@ static_assert(OFF_CG % 16 == 0 && OFF_THRX % 16 == 0 && OFF_CMD % 16 == 0 && OFF
 
 constexpr int MAX_GRID = 160;          // one persistent CTA per SM
 constexpr int VAR_RANK = 6;            // kernel variant: rank of one designated gallery item per query
+
+// The work decomposition, cost-balanced on the host: CTA b of nb sweeps the linearised tiles [tb[b], tb[b+1]).
+// A query tile's sweep is shared by consecutive CTAs, its rows' "pieces", each of which writes 4 sub-lists
+// per row (count + group maxima, every call).  Slots beyond a row's pieces hold stale data from other problem
+// shapes and are never looked at -- so nothing has to be reset between calls.
+struct TilePlan {
+  int ntiles_n, nb;
+  int tb[MAX_GRID + 1];
+};
+
+// the CTA whose (non-empty) range contains tile t: the largest b with tb[b] <= t
+__device__ __forceinline__ int cta_of_tile(const TilePlan& pl, long long t) {
+  int lo = 0, hi = pl.nb - 1;
+  while (lo < hi) {
+    const int mid = (lo + hi + 1) >> 1;
+    if ((long long)pl.tb[mid] <= t) lo = mid;
+    else hi = mid - 1;
+  }
+  return lo;
+}
+// the number of CTAs that swept query row qi's gallery tiles
+__device__ __forceinline__ int pieces_of_row(const TilePlan& pl, int qi) {
+  const long long r0 = (long long)(qi / BM) * pl.ntiles_n;
+  return cta_of_tile(pl, r0 + pl.ntiles_n - 1) - cta_of_tile(pl, r0) + 1;
+}
+
 struct Params {
-  int Q, G, num_mtiles, ntiles_n;
-  long long total_tiles;
+  int Q, G;
   int P;                      // sub-list slots per row: max CTAs sharing one query tile's sweep
   int CAP;                    // entries per sub-list
   int nseed;                  // threshold-only sample tiles at the start of a segment
@@ -82,24 +107,13 @@ struct Params {
   uint32_t* rowflag;          // (Q) nonzero: the row lost candidates, must be ranked exhaustively
   uint2* rowbuf;              // (Q, P, 4, CAP x 8 bytes) = CAP/2 quad records {w0,w1,w2,w3} per sub-list
   float* gmax;                // (Q, P, 4, 16) final group maxima of each thread (disjoint column groups)
-  int tb[MAX_GRID + 1];       // CTA b sweeps the linearised tiles [tb[b], tb[b+1]) (cost-balanced on the host)
+  TilePlan plan;
   // rank-of-target variant (VAR_RANK): per-row band (lo, hi] around the target's value and, per sub-list,
   // the number of elements certainly above it
   const float* rank_lo;       // (Q)
   const float* rank_hi;       // (Q)
   int32_t* rank_above;        // (Q, P, 4)
 };
-
-// the CTA whose (non-empty) range contains tile t: the largest b with tb[b] <= t
-__device__ __forceinline__ int cta_of_tile(const Params& p, int nb, long long t) {
-  int lo = 0, hi = nb - 1;
-  while (lo < hi) {
-    const int mid = (lo + hi + 1) >> 1;
-    if ((long long)p.tb[mid] <= t) lo = mid;
-    else hi = mid - 1;
-  }
-  return lo;
-}
 
 // One segment = query tile m, gallery tiles [nt0, nt0 + n_main), preceded by n_seed sample tiles
 // (threshold-only previews of tiles spread over the same range).
@@ -123,13 +137,13 @@ constexpr int NSEED = 4;               // sample tiles of a sampled segment (the
 __device__ __forceinline__ Segment segment_before(const Params& p, long long t_begin, long long t_hi, long long t_end,
                                                   long long& next_hi) {
   Segment s;
-  s.m = (int)((t_hi - 1) / p.ntiles_n);
-  const long long row0 = (long long)s.m * p.ntiles_n;
+  s.m = (int)((t_hi - 1) / p.plan.ntiles_n);
+  const long long row0 = (long long)s.m * p.plan.ntiles_n;
   const long long start = max(t_begin, row0);
   s.nt0 = (int)(start - row0);
   s.n_main = (int)(t_hi - start);
   s.n_seed = (t_hi == t_end || start == row0) ? min(p.nseed, s.n_main) : 0;
-  s.ntiles_n = p.ntiles_n;
+  s.ntiles_n = p.plan.ntiles_n;
   next_hi = start;
   return s;
 }
@@ -192,6 +206,14 @@ __device__ __forceinline__ float eighth_largest_of_16(const float (&gm)[16]) {
 // compared and recorded as group maximum too: the whole filter is consistent in "w space".
 constexpr uint32_t TAG_MASK = 63u;
 constexpr int TAG_BITS = 6;
+constexpr int TAG_TILES = 1 << (3 * TAG_BITS);   // gallery tiles a record can name
+// The gallery column of w0 of a record read from sub-list l of its row; w1..w3 are the next three.  The
+// inverse of the tagging in filter16 / filter16_rank: the sub-list gives the column quarter.
+__device__ __forceinline__ uint32_t quad_first_col(const uint4& rec, int l) {
+  const uint32_t tile =
+      (rec.y & TAG_MASK) | ((rec.z & TAG_MASK) << TAG_BITS) | ((rec.w & TAG_MASK) << (2 * TAG_BITS));
+  return tile * BN + ((uint32_t)l % NQ) * QCOLS + (rec.x & TAG_MASK) * 4u;
+}
 template <int Q4>
 __device__ __forceinline__ float tagged_imm(uint32_t acc, float cg, uint32_t keep) {
   float w;
@@ -386,8 +408,8 @@ score_topk_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant
   const uint32_t tmem_base = *tmem_ptr_s;
 
   long long t_begin, t_end;
-  t_begin = p.tb[blockIdx.x];
-  t_end = p.tb[blockIdx.x + 1];
+  t_begin = p.plan.tb[blockIdx.x];
+  t_end = p.plan.tb[blockIdx.x + 1];
 
   if (warp == 0) {
     // ================================================================= TMA producer
@@ -480,7 +502,7 @@ score_topk_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant
     while (t > t_begin) {
       const Segment sg = segment_before(p, t_begin, t, t_end, next);
       const int n = sg.count();
-      const int piece = blockIdx.x - cta_of_tile(p, gridDim.x, (long long)sg.m * p.ntiles_n);
+      const int piece = blockIdx.x - cta_of_tile(p.plan, (long long)sg.m * p.plan.ntiles_n);
       for (int i = 0; i < n; ++i) {
         const int nt = sg.tile(i);
         const int j0 = nt * BN + lane * 8;

@@ -74,7 +74,6 @@ struct ProfileScope {
   }
 };
 
-static_assert(exact::PLAN_MAX_GRID == score::MAX_GRID, "the re-score kernels carry a copy of the scorer's CTA ranges");
 static thread_local char g_create_err[256] = "";
 
 static unsigned int* g_watchdog_host[64] = {};
@@ -523,9 +522,9 @@ int seam_prepare_gallery(seam_handle* h, const float* g, int G, void* g16, float
 }
 
 struct ScorePlan {
-  int num_mtiles, ntiles_n, grid, P, CAP, nseed;
-  int tb[score::MAX_GRID + 1];
-  long long total_tiles;
+  int num_mtiles, P, CAP, nseed;
+  score::TilePlan tiles;
+  size_t xunits;   // the exhaustive kernel's partial-list units (off_xpart)
   size_t off_a16, off_rq, off_anorm, off_thr, off_rowcnt, off_gmax, off_rowflag, off_rowbuf, off_cnt, off_rows, off_xpart, off_xdone, total;
 };
 
@@ -535,27 +534,29 @@ struct ScorePlan {
 // the row) of CAP entries, CAP >= 3 times the expected number of appends.
 static ScorePlan plan_score(int num_sms, int Q, int G, bool rank) {
   ScorePlan s;
+  score::TilePlan& tp = s.tiles;
   s.num_mtiles = (Q + score::BM - 1) / score::BM;
-  s.ntiles_n = (G + score::BN - 1) / score::BN;
+  tp.ntiles_n = (G + score::BN - 1) / score::BN;
   if (s.num_mtiles < 1) s.num_mtiles = 1;
-  if (s.ntiles_n < 1) s.ntiles_n = 1;
-  s.total_tiles = (long long)s.num_mtiles * s.ntiles_n;
-  s.grid = s.total_tiles < num_sms ? (int)s.total_tiles : num_sms;
-  if (s.grid > score::MAX_GRID) s.grid = score::MAX_GRID;
+  if (tp.ntiles_n < 1) tp.ntiles_n = 1;
+  const long long ntn = tp.ntiles_n, total = (long long)s.num_mtiles * ntn;
+  tp.nb = total < num_sms ? (int)total : num_sms;
+  if (tp.nb > score::MAX_GRID) tp.nb = score::MAX_GRID;
+  const int grid = tp.nb;
+  int* tb = tp.tb;
   s.nseed = rank ? 0 : score::NSEED;
   // Cost-balanced contiguous ranges.  A tile costs 1; a segment start costs SEG_COST (query tile load,
   // epilogue hand-over); a segment that holds its row's first gallery tile -- or is all a CTA has --
   // also sweeps min(nseed, length) threshold-only sample tiles (score_tc.cuh, segment_before).  walk()
   // cuts ranges of cost <= target; the smallest target whose last range also fits is found by bisection.
   const double SEG_COST = 0.35;
-  const long long ntn = s.ntiles_n, total = s.total_tiles;
-  auto walk = [&](double target, int* tb) -> double {   // returns the cost of the last CTA's range
+  auto walk = [&](double target) -> double {   // returns the cost of the last CTA's range
     long long pos = 0;
     tb[0] = 0;
-    for (int b = 0; b < s.grid; ++b) {
+    for (int b = 0; b < grid; ++b) {
       const long long t0 = pos;
       double cost = 0.0;
-      const bool last = b == s.grid - 1;
+      const bool last = b == grid - 1;
       while (pos < total) {
         const long long row_end = (pos / ntn + 1) * ntn;
         const long long seg_len = row_end - pos;
@@ -582,15 +583,15 @@ static ScorePlan plan_score(int num_sms, int Q, int G, bool rank) {
   };
   {
     // every query tile starts a segment, every CTA boundary at most one more
-    const double all = (double)total + ((double)s.num_mtiles + s.grid) * (SEG_COST + s.nseed);
-    double lo = (double)total / s.grid, hi = 2.0 * all / s.grid + s.nseed + 2.0;
+    const double all = (double)total + ((double)s.num_mtiles + grid) * (SEG_COST + s.nseed);
+    double lo = (double)total / grid, hi = 2.0 * all / grid + s.nseed + 2.0;
     for (int it = 0; it < 40; ++it) {
       const double mid = 0.5 * (lo + hi);
-      if (walk(mid, s.tb) <= mid) hi = mid;
+      if (walk(mid) <= mid) hi = mid;
       else lo = mid;
     }
-    walk(hi, s.tb);
-    s.tb[s.grid] = (int)total;
+    walk(hi);
+    tb[grid] = (int)total;
   }
   // sub-list slots per row = most CTAs whose ranges touch one query tile's sweep (pieces are numbered
   // from the first CTA that touches the row)
@@ -600,13 +601,13 @@ static ScorePlan plan_score(int num_sms, int Q, int G, bool rank) {
     int b_first = 0;
     for (long long m = 0; m < s.num_mtiles; ++m) {
       const long long r0 = m * ntn, r1 = r0 + ntn;
-      while (b_first + 1 < s.grid && s.tb[b_first + 1] <= r0) ++b_first;   // first CTA with tb[b+1] > r0
+      while (b_first + 1 < grid && tb[b_first + 1] <= r0) ++b_first;   // first CTA with tb[b+1] > r0
       int b_last = b_first;
-      while (b_last + 1 < s.grid && s.tb[b_last + 1] < r1) ++b_last;
+      while (b_last + 1 < grid && tb[b_last + 1] < r1) ++b_last;
       if (b_last - b_first + 1 > pmax) pmax = b_last - b_first + 1;
     }
-    for (int b = 0; b < s.grid; ++b)
-      if (s.tb[b + 1] - s.tb[b] > max_range) max_range = s.tb[b + 1] - s.tb[b];
+    for (int b = 0; b < grid; ++b)
+      if (tb[b + 1] - tb[b] > max_range) max_range = tb[b + 1] - tb[b];
   }
   s.P = pmax;
   // Expected bytes one epilogue thread appends over a piece of T tiles.  A record is a quad of 4 adjacent
@@ -615,7 +616,7 @@ static ScorePlan plan_score(int num_sms, int Q, int G, bool rank) {
   // bound, a quarter of them in this thread's columns), nearly all in different quads; seeded pieces start
   // at the rate of tile nseed+1.  Segments shorter than 4*nseed tiles run unseeded and may append whole
   // tiles.  3x margin on the sparse part.
-  const double T = (double)(max_range < s.ntiles_n ? max_range : s.ntiles_n);
+  const double T = (double)(max_range < ntn ? max_range : ntn);
   const double tile_bytes = score::QCOLS / 4 * 16.0;
   double need;
   if (s.nseed > 0) {
@@ -652,8 +653,8 @@ static ScorePlan plan_score(int num_sms, int Q, int G, bool rank) {
   s.off_cnt = o;     o += 256;
   s.off_rows = o;    o += align_up((size_t)Q * 4, 256);
   // exhaustive kernel: per-slice lists of rows split over several CTAs (units <= max(its grid, Q)), per-row counts
-  const size_t xunits = (size_t)(Q > 2 * num_sms ? Q : 2 * num_sms);
-  s.off_xpart = o;   o += align_up(xunits * 32 * 8, 256);
+  s.xunits = (size_t)(Q > 2 * num_sms ? Q : 2 * num_sms);
+  s.off_xpart = o;   o += align_up(s.xunits * 32 * 8, 256);
   s.off_xdone = o;   o += align_up((size_t)Q * 4, 256);
   s.total = o;
   return s;
@@ -668,7 +669,7 @@ size_t seam_score_workspace_bytes(const seam_handle* h, int Q, int G, int k) {
 int seam_score_plan(const seam_handle* h, int Q, int G, int64_t* out) {
   if (!h || !out || Q <= 0 || G <= 0) return SEAM_ERR_BAD_ARG;
   const ScorePlan s = plan_score(h->num_sms, Q, G, false);
-  const int64_t v[14] = {s.num_mtiles, s.ntiles_n, s.grid, s.P, s.CAP, (int64_t)s.off_a16,
+  const int64_t v[14] = {s.num_mtiles, s.tiles.ntiles_n, s.tiles.nb, s.P, s.CAP, (int64_t)s.off_a16,
                          (int64_t)s.off_rq, (int64_t)s.off_anorm, (int64_t)s.off_thr, (int64_t)s.off_rowcnt,
                          (int64_t)s.off_rowbuf, (int64_t)s.off_cnt, (int64_t)s.off_rows, (int64_t)s.total};
   for (int i = 0; i < 14; ++i) out[i] = v[i];
@@ -679,11 +680,11 @@ int seam_score_plan(const seam_handle* h, int Q, int G, int64_t* out) {
 int seam_score_partition(int num_sms, int Q, int G, int rank_variant, int32_t* bounds, int bounds_len, int32_t* out6) {
   if (num_sms < 1 || Q <= 0 || G <= 0 || !bounds || !out6) return SEAM_ERR_BAD_ARG;
   const ScorePlan s = plan_score(num_sms, Q, G, rank_variant != 0);
-  if (bounds_len < s.grid + 1) return SEAM_ERR_BAD_ARG;
-  for (int b = 0; b <= s.grid; ++b) bounds[b] = s.tb[b];
+  if (bounds_len < s.tiles.nb + 1) return SEAM_ERR_BAD_ARG;
+  for (int b = 0; b <= s.tiles.nb; ++b) bounds[b] = s.tiles.tb[b];
   out6[0] = s.num_mtiles;
-  out6[1] = s.ntiles_n;
-  out6[2] = s.grid;
+  out6[1] = s.tiles.ntiles_n;
+  out6[2] = s.tiles.nb;
   out6[3] = s.P;
   out6[4] = s.CAP;
   out6[5] = s.nseed;
@@ -708,6 +709,82 @@ static int encode_map_fp16_rows(seam_handle* h, CUtensorMap* map, const void* ba
                          CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
                          CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
   if (r != CUDA_SUCCESS) return fail(h, SEAM_ERR_CUDA, "cuTensorMapEncodeTiled failed with CUresult %d", (int)r);
+  return SEAM_OK;
+}
+
+// The scorer's workspace, carved by plan_score's offsets into typed buffers.
+struct ScoreWorkspace {
+  ScorePlan plan;
+  __half* a16;
+  float *rq, *anorm, *gmax;
+  uint32_t *thr, *rowcnt, *rowflag;
+  uint2* rowbuf;
+  int32_t *counters, *frows;
+  float* xpart_d;              // exhaustive kernel
+  int32_t *xpart_i, *xdone;
+  // rank variant only (null otherwise): it keeps no group maxima, and its per-sub-list counts of the elements
+  // above the band (Q x nlists), the band (lo, hi] and the target margins (Q each) live in that region
+  int32_t* above;
+  float *lo, *hi, *dtarget;
+};
+
+// Checks what both scorer variants take, plans the work and carves the workspace; fn names the entry point.
+static int carve_score_workspace(seam_handle* h, const char* fn, bool rank, const float* q, int Q, const float* g,
+                                 const void* g16, const float* cg, const float* gstat, int G, void* workspace,
+                                 size_t workspace_bytes, ScoreWorkspace* w) {
+  if (!q || !g || !g16 || !cg || !gstat || !workspace) return fail(h, SEAM_ERR_BAD_ARG, "%s: null pointer", fn);
+  if (!aligned16(q) || !aligned16(g) || !aligned16(g16) || (reinterpret_cast<uintptr_t>(workspace) & 255u))
+    return fail(h, SEAM_ERR_UNSUPPORTED, "%s: q/g/g16 need 16-byte, workspace 256-byte alignment", fn);
+  const ScorePlan& s = w->plan = plan_score(h->num_sms, Q, G, rank);
+  if (s.tiles.ntiles_n > score::TAG_TILES)
+    return fail(h, SEAM_ERR_UNSUPPORTED, "%s: G=%d exceeds the %d gallery rows one shard may hold", fn, G,
+                score::TAG_TILES * score::BN);
+  if (workspace_bytes < s.total)
+    return fail(h, SEAM_ERR_STATE, "%s: workspace too small (%zu < %zu)", fn, workspace_bytes, s.total);
+  uint8_t* ws = static_cast<uint8_t*>(workspace);
+  w->a16 = reinterpret_cast<__half*>(ws + s.off_a16);
+  w->rq = reinterpret_cast<float*>(ws + s.off_rq);
+  w->anorm = reinterpret_cast<float*>(ws + s.off_anorm);
+  w->thr = reinterpret_cast<uint32_t*>(ws + s.off_thr);
+  w->rowcnt = reinterpret_cast<uint32_t*>(ws + s.off_rowcnt);
+  w->gmax = reinterpret_cast<float*>(ws + s.off_gmax);
+  w->rowflag = reinterpret_cast<uint32_t*>(ws + s.off_rowflag);
+  // sub-lists are aligned to their (power-of-two) size so that none straddles a 4 GiB boundary
+  w->rowbuf = reinterpret_cast<uint2*>(align_up(reinterpret_cast<uintptr_t>(ws + s.off_rowbuf), (size_t)s.CAP * 8));
+  w->counters = reinterpret_cast<int32_t*>(ws + s.off_cnt);
+  w->frows = reinterpret_cast<int32_t*>(ws + s.off_rows);
+  w->xpart_d = reinterpret_cast<float*>(ws + s.off_xpart);
+  w->xpart_i = reinterpret_cast<int32_t*>(ws + s.off_xpart + s.xunits * 32 * 4);
+  w->xdone = reinterpret_cast<int32_t*>(ws + s.off_xdone);
+  const size_t nlists = (size_t)s.P * score::NQ;
+  w->above = rank ? reinterpret_cast<int32_t*>(w->gmax) : nullptr;
+  w->lo = rank ? w->gmax + Q * nlists : nullptr;
+  w->hi = rank ? w->lo + Q : nullptr;
+  w->dtarget = rank ? w->hi + Q : nullptr;
+  return SEAM_OK;
+}
+
+// The tensor maps of the fp16 query and gallery operands and score_topk_kernel's parameters, for either variant.
+static int score_kernel_args(seam_handle* h, const ScoreWorkspace& w, int Q, const void* g16, const float* cg, int G,
+                             CUtensorMap* tmA, CUtensorMap* tmB, score::Params* sp) {
+  int rc;
+  if ((rc = encode_map_fp16_rows(h, tmA, w.a16, Q, score::BM)) != SEAM_OK) return rc;
+  if ((rc = encode_map_fp16_rows(h, tmB, g16, G, score::BN)) != SEAM_OK) return rc;
+  sp->Q = Q;
+  sp->G = G;
+  sp->P = w.plan.P;
+  sp->CAP = w.plan.CAP;
+  sp->nseed = w.plan.nseed;
+  sp->cg = cg;
+  sp->thr_global = w.thr;
+  sp->rowcnt = w.rowcnt;
+  sp->rowflag = w.rowflag;
+  sp->rowbuf = w.rowbuf;
+  sp->gmax = w.gmax;
+  sp->plan = w.plan.tiles;
+  sp->rank_lo = w.lo;
+  sp->rank_hi = w.hi;
+  sp->rank_above = w.above;
   return SEAM_OK;
 }
 
@@ -736,64 +813,23 @@ static int score_topk_impl(seam_handle* h, const xchg::Exchange* x, const float*
     SEAM_LAUNCHED(h, "fill_empty_topk_kernel");
     return SEAM_OK;
   }
-  if (!q || !g || !g16 || !cg || !gstat || !workspace) return fail(h, SEAM_ERR_BAD_ARG, "seam_score_topk: null pointer");
-  if (!aligned16(q) || !aligned16(g) || !aligned16(g16) || (reinterpret_cast<uintptr_t>(workspace) & 255u))
-    return fail(h, SEAM_ERR_UNSUPPORTED, "seam_score_topk: q/g/g16 need 16-byte, workspace 256-byte alignment");
-  const ScorePlan s = plan_score(h->num_sms, Q, G, false);
-  if (s.ntiles_n > (1 << 18))
-    return fail(h, SEAM_ERR_UNSUPPORTED, "seam_score_topk: G=%d exceeds the 2^26 gallery rows one shard may hold", G);
-  if (workspace_bytes < s.total)
-    return fail(h, SEAM_ERR_STATE, "seam_score_topk: workspace too small (%zu < %zu)", workspace_bytes, s.total);
-  uint8_t* ws = static_cast<uint8_t*>(workspace);
-  __half* a16 = reinterpret_cast<__half*>(ws + s.off_a16);
-  float* rq = reinterpret_cast<float*>(ws + s.off_rq);
-  float* anorm = reinterpret_cast<float*>(ws + s.off_anorm);
-  uint32_t* thr = reinterpret_cast<uint32_t*>(ws + s.off_thr);
-  uint32_t* rowcnt = reinterpret_cast<uint32_t*>(ws + s.off_rowcnt);
-  float* gmax = reinterpret_cast<float*>(ws + s.off_gmax);
-  uint32_t* rowflag = reinterpret_cast<uint32_t*>(ws + s.off_rowflag);
-  // sub-lists are aligned to their (power-of-two) size so that none straddles a 4 GiB boundary
-  uint2* rowbuf = reinterpret_cast<uint2*>(
-      align_up(reinterpret_cast<uintptr_t>(ws + s.off_rowbuf), (size_t)s.CAP * 8));
-  int32_t* counters = reinterpret_cast<int32_t*>(ws + s.off_cnt);
-  int32_t* frows = reinterpret_cast<int32_t*>(ws + s.off_rows);
-  const size_t xunits = (size_t)(Q > 2 * h->num_sms ? Q : 2 * h->num_sms);
-  float* xpart_d = reinterpret_cast<float*>(ws + s.off_xpart);
-  int32_t* xpart_i = reinterpret_cast<int32_t*>(ws + s.off_xpart + xunits * 32 * 4);
-  int32_t* xdone = reinterpret_cast<int32_t*>(ws + s.off_xdone);
+  ScoreWorkspace w;
+  int rc = carve_score_workspace(h, "seam_score_topk", false, q, Q, g, g16, cg, gstat, G, workspace, workspace_bytes, &w);
+  if (rc != SEAM_OK) return rc;
 
   {
     ProfileScope prof(h, SEAM_KERNEL_PREP_QUERIES, stream);
-    exact::prep_queries_kernel<<<(Q + 7) / 8, 256, 0, stream>>>(q, Q, h->fold, a16, rq, anorm, thr, rowflag, counters, xdone, x_on, xe);
+    exact::prep_queries_kernel<<<(Q + 7) / 8, 256, 0, stream>>>(q, Q, h->fold, w.a16, w.rq, w.anorm, w.thr, w.rowflag,
+                                                                w.counters, w.xdone, x_on, xe);
     SEAM_LAUNCHED(h, "prep_queries_kernel");
   }
 
   CUtensorMap tmA, tmB;
-  int rc;
-  if ((rc = encode_map_fp16_rows(h, &tmA, a16, Q, score::BM)) != SEAM_OK) return rc;
-  if ((rc = encode_map_fp16_rows(h, &tmB, g16, G, score::BN)) != SEAM_OK) return rc;
   score::Params sp;
-  sp.Q = Q;
-  sp.G = G;
-  sp.num_mtiles = s.num_mtiles;
-  sp.ntiles_n = s.ntiles_n;
-  sp.total_tiles = s.total_tiles;
-  sp.P = s.P;
-  sp.CAP = s.CAP;
-  sp.nseed = s.nseed;
-  for (int b = 0; b <= s.grid; ++b) sp.tb[b] = s.tb[b];
-  sp.cg = cg;
-  sp.thr_global = thr;
-  sp.rowcnt = rowcnt;
-  sp.rowflag = rowflag;
-  sp.rowbuf = rowbuf;
-  sp.gmax = gmax;
-  sp.rank_lo = nullptr;
-  sp.rank_hi = nullptr;
-  sp.rank_above = nullptr;
+  if ((rc = score_kernel_args(h, w, Q, g16, cg, G, &tmA, &tmB, &sp)) != SEAM_OK) return rc;
   {
     ProfileScope prof(h, SEAM_KERNEL_SCORE, stream);
-    score::score_topk_kernel<0><<<s.grid, score::THREADS, score::SMEM_BYTES, stream>>>(tmA, tmB, sp);
+    score::score_topk_kernel<0><<<w.plan.tiles.nb, score::THREADS, score::SMEM_BYTES, stream>>>(tmA, tmB, sp);
     SEAM_LAUNCHED(h, "score_topk_kernel");
   }
 
@@ -801,30 +837,28 @@ static int score_topk_impl(seam_handle* h, const xchg::Exchange* x, const float*
   rp.q = q;
   rp.g = g;
   rp.fold = h->fold;
-  rp.rowbuf = rowbuf;
-  rp.rowcnt = rowcnt;
-  rp.rowflag = rowflag;
-  rp.thr_global = thr;
-  rp.gmax = gmax;
-  rp.rq = rq;
-  rp.anorm = anorm;
+  rp.rowbuf = w.rowbuf;
+  rp.rowcnt = w.rowcnt;
+  rp.rowflag = w.rowflag;
+  rp.thr_global = w.thr;
+  rp.gmax = w.gmax;
+  rp.rq = w.rq;
+  rp.anorm = w.anorm;
   rp.gstat = gstat;
   rp.Q = Q;
   rp.G = G;
-  rp.nlists = s.P * score::NQ;
-  rp.CAP = s.CAP;
+  rp.nlists = w.plan.P * score::NQ;
+  rp.CAP = w.plan.CAP;
   rp.k = k;
   rp.index_offset = index_offset;
   rp.out_score = out_score;
   rp.out_margin = out_margin;
   rp.out_idx = out_idx;
-  rp.counters = counters;
-  rp.fallback_rows = frows;
+  rp.counters = w.counters;
+  rp.fallback_rows = w.frows;
   rp.x_on = x_on;
   rp.x = xe;
-  rp.plan.ntiles_n = s.ntiles_n;
-  rp.plan.nb = s.grid;
-  for (int b = 0; b <= s.grid; ++b) rp.plan.tb[b] = s.tb[b];
+  rp.plan = w.plan.tiles;
   {
     ProfileScope prof(h, SEAM_KERNEL_RESCORE, stream);
     exact::rescore_kernel<<<(Q + 7) / 8, 256, 0, stream>>>(rp);
@@ -839,14 +873,14 @@ static int score_topk_impl(seam_handle* h, const xchg::Exchange* x, const float*
   ep.G = G;
   ep.k = k;
   ep.index_offset = index_offset;
-  ep.count = counters;
-  ep.rows = frows;
+  ep.count = w.counters;
+  ep.rows = w.frows;
   ep.out_score = out_score;
   ep.out_margin = out_margin;
   ep.out_idx = out_idx;
-  ep.part_d = xpart_d;
-  ep.part_i = xpart_i;
-  ep.done = xdone;
+  ep.part_d = w.xpart_d;
+  ep.part_i = w.xpart_i;
+  ep.done = w.xdone;
   ep.x_on = x_on;
   ep.x = xe;
   {
@@ -854,7 +888,7 @@ static int score_topk_impl(seam_handle* h, const xchg::Exchange* x, const float*
     exact::exact_topk_kernel<<<2 * h->num_sms, 256, 0, stream>>>(ep);
     SEAM_LAUNCHED(h, "exact_topk_kernel");
   }
-  if (stats) SEAM_CUDA(h, cudaMemcpyAsync(stats, counters, 4, cudaMemcpyDeviceToDevice, stream));
+  if (stats) SEAM_CUDA(h, cudaMemcpyAsync(stats, w.counters, 4, cudaMemcpyDeviceToDevice, stream));
   return SEAM_OK;
 }
 
@@ -989,8 +1023,7 @@ size_t seam_rank_workspace_bytes(const seam_handle* h, int Q, int G) {
 
 // Tensor-core path: prepare queries -> exact target margins + bands -> score_topk_kernel<VAR_RANK> (counts
 // what is certainly above, appends what is inside the band) -> rank_resolve_kernel -> exhaustive kernel for
-// the rows that could not be certified.  The workspace is laid out like seam_score_topk's (no sample
-// tiles); the band, the target margins and the per-sub-list counts live in its group-maxima region.
+// the rows that could not be certified.  The workspace is laid out like seam_score_topk's (no sample tiles).
 int seam_rank_of_target_prepared(seam_handle* h, const float* q, int Q, const float* g, const void* g16,
                                  const float* cg, const float* gstat, int G, const int32_t* target, int32_t* out_rank,
                                  float* out_margin, int32_t* stats, void* workspace, size_t workspace_bytes,
@@ -1002,98 +1035,57 @@ int seam_rank_of_target_prepared(seam_handle* h, const float* q, int Q, const fl
   DeviceGuard guard(h->device);
   if (stats) SEAM_CUDA(h, cudaMemsetAsync(stats, 0, 16, stream));
   if (Q == 0) return SEAM_OK;
-  if (!q || !g || !g16 || !cg || !gstat || !target || !out_rank || !workspace)
-    return fail(h, SEAM_ERR_BAD_ARG, "seam_rank_of_target_prepared: null pointer");
-  if (!aligned16(q) || !aligned16(g) || !aligned16(g16) || (reinterpret_cast<uintptr_t>(workspace) & 255u))
-    return fail(h, SEAM_ERR_UNSUPPORTED, "seam_rank_of_target_prepared: q/g/g16 need 16-byte, workspace 256-byte alignment");
-  const ScorePlan s = plan_score(h->num_sms, Q, G, true);
-  if (s.ntiles_n > (1 << 18))
-    return fail(h, SEAM_ERR_UNSUPPORTED, "seam_rank_of_target_prepared: G=%d exceeds the 2^26 gallery rows one shard may hold", G);
-  if (workspace_bytes < s.total)
-    return fail(h, SEAM_ERR_STATE, "seam_rank_of_target_prepared: workspace too small (%zu < %zu)", workspace_bytes, s.total);
-  uint8_t* ws = static_cast<uint8_t*>(workspace);
-  __half* a16 = reinterpret_cast<__half*>(ws + s.off_a16);
-  float* rq = reinterpret_cast<float*>(ws + s.off_rq);
-  float* anorm = reinterpret_cast<float*>(ws + s.off_anorm);
-  uint32_t* thr = reinterpret_cast<uint32_t*>(ws + s.off_thr);
-  uint32_t* rowcnt = reinterpret_cast<uint32_t*>(ws + s.off_rowcnt);
-  float* gmax = reinterpret_cast<float*>(ws + s.off_gmax);
-  uint32_t* rowflag = reinterpret_cast<uint32_t*>(ws + s.off_rowflag);
-  uint2* rowbuf = reinterpret_cast<uint2*>(align_up(reinterpret_cast<uintptr_t>(ws + s.off_rowbuf), (size_t)s.CAP * 8));
-  int32_t* counters = reinterpret_cast<int32_t*>(ws + s.off_cnt);
-  int32_t* frows = reinterpret_cast<int32_t*>(ws + s.off_rows);
-  const int nlists = s.P * score::NQ;
-  // the group-maxima region (Q x nlists x 16 words) is free in this variant
-  int32_t* above = reinterpret_cast<int32_t*>(gmax);
-  float* lo = gmax + (size_t)Q * nlists;
-  float* hi = lo + Q;
-  float* dtarget = hi + Q;
+  if (!target || !out_rank) return fail(h, SEAM_ERR_BAD_ARG, "seam_rank_of_target_prepared: null pointer");
+  ScoreWorkspace w;
+  int rc = carve_score_workspace(h, "seam_rank_of_target_prepared", true, q, Q, g, g16, cg, gstat, G, workspace,
+                                 workspace_bytes, &w);
+  if (rc != SEAM_OK) return rc;
+  const int nlists = w.plan.P * score::NQ;
 
   xchg::Exchange no_x;
   memset(&no_x, 0, sizeof(no_x));
-  exact::prep_queries_kernel<<<(Q + 7) / 8, 256, 0, stream>>>(q, Q, h->fold, a16, rq, anorm, thr, rowflag, counters, nullptr, 0, no_x);
+  exact::prep_queries_kernel<<<(Q + 7) / 8, 256, 0, stream>>>(q, Q, h->fold, w.a16, w.rq, w.anorm, w.thr, w.rowflag,
+                                                              w.counters, nullptr, 0, no_x);
   SEAM_LAUNCHED(h, "prep_queries_kernel");
-  exact::rank_prep_kernel<<<(Q + 7) / 8, 256, 0, stream>>>(q, Q, g, target, h->fold, rq, anorm, gstat, lo, hi, dtarget,
-                                                          above, nlists);
+  exact::rank_prep_kernel<<<(Q + 7) / 8, 256, 0, stream>>>(q, Q, g, target, h->fold, w.rq, w.anorm, gstat, w.lo, w.hi,
+                                                          w.dtarget, w.above, nlists);
   SEAM_LAUNCHED(h, "rank_prep_kernel");
 
   CUtensorMap tmA, tmB;
-  int rc;
-  if ((rc = encode_map_fp16_rows(h, &tmA, a16, Q, score::BM)) != SEAM_OK) return rc;
-  if ((rc = encode_map_fp16_rows(h, &tmB, g16, G, score::BN)) != SEAM_OK) return rc;
   score::Params sp;
-  sp.Q = Q;
-  sp.G = G;
-  sp.num_mtiles = s.num_mtiles;
-  sp.ntiles_n = s.ntiles_n;
-  sp.total_tiles = s.total_tiles;
-  sp.P = s.P;
-  sp.CAP = s.CAP;
-  sp.nseed = 0;
-  for (int b = 0; b <= s.grid; ++b) sp.tb[b] = s.tb[b];
-  sp.cg = cg;
-  sp.thr_global = thr;
-  sp.rowcnt = rowcnt;
-  sp.rowflag = rowflag;
-  sp.rowbuf = rowbuf;
-  sp.gmax = gmax;
-  sp.rank_lo = lo;
-  sp.rank_hi = hi;
-  sp.rank_above = above;
-  score::score_topk_kernel<score::VAR_RANK><<<s.grid, score::THREADS, score::SMEM_BYTES, stream>>>(tmA, tmB, sp);
+  if ((rc = score_kernel_args(h, w, Q, g16, cg, G, &tmA, &tmB, &sp)) != SEAM_OK) return rc;
+  score::score_topk_kernel<score::VAR_RANK><<<w.plan.tiles.nb, score::THREADS, score::SMEM_BYTES, stream>>>(tmA, tmB, sp);
   SEAM_LAUNCHED(h, "score_topk_kernel<rank>");
 
   exact::RankResolveParams rp;
   rp.q = q;
   rp.g = g;
   rp.fold = h->fold;
-  rp.rowbuf = rowbuf;
-  rp.rowcnt = rowcnt;
-  rp.rowflag = rowflag;
-  rp.above = above;
-  rp.lo = lo;
-  rp.hi = hi;
-  rp.dtarget = dtarget;
-  rp.rq = rq;
+  rp.rowbuf = w.rowbuf;
+  rp.rowcnt = w.rowcnt;
+  rp.rowflag = w.rowflag;
+  rp.above = w.above;
+  rp.lo = w.lo;
+  rp.hi = w.hi;
+  rp.dtarget = w.dtarget;
+  rp.rq = w.rq;
   rp.gstat = gstat;
   rp.target = target;
   rp.Q = Q;
   rp.G = G;
   rp.nlists = nlists;
-  rp.CAP = s.CAP;
+  rp.CAP = w.plan.CAP;
   rp.out_rank = out_rank;
   rp.out_margin = out_margin;
-  rp.counters = counters;
-  rp.fallback_rows = frows;
-  rp.plan.ntiles_n = s.ntiles_n;
-  rp.plan.nb = s.grid;
-  for (int b = 0; b <= s.grid; ++b) rp.plan.tb[b] = s.tb[b];
+  rp.counters = w.counters;
+  rp.fallback_rows = w.frows;
+  rp.plan = w.plan.tiles;
   exact::rank_resolve_kernel<<<(Q + 7) / 8, 256, 0, stream>>>(rp);
   SEAM_LAUNCHED(h, "rank_resolve_kernel");
-  exact::rank_of_target_kernel<<<2 * h->num_sms, 256, 0, stream>>>(q, Q, g, G, target, h->fold, counters, frows, out_rank,
-                                                                  out_margin);
+  exact::rank_of_target_kernel<<<2 * h->num_sms, 256, 0, stream>>>(q, Q, g, G, target, h->fold, w.counters, w.frows,
+                                                                  out_rank, out_margin);
   SEAM_LAUNCHED(h, "rank_of_target_kernel");
-  if (stats) SEAM_CUDA(h, cudaMemcpyAsync(stats, counters, 4, cudaMemcpyDeviceToDevice, stream));
+  if (stats) SEAM_CUDA(h, cudaMemcpyAsync(stats, w.counters, 4, cudaMemcpyDeviceToDevice, stream));
   return SEAM_OK;
 }
 
