@@ -38,7 +38,7 @@ enum seam_status {
 
 enum { SEAM_D = 256, SEAM_DI = 128, SEAM_MAX_T = 64, SEAM_MAX_K = 32, SEAM_MAX_WORLD = 8 };
 
-/* ABI version of this header (bumped on any signature change). */
+/* ABI version of this header: bumped when an existing signature changes, not when an entry point is added. */
 int seam_abi_version(void);
 
 /* One handle per device.  Not thread-safe; distinct handles are independent. */
@@ -121,6 +121,15 @@ size_t seam_aggregate_workspace_bytes(int Q);
 int seam_aggregate(seam_handle* h, const float* seq, const uint8_t* mask, const int32_t* lens, int Tmax, int Q,
                    int64_t frame_stride, int64_t track_stride, float* out, float* att, void* workspace,
                    size_t workspace_bytes, void* stream);
+/* seam_aggregate for fp16 tracks: seq (1+Tmax, Q, 256) holds IEEE fp16 bit patterns (the dtype torch.autocast
+ * and the reference's host-side feature store, evaluate_movingfashion.py:82-92, produce), strides in fp16
+ * elements and multiples of 8 (16 bytes), seq 16-byte aligned; otherwise SEAM_ERR_UNSUPPORTED.  The kernel
+ * widens each frame to fp32 as it leaves shared memory (exact) and runs the fp32 arithmetic from there on:
+ * out / att are bit-identical to seam_aggregate on the widened tracks, for half the bytes read.  Same outputs
+ * (fp32) and workspace as seam_aggregate. */
+int seam_aggregate_f16(seam_handle* h, const void* seq, const uint8_t* mask, const int32_t* lens, int Tmax, int Q,
+                       int64_t frame_stride, int64_t track_stride, float* out, float* att, void* workspace,
+                       size_t workspace_bytes, void* stream);
 
 /* Full non-local block output (not pooled): NONLocalBlock1D.forward, models/nlb.py:66-101.
  *   x, z  (B, 256, T) fp32 channel-major as in the reference; T <= 64.
@@ -176,6 +185,13 @@ int seam_search(seam_handle* h, const float* seq, const uint8_t* mask, const int
                 int64_t frame_stride, int64_t track_stride, float* q_out, const float* g, const void* g16, const float* cg,
                 const float* gstat, int G, int index_offset, int k, float* out_score, float* out_margin, int32_t* out_idx,
                 int32_t* stats, void* workspace, size_t workspace_bytes, void* stream);
+/* seam_search for fp16 tracks (seq, strides and alignment as seam_aggregate_f16); everything else, q_out
+ * included, as seam_search, and bit-identical to it on the widened tracks. */
+int seam_search_f16(seam_handle* h, const void* seq, const uint8_t* mask, const int32_t* lens, int Tmax, int Q,
+                    int64_t frame_stride, int64_t track_stride, float* q_out, const float* g, const void* g16,
+                    const float* cg, const float* gstat, int G, int index_offset, int k, float* out_score,
+                    float* out_margin, int32_t* out_idx, int32_t* stats, void* workspace, size_t workspace_bytes,
+                    void* stream);
 
 /* Dense logits (parity / small problems): x5 (Q,G,2) fp32 = last((q-g)^2).
  * models/match_head.py:160-162 and MatchPredictor.forward :70-74. */
@@ -268,6 +284,10 @@ size_t seam_exchange_sizeof(void);
 int seam_sharded_aggregate(seam_handle* h, const seam_exchange* x, const float* seq, const uint8_t* mask,
                            const int32_t* lens, int Tmax, int Qlocal, int64_t frame_stride, int64_t track_stride,
                            int row0, int last, float* att, void* stream);
+/* seam_sharded_aggregate for fp16 tracks (seq, strides and alignment as seam_aggregate_f16). */
+int seam_sharded_aggregate_f16(seam_handle* h, const seam_exchange* x, const void* seq, const uint8_t* mask,
+                               const int32_t* lens, int Tmax, int Qlocal, int64_t frame_stride, int64_t track_stride,
+                               int row0, int last, float* att, void* stream);
 /* seam_score_topk of all Q queries (this rank's q_all, once every rank's descriptors have landed) against the
  * rank's prepared gallery shard; the top-k rows go to the queries' owners.  Workspace as seam_score_topk. */
 int seam_sharded_score_topk(seam_handle* h, const seam_exchange* x, const float* g, const void* g16, const float* cg,
@@ -334,6 +354,10 @@ int seam_tower_forward(seam_handle* h, const float* x, int K, float* out, const 
  * models/match_head.py:101-111) is neither read nor written.  Pinned host memory makes it asynchronous. */
 int seam_upload_tracks(seam_handle* h, const float* seq_host, int Tmax, int Q, int lo, int hi, float* seq_dev,
                        void* stream);
+/* seam_upload_tracks for an fp16 host x3_1_seq: the same single pitched copy with 512-byte rows into an fp16
+ * device tensor (1+Tmax, hi-lo, 256) -- half the PCIe bytes; feed the result to the _f16 entry points. */
+int seam_upload_tracks_f16(seam_handle* h, const void* seq_host, int Tmax, int Q, int lo, int hi, void* seq_dev,
+                           void* stream);
 
 #ifdef __cplusplus
 }

@@ -109,6 +109,8 @@ def _declare(lib: C.CDLL) -> None:
     lib.seam_aggregate_workspace_bytes.argtypes = [i32]
     lib.seam_aggregate.restype = i32
     lib.seam_aggregate.argtypes = [vp, vp, vp, vp, i32, i32, i64, i64, vp, vp, vp, sz, vp]
+    lib.seam_aggregate_f16.restype = i32
+    lib.seam_aggregate_f16.argtypes = lib.seam_aggregate.argtypes
     lib.seam_nlb_workspace_bytes.restype = sz
     lib.seam_nlb_workspace_bytes.argtypes = [i32, i32]
     lib.seam_nlb_forward.restype = i32
@@ -125,6 +127,8 @@ def _declare(lib: C.CDLL) -> None:
     lib.seam_score_topk.argtypes = [vp, vp, i32, vp, vp, vp, vp, i32, i32, i32, vp, vp, vp, vp, vp, sz, vp]
     lib.seam_search.restype = i32
     lib.seam_search.argtypes = [vp, vp, vp, vp, i32, i32, i64, i64, vp, vp, vp, vp, vp, i32, i32, i32, vp, vp, vp, vp, vp, sz, vp]
+    lib.seam_search_f16.restype = i32
+    lib.seam_search_f16.argtypes = lib.seam_search.argtypes
     lib.seam_score_dense.restype = i32
     lib.seam_score_dense.argtypes = [vp, vp, i32, vp, i32, vp, vp]
     lib.seam_score_prob.restype = i32
@@ -140,6 +144,8 @@ def _declare(lib: C.CDLL) -> None:
     xp = C.POINTER(SeamExchange)
     lib.seam_sharded_aggregate.restype = i32
     lib.seam_sharded_aggregate.argtypes = [vp, xp, vp, vp, vp, i32, i32, i64, i64, i32, i32, vp, vp]
+    lib.seam_sharded_aggregate_f16.restype = i32
+    lib.seam_sharded_aggregate_f16.argtypes = lib.seam_sharded_aggregate.argtypes
     lib.seam_sharded_score_topk.restype = i32
     lib.seam_sharded_score_topk.argtypes = [vp, xp, vp, vp, vp, vp, i32, i32, vp, vp, sz, vp]
     lib.seam_sharded_merge.restype = i32
@@ -157,6 +163,8 @@ def _declare(lib: C.CDLL) -> None:
     lib.seam_tower_forward.argtypes = [vp, vp, i32, vp, vp, vp, sz, vp]
     lib.seam_upload_tracks.restype = i32
     lib.seam_upload_tracks.argtypes = [vp, vp, i32, i32, i32, i32, vp, vp]
+    lib.seam_upload_tracks_f16.restype = i32
+    lib.seam_upload_tracks_f16.argtypes = lib.seam_upload_tracks.argtypes
     lib.seam_merge_topk.restype = i32
     lib.seam_merge_topk.argtypes = [vp, vp, vp, vp, i32, i32, i32, vp, vp, vp, vp]
 

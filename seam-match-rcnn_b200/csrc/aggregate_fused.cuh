@@ -23,6 +23,10 @@
 // Results do not depend on how tracks are grouped into batches (a column of D depends on its own track
 // only; the accumulation order over k is fixed), nor on which slot a track lands in.
 //
+// Tracks are fp32 or fp16 (template parameter In): only the track buffers and the copies into them follow the element
+// size; load_frame widens an fp16 frame to fp32 as it leaves shared memory (exact), so the fp16 instantiations give
+// bit for bit what the fp32 ones give on the widened tracks.
+//
 // A producer's iteration is a LATENCY CHAIN (2-3 producer warps per scheduler: shuffle rounds, named barriers,
 // shared-memory atomics, mbarrier polls and the hand-over of a copy to the copy engine all sit on one warp's
 // critical path), so the code below trades instructions for fewer dependent steps: reductions are folded into
@@ -76,11 +80,11 @@ __host__ __device__ constexpr uint32_t fused_bytes() {
 }
 
 struct Params {
-  const float* seq;
+  const void* seq;         // float or __half: the kernels' In
   const uint8_t* mask;     // (Q, 1+Tmax) or null
   const int32_t* lens;     // (Q) or null
   int Tmax, Q;
-  long long frame_stride, track_stride;   // floats
+  long long frame_stride, track_stride;   // elements of seq
   const float* fold;
   float* out;      // (Q,256)
   float* att;      // (Q,Tmax) or null
@@ -129,6 +133,23 @@ __device__ __forceinline__ Vec8 load_vec8(const float* row, int lane) {
   const ulonglong2 lo = *reinterpret_cast<const ulonglong2*>(row + 4 * lane);
   const ulonglong2 hi = *reinterpret_cast<const ulonglong2*>(row + 128 + 4 * lane);
   return Vec8{lo.x, lo.y, hi.x, hi.y};
+}
+// a frame of the track buffer (In = float or __half) -> registers, with the lane -> channel mapping of load_vec8.
+// fp16 frames are widened here (exact), so every instruction after this load is the fp32 path's.
+__device__ __forceinline__ u64 widen2(uint32_t h2) {
+  const float2 f = __half22float2(*reinterpret_cast<const __half2*>(&h2));
+  return pk(f.x, f.y);
+}
+template <typename In>
+__device__ __forceinline__ Vec8 load_frame(const In* row, int lane) {
+  if constexpr (std::is_same<In, float>::value) {
+    return load_vec8(row, lane);
+  } else {
+    static_assert(std::is_same<In, __half>::value, "frames are float or __half");
+    const uint2 lo = *reinterpret_cast<const uint2*>(row + 4 * lane);
+    const uint2 hi = *reinterpret_cast<const uint2*>(row + 128 + 4 * lane);
+    return Vec8{widen2(lo.x), widen2(lo.y), widen2(hi.x), widen2(hi.y)};
+  }
 }
 __device__ __forceinline__ Vec8 zero_vec8() { return Vec8{0ull, 0ull, 0ull, 0ull}; }
 __device__ __forceinline__ float dot8(const Vec8& x, const Vec8& u) {
@@ -463,9 +484,10 @@ struct Cfg<10> { static constexpr int NW = 11, SLOTS = 1, LOADER = 1, REGS_P = 1
 template <>
 struct Cfg<16> { static constexpr int NW = 8, SLOTS = 1, LOADER = 0, REGS_P = 224, REGS_H = 56; };
 
-template <int TR>
+// In: the element type of the tracks (float or __half); only the track buffers and the copies into them depend on it
+template <int TR, typename In>
 constexpr size_t warp_smem_bytes() {
-  return 1024 + fused_bytes<true>() + (size_t)Cfg<TR>::NW * Cfg<TR>::SLOTS * TR * D * 4   // track buffers
+  return 1024 + fused_bytes<true>() + (size_t)Cfg<TR>::NW * Cfg<TR>::SLOTS * TR * D * sizeof(In)   // track buffers
          + (size_t)Cfg<TR>::NW * 64 * 4                                                   // per-warp scalars
          + (size_t)Cfg<TR>::NW * Cfg<TR>::SLOTS * 8                                       // mbarriers
          + (size_t)Cfg<TR>::NW * 8                                                        // "buffer is free" mbarriers
@@ -474,13 +496,16 @@ constexpr size_t warp_smem_bytes() {
 template <int TR>
 constexpr int warp_threads() { return (Cfg<TR>::NW + HELPER_WARPS + Cfg<TR>::LOADER) * 32; }
 
-template <int TR>
+template <int TR, typename In>
 __global__ void __launch_bounds__((Cfg<TR>::NW + HELPER_WARPS + Cfg<TR>::LOADER) * 32, 1)
 aggregate_fused_warp_kernel(const __grid_constant__ CUtensorMap tmSeq, const Params p) {
   constexpr int NW = Cfg<TR>::NW, SLOTS = Cfg<TR>::SLOTS;
   constexpr bool LOADER = Cfg<TR>::LOADER != 0;
   static_assert(!LOADER || SLOTS == 1, "the loader warp serves single-buffer producers");
   constexpr int M_INFLIGHT = TR >= 10 ? 4 : 2;     // chunks of M a producer warp has in flight at start
+  constexpr uint32_t FRAME_BYTES = D * sizeof(In);
+  constexpr size_t XBUF_BYTES = (size_t)NW * SLOTS * TR * FRAME_BYTES;   // every producer's track buffers
+  const In* const seq = static_cast<const In*>(p.seq);
   extern __shared__ uint8_t smem_raw[];
   const uint32_t raw_addr = ptx::smem_u32(smem_raw);
   uint8_t* fz = smem_raw + (((raw_addr + 1023u) & ~1023u) - raw_addr);        // fused area (1 KB aligned), then producers
@@ -494,15 +519,15 @@ aggregate_fused_warp_kernel(const __grid_constant__ CUtensorMap tmSeq, const Par
   const long long stride = (long long)gridDim.x * NW;
   const long long first0 = (long long)blockIdx.x * NW;
 
-  float* xbuf = reinterpret_cast<float*>(pz) + (size_t)(warp < NW ? warp : 0) * SLOTS * TR * D;
-  float* scal = reinterpret_cast<float*>(pz) + (size_t)NW * SLOTS * TR * D + (warp < NW ? warp : 0) * 64;
-  uint64_t* bars = reinterpret_cast<uint64_t*>(pz + (size_t)NW * SLOTS * TR * D * 4 + (size_t)NW * 64 * 4) +
+  In* xbuf = reinterpret_cast<In*>(pz) + (size_t)(warp < NW ? warp : 0) * SLOTS * TR * D;
+  float* scal = reinterpret_cast<float*>(pz + XBUF_BYTES) + (warp < NW ? warp : 0) * 64;
+  uint64_t* bars = reinterpret_cast<uint64_t*>(pz + XBUF_BYTES + (size_t)NW * 64 * 4) +
                    (warp < NW ? warp : 0) * SLOTS;
-  int* slot_len = reinterpret_cast<int*>(pz + (size_t)NW * SLOTS * TR * D * 4 + (size_t)NW * 64 * 4 +
+  int* slot_len = reinterpret_cast<int*>(pz + XBUF_BYTES + (size_t)NW * 64 * 4 +
                                          (size_t)NW * SLOTS * 8 + (size_t)NW * 8) + (warp < NW ? warp : 0) * SLOTS;
   // loader's view: every producer's buffer, barriers and track length
-  float* const xbuf_all = reinterpret_cast<float*>(pz);
-  uint64_t* const bars_all = reinterpret_cast<uint64_t*>(pz + (size_t)NW * SLOTS * TR * D * 4 + (size_t)NW * 64 * 4);
+  In* const xbuf_all = reinterpret_cast<In*>(pz);
+  uint64_t* const bars_all = reinterpret_cast<uint64_t*>(pz + XBUF_BYTES + (size_t)NW * 64 * 4);
   uint64_t* const empty_all = bars_all + NW * SLOTS;                                    // producer -> loader: frames are in registers
   int* const slot_len_all = reinterpret_cast<int*>(empty_all + NW);
   if (warp < NW && lane == 0) {
@@ -540,7 +565,7 @@ aggregate_fused_warp_kernel(const __grid_constant__ CUtensorMap tmSeq, const Par
     }
     if (lane == 0) {
       slot_len[slot] = len;
-      if (len > 0) ptx::mbar_arrive_expect_tx(&bars[slot], (uint32_t)len * (D * 4));
+      if (len > 0) ptx::mbar_arrive_expect_tx(&bars[slot], (uint32_t)len * FRAME_BYTES);
       else ptx::mbar_arrive(&bars[slot]);
     }
     __syncwarp();
@@ -550,8 +575,8 @@ aggregate_fused_warp_kernel(const __grid_constant__ CUtensorMap tmSeq, const Par
       if (ptx::elect_one()) ptx::tma_load_3d_hint(xbuf + (size_t)slot * TR * D, &tmSeq, &bars[slot], 0, (int)track, 1, pol);
       __syncwarp();
     } else if (lane < len) {
-      const float* src = p.seq + (long long)(lane + 1) * p.frame_stride + track * p.track_stride;
-      ptx::bulk_load_1d_hint(xbuf + ((size_t)slot * TR + lane) * D, src, D * 4, &bars[slot], pol);
+      const In* src = seq + (long long)(lane + 1) * p.frame_stride + track * p.track_stride;
+      ptx::bulk_load_1d_hint(xbuf + ((size_t)slot * TR + lane) * D, src, FRAME_BYTES, &bars[slot], pol);
     }
   };
 
@@ -593,16 +618,16 @@ aggregate_fused_warp_kernel(const __grid_constant__ CUtensorMap tmSeq, const Par
       const bool ready = active && ptx::mbar_test_wait(&empty_all[lane < NW ? lane : 0], ph);
       if (ready) {
         uint64_t* bar = &bars_all[lane];
-        float* dst = xbuf_all + (size_t)lane * TR * D;
+        In* dst = xbuf_all + (size_t)lane * TR * D;
         slot_len_all[lane] = len_next;
-        if (len_next > 0) ptx::mbar_arrive_expect_tx(bar, (uint32_t)len_next * (D * 4));
+        if (len_next > 0) ptx::mbar_arrive_expect_tx(bar, (uint32_t)len_next * FRAME_BYTES);
         else ptx::mbar_arrive(bar);
         if (TR >= 10 && p.use_tm && len_next == TR) {
           ptx::tma_load_3d_hint(dst, &tmSeq, bar, 0, (int)next, 1, pol);
         } else {
           for (int t = 0; t < len_next; ++t)
-            ptx::bulk_load_1d_hint(dst + (size_t)t * D, p.seq + (long long)(t + 1) * p.frame_stride + next * p.track_stride,
-                                   D * 4, bar, pol);
+            ptx::bulk_load_1d_hint(dst + (size_t)t * D, seq + (long long)(t + 1) * p.frame_stride + next * p.track_stride,
+                                   FRAME_BYTES, bar, pol);
         }
         next += stride;
         ph ^= 1u;
@@ -650,7 +675,7 @@ aggregate_fused_warp_kernel(const __grid_constant__ CUtensorMap tmSeq, const Par
       }
       ptx::mbar_wait(&bars[slot], phase, 105);
       const int len = slot_len[slot];
-      const float* xs = xbuf + (size_t)slot * TR * D;
+      const In* xs = xbuf + (size_t)slot * TR * D;
 
       // One body, two instantiations: tracks with all TR frames (the common case) run without
       // per-frame guards and with unrolled T x T loops.
@@ -673,7 +698,7 @@ aggregate_fused_warp_kernel(const __grid_constant__ CUtensorMap tmSeq, const Par
           for (int u = 0; u < 8; ++u) {
             const int t = t0 + u;
             if (u < nf) {
-              if (FULL || t < len) x[t] = load_vec8(xs + t * D, lane);
+              if (FULL || t < len) x[t] = load_frame(xs + t * D, lane);
               else x[t] = zero_vec8();
               acc[4 * u + 0] = dot8(x[t], ut);
               acc[4 * u + 1] = dot8(x[t], wa);
@@ -830,23 +855,25 @@ struct alignas(16) GroupSmem {
   unsigned int slot;
   float pad[3];
 };
-template <int GW>
+template <int GW, typename In>
 struct GSmem {
-  float x[GWARPS][FB][D];              // 8 x 16 KB
+  In x[GWARPS][FB][D];                 // 8 x 16 KB (fp32) / 8 x 8 KB (fp16)
   GroupSmem<GW> g[GWARPS / GW];
   uint64_t bar[GWARPS];
 };
-template <int GW>
-constexpr size_t group_smem_bytes() { return 1024 + fused_bytes<false>() + sizeof(GSmem<GW>); }
+template <int GW, typename In>
+constexpr size_t group_smem_bytes() { return 1024 + fused_bytes<false>() + sizeof(GSmem<GW, In>); }
 
-template <int GW>
+template <int GW, typename In>
 __global__ void __launch_bounds__(GTHREADS, 1)
 aggregate_fused_group_kernel(const __grid_constant__ CUtensorMap tmSeq, const Params p) {
   constexpr int GROUPS_PER_CTA = GWARPS / GW;
+  constexpr uint32_t FRAME_BYTES = D * sizeof(In);
+  const In* const seq = static_cast<const In*>(p.seq);
   extern __shared__ uint8_t smem_raw[];
   const uint32_t raw_addr = ptx::smem_u32(smem_raw);
   uint8_t* fz = smem_raw + (((raw_addr + 1023u) & ~1023u) - raw_addr);
-  GSmem<GW>& s = *reinterpret_cast<GSmem<GW>*>(fz + fused_bytes<false>());
+  GSmem<GW, In>& s = *reinterpret_cast<GSmem<GW, In>*>(fz + fused_bytes<false>());
   const int lane = threadIdx.x & 31;
   const int warp = __shfl_sync(ptx::FULL_MASK, threadIdx.x >> 5, 0);
   Meta* meta = reinterpret_cast<Meta*>(fz + OFF_META);
@@ -863,7 +890,7 @@ aggregate_fused_group_kernel(const __grid_constant__ CUtensorMap tmSeq, const Pa
   const int pw = warp < GWARPS ? warp : 0;            // helper warps never use what follows
   const int grp = pw / GW, wg = pw % GW;
   GroupSmem<GW>& gs = s.g[grp];
-  float* xs = &s.x[pw][0][0];
+  In* xs = &s.x[pw][0][0];
   uint64_t* bar = &s.bar[pw];
   const int Tmax = p.Tmax;
   const uint32_t bar_id = 2 + grp;                     // named barrier 1 belongs to the helpers
@@ -909,13 +936,13 @@ aggregate_fused_group_kernel(const __grid_constant__ CUtensorMap tmSeq, const Pa
   auto issue = [&](long long track, int len) {
     const int nw = max(0, min(len - FB * wg, FB));
     if (nw < nw_buf) {                 // warp-uniform
-      float4* z = reinterpret_cast<float4*>(xs + (size_t)nw * D);
-      for (int i = lane; i < (nw_buf - nw) * (D / 4); i += 32) z[i] = make_float4(0.f, 0.f, 0.f, 0.f);
+      float4* z = reinterpret_cast<float4*>(xs + (size_t)nw * D);   // 16-byte chunks of zeros
+      for (int i = lane; i < (nw_buf - nw) * (int)(FRAME_BYTES / 16); i += 32) z[i] = make_float4(0.f, 0.f, 0.f, 0.f);
       ptx::fence_proxy_async_smem();   // these generic-proxy writes come before any later copy into the same bytes
     }
     nw_buf = nw;
     if (lane == 0) {
-      if (nw > 0) ptx::mbar_arrive_expect_tx(bar, (uint32_t)nw * (D * 4));
+      if (nw > 0) ptx::mbar_arrive_expect_tx(bar, (uint32_t)nw * FRAME_BYTES);
       else ptx::mbar_arrive(bar);
     }
     __syncwarp();
@@ -925,8 +952,8 @@ aggregate_fused_group_kernel(const __grid_constant__ CUtensorMap tmSeq, const Pa
       if (ptx::elect_one()) ptx::tma_load_3d_hint(xs, &tmSeq, bar, 0, (int)track, FB * wg + 1, pol);
       __syncwarp();
     } else if (lane < nw) {
-      const float* src = p.seq + (long long)(FB * wg + lane + 1) * p.frame_stride + track * p.track_stride;
-      ptx::bulk_load_1d_hint(xs + (size_t)lane * D, src, D * 4, bar, pol);
+      const In* src = seq + (long long)(FB * wg + lane + 1) * p.frame_stride + track * p.track_stride;
+      ptx::bulk_load_1d_hint(xs + (size_t)lane * D, src, FRAME_BYTES, bar, pol);
     }
   };
   // the first track is requested before the CTA-wide set-up
@@ -973,7 +1000,7 @@ aggregate_fused_group_kernel(const __grid_constant__ CUtensorMap tmSeq, const Pa
 #pragma unroll
         for (int u = 0; u < 8; ++u) {
           const int t = t0 + u;
-          x[t] = load_vec8(xs + t * D, lane);
+          x[t] = load_frame(xs + t * D, lane);
           acc[4 * u + 0] = dot8(x[t], ut);
           acc[4 * u + 1] = dot8(x[t], wa);
           acc[4 * u + 2] = dot8(x[t], up);

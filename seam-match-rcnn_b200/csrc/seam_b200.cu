@@ -119,38 +119,65 @@ static inline size_t align_up(size_t x, size_t a) { return (x + a - 1) / a * a; 
 static inline bool aligned16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15u) == 0; }
 
 // Full tracks / full frame blocks are fetched with one 3-D tensor-map copy: box {256, 1 track, frames} over seq viewed as
-// (1+Tmax, Q, 256) with the caller's strides.  Returns whether the map is usable.
+// (1+Tmax, Q, 256) with the caller's strides (elements of In: float or __half).  Returns whether the map is usable.
+template <typename In>
 static int encode_seq_map(seam_handle* h, const aggf::Params& p, int box_frames, CUtensorMap* tm) {
+  constexpr long long ES = sizeof(In);
   memset(tm, 0, sizeof(*tm));
-  if (!p.seq || p.Q <= 0 || (p.track_stride * 4) % 16 != 0 || (p.frame_stride * 4) % 16 != 0 || p.track_stride < 256 ||
+  if (!p.seq || p.Q <= 0 || (p.track_stride * ES) % 16 != 0 || (p.frame_stride * ES) % 16 != 0 || p.track_stride < 256 ||
       p.frame_stride < 256 || box_frames > p.Tmax)
     return 0;
   const cuuint64_t dims[3] = {256, (cuuint64_t)p.Q, (cuuint64_t)(1 + p.Tmax)};
-  const cuuint64_t strides[2] = {(cuuint64_t)p.track_stride * 4, (cuuint64_t)p.frame_stride * 4};
+  const cuuint64_t strides[2] = {(cuuint64_t)(p.track_stride * ES), (cuuint64_t)(p.frame_stride * ES)};
   const cuuint32_t box[3] = {256, 1, (cuuint32_t)box_frames};
   const cuuint32_t estr[3] = {1, 1, 1};
-  return h->encode(tm, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 3, const_cast<float*>(p.seq), dims, strides, box, estr,
-                   CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
+  const CUtensorMapDataType dt = ES == 2 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT16 : CU_TENSOR_MAP_DATA_TYPE_FLOAT32;
+  return h->encode(tm, dt, 3, const_cast<void*>(p.seq), dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
+                   CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
                    CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
 }
 
-template <int TR>
+template <int TR, typename In>
 static void launch_aggregate_warp(seam_handle* h, aggf::Params& p, cudaStream_t stream) {
   constexpr int NW = aggf::Cfg<TR>::NW;
   const int want = (p.Q + NW - 1) / NW;
   const int grid = want < h->num_sms ? want : h->num_sms;
   CUtensorMap tm;
-  p.use_tm = p.Tmax == TR ? encode_seq_map(h, p, TR, &tm) : (memset(&tm, 0, sizeof(tm)), 0);
-  aggf::aggregate_fused_warp_kernel<TR><<<grid, aggf::warp_threads<TR>(), aggf::warp_smem_bytes<TR>(), stream>>>(tm, p);
+  p.use_tm = p.Tmax == TR ? encode_seq_map<In>(h, p, TR, &tm) : (memset(&tm, 0, sizeof(tm)), 0);
+  aggf::aggregate_fused_warp_kernel<TR, In>
+      <<<grid, aggf::warp_threads<TR>(), aggf::warp_smem_bytes<TR, In>(), stream>>>(tm, p);
 }
-template <int GW>
+template <int GW, typename In>
 static void launch_aggregate_group(seam_handle* h, aggf::Params& p, cudaStream_t stream) {
   constexpr int GPC = aggf::GWARPS / GW;
   const int want = (p.Q + GPC - 1) / GPC;
   const int grid = want < h->num_sms ? want : h->num_sms;
   CUtensorMap tm;
-  p.use_tm = encode_seq_map(h, p, aggf::FB, &tm);
-  aggf::aggregate_fused_group_kernel<GW><<<grid, aggf::GTHREADS, aggf::group_smem_bytes<GW>(), stream>>>(tm, p);
+  p.use_tm = encode_seq_map<In>(h, p, aggf::FB, &tm);
+  aggf::aggregate_fused_group_kernel<GW, In><<<grid, aggf::GTHREADS, aggf::group_smem_bytes<GW, In>(), stream>>>(tm, p);
+}
+template <typename In>
+static void launch_aggregate(seam_handle* h, aggf::Params& p, cudaStream_t stream) {
+  const int Tmax = p.Tmax;
+  if (Tmax <= 4) launch_aggregate_warp<4, In>(h, p, stream);
+  else if (Tmax <= 10) launch_aggregate_warp<10, In>(h, p, stream);
+  else if (Tmax <= 16) launch_aggregate_warp<16, In>(h, p, stream);
+  else if (Tmax <= 32) launch_aggregate_group<2, In>(h, p, stream);   // two warps per track
+  else launch_aggregate_group<4, In>(h, p, stream);                   // 33..64 frames: four warps per track
+}
+// large dynamic shared memory for the aggregation kernels of one element type
+template <typename In>
+static void opt_in_aggregate_smem() {
+  cudaFuncSetAttribute(aggf::aggregate_fused_warp_kernel<4, In>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                       (int)aggf::warp_smem_bytes<4, In>());
+  cudaFuncSetAttribute(aggf::aggregate_fused_warp_kernel<10, In>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                       (int)aggf::warp_smem_bytes<10, In>());
+  cudaFuncSetAttribute(aggf::aggregate_fused_warp_kernel<16, In>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                       (int)aggf::warp_smem_bytes<16, In>());
+  cudaFuncSetAttribute(aggf::aggregate_fused_group_kernel<2, In>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                       (int)aggf::group_smem_bytes<2, In>());
+  cudaFuncSetAttribute(aggf::aggregate_fused_group_kernel<4, In>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                       (int)aggf::group_smem_bytes<4, In>());
 }
 
 static int import_exchange(seam_handle* h, const seam_exchange* x, xchg::Exchange* e, const char* who) {
@@ -257,16 +284,8 @@ int seam_create(seam_handle** out, int device) {
                        (int)score::SMEM_BYTES);
   cudaFuncSetAttribute(score::score_topk_kernel<score::VAR_RANK>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                        (int)score::SMEM_BYTES);
-  cudaFuncSetAttribute(aggf::aggregate_fused_warp_kernel<4>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                       (int)aggf::warp_smem_bytes<4>());
-  cudaFuncSetAttribute(aggf::aggregate_fused_warp_kernel<10>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                       (int)aggf::warp_smem_bytes<10>());
-  cudaFuncSetAttribute(aggf::aggregate_fused_warp_kernel<16>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                       (int)aggf::warp_smem_bytes<16>());
-  cudaFuncSetAttribute(aggf::aggregate_fused_group_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                       (int)aggf::group_smem_bytes<2>());
-  cudaFuncSetAttribute(aggf::aggregate_fused_group_kernel<4>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                       (int)aggf::group_smem_bytes<4>());
+  opt_in_aggregate_smem<float>();
+  opt_in_aggregate_smem<__half>();
   cudaFuncSetAttribute(bwd::agg_backward_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
                        (int)bwd::agg_bwd_smem_bytes(bwd::BWD_MAX_T));
   cudaFuncSetAttribute(tower::conv3x3_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tower::SMEM_BYTES);
@@ -379,7 +398,8 @@ size_t seam_aggregate_workspace_bytes(int Q) {
   return 256;   // the fused kernel keeps every intermediate on the SM
 }
 
-static int aggregate_impl(seam_handle* h, const xchg::Exchange* x, int row0, int last, const float* seq,
+// seq holds fp32 values, or fp16 bit patterns when f16 is set (strides in elements either way)
+static int aggregate_impl(seam_handle* h, const xchg::Exchange* x, int row0, int last, const void* seq, bool f16,
                           const uint8_t* mask, const int32_t* lens, int Tmax, int Q, int64_t frame_stride,
                           int64_t track_stride, float* out, float* att, cudaStream_t stream, const char* who) {
   if (!h->have_aggregator) return fail(h, SEAM_ERR_STATE, "%s: weights not loaded", who);
@@ -393,8 +413,11 @@ static int aggregate_impl(seam_handle* h, const xchg::Exchange* x, int row0, int
     return SEAM_OK;
   }
   if (Q > 0 && Tmax > 0 && !seq) return fail(h, SEAM_ERR_BAD_ARG, "%s: null pointer", who);
-  if (!aligned16(seq) || (out && !aligned16(out)) || (frame_stride & 3) || (track_stride & 3))
-    return fail(h, SEAM_ERR_UNSUPPORTED, "%s: seq/out must be 16-byte aligned, strides multiples of 4", who);
+  // the bulk copies and the tensor map move whole frames: 16-byte aligned rows
+  const int64_t stride_mask = f16 ? 7 : 3;
+  if (!aligned16(seq) || (out && !aligned16(out)) || (frame_stride & stride_mask) || (track_stride & stride_mask))
+    return fail(h, SEAM_ERR_UNSUPPORTED, "%s: seq/out must be 16-byte aligned, strides multiples of %s", who,
+                f16 ? "8 fp16 elements" : "4");
   ProfileScope prof(h, SEAM_KERNEL_AGGREGATE, stream);
   aggf::Params p;
   memset(&p, 0, sizeof(p));
@@ -426,11 +449,8 @@ static int aggregate_impl(seam_handle* h, const xchg::Exchange* x, int row0, int
     }
     return SEAM_OK;
   }
-  if (Tmax <= 4) launch_aggregate_warp<4>(h, p, stream);
-  else if (Tmax <= 10) launch_aggregate_warp<10>(h, p, stream);
-  else if (Tmax <= 16) launch_aggregate_warp<16>(h, p, stream);
-  else if (Tmax <= 32) launch_aggregate_group<2>(h, p, stream);   // two warps per track
-  else launch_aggregate_group<4>(h, p, stream);                   // 33..64 frames: four warps per track
+  if (f16) launch_aggregate<__half>(h, p, stream);
+  else launch_aggregate<float>(h, p, stream);
   SEAM_LAUNCHED(h, "aggregate kernel");
   return SEAM_OK;
 }
@@ -441,21 +461,45 @@ int seam_aggregate(seam_handle* h, const float* seq, const uint8_t* mask, const 
   (void)workspace;
   (void)workspace_bytes;
   if (!h) return SEAM_ERR_BAD_ARG;
-  return aggregate_impl(h, nullptr, 0, 0, seq, mask, lens, Tmax, Q, frame_stride, track_stride, out, att,
+  return aggregate_impl(h, nullptr, 0, 0, seq, false, mask, lens, Tmax, Q, frame_stride, track_stride, out, att,
                         static_cast<cudaStream_t>(stream_), "seam_aggregate");
+}
+
+int seam_aggregate_f16(seam_handle* h, const void* seq, const uint8_t* mask, const int32_t* lens, int Tmax, int Q,
+                       int64_t frame_stride, int64_t track_stride, float* out, float* att, void* workspace,
+                       size_t workspace_bytes, void* stream_) {
+  (void)workspace;
+  (void)workspace_bytes;
+  if (!h) return SEAM_ERR_BAD_ARG;
+  return aggregate_impl(h, nullptr, 0, 0, seq, true, mask, lens, Tmax, Q, frame_stride, track_stride, out, att,
+                        static_cast<cudaStream_t>(stream_), "seam_aggregate_f16");
+}
+
+static int sharded_aggregate_impl(seam_handle* h, const seam_exchange* x, const void* seq, bool f16, const uint8_t* mask,
+                                  const int32_t* lens, int Tmax, int Qlocal, int64_t frame_stride, int64_t track_stride,
+                                  int row0, int last, float* att, void* stream_, const char* who) {
+  if (!h) return SEAM_ERR_BAD_ARG;
+  xchg::Exchange e;
+  int rc = import_exchange(h, x, &e, who);
+  if (rc != SEAM_OK) return rc;
+  if (row0 < 0 || Qlocal < 0 || row0 + Qlocal > x->Q)
+    return fail(h, SEAM_ERR_BAD_ARG, "%s: rows [%d,%d) outside the %d queries", who, row0, row0 + Qlocal, x->Q);
+  return aggregate_impl(h, &e, row0, last ? 1 : 0, seq, f16, mask, lens, Tmax, Qlocal, frame_stride, track_stride, nullptr,
+                        att, static_cast<cudaStream_t>(stream_), who);
 }
 
 int seam_sharded_aggregate(seam_handle* h, const seam_exchange* x, const float* seq, const uint8_t* mask,
                            const int32_t* lens, int Tmax, int Qlocal, int64_t frame_stride, int64_t track_stride,
                            int row0, int last, float* att, void* stream_) {
-  if (!h) return SEAM_ERR_BAD_ARG;
-  xchg::Exchange e;
-  int rc = import_exchange(h, x, &e, "seam_sharded_aggregate");
-  if (rc != SEAM_OK) return rc;
-  if (row0 < 0 || Qlocal < 0 || row0 + Qlocal > x->Q)
-    return fail(h, SEAM_ERR_BAD_ARG, "seam_sharded_aggregate: rows [%d,%d) outside the %d queries", row0, row0 + Qlocal, x->Q);
-  return aggregate_impl(h, &e, row0, last ? 1 : 0, seq, mask, lens, Tmax, Qlocal, frame_stride, track_stride, nullptr, att,
-                        static_cast<cudaStream_t>(stream_), "seam_sharded_aggregate");
+  return sharded_aggregate_impl(h, x, seq, false, mask, lens, Tmax, Qlocal, frame_stride, track_stride, row0, last, att,
+                                stream_, "seam_sharded_aggregate");
+}
+
+int seam_sharded_aggregate_f16(seam_handle* h, const seam_exchange* x, const void* seq, const uint8_t* mask,
+                               const int32_t* lens, int Tmax, int Qlocal, int64_t frame_stride, int64_t track_stride,
+                               int row0, int last, float* att, void* stream_) {
+  return sharded_aggregate_impl(h, x, seq, true, mask, lens, Tmax, Qlocal, frame_stride, track_stride, row0, last, att,
+                                stream_, "seam_sharded_aggregate_f16");
 }
 
 size_t seam_nlb_workspace_bytes(int B, int T) {
@@ -900,17 +944,37 @@ int seam_score_topk(seam_handle* h, const float* q, int Q, const float* g, const
                          workspace, workspace_bytes, stream_);
 }
 
+static int search_impl(seam_handle* h, const void* seq, bool f16, const uint8_t* mask, const int32_t* lens, int Tmax,
+                       int Q, int64_t frame_stride, int64_t track_stride, float* q_out, const float* g, const void* g16,
+                       const float* cg, const float* gstat, int G, int index_offset, int k, float* out_score,
+                       float* out_margin, int32_t* out_idx, int32_t* stats, void* workspace, size_t workspace_bytes,
+                       void* stream_, const char* who) {
+  if (!h) return SEAM_ERR_BAD_ARG;
+  if (!q_out && Q > 0) return fail(h, SEAM_ERR_BAD_ARG, "%s: q_out is null", who);
+  int rc = aggregate_impl(h, nullptr, 0, 0, seq, f16, mask, lens, Tmax, Q, frame_stride, track_stride, q_out, nullptr,
+                          static_cast<cudaStream_t>(stream_), who);
+  if (rc != SEAM_OK) return rc;
+  return score_topk_impl(h, nullptr, q_out, Q, g, g16, cg, gstat, G, index_offset, k, out_score, out_margin, out_idx, stats,
+                         workspace, workspace_bytes, stream_);
+}
+
 int seam_search(seam_handle* h, const float* seq, const uint8_t* mask, const int32_t* lens, int Tmax, int Q,
                 int64_t frame_stride, int64_t track_stride, float* q_out, const float* g, const void* g16, const float* cg,
                 const float* gstat, int G, int index_offset, int k, float* out_score, float* out_margin, int32_t* out_idx,
                 int32_t* stats, void* workspace, size_t workspace_bytes, void* stream_) {
-  if (!h) return SEAM_ERR_BAD_ARG;
-  if (!q_out && Q > 0) return fail(h, SEAM_ERR_BAD_ARG, "seam_search: q_out is null");
-  int rc = aggregate_impl(h, nullptr, 0, 0, seq, mask, lens, Tmax, Q, frame_stride, track_stride, q_out, nullptr,
-                          static_cast<cudaStream_t>(stream_), "seam_search");
-  if (rc != SEAM_OK) return rc;
-  return score_topk_impl(h, nullptr, q_out, Q, g, g16, cg, gstat, G, index_offset, k, out_score, out_margin, out_idx, stats,
-                         workspace, workspace_bytes, stream_);
+  return search_impl(h, seq, false, mask, lens, Tmax, Q, frame_stride, track_stride, q_out, g, g16, cg, gstat, G,
+                     index_offset, k, out_score, out_margin, out_idx, stats, workspace, workspace_bytes, stream_,
+                     "seam_search");
+}
+
+int seam_search_f16(seam_handle* h, const void* seq, const uint8_t* mask, const int32_t* lens, int Tmax, int Q,
+                    int64_t frame_stride, int64_t track_stride, float* q_out, const float* g, const void* g16,
+                    const float* cg, const float* gstat, int G, int index_offset, int k, float* out_score,
+                    float* out_margin, int32_t* out_idx, int32_t* stats, void* workspace, size_t workspace_bytes,
+                    void* stream_) {
+  return search_impl(h, seq, true, mask, lens, Tmax, Q, frame_stride, track_stride, q_out, g, g16, cg, gstat, G,
+                     index_offset, k, out_score, out_margin, out_idx, stats, workspace, workspace_bytes, stream_,
+                     "seam_search_f16");
 }
 
 int seam_sharded_score_topk(seam_handle* h, const seam_exchange* x, const float* g, const void* g16, const float* cg,
@@ -1259,18 +1323,29 @@ int seam_tower_forward(seam_handle* h, const float* x, int K, float* out, const 
   return SEAM_OK;
 }
 
+// es: bytes per element (4: fp32, 2: fp16); a frame row of one track is 256 * es bytes
+static int upload_tracks_impl(seam_handle* h, const void* seq_host, size_t es, int Tmax, int Q, int lo, int hi,
+                              void* seq_dev, void* stream_, const char* who) {
+  if (!h) return SEAM_ERR_BAD_ARG;
+  if (Tmax < 0 || Q < 0 || lo < 0 || hi < lo || hi > Q) return fail(h, SEAM_ERR_BAD_ARG, "%s: bad range", who);
+  if (Tmax == 0 || hi == lo) return SEAM_OK;
+  if (!seq_host || !seq_dev) return fail(h, SEAM_ERR_BAD_ARG, "%s: null pointer", who);
+  DeviceGuard guard(h->device);
+  const size_t n = (size_t)(hi - lo), row = 256 * es;
+  SEAM_CUDA(h, cudaMemcpy2DAsync(static_cast<uint8_t*>(seq_dev) + n * row, n * row,
+                                 static_cast<const uint8_t*>(seq_host) + ((size_t)Q + (size_t)lo) * row, (size_t)Q * row,
+                                 n * row, (size_t)Tmax, cudaMemcpyHostToDevice, static_cast<cudaStream_t>(stream_)));
+  return SEAM_OK;
+}
+
 int seam_upload_tracks(seam_handle* h, const float* seq_host, int Tmax, int Q, int lo, int hi, float* seq_dev,
                        void* stream_) {
-  if (!h) return SEAM_ERR_BAD_ARG;
-  if (Tmax < 0 || Q < 0 || lo < 0 || hi < lo || hi > Q) return fail(h, SEAM_ERR_BAD_ARG, "seam_upload_tracks: bad range");
-  if (Tmax == 0 || hi == lo) return SEAM_OK;
-  if (!seq_host || !seq_dev) return fail(h, SEAM_ERR_BAD_ARG, "seam_upload_tracks: null pointer");
-  DeviceGuard guard(h->device);
-  const size_t n = (size_t)(hi - lo);
-  SEAM_CUDA(h, cudaMemcpy2DAsync(seq_dev + n * 256, n * 1024, seq_host + ((size_t)Q + (size_t)lo) * 256,
-                                 (size_t)Q * 1024, n * 1024, (size_t)Tmax, cudaMemcpyHostToDevice,
-                                 static_cast<cudaStream_t>(stream_)));
-  return SEAM_OK;
+  return upload_tracks_impl(h, seq_host, 4, Tmax, Q, lo, hi, seq_dev, stream_, "seam_upload_tracks");
+}
+
+int seam_upload_tracks_f16(seam_handle* h, const void* seq_host, int Tmax, int Q, int lo, int hi, void* seq_dev,
+                           void* stream_) {
+  return upload_tracks_impl(h, seq_host, 2, Tmax, Q, lo, hi, seq_dev, stream_, "seam_upload_tracks_f16");
 }
 
 int seam_merge_topk(seam_handle* h, const float* scores, const float* margins, const int32_t* idx, int N, int Q,

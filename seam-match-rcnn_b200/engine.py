@@ -188,7 +188,7 @@ class SeamEngine:
     def aggregate_backward(self, seq: torch.Tensor, mask, lens, params: Mapping[str, torch.Tensor], dout: torch.Tensor):
         """Vector-Jacobian product of ``aggregate``: ``dout (Q,256)`` -> ``(dseq (1+Tmax,Q,256), {field: grad})`` for
         the 11 aggregator parameters (fields of ``struct seam_weights``, un-folded fp32 tensors in ``params``)."""
-        seq, m8, l32, Tmax, Q = self._tracks(seq, mask, lens)
+        seq, m8, l32, Tmax, Q = self._tracks(seq, mask, lens, keep_f16=False)     # the backward kernel reads fp32
         dout = self._f32(dout, "dout")
         tensors = {f: self._f32(params[f].detach(), f) for f in SeamWeightGrads.FIELDS}
         w = SeamWeights(**{f: (tensors[f].data_ptr() if f in tensors else 0) for f in SeamWeights.FIELDS})
@@ -281,41 +281,31 @@ class SeamEngine:
 
         seq (1+Tmax, Q, 256) fp32 with dummy row 0, mask (Q, 1+Tmax) bool (True = padding):
         the arguments ``x3_1_seq`` / ``x3_1_mask`` of models/match_head.py:90, :133-154.
+        An fp16 ``seq`` on this device is read as fp16 (``seam_aggregate_f16``: no conversion pass, same results as
+        on ``seq.float()``); other dtypes are converted to fp32.
         """
-        if seq.dim() != 3 or seq.shape[2] != D_MODEL:
-            raise ValueError(f"x3_1_seq must be (1+Tmax, Q, 256), got {tuple(seq.shape)}")
-        if seq.device != self.device or seq.dtype != torch.float32:
-            seq = seq.to(device=self.device, dtype=torch.float32)
-        if seq.stride(2) != 1 or seq.stride(0) % 4 or seq.stride(1) % 4:
-            seq = seq.contiguous()
-        Tmax, Q = seq.shape[0] - 1, seq.shape[1]
-        if Tmax > _lib.SEAM_MAX_T:
-            raise SeamError(2, f"Tmax={Tmax} exceeds the supported {_lib.SEAM_MAX_T} frames per track")
-        m8 = None
-        if mask is not None:
-            if tuple(mask.shape) != (Q, 1 + Tmax):
-                raise ValueError(f"x3_1_mask must be (Q, 1+Tmax)={Q, 1 + Tmax}, got {tuple(mask.shape)}")
-            m8 = mask.to(device=self.device, dtype=torch.bool).contiguous().view(torch.uint8)
-        l32 = None
-        if lens is not None:
-            l32 = lens.to(device=self.device, dtype=torch.int32).contiguous()
+        seq, m8, l32, Tmax, Q = self._tracks(seq, mask, lens)
         out = self._out(out, (Q, D_MODEL), torch.float32, "aggregate")
         att = torch.empty((Q, Tmax), dtype=torch.float32, device=self.device) if getatt else None
         nbytes = int(self._lib.seam_aggregate_workspace_bytes(Q))
         ws = self._workspace("agg", nbytes)
-        self._check(self._lib.seam_aggregate(self._h, seq.data_ptr(), _ptr(m8), _ptr(l32), Tmax, Q,
-                                             seq.stride(0), seq.stride(1), out.data_ptr(), _ptr(att),
-                                             ws.data_ptr(), ws.numel(), self._stream()))
+        fn = self._lib.seam_aggregate_f16 if seq.dtype == torch.float16 else self._lib.seam_aggregate
+        self._check(fn(self._h, seq.data_ptr(), _ptr(m8), _ptr(l32), Tmax, Q, seq.stride(0), seq.stride(1),
+                       out.data_ptr(), _ptr(att), ws.data_ptr(), ws.numel(), self._stream()))
         return (out, att) if getatt else out
 
     # ------------------------------------------------------------------ gallery-sharded search (exchange in the kernels)
-    def _tracks(self, seq, mask, lens):
-        """Argument normalisation shared by aggregate / sharded_aggregate."""
+    def _tracks(self, seq, mask, lens, keep_f16: bool = True):
+        """Argument normalisation shared by aggregate / search / sharded_aggregate / aggregate_backward.  ``seq`` comes
+        back fp32, or fp16 when it is fp16 on this device and ``keep_f16`` (the ``_f16`` entry points read it as it
+        is), with 16-byte strides: copied only when its own strides do not allow that."""
         if seq.dim() != 3 or seq.shape[2] != D_MODEL:
             raise ValueError(f"x3_1_seq must be (1+Tmax, Q, 256), got {tuple(seq.shape)}")
-        if seq.device != self.device or seq.dtype != torch.float32:
+        if not (keep_f16 and seq.dtype == torch.float16 and seq.device == self.device) and (
+                seq.device != self.device or seq.dtype != torch.float32):
             seq = seq.to(device=self.device, dtype=torch.float32)
-        if seq.stride(2) != 1 or seq.stride(0) % 4 or seq.stride(1) % 4:
+        per16 = 16 // seq.element_size()                 # elements per 16 bytes: 4 (fp32) / 8 (fp16)
+        if seq.stride(2) != 1 or seq.stride(0) % per16 or seq.stride(1) % per16:
             seq = seq.contiguous()
         Tmax, Q = seq.shape[0] - 1, seq.shape[1]
         if Tmax > _lib.SEAM_MAX_T:
@@ -336,9 +326,9 @@ class SeamEngine:
         seq, m8, l32, Tmax, Q = self._tracks(seq, mask, lens)
         row0 = x.q_lo[x.rank] if row0 is None else int(row0)
         att = torch.empty((Q, Tmax), dtype=torch.float32, device=self.device) if getatt else None
-        self._check(self._lib.seam_sharded_aggregate(self._h, C.byref(x.struct), seq.data_ptr() if Q else 0, _ptr(m8),
-                                                     _ptr(l32), Tmax, Q, seq.stride(0), seq.stride(1), row0,
-                                                     1 if last else 0, _ptr(att), self._stream()))
+        fn = self._lib.seam_sharded_aggregate_f16 if seq.dtype == torch.float16 else self._lib.seam_sharded_aggregate
+        self._check(fn(self._h, C.byref(x.struct), seq.data_ptr() if Q else 0, _ptr(m8), _ptr(l32), Tmax, Q,
+                       seq.stride(0), seq.stride(1), row0, 1 if last else 0, _ptr(att), self._stream()))
         return att
 
     def sharded_score_topk(self, x, gallery: PreparedGallery, return_stats: bool = False):
@@ -464,11 +454,11 @@ class SeamEngine:
         ix = torch.empty((Q, k), dtype=torch.int32, device=self.device)
         stats = torch.zeros((4,), dtype=torch.int32, device=self.device) if return_stats else None
         ws = self._workspace("score", nbytes)
-        self._check(self._lib.seam_search(self._h, seq.data_ptr() if Q else 0, _ptr(m8), _ptr(l32), Tmax, Q, seq.stride(0),
-                                          seq.stride(1), q.data_ptr(), gallery.g.data_ptr(), gallery.g16.data_ptr(),
-                                          gallery.cg.data_ptr(), gallery.gstat.data_ptr(), G, int(gallery.index_offset), k,
-                                          sc.data_ptr(), mg.data_ptr(), ix.data_ptr(), _ptr(stats), ws.data_ptr(),
-                                          ws.numel(), self._stream()))
+        fn = self._lib.seam_search_f16 if seq.dtype == torch.float16 else self._lib.seam_search
+        self._check(fn(self._h, seq.data_ptr() if Q else 0, _ptr(m8), _ptr(l32), Tmax, Q, seq.stride(0), seq.stride(1),
+                       q.data_ptr(), gallery.g.data_ptr(), gallery.g16.data_ptr(), gallery.cg.data_ptr(),
+                       gallery.gstat.data_ptr(), G, int(gallery.index_offset), k, sc.data_ptr(), mg.data_ptr(),
+                       ix.data_ptr(), _ptr(stats), ws.data_ptr(), ws.numel(), self._stream()))
         return (q, sc, mg, ix, stats) if return_stats else (q, sc, mg, ix)
 
     def score_plan(self, Q: int, G: int) -> Dict[str, int]:
@@ -550,15 +540,18 @@ class SeamEngine:
 
     def upload_tracks(self, seq_host: torch.Tensor, lo: int, hi: int) -> torch.Tensor:
         """Tracks [lo, hi) of a HOST ``x3_1_seq (1+Tmax, Q, 256)`` -> device ``(1+Tmax, hi-lo, 256)`` on the
-        current stream with one pitched copy of the frame rows (row 0, the dummy frame, stays untouched)."""
-        if seq_host.device.type != "cpu" or seq_host.dtype != torch.float32 or not seq_host.is_contiguous():
-            raise SeamError(2, "upload_tracks: seq_host must be a contiguous fp32 host tensor")
+        current stream with one pitched copy of the frame rows (row 0, the dummy frame, stays untouched).  fp32 or fp16:
+        the device tensor has the host tensor's dtype (fp16 tracks cross the bus at half the bytes and are aggregated
+        as fp16)."""
+        if (seq_host.device.type != "cpu" or seq_host.dtype not in (torch.float32, torch.float16)
+                or not seq_host.is_contiguous()):
+            raise SeamError(2, "upload_tracks: seq_host must be a contiguous fp32 or fp16 host tensor")
         T1, Q, D = seq_host.shape
         if D != D_MODEL:
             raise SeamError(3, f"upload_tracks: feature size {D} != {D_MODEL}")
-        out = torch.empty((T1, hi - lo, D), dtype=torch.float32, device=self.device)
-        self._check(self._lib.seam_upload_tracks(self._h, seq_host.data_ptr(), T1 - 1, Q, lo, hi, out.data_ptr(),
-                                                 self._stream()))
+        out = torch.empty((T1, hi - lo, D), dtype=seq_host.dtype, device=self.device)
+        fn = self._lib.seam_upload_tracks_f16 if seq_host.dtype == torch.float16 else self._lib.seam_upload_tracks
+        self._check(fn(self._h, seq_host.data_ptr(), T1 - 1, Q, lo, hi, out.data_ptr(), self._stream()))
         return out
 
     def merge_topk(self, scores: Optional[torch.Tensor], margins: torch.Tensor, idx: torch.Tensor):
