@@ -143,6 +143,13 @@ int seam_nlb_forward(seam_handle* h, const float* x, int B, int T, float* z, voi
  * per-item term cg_j = sum_k dw_k g_jk^2 (dw = last.weight[1]-last.weight[0]) and
  * gstat[0] = max_j ||g_j||_2.  g (G,256) fp32 -> g16 (G,256) fp16, cg (G) fp32, gstat (4) fp32. */
 int seam_prepare_gallery(seam_handle* h, const float* g, int G, void* g16, float* cg, float* gstat, void* stream);
+/* Preparation of an fp16 gallery (the dtype the reference's shop-descriptor store, evaluate_movingfashion.py:82-92, and
+ * torch.autocast produce): g16 (G,256) fp16, 256 contiguous halves per row, 16-byte aligned (otherwise
+ * SEAM_ERR_UNSUPPORTED), is read only -- it IS the tensor-core operand, and the direct form reads it as the gallery rows,
+ * so neither an fp32 copy nor a second fp16 copy exists (516 instead of 1,540 bytes per prepared row).  Writes cg and
+ * gstat, bit-identical to seam_prepare_gallery of the widened rows (overflow flag included).  A gallery prepared this
+ * way is scored through the _g16 entry points below. */
+int seam_prepare_gallery_f16(seam_handle* h, const void* g16, int G, float* cg, float* gstat, void* stream);
 
 /* Fused scorer + top-k.  Replaces, for all queries at once, the per-query loop body
  * evaluate_movingfashion.py:263-269 (evaluate_multiDF2.py:220-226):
@@ -175,6 +182,15 @@ int seam_score_partition(int num_sms, int Q, int G, int rank_variant, int32_t* b
 int seam_score_topk(seam_handle* h, const float* q, int Q, const float* g, const void* g16, const float* cg,
                     const float* gstat, int G, int index_offset, int k, float* out_score, float* out_margin,
                     int32_t* out_idx, int32_t* stats, void* workspace, size_t workspace_bytes, void* stream);
+/* The _g16 entry points take an fp16 gallery: there is no g argument, the gallery IS g16 (prepared by
+ * seam_prepare_gallery_f16) -- the tensor-core operand and the rows the fp32 direct form reads, widened exactly.  Results
+ * are bit-identical to the fp32 entry on the widened gallery g16.float().  (Given the g16 that seam_prepare_gallery
+ * made of an fp32 gallery, they score the rounded rows.)  g16 16-byte aligned with rows of 256 contiguous halves,
+ * otherwise SEAM_ERR_UNSUPPORTED; everything else as the fp32 twin.
+ * seam_score_topk for an fp16 gallery: */
+int seam_score_topk_g16(seam_handle* h, const float* q, int Q, const void* g16, const float* cg, const float* gstat,
+                        int G, int index_offset, int k, float* out_score, float* out_margin, int32_t* out_idx,
+                        int32_t* stats, void* workspace, size_t workspace_bytes, void* stream);
 
 /* seam_aggregate + seam_score_topk in one call: tracks in, descriptors (q_out (Q,256) = x3_1b) and per-query top-k
  * out -- the whole per-product loop body evaluate_movingfashion.py:252-277 for all products at once; same results as
@@ -192,6 +208,15 @@ int seam_search_f16(seam_handle* h, const void* seq, const uint8_t* mask, const 
                     const float* cg, const float* gstat, int G, int index_offset, int k, float* out_score,
                     float* out_margin, int32_t* out_idx, int32_t* stats, void* workspace, size_t workspace_bytes,
                     void* stream);
+/* seam_search / seam_search_f16 (fp32 / fp16 tracks) for an fp16 gallery (see seam_score_topk_g16). */
+int seam_search_g16(seam_handle* h, const float* seq, const uint8_t* mask, const int32_t* lens, int Tmax, int Q,
+                    int64_t frame_stride, int64_t track_stride, float* q_out, const void* g16, const float* cg,
+                    const float* gstat, int G, int index_offset, int k, float* out_score, float* out_margin,
+                    int32_t* out_idx, int32_t* stats, void* workspace, size_t workspace_bytes, void* stream);
+int seam_search_f16_g16(seam_handle* h, const void* seq, const uint8_t* mask, const int32_t* lens, int Tmax, int Q,
+                        int64_t frame_stride, int64_t track_stride, float* q_out, const void* g16, const float* cg,
+                        const float* gstat, int G, int index_offset, int k, float* out_score, float* out_margin,
+                        int32_t* out_idx, int32_t* stats, void* workspace, size_t workspace_bytes, void* stream);
 
 /* Dense logits (parity / small problems): x5 (Q,G,2) fp32 = last((q-g)^2).
  * models/match_head.py:160-162 and MatchPredictor.forward :70-74. */
@@ -229,6 +254,12 @@ int seam_rank_of_target_prepared(seam_handle* h, const float* q, int Q, const fl
                                  const float* cg, const float* gstat, int G, const int32_t* target, int32_t* out_rank,
                                  float* out_margin, int32_t* stats, void* workspace, size_t workspace_bytes,
                                  void* stream);
+/* seam_rank_of_target_prepared for an fp16 gallery (see seam_score_topk_g16): same ranks and margins as the fp32 entry
+ * on the widened gallery, its exhaustive fallback included. */
+int seam_rank_of_target_prepared_g16(seam_handle* h, const float* q, int Q, const void* g16, const float* cg,
+                                     const float* gstat, int G, const int32_t* target, int32_t* out_rank,
+                                     float* out_margin, int32_t* stats, void* workspace, size_t workspace_bytes,
+                                     void* stream);
 
 /* Merge N per-shard top-k lists (after the all-gather) into one: lists are (N,Q,k)
  * contiguous; entries with idx < 0 are invalid.  Same ordering contract as seam_score_topk.
@@ -293,6 +324,10 @@ int seam_sharded_aggregate_f16(seam_handle* h, const seam_exchange* x, const voi
 int seam_sharded_score_topk(seam_handle* h, const seam_exchange* x, const float* g, const void* g16, const float* cg,
                             const float* gstat, int G, int index_offset, int32_t* stats, void* workspace,
                             size_t workspace_bytes, void* stream);
+/* seam_sharded_score_topk for an fp16 gallery shard (see seam_score_topk_g16). */
+int seam_sharded_score_topk_g16(seam_handle* h, const seam_exchange* x, const void* g16, const float* cg,
+                                const float* gstat, int G, int index_offset, int32_t* stats, void* workspace,
+                                size_t workspace_bytes, void* stream);
 /* Merges the world lists of the queries this rank owns and ends the step.  With final buffers in the exchange every
  * rank holds the complete (Q,k) result when its stream reaches the end of this call; without, out_* (own,k) receive
  * the owner's rows. */

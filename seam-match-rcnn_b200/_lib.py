@@ -117,6 +117,8 @@ def _declare(lib: C.CDLL) -> None:
     lib.seam_nlb_forward.argtypes = [vp, vp, i32, i32, vp, vp, sz, vp]
     lib.seam_prepare_gallery.restype = i32
     lib.seam_prepare_gallery.argtypes = [vp, vp, i32, vp, vp, vp, vp]
+    lib.seam_prepare_gallery_f16.restype = i32
+    lib.seam_prepare_gallery_f16.argtypes = [vp, vp, i32, vp, vp, vp]
     lib.seam_score_workspace_bytes.restype = sz
     lib.seam_score_workspace_bytes.argtypes = [vp, i32, i32, i32]
     lib.seam_score_partition.restype = i32
@@ -125,10 +127,16 @@ def _declare(lib: C.CDLL) -> None:
     lib.seam_score_plan.argtypes = [vp, i32, i32, C.POINTER(C.c_int64)]
     lib.seam_score_topk.restype = i32
     lib.seam_score_topk.argtypes = [vp, vp, i32, vp, vp, vp, vp, i32, i32, i32, vp, vp, vp, vp, vp, sz, vp]
+    lib.seam_score_topk_g16.restype = i32
+    lib.seam_score_topk_g16.argtypes = [vp, vp, i32, vp, vp, vp, i32, i32, i32, vp, vp, vp, vp, vp, sz, vp]
     lib.seam_search.restype = i32
     lib.seam_search.argtypes = [vp, vp, vp, vp, i32, i32, i64, i64, vp, vp, vp, vp, vp, i32, i32, i32, vp, vp, vp, vp, vp, sz, vp]
     lib.seam_search_f16.restype = i32
     lib.seam_search_f16.argtypes = lib.seam_search.argtypes
+    lib.seam_search_g16.restype = i32
+    lib.seam_search_g16.argtypes = [vp, vp, vp, vp, i32, i32, i64, i64, vp, vp, vp, vp, i32, i32, i32, vp, vp, vp, vp, vp, sz, vp]
+    lib.seam_search_f16_g16.restype = i32
+    lib.seam_search_f16_g16.argtypes = lib.seam_search_g16.argtypes
     lib.seam_score_dense.restype = i32
     lib.seam_score_dense.argtypes = [vp, vp, i32, vp, i32, vp, vp]
     lib.seam_score_prob.restype = i32
@@ -141,6 +149,8 @@ def _declare(lib: C.CDLL) -> None:
     lib.seam_rank_workspace_bytes.argtypes = [vp, i32, i32]
     lib.seam_rank_of_target_prepared.restype = i32
     lib.seam_rank_of_target_prepared.argtypes = [vp, vp, i32, vp, vp, vp, vp, i32, vp, vp, vp, vp, vp, sz, vp]
+    lib.seam_rank_of_target_prepared_g16.restype = i32
+    lib.seam_rank_of_target_prepared_g16.argtypes = [vp, vp, i32, vp, vp, vp, i32, vp, vp, vp, vp, vp, sz, vp]
     xp = C.POINTER(SeamExchange)
     lib.seam_sharded_aggregate.restype = i32
     lib.seam_sharded_aggregate.argtypes = [vp, xp, vp, vp, vp, i32, i32, i64, i64, i32, i32, vp, vp]
@@ -148,6 +158,8 @@ def _declare(lib: C.CDLL) -> None:
     lib.seam_sharded_aggregate_f16.argtypes = lib.seam_sharded_aggregate.argtypes
     lib.seam_sharded_score_topk.restype = i32
     lib.seam_sharded_score_topk.argtypes = [vp, xp, vp, vp, vp, vp, i32, i32, vp, vp, sz, vp]
+    lib.seam_sharded_score_topk_g16.restype = i32
+    lib.seam_sharded_score_topk_g16.argtypes = [vp, xp, vp, vp, vp, i32, i32, vp, vp, sz, vp]
     lib.seam_sharded_merge.restype = i32
     lib.seam_sharded_merge.argtypes = [vp, xp, vp, vp, vp, vp]
     lib.seam_aggregate_backward.restype = i32

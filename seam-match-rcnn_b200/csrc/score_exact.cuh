@@ -41,6 +41,18 @@ __device__ __forceinline__ Slice load_slice(const float* row, int lane) {
   s.hi = *reinterpret_cast<const float4*>(row + 128 + 4 * lane);
   return s;
 }
+// the same slice of an fp16 row: two 8-byte loads, widened exactly (every later instruction is the fp32 path's)
+__device__ __forceinline__ float4 widen4(uint2 v) {
+  const float2 a = __half22float2(*reinterpret_cast<const __half2*>(&v.x));
+  const float2 b = __half22float2(*reinterpret_cast<const __half2*>(&v.y));
+  return make_float4(a.x, a.y, b.x, b.y);
+}
+__device__ __forceinline__ Slice load_slice(const __half* row, int lane) {
+  Slice s;
+  s.lo = widen4(*reinterpret_cast<const uint2*>(row + 4 * lane));
+  s.hi = widen4(*reinterpret_cast<const uint2*>(row + 128 + 4 * lane));
+  return s;
+}
 // Packed fp32 pairs (sub/mul/fma .f32x2 = one issue slot for two IEEE fp32 operations: every kernel
 // here is bound by instruction issue).  Each lane forms two partial sums per logit (even / odd
 // channels of its slice) and adds them at the end.
@@ -73,8 +85,9 @@ __device__ __forceinline__ void sqdiff_dot2(const Slice& q, const Slice& g, cons
   p0 = sum2(a0);
   p1 = sum2(a1);
 }
-// both logits of one pair, all lanes get the result
-__device__ __forceinline__ void pair_logits(const Slice& q, const float* grow, const Slice& w0, const Slice& w1,
+// both logits of one pair, all lanes get the result; Row: float or __half gallery rows
+template <typename Row>
+__device__ __forceinline__ void pair_logits(const Slice& q, const Row* grow, const Slice& w0, const Slice& w1,
                                             float b0, float b1, int lane, float& l0, float& l1) {
   const Slice g = load_slice(grow, lane);
   float p0, p1;
@@ -84,8 +97,10 @@ __device__ __forceinline__ void pair_logits(const Slice& q, const float* grow, c
 }
 
 // ---------------------------------------------------------------- gallery preparation
-// warp per gallery row: fp16 copy, cg_j = dw . g_j^2, max_j ||g_j|| (gstat[0]), overflow flag (gstat[1])
-__global__ void __launch_bounds__(256) prep_gallery_kernel(const float* __restrict__ g, int G,
+// warp per gallery row: fp16 copy, cg_j = dw . g_j^2, max_j ||g_j|| (gstat[0]), overflow flag (gstat[1]).
+// Row = __half: the caller's rows are the fp16 operand already -- cg and gstat only (g16 is not written).
+template <typename Row>
+__global__ void __launch_bounds__(256) prep_gallery_kernel(const Row* __restrict__ g, int G,
                                                            const float* __restrict__ fold, __half* __restrict__ g16,
                                                            float* __restrict__ cg, float* __restrict__ gstat) {
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -104,9 +119,11 @@ __global__ void __launch_bounds__(256) prep_gallery_kernel(const float* __restri
     amax = fmaxf(amax, fabsf(xs[e]));
     h[e] = __float2half_rn(xs[e]);
   }
-  __half* dst = g16 + (size_t)j * 256;
-  *reinterpret_cast<uint2*>(dst + 4 * lane) = *reinterpret_cast<const uint2*>(&h[0]);
-  *reinterpret_cast<uint2*>(dst + 128 + 4 * lane) = *reinterpret_cast<const uint2*>(&h[4]);
+  if constexpr (std::is_same<Row, float>::value) {
+    __half* dst = g16 + (size_t)j * 256;
+    *reinterpret_cast<uint2*>(dst + 4 * lane) = *reinterpret_cast<const uint2*>(&h[0]);
+    *reinterpret_cast<uint2*>(dst + 128 + 4 * lane) = *reinterpret_cast<const uint2*>(&h[4]);
+  }
   c = ptx::warp_sum(c);
   n2 = ptx::warp_sum(n2);
   amax = ptx::warp_max(amax);
@@ -172,7 +189,7 @@ __global__ void __launch_bounds__(256) prep_queries_kernel(const float* q, int Q
 // ---------------------------------------------------------------- re-score + certify
 struct RescoreParams {
   const float* q;        // (Q,256)
-  const float* g;        // (G,256)
+  const void* g;         // (G,256) rows of the kernel's Row type (float or __half)
   const float* fold;
   const uint2* rowbuf;         // (Q,nlists,CAP x 8 bytes): CAP/2 quad records {w0,w1,w2,w3} per sub-list
   const uint32_t* rowcnt;      // (Q,nlists) quad records in each sub-list
@@ -257,6 +274,7 @@ __device__ __forceinline__ void rescore_merge32(const uint2* wb, int begin, int 
 }
 
 // (other occupancies were measured: 5 CTAs per SM = 48 registers, 168 bytes of spills: 70 -> 83 us; 3 CTAs = 80 registers: 78 us)
+template <typename Row>
 __global__ void __launch_bounds__(256) rescore_kernel(const RescoreParams p) {
   __shared__ uint2 wbuf[8][RESCORE_WBUF];
   __shared__ uint4 qbuf[8][64];
@@ -444,7 +462,7 @@ __global__ void __launch_bounds__(256) rescore_kernel(const RescoreParams p) {
 #pragma unroll
       for (int u = 0; u < 4; ++u) {
         const int idx = __shfl_sync(ptx::FULL_MASK, (int)cidx, min(c0 + u, ns - 1));
-        gs[u] = load_slice(p.g + (size_t)idx * 256, lane);
+        gs[u] = load_slice(static_cast<const Row*>(p.g) + (size_t)idx * 256, lane);
       }
       float part[8];
 #pragma unroll
@@ -485,7 +503,7 @@ __global__ void __launch_bounds__(256) rescore_kernel(const RescoreParams p) {
 // ---------------------------------------------------------------- exhaustive fp32 ranking
 struct ExactParams {
   const float* q;
-  const float* g;
+  const void* g;          // rows of the kernel's Row type
   const float* fold;
   int Q, G, k, index_offset;
   const int32_t* count;   // number of rows to process (device), or null: all Q rows
@@ -508,6 +526,7 @@ constexpr int EXACT_MIN_SLICE = 128;   // gallery rows per slice at least (16 pe
 // sweep by ONE CTA each (15,000 items: 0.87 ms for a single row, four times the whole step): with fewer rows than CTAs
 // a row's gallery is cut into S = grid / rows slices, every slice's list goes to global memory and the CTA that
 // finishes a row's last slice merges them.  The result is independent of S: (margin desc, index asc) is a total order.
+template <typename Row>
 __global__ void __launch_bounds__(256) exact_topk_kernel(const ExactParams p) {
   __shared__ float sd[8][32];
   __shared__ int si[8][32];
@@ -566,7 +585,7 @@ __global__ void __launch_bounds__(256) exact_topk_kernel(const ExactParams p) {
     for (int j0 = j_lo + 4 * warp; j0 < j_hi; j0 += 32) {
       Slice gs[4];
 #pragma unroll
-      for (int u = 0; u < 4; ++u) gs[u] = load_slice(p.g + (size_t)min(j0 + u, j_hi - 1) * 256, lane);
+      for (int u = 0; u < 4; ++u) gs[u] = load_slice(static_cast<const Row*>(p.g) + (size_t)min(j0 + u, j_hi - 1) * 256, lane);
       float part[8];
 #pragma unroll
       for (int u = 0; u < 4; ++u) sqdiff_dot2(qs, gs[u], w0, w1, part[2 * u], part[2 * u + 1]);
@@ -797,8 +816,9 @@ __global__ void __launch_bounds__(256) fused_dist_rank_kernel(const FusedDistPar
 // CTA per query: margin of the target, then count items ranking before it -- exhaustive, fp32 direct
 // form.  With a row list (count, rows) only those queries are processed (the rows the tensor-core
 // path below could not certify).
+template <typename Row>
 __global__ void __launch_bounds__(256) rank_of_target_kernel(const float* __restrict__ q, int Q,
-                                                             const float* __restrict__ g, int G,
+                                                             const Row* __restrict__ g, int G,
                                                              const int32_t* __restrict__ target,
                                                              const float* __restrict__ fold,
                                                              const int32_t* __restrict__ count,
@@ -844,7 +864,8 @@ __global__ void __launch_bounds__(256) rank_of_target_kernel(const float* __rest
 // warp per query: exact margin of the target, its image v* in the space of the tensor-core values
 // (v = d - rq - db), and the band v* +- E with E >= |w - v| for every element near the band:
 // EPS_COEFF ||a_i|| max_j ||g_j||  (fp16 operands)  +  TAG_REL_ERR (|v*| + that)  (column tag)  +  fp32 slack.
-__global__ void __launch_bounds__(256) rank_prep_kernel(const float* __restrict__ q, int Q, const float* __restrict__ g,
+template <typename Row>
+__global__ void __launch_bounds__(256) rank_prep_kernel(const float* __restrict__ q, int Q, const Row* __restrict__ g,
                                                         const int32_t* __restrict__ target,
                                                         const float* __restrict__ fold, const float* __restrict__ rq,
                                                         const float* __restrict__ anorm,
@@ -874,7 +895,7 @@ __global__ void __launch_bounds__(256) rank_prep_kernel(const float* __restrict_
 
 struct RankResolveParams {
   const float* q;
-  const float* g;
+  const void* g;             // rows of the kernel's Row type
   const float* fold;
   const uint2* rowbuf;
   const uint32_t* rowcnt;
@@ -898,6 +919,7 @@ constexpr int RANK_CAND = 96;    // in-band candidates gathered before they are 
 // warp per query: certain count from the tensor-core pass + exact verdicts for the elements in the band
 // (a target in the bulk of the ranking has about 1 % of the gallery inside its band; one near the top,
 // the case the eval cares about, a handful)
+template <typename Row>
 __global__ void __launch_bounds__(256) rank_resolve_kernel(const RankResolveParams p) {
   __shared__ uint2 cand[8][RANK_CAND + 128];   // {approximate value, gallery row}
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -926,7 +948,7 @@ __global__ void __launch_bounds__(256) rank_resolve_kernel(const RankResolvePara
 #pragma unroll
       for (int u = 0; u < 4; ++u) {
         ce[u] = cb[min(c0 + u, fill - 1)];
-        gs[u] = load_slice(p.g + (size_t)ce[u].y * 256, lane);
+        gs[u] = load_slice(static_cast<const Row*>(p.g) + (size_t)ce[u].y * 256, lane);
       }
       float part[8];
 #pragma unroll

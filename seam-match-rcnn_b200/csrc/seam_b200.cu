@@ -546,23 +546,39 @@ int seam_nlb_forward(seam_handle* h, const float* x, int B, int T, float* z, voi
 }
 
 // ------------------------------------------------------------------------------ scorer
-int seam_prepare_gallery(seam_handle* h, const float* g, int G, void* g16, float* cg, float* gstat, void* stream_) {
+// rows: the gallery's (G,256) rows, fp32 or (rows_f16) fp16.  An fp16 gallery is its own tensor-core operand: g16 is
+// then the same pointer and is not written.
+static int prepare_gallery_impl(seam_handle* h, const void* rows, bool rows_f16, void* g16, int G, float* cg,
+                                float* gstat, void* stream_, const char* who) {
   if (!h) return SEAM_ERR_BAD_ARG;
-  if (!h->have_scorer) return fail(h, SEAM_ERR_STATE, "seam_prepare_gallery: scorer weights not loaded");
-  if (G < 0) return fail(h, SEAM_ERR_BAD_ARG, "seam_prepare_gallery: negative size");
-  if (!gstat) return fail(h, SEAM_ERR_BAD_ARG, "seam_prepare_gallery: gstat is null");
+  if (!h->have_scorer) return fail(h, SEAM_ERR_STATE, "%s: scorer weights not loaded", who);
+  if (G < 0) return fail(h, SEAM_ERR_BAD_ARG, "%s: negative size", who);
+  if (!gstat) return fail(h, SEAM_ERR_BAD_ARG, "%s: gstat is null", who);
   cudaStream_t stream = static_cast<cudaStream_t>(stream_);
   DeviceGuard guard(h->device);
   SEAM_CUDA(h, cudaMemsetAsync(gstat, 0, 16, stream));
   if (G == 0) return SEAM_OK;
-  if (!g || !g16 || !cg) return fail(h, SEAM_ERR_BAD_ARG, "seam_prepare_gallery: null pointer");
-  if (!aligned16(g) || !aligned16(g16)) return fail(h, SEAM_ERR_UNSUPPORTED, "seam_prepare_gallery: 16-byte alignment");
+  if (!rows || !g16 || !cg) return fail(h, SEAM_ERR_BAD_ARG, "%s: null pointer", who);
+  if (!aligned16(rows) || !aligned16(g16)) return fail(h, SEAM_ERR_UNSUPPORTED, "%s: 16-byte alignment", who);
   {
     ProfileScope prof(h, SEAM_KERNEL_PREP_GALLERY, stream);
-    exact::prep_gallery_kernel<<<(G + 7) / 8, 256, 0, stream>>>(g, G, h->fold, static_cast<__half*>(g16), cg, gstat);
+    if (rows_f16)
+      exact::prep_gallery_kernel<__half><<<(G + 7) / 8, 256, 0, stream>>>(static_cast<const __half*>(rows), G, h->fold,
+                                                                          nullptr, cg, gstat);
+    else
+      exact::prep_gallery_kernel<float><<<(G + 7) / 8, 256, 0, stream>>>(static_cast<const float*>(rows), G, h->fold,
+                                                                         static_cast<__half*>(g16), cg, gstat);
     SEAM_LAUNCHED(h, "prep_gallery_kernel");
   }
   return SEAM_OK;
+}
+
+int seam_prepare_gallery(seam_handle* h, const float* g, int G, void* g16, float* cg, float* gstat, void* stream_) {
+  return prepare_gallery_impl(h, g, false, g16, G, cg, gstat, stream_, "seam_prepare_gallery");
+}
+
+int seam_prepare_gallery_f16(seam_handle* h, const void* g16, int G, float* cg, float* gstat, void* stream_) {
+  return prepare_gallery_impl(h, g16, true, const_cast<void*>(g16), G, cg, gstat, stream_, "seam_prepare_gallery_f16");
 }
 
 struct ScorePlan {
@@ -772,12 +788,13 @@ struct ScoreWorkspace {
   float *lo, *hi, *dtarget;
 };
 
-// Checks what both scorer variants take, plans the work and carves the workspace; fn names the entry point.
-static int carve_score_workspace(seam_handle* h, const char* fn, bool rank, const float* q, int Q, const float* g,
+// Checks what both scorer variants take, plans the work and carves the workspace; fn names the entry point, rows are
+// the gallery rows the direct form reads (g, or g16 itself for an fp16 gallery).
+static int carve_score_workspace(seam_handle* h, const char* fn, bool rank, const float* q, int Q, const void* rows,
                                  const void* g16, const float* cg, const float* gstat, int G, void* workspace,
                                  size_t workspace_bytes, ScoreWorkspace* w) {
-  if (!q || !g || !g16 || !cg || !gstat || !workspace) return fail(h, SEAM_ERR_BAD_ARG, "%s: null pointer", fn);
-  if (!aligned16(q) || !aligned16(g) || !aligned16(g16) || (reinterpret_cast<uintptr_t>(workspace) & 255u))
+  if (!q || !rows || !g16 || !cg || !gstat || !workspace) return fail(h, SEAM_ERR_BAD_ARG, "%s: null pointer", fn);
+  if (!aligned16(q) || !aligned16(rows) || !aligned16(g16) || (reinterpret_cast<uintptr_t>(workspace) & 255u))
     return fail(h, SEAM_ERR_UNSUPPORTED, "%s: q/g/g16 need 16-byte, workspace 256-byte alignment", fn);
   const ScorePlan& s = w->plan = plan_score(h->num_sms, Q, G, rank);
   if (s.tiles.ntiles_n > score::TAG_TILES)
@@ -832,20 +849,22 @@ static int score_kernel_args(seam_handle* h, const ScoreWorkspace& w, int Q, con
   return SEAM_OK;
 }
 
-static int score_topk_impl(seam_handle* h, const xchg::Exchange* x, const float* q, int Q, const float* g,
-                           const void* g16, const float* cg, const float* gstat, int G, int index_offset, int k,
-                           float* out_score, float* out_margin, int32_t* out_idx, int32_t* stats, void* workspace,
-                           size_t workspace_bytes, void* stream_) {
-  if (!h->have_scorer) return fail(h, SEAM_ERR_STATE, "seam_score_topk: scorer weights not loaded");
-  if (Q < 0 || G < 0) return fail(h, SEAM_ERR_BAD_ARG, "seam_score_topk: negative size");
-  if (k < 1 || k > SEAM_MAX_K) return fail(h, SEAM_ERR_UNSUPPORTED, "seam_score_topk: k=%d outside [1,%d]", k, SEAM_MAX_K);
+// rows: the gallery rows of the direct form, fp32 or (rows_f16) fp16 -- then the same pointer as g16.  who names the
+// entry point in errors, xwho the sharded entry in the check only a sharded call can fail.
+static int score_topk_impl(seam_handle* h, const xchg::Exchange* x, const float* q, int Q, const void* rows,
+                           bool rows_f16, const void* g16, const float* cg, const float* gstat, int G, int index_offset,
+                           int k, float* out_score, float* out_margin, int32_t* out_idx, int32_t* stats, void* workspace,
+                           size_t workspace_bytes, void* stream_, const char* who, const char* xwho) {
+  if (!h->have_scorer) return fail(h, SEAM_ERR_STATE, "%s: scorer weights not loaded", who);
+  if (Q < 0 || G < 0) return fail(h, SEAM_ERR_BAD_ARG, "%s: negative size", who);
+  if (k < 1 || k > SEAM_MAX_K) return fail(h, SEAM_ERR_UNSUPPORTED, "%s: k=%d outside [1,%d]", who, k, SEAM_MAX_K);
   if (Q == 0 && !x) return SEAM_OK;
-  if (!x && (!out_score || !out_margin || !out_idx)) return fail(h, SEAM_ERR_BAD_ARG, "seam_score_topk: null output");
+  if (!x && (!out_score || !out_margin || !out_idx)) return fail(h, SEAM_ERR_BAD_ARG, "%s: null output", who);
   cudaStream_t stream = static_cast<cudaStream_t>(stream_);
   DeviceGuard guard(h->device);
   if (stats) SEAM_CUDA(h, cudaMemsetAsync(stats, 0, 16, stream));
   if (x && (Q == 0 || G == 0))
-    return fail(h, SEAM_ERR_UNSUPPORTED, "seam_sharded_score_topk: every rank needs queries and a non-empty gallery shard");
+    return fail(h, SEAM_ERR_UNSUPPORTED, "%s: every rank needs queries and a non-empty gallery shard", xwho);
   const int x_on = x ? 1 : 0;
   xchg::Exchange xe;
   memset(&xe, 0, sizeof(xe));
@@ -858,7 +877,7 @@ static int score_topk_impl(seam_handle* h, const xchg::Exchange* x, const float*
     return SEAM_OK;
   }
   ScoreWorkspace w;
-  int rc = carve_score_workspace(h, "seam_score_topk", false, q, Q, g, g16, cg, gstat, G, workspace, workspace_bytes, &w);
+  int rc = carve_score_workspace(h, who, false, q, Q, rows, g16, cg, gstat, G, workspace, workspace_bytes, &w);
   if (rc != SEAM_OK) return rc;
 
   {
@@ -879,7 +898,7 @@ static int score_topk_impl(seam_handle* h, const xchg::Exchange* x, const float*
 
   exact::RescoreParams rp;
   rp.q = q;
-  rp.g = g;
+  rp.g = rows;
   rp.fold = h->fold;
   rp.rowbuf = w.rowbuf;
   rp.rowcnt = w.rowcnt;
@@ -905,13 +924,14 @@ static int score_topk_impl(seam_handle* h, const xchg::Exchange* x, const float*
   rp.plan = w.plan.tiles;
   {
     ProfileScope prof(h, SEAM_KERNEL_RESCORE, stream);
-    exact::rescore_kernel<<<(Q + 7) / 8, 256, 0, stream>>>(rp);
+    if (rows_f16) exact::rescore_kernel<__half><<<(Q + 7) / 8, 256, 0, stream>>>(rp);
+    else exact::rescore_kernel<float><<<(Q + 7) / 8, 256, 0, stream>>>(rp);
     SEAM_LAUNCHED(h, "rescore_kernel");
   }
 
   exact::ExactParams ep;
   ep.q = q;
-  ep.g = g;
+  ep.g = rows;
   ep.fold = h->fold;
   ep.Q = Q;
   ep.G = G;
@@ -929,7 +949,8 @@ static int score_topk_impl(seam_handle* h, const xchg::Exchange* x, const float*
   ep.x = xe;
   {
     ProfileScope prof(h, SEAM_KERNEL_EXACT, stream);
-    exact::exact_topk_kernel<<<2 * h->num_sms, 256, 0, stream>>>(ep);
+    if (rows_f16) exact::exact_topk_kernel<__half><<<2 * h->num_sms, 256, 0, stream>>>(ep);
+    else exact::exact_topk_kernel<float><<<2 * h->num_sms, 256, 0, stream>>>(ep);
     SEAM_LAUNCHED(h, "exact_topk_kernel");
   }
   if (stats) SEAM_CUDA(h, cudaMemcpyAsync(stats, w.counters, 4, cudaMemcpyDeviceToDevice, stream));
@@ -940,31 +961,40 @@ int seam_score_topk(seam_handle* h, const float* q, int Q, const float* g, const
                     const float* gstat, int G, int index_offset, int k, float* out_score, float* out_margin,
                     int32_t* out_idx, int32_t* stats, void* workspace, size_t workspace_bytes, void* stream_) {
   if (!h) return SEAM_ERR_BAD_ARG;
-  return score_topk_impl(h, nullptr, q, Q, g, g16, cg, gstat, G, index_offset, k, out_score, out_margin, out_idx, stats,
-                         workspace, workspace_bytes, stream_);
+  return score_topk_impl(h, nullptr, q, Q, g, false, g16, cg, gstat, G, index_offset, k, out_score, out_margin, out_idx,
+                         stats, workspace, workspace_bytes, stream_, "seam_score_topk", "seam_score_topk");
 }
 
+int seam_score_topk_g16(seam_handle* h, const float* q, int Q, const void* g16, const float* cg, const float* gstat,
+                        int G, int index_offset, int k, float* out_score, float* out_margin, int32_t* out_idx,
+                        int32_t* stats, void* workspace, size_t workspace_bytes, void* stream_) {
+  if (!h) return SEAM_ERR_BAD_ARG;
+  return score_topk_impl(h, nullptr, q, Q, g16, true, g16, cg, gstat, G, index_offset, k, out_score, out_margin, out_idx,
+                         stats, workspace, workspace_bytes, stream_, "seam_score_topk_g16", "seam_score_topk_g16");
+}
+
+// f16: fp16 tracks; rows / rows_f16: the gallery rows as in score_topk_impl.  Scorer errors name score_who.
 static int search_impl(seam_handle* h, const void* seq, bool f16, const uint8_t* mask, const int32_t* lens, int Tmax,
-                       int Q, int64_t frame_stride, int64_t track_stride, float* q_out, const float* g, const void* g16,
-                       const float* cg, const float* gstat, int G, int index_offset, int k, float* out_score,
-                       float* out_margin, int32_t* out_idx, int32_t* stats, void* workspace, size_t workspace_bytes,
-                       void* stream_, const char* who) {
+                       int Q, int64_t frame_stride, int64_t track_stride, float* q_out, const void* rows, bool rows_f16,
+                       const void* g16, const float* cg, const float* gstat, int G, int index_offset, int k,
+                       float* out_score, float* out_margin, int32_t* out_idx, int32_t* stats, void* workspace,
+                       size_t workspace_bytes, void* stream_, const char* who, const char* score_who) {
   if (!h) return SEAM_ERR_BAD_ARG;
   if (!q_out && Q > 0) return fail(h, SEAM_ERR_BAD_ARG, "%s: q_out is null", who);
   int rc = aggregate_impl(h, nullptr, 0, 0, seq, f16, mask, lens, Tmax, Q, frame_stride, track_stride, q_out, nullptr,
                           static_cast<cudaStream_t>(stream_), who);
   if (rc != SEAM_OK) return rc;
-  return score_topk_impl(h, nullptr, q_out, Q, g, g16, cg, gstat, G, index_offset, k, out_score, out_margin, out_idx, stats,
-                         workspace, workspace_bytes, stream_);
+  return score_topk_impl(h, nullptr, q_out, Q, rows, rows_f16, g16, cg, gstat, G, index_offset, k, out_score, out_margin,
+                         out_idx, stats, workspace, workspace_bytes, stream_, score_who, score_who);
 }
 
 int seam_search(seam_handle* h, const float* seq, const uint8_t* mask, const int32_t* lens, int Tmax, int Q,
                 int64_t frame_stride, int64_t track_stride, float* q_out, const float* g, const void* g16, const float* cg,
                 const float* gstat, int G, int index_offset, int k, float* out_score, float* out_margin, int32_t* out_idx,
                 int32_t* stats, void* workspace, size_t workspace_bytes, void* stream_) {
-  return search_impl(h, seq, false, mask, lens, Tmax, Q, frame_stride, track_stride, q_out, g, g16, cg, gstat, G,
+  return search_impl(h, seq, false, mask, lens, Tmax, Q, frame_stride, track_stride, q_out, g, false, g16, cg, gstat, G,
                      index_offset, k, out_score, out_margin, out_idx, stats, workspace, workspace_bytes, stream_,
-                     "seam_search");
+                     "seam_search", "seam_score_topk");
 }
 
 int seam_search_f16(seam_handle* h, const void* seq, const uint8_t* mask, const int32_t* lens, int Tmax, int Q,
@@ -972,20 +1002,53 @@ int seam_search_f16(seam_handle* h, const void* seq, const uint8_t* mask, const 
                     const float* cg, const float* gstat, int G, int index_offset, int k, float* out_score,
                     float* out_margin, int32_t* out_idx, int32_t* stats, void* workspace, size_t workspace_bytes,
                     void* stream_) {
-  return search_impl(h, seq, true, mask, lens, Tmax, Q, frame_stride, track_stride, q_out, g, g16, cg, gstat, G,
+  return search_impl(h, seq, true, mask, lens, Tmax, Q, frame_stride, track_stride, q_out, g, false, g16, cg, gstat, G,
                      index_offset, k, out_score, out_margin, out_idx, stats, workspace, workspace_bytes, stream_,
-                     "seam_search_f16");
+                     "seam_search_f16", "seam_score_topk");
+}
+
+int seam_search_g16(seam_handle* h, const float* seq, const uint8_t* mask, const int32_t* lens, int Tmax, int Q,
+                    int64_t frame_stride, int64_t track_stride, float* q_out, const void* g16, const float* cg,
+                    const float* gstat, int G, int index_offset, int k, float* out_score, float* out_margin,
+                    int32_t* out_idx, int32_t* stats, void* workspace, size_t workspace_bytes, void* stream_) {
+  return search_impl(h, seq, false, mask, lens, Tmax, Q, frame_stride, track_stride, q_out, g16, true, g16, cg, gstat, G,
+                     index_offset, k, out_score, out_margin, out_idx, stats, workspace, workspace_bytes, stream_,
+                     "seam_search_g16", "seam_search_g16");
+}
+
+int seam_search_f16_g16(seam_handle* h, const void* seq, const uint8_t* mask, const int32_t* lens, int Tmax, int Q,
+                        int64_t frame_stride, int64_t track_stride, float* q_out, const void* g16, const float* cg,
+                        const float* gstat, int G, int index_offset, int k, float* out_score, float* out_margin,
+                        int32_t* out_idx, int32_t* stats, void* workspace, size_t workspace_bytes, void* stream_) {
+  return search_impl(h, seq, true, mask, lens, Tmax, Q, frame_stride, track_stride, q_out, g16, true, g16, cg, gstat, G,
+                     index_offset, k, out_score, out_margin, out_idx, stats, workspace, workspace_bytes, stream_,
+                     "seam_search_f16_g16", "seam_search_f16_g16");
+}
+
+static int sharded_score_topk_impl(seam_handle* h, const seam_exchange* x, const void* rows, bool rows_f16,
+                                   const void* g16, const float* cg, const float* gstat, int G, int index_offset,
+                                   int32_t* stats, void* workspace, size_t workspace_bytes, void* stream_,
+                                   const char* who, const char* score_who) {
+  if (!h) return SEAM_ERR_BAD_ARG;
+  xchg::Exchange e;
+  int rc = import_exchange(h, x, &e, who);
+  if (rc != SEAM_OK) return rc;
+  return score_topk_impl(h, &e, nullptr, x->Q, rows, rows_f16, g16, cg, gstat, G, index_offset, x->k, nullptr, nullptr,
+                         nullptr, stats, workspace, workspace_bytes, stream_, score_who, who);
 }
 
 int seam_sharded_score_topk(seam_handle* h, const seam_exchange* x, const float* g, const void* g16, const float* cg,
                             const float* gstat, int G, int index_offset, int32_t* stats, void* workspace,
                             size_t workspace_bytes, void* stream_) {
-  if (!h) return SEAM_ERR_BAD_ARG;
-  xchg::Exchange e;
-  int rc = import_exchange(h, x, &e, "seam_sharded_score_topk");
-  if (rc != SEAM_OK) return rc;
-  return score_topk_impl(h, &e, nullptr, x->Q, g, g16, cg, gstat, G, index_offset, x->k, nullptr, nullptr, nullptr, stats,
-                         workspace, workspace_bytes, stream_);
+  return sharded_score_topk_impl(h, x, g, false, g16, cg, gstat, G, index_offset, stats, workspace, workspace_bytes,
+                                 stream_, "seam_sharded_score_topk", "seam_score_topk");
+}
+
+int seam_sharded_score_topk_g16(seam_handle* h, const seam_exchange* x, const void* g16, const float* cg,
+                                const float* gstat, int G, int index_offset, int32_t* stats, void* workspace,
+                                size_t workspace_bytes, void* stream_) {
+  return sharded_score_topk_impl(h, x, g16, true, g16, cg, gstat, G, index_offset, stats, workspace, workspace_bytes,
+                                 stream_, "seam_sharded_score_topk_g16", "seam_sharded_score_topk_g16");
 }
 
 int seam_sharded_merge(seam_handle* h, const seam_exchange* x, float* out_score, float* out_margin, int32_t* out_idx,
@@ -1074,8 +1137,9 @@ int seam_rank_of_target(seam_handle* h, const float* q, int Q, const float* g, i
   if (!q || !g || !target || !out_rank) return fail(h, SEAM_ERR_BAD_ARG, "seam_rank_of_target: null pointer");
   if (!aligned16(q) || !aligned16(g)) return fail(h, SEAM_ERR_UNSUPPORTED, "seam_rank_of_target: 16-byte alignment");
   DeviceGuard guard(h->device);
-  exact::rank_of_target_kernel<<<Q, 256, 0, static_cast<cudaStream_t>(stream_)>>>(q, Q, g, G, target, h->fold, nullptr,
-                                                                                   nullptr, out_rank, out_margin);
+  exact::rank_of_target_kernel<float><<<Q, 256, 0, static_cast<cudaStream_t>(stream_)>>>(q, Q, g, G, target, h->fold,
+                                                                                          nullptr, nullptr, out_rank,
+                                                                                          out_margin);
   SEAM_LAUNCHED(h, "rank_of_target_kernel");
   return SEAM_OK;
 }
@@ -1088,21 +1152,21 @@ size_t seam_rank_workspace_bytes(const seam_handle* h, int Q, int G) {
 // Tensor-core path: prepare queries -> exact target margins + bands -> score_topk_kernel<VAR_RANK> (counts
 // what is certainly above, appends what is inside the band) -> rank_resolve_kernel -> exhaustive kernel for
 // the rows that could not be certified.  The workspace is laid out like seam_score_topk's (no sample tiles).
-int seam_rank_of_target_prepared(seam_handle* h, const float* q, int Q, const float* g, const void* g16,
-                                 const float* cg, const float* gstat, int G, const int32_t* target, int32_t* out_rank,
-                                 float* out_margin, int32_t* stats, void* workspace, size_t workspace_bytes,
-                                 void* stream_) {
+// rows / rows_f16 as in score_topk_impl
+static int rank_prepared_impl(seam_handle* h, const float* q, int Q, const void* rows, bool rows_f16, const void* g16,
+                              const float* cg, const float* gstat, int G, const int32_t* target, int32_t* out_rank,
+                              float* out_margin, int32_t* stats, void* workspace, size_t workspace_bytes, void* stream_,
+                              const char* who) {
   if (!h) return SEAM_ERR_BAD_ARG;
-  if (!h->have_scorer) return fail(h, SEAM_ERR_STATE, "seam_rank_of_target_prepared: scorer weights not loaded");
-  if (Q < 0 || G <= 0) return fail(h, SEAM_ERR_BAD_ARG, "seam_rank_of_target_prepared: bad size");
+  if (!h->have_scorer) return fail(h, SEAM_ERR_STATE, "%s: scorer weights not loaded", who);
+  if (Q < 0 || G <= 0) return fail(h, SEAM_ERR_BAD_ARG, "%s: bad size", who);
   cudaStream_t stream = static_cast<cudaStream_t>(stream_);
   DeviceGuard guard(h->device);
   if (stats) SEAM_CUDA(h, cudaMemsetAsync(stats, 0, 16, stream));
   if (Q == 0) return SEAM_OK;
-  if (!target || !out_rank) return fail(h, SEAM_ERR_BAD_ARG, "seam_rank_of_target_prepared: null pointer");
+  if (!target || !out_rank) return fail(h, SEAM_ERR_BAD_ARG, "%s: null pointer", who);
   ScoreWorkspace w;
-  int rc = carve_score_workspace(h, "seam_rank_of_target_prepared", true, q, Q, g, g16, cg, gstat, G, workspace,
-                                 workspace_bytes, &w);
+  int rc = carve_score_workspace(h, who, true, q, Q, rows, g16, cg, gstat, G, workspace, workspace_bytes, &w);
   if (rc != SEAM_OK) return rc;
   const int nlists = w.plan.P * score::NQ;
 
@@ -1111,8 +1175,14 @@ int seam_rank_of_target_prepared(seam_handle* h, const float* q, int Q, const fl
   exact::prep_queries_kernel<<<(Q + 7) / 8, 256, 0, stream>>>(q, Q, h->fold, w.a16, w.rq, w.anorm, w.thr, w.rowflag,
                                                               w.counters, nullptr, 0, no_x);
   SEAM_LAUNCHED(h, "prep_queries_kernel");
-  exact::rank_prep_kernel<<<(Q + 7) / 8, 256, 0, stream>>>(q, Q, g, target, h->fold, w.rq, w.anorm, gstat, w.lo, w.hi,
-                                                          w.dtarget, w.above, nlists);
+  if (rows_f16)
+    exact::rank_prep_kernel<__half><<<(Q + 7) / 8, 256, 0, stream>>>(q, Q, static_cast<const __half*>(rows), target,
+                                                                     h->fold, w.rq, w.anorm, gstat, w.lo, w.hi,
+                                                                     w.dtarget, w.above, nlists);
+  else
+    exact::rank_prep_kernel<float><<<(Q + 7) / 8, 256, 0, stream>>>(q, Q, static_cast<const float*>(rows), target,
+                                                                    h->fold, w.rq, w.anorm, gstat, w.lo, w.hi,
+                                                                    w.dtarget, w.above, nlists);
   SEAM_LAUNCHED(h, "rank_prep_kernel");
 
   CUtensorMap tmA, tmB;
@@ -1123,7 +1193,7 @@ int seam_rank_of_target_prepared(seam_handle* h, const float* q, int Q, const fl
 
   exact::RankResolveParams rp;
   rp.q = q;
-  rp.g = g;
+  rp.g = rows;
   rp.fold = h->fold;
   rp.rowbuf = w.rowbuf;
   rp.rowcnt = w.rowcnt;
@@ -1144,13 +1214,36 @@ int seam_rank_of_target_prepared(seam_handle* h, const float* q, int Q, const fl
   rp.counters = w.counters;
   rp.fallback_rows = w.frows;
   rp.plan = w.plan.tiles;
-  exact::rank_resolve_kernel<<<(Q + 7) / 8, 256, 0, stream>>>(rp);
+  if (rows_f16) exact::rank_resolve_kernel<__half><<<(Q + 7) / 8, 256, 0, stream>>>(rp);
+  else exact::rank_resolve_kernel<float><<<(Q + 7) / 8, 256, 0, stream>>>(rp);
   SEAM_LAUNCHED(h, "rank_resolve_kernel");
-  exact::rank_of_target_kernel<<<2 * h->num_sms, 256, 0, stream>>>(q, Q, g, G, target, h->fold, w.counters, w.frows,
-                                                                  out_rank, out_margin);
+  if (rows_f16)
+    exact::rank_of_target_kernel<__half><<<2 * h->num_sms, 256, 0, stream>>>(q, Q, static_cast<const __half*>(rows), G,
+                                                                              target, h->fold, w.counters, w.frows,
+                                                                              out_rank, out_margin);
+  else
+    exact::rank_of_target_kernel<float><<<2 * h->num_sms, 256, 0, stream>>>(q, Q, static_cast<const float*>(rows), G,
+                                                                             target, h->fold, w.counters, w.frows,
+                                                                             out_rank, out_margin);
   SEAM_LAUNCHED(h, "rank_of_target_kernel");
   if (stats) SEAM_CUDA(h, cudaMemcpyAsync(stats, w.counters, 4, cudaMemcpyDeviceToDevice, stream));
   return SEAM_OK;
+}
+
+int seam_rank_of_target_prepared(seam_handle* h, const float* q, int Q, const float* g, const void* g16,
+                                 const float* cg, const float* gstat, int G, const int32_t* target, int32_t* out_rank,
+                                 float* out_margin, int32_t* stats, void* workspace, size_t workspace_bytes,
+                                 void* stream_) {
+  return rank_prepared_impl(h, q, Q, g, false, g16, cg, gstat, G, target, out_rank, out_margin, stats, workspace,
+                            workspace_bytes, stream_, "seam_rank_of_target_prepared");
+}
+
+int seam_rank_of_target_prepared_g16(seam_handle* h, const float* q, int Q, const void* g16, const float* cg,
+                                     const float* gstat, int G, const int32_t* target, int32_t* out_rank,
+                                     float* out_margin, int32_t* stats, void* workspace, size_t workspace_bytes,
+                                     void* stream_) {
+  return rank_prepared_impl(h, q, Q, g16, true, g16, cg, gstat, G, target, out_rank, out_margin, stats, workspace,
+                            workspace_bytes, stream_, "seam_rank_of_target_prepared_g16");
 }
 
 // ------------------------------------------------------------------------------ backward (f4)

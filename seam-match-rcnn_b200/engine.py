@@ -33,10 +33,14 @@ def _ptr(t: Optional[torch.Tensor]) -> Optional[int]:
 class PreparedGallery:
     """A gallery shard resident on the device with its tensor-core operands.
 
-    g    (G,256) fp32   the shop descriptors (x3_2 of models/match_head.py:131/156)
-    g16  (G,256) fp16   operand of the tcgen05 pass
+    g    (G,256) fp32   the shop descriptors (x3_2 of models/match_head.py:131/156), or fp16 when the caller's
+                        gallery is fp16: then it is the caller's tensor (or one contiguous copy of it) and
+    g16  (G,256) fp16   operand of the tcgen05 pass -- the same tensor as ``g`` for an fp16 gallery
     cg   (G)     fp32   dw . g_j^2
     gstat (4)    fp32   [max_j ||g_j||, fp16-overflow flag, -, -]
+
+    An fp32 gallery holds 1,540 bytes per row (g, g16, cg), an fp16 one 516 (g16, cg); both score the same: the fp16
+    rows are widened exactly wherever the fp32 direct form reads them.
     """
     g: torch.Tensor
     g16: torch.Tensor
@@ -48,6 +52,11 @@ class PreparedGallery:
     @property
     def G(self) -> int:
         return self.g.shape[0]
+
+    @property
+    def rows_f16(self) -> bool:
+        """The gallery rows are fp16 (``g is g16``): scored through the ``_g16`` entry points."""
+        return self.g.dtype == torch.float16
 
 
 class SeamEngine:
@@ -339,10 +348,16 @@ class SeamEngine:
         stats = torch.zeros((4,), dtype=torch.int32, device=self.device) if return_stats else None
         nbytes = int(self._lib.seam_score_workspace_bytes(self._h, x.Q, gallery.G, x.k))
         ws = self._workspace("score", nbytes)
-        self._check(self._lib.seam_sharded_score_topk(self._h, C.byref(x.struct), gallery.g.data_ptr(),
-                                                      gallery.g16.data_ptr(), gallery.cg.data_ptr(),
-                                                      gallery.gstat.data_ptr(), gallery.G, int(gallery.index_offset),
-                                                      _ptr(stats), ws.data_ptr(), ws.numel(), self._stream()))
+        if gallery.rows_f16:
+            self._check(self._lib.seam_sharded_score_topk_g16(self._h, C.byref(x.struct), gallery.g16.data_ptr(),
+                                                              gallery.cg.data_ptr(), gallery.gstat.data_ptr(), gallery.G,
+                                                              int(gallery.index_offset), _ptr(stats), ws.data_ptr(),
+                                                              ws.numel(), self._stream()))
+        else:
+            self._check(self._lib.seam_sharded_score_topk(self._h, C.byref(x.struct), gallery.g.data_ptr(),
+                                                          gallery.g16.data_ptr(), gallery.cg.data_ptr(),
+                                                          gallery.gstat.data_ptr(), gallery.G, int(gallery.index_offset),
+                                                          _ptr(stats), ws.data_ptr(), ws.numel(), self._stream()))
         return stats
 
     def sharded_merge(self, x):
@@ -377,25 +392,41 @@ class SeamEngine:
 
     # ------------------------------------------------------------------ (b)+(c) scorer
     def prepare_gallery(self, g: torch.Tensor, index_offset: int = 0) -> PreparedGallery:
+        """Device-resident gallery with its tensor-core operands.  An fp16 ``g`` stays fp16: used in place when it is
+        on this device, contiguous and 16-byte aligned (``seam_prepare_gallery_f16``: no fp32 copy, no second fp16
+        copy), else copied once to a contiguous fp16 tensor here.  Other dtypes are converted to fp32."""
         if g.dim() != 2 or g.shape[1] != D_MODEL:
             raise ValueError(f"gallery must be (G,256), got {tuple(g.shape)}")
-        g = self._f32(g, "gallery")
+        if g.dtype == torch.float16:
+            g = g.to(self.device)
+            if not g.is_contiguous() or g.data_ptr() % 16:
+                g = g.clone(memory_format=torch.contiguous_format)
+            g16 = g
+        else:
+            g = self._f32(g, "gallery")
+            g16 = torch.empty((g.shape[0], D_MODEL), dtype=torch.float16, device=self.device)
         G = g.shape[0]
-        g16 = torch.empty((G, D_MODEL), dtype=torch.float16, device=self.device)
         cg = torch.empty((max(G, 1),), dtype=torch.float32, device=self.device)
         gstat = torch.empty((4,), dtype=torch.float32, device=self.device)
-        self._check(self._lib.seam_prepare_gallery(self._h, g.data_ptr(), G, g16.data_ptr(), cg.data_ptr(),
-                                                   gstat.data_ptr(), self._stream()))
-        return PreparedGallery(g=g, g16=g16, cg=cg, gstat=gstat, index_offset=index_offset,
-                               scorer_epoch=self.scorer_epoch)
+        gallery = PreparedGallery(g=g, g16=g16, cg=cg, gstat=gstat, index_offset=index_offset,
+                                  scorer_epoch=self.scorer_epoch)
+        self._prepare(gallery)
+        return gallery
+
+    def _prepare(self, gallery: PreparedGallery) -> None:
+        if gallery.rows_f16:
+            self._check(self._lib.seam_prepare_gallery_f16(self._h, gallery.g16.data_ptr(), gallery.G,
+                                                           gallery.cg.data_ptr(), gallery.gstat.data_ptr(),
+                                                           self._stream()))
+        else:
+            self._check(self._lib.seam_prepare_gallery(self._h, gallery.g.data_ptr(), gallery.G, gallery.g16.data_ptr(),
+                                                       gallery.cg.data_ptr(), gallery.gstat.data_ptr(), self._stream()))
 
     def _fresh(self, gallery: PreparedGallery) -> PreparedGallery:
         """A gallery prepared under another scorer (its cg = dw . g^2 and overflow statistics are stale after
-        load_weights / load_scorer) is prepared again in place: one pass over its fp32 rows."""
+        load_weights / load_scorer) is prepared again in place: one pass over its rows."""
         if gallery.scorer_epoch != self.scorer_epoch:
-            G = gallery.G
-            self._check(self._lib.seam_prepare_gallery(self._h, gallery.g.data_ptr(), G, gallery.g16.data_ptr(),
-                                                       gallery.cg.data_ptr(), gallery.gstat.data_ptr(), self._stream()))
+            self._prepare(gallery)
             gallery.scorer_epoch = self.scorer_epoch
         return gallery
 
@@ -426,12 +457,13 @@ class SeamEngine:
             nbytes = int(self._lib.seam_score_workspace_bytes(self._h, n, G, k))
             ws = self._workspace("score", nbytes)
             st = stats if (slab == Q or stats is None) else torch.zeros((4,), dtype=torch.int32, device=self.device)
-            self._check(self._lib.seam_score_topk(self._h, q[lo:hi].data_ptr() if n else 0, n, gallery.g.data_ptr(),
-                                                  gallery.g16.data_ptr(), gallery.cg.data_ptr(),
-                                                  gallery.gstat.data_ptr(), G, int(gallery.index_offset), k,
-                                                  sc[lo:hi].data_ptr() if n else 0, mg[lo:hi].data_ptr() if n else 0,
-                                                  ix[lo:hi].data_ptr() if n else 0, _ptr(st),
-                                                  ws.data_ptr(), ws.numel(), self._stream()))
+            # an fp16 gallery has no separate rows: the _g16 entry reads g16 for both the operand and the direct form
+            fn, rows = ((self._lib.seam_score_topk_g16, ()) if gallery.rows_f16
+                        else (self._lib.seam_score_topk, (gallery.g.data_ptr(),)))
+            self._check(fn(self._h, q[lo:hi].data_ptr() if n else 0, n, *rows, gallery.g16.data_ptr(),
+                           gallery.cg.data_ptr(), gallery.gstat.data_ptr(), G, int(gallery.index_offset), k,
+                           sc[lo:hi].data_ptr() if n else 0, mg[lo:hi].data_ptr() if n else 0,
+                           ix[lo:hi].data_ptr() if n else 0, _ptr(st), ws.data_ptr(), ws.numel(), self._stream()))
             if st is not stats:
                 stats += st
         if return_stats:
@@ -454,9 +486,13 @@ class SeamEngine:
         ix = torch.empty((Q, k), dtype=torch.int32, device=self.device)
         stats = torch.zeros((4,), dtype=torch.int32, device=self.device) if return_stats else None
         ws = self._workspace("score", nbytes)
-        fn = self._lib.seam_search_f16 if seq.dtype == torch.float16 else self._lib.seam_search
+        f16 = seq.dtype == torch.float16
+        if gallery.rows_f16:
+            fn, rows = (self._lib.seam_search_f16_g16 if f16 else self._lib.seam_search_g16), ()
+        else:
+            fn, rows = (self._lib.seam_search_f16 if f16 else self._lib.seam_search), (gallery.g.data_ptr(),)
         self._check(fn(self._h, seq.data_ptr() if Q else 0, _ptr(m8), _ptr(l32), Tmax, Q, seq.stride(0), seq.stride(1),
-                       q.data_ptr(), gallery.g.data_ptr(), gallery.g16.data_ptr(), gallery.cg.data_ptr(),
+                       q.data_ptr(), *rows, gallery.g16.data_ptr(), gallery.cg.data_ptr(),
                        gallery.gstat.data_ptr(), G, int(gallery.index_offset), k, sc.data_ptr(), mg.data_ptr(),
                        ix.data_ptr(), _ptr(stats), ws.data_ptr(), ws.numel(), self._stream()))
         return (q, sc, mg, ix, stats) if return_stats else (q, sc, mg, ix)
@@ -526,10 +562,11 @@ class SeamEngine:
         if prepared and Q > 0:
             nbytes = int(self._lib.seam_rank_workspace_bytes(self._h, Q, G))
             ws = self._workspace("score", nbytes)
-            self._check(self._lib.seam_rank_of_target_prepared(
-                self._h, q.data_ptr(), Q, gm.data_ptr(), g.g16.data_ptr(), g.cg.data_ptr(), g.gstat.data_ptr(), G,
-                t32.data_ptr(), rank.data_ptr(), margin.data_ptr(), stats.data_ptr(), ws.data_ptr(), ws.numel(),
-                self._stream()))
+            fn, rows = ((self._lib.seam_rank_of_target_prepared_g16, ()) if g.rows_f16
+                        else (self._lib.seam_rank_of_target_prepared, (gm.data_ptr(),)))
+            self._check(fn(self._h, q.data_ptr(), Q, *rows, g.g16.data_ptr(), g.cg.data_ptr(), g.gstat.data_ptr(), G,
+                           t32.data_ptr(), rank.data_ptr(), margin.data_ptr(), stats.data_ptr(), ws.data_ptr(), ws.numel(),
+                           self._stream()))
         else:
             self._check(self._lib.seam_rank_of_target(self._h, q.data_ptr(), Q, gm.data_ptr(), G,
                                                       t32.data_ptr(), rank.data_ptr(), margin.data_ptr(),

@@ -457,7 +457,6 @@ def evaluate_products(engine: SeamEngine, frame_desc: torch.Tensor, frame_produc
     fp = frame_product.to(dev, torch.int64)
     target = target.to(dev, torch.int64)
     P = int(target.shape[0])
-    shop_desc = shop_desc.to(dev, torch.float32).contiguous()
     ks = list(k_thresholds)
 
     big = torch.iinfo(torch.int32).max
