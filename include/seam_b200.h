@@ -261,6 +261,33 @@ int seam_rank_of_target_prepared_g16(seam_handle* h, const float* q, int Q, cons
                                      float* out_margin, int32_t* stats, void* workspace, size_t workspace_bytes,
                                      void* stream);
 
+/* Rank of the target over a gallery split into shards (one per GPU), exactly: for global target t,
+ *   rank_i = sum over shards s of #{ j in s : (d_ij, j) ranks before (d_it, t) }   (ties by GLOBAL row).
+ * Only the shard holding row t can compute d_it, so a sharded rank is three steps per shard:
+ *   1. seam_shard_target_margin: out_margin (Q) fp32 = d_it where global row target[i] lies in
+ *      [index_offset, index_offset + G), else -inf -- bit for bit the margin seam_rank_of_target[_prepared] reports;
+ *   2. all-reduce MAX of the margins over the shards (every shard now holds every d_it);
+ *   3. seam_shard_rank_count_prepared: out_count (Q) int32 = this shard's count against target_margin, by the
+ *      tensor-core path of seam_rank_of_target_prepared on this shard's PREPARED rows (same workspace:
+ *      seam_rank_workspace_bytes(h, Q, G)); queries it cannot certify on this shard are counted exhaustively here
+ *      (their number in stats[0]);
+ * then an all-reduce SUM of the counts gives the unsharded rank, integer for integer.
+ *   target (Q) int32 GLOBAL gallery rows; index_offset >= 0 (else SEAM_ERR_BAD_ARG); target_margin must not be null
+ *   (SEAM_ERR_BAD_ARG); Q == 0 is a no-op.  The _g16 forms take an fp16 shard (see seam_score_topk_g16), 16-byte
+ *   aligned (else SEAM_ERR_UNSUPPORTED), and give the fp32 forms' results on the widened rows. */
+int seam_shard_target_margin(seam_handle* h, const float* q, int Q, const float* g, int G, int index_offset,
+                             const int32_t* target, float* out_margin, void* stream);
+int seam_shard_target_margin_g16(seam_handle* h, const float* q, int Q, const void* g16, int G, int index_offset,
+                                 const int32_t* target, float* out_margin, void* stream);
+int seam_shard_rank_count_prepared(seam_handle* h, const float* q, int Q, const float* g, const void* g16,
+                                   const float* cg, const float* gstat, int G, int index_offset, const int32_t* target,
+                                   const float* target_margin, int32_t* out_count, int32_t* stats, void* workspace,
+                                   size_t workspace_bytes, void* stream);
+int seam_shard_rank_count_prepared_g16(seam_handle* h, const float* q, int Q, const void* g16, const float* cg,
+                                       const float* gstat, int G, int index_offset, const int32_t* target,
+                                       const float* target_margin, int32_t* out_count, int32_t* stats,
+                                       void* workspace, size_t workspace_bytes, void* stream);
+
 /* Merge N per-shard top-k lists (after the all-gather) into one: lists are (N,Q,k)
  * contiguous; entries with idx < 0 are invalid.  Same ordering contract as seam_score_topk.
  * No reference counterpart (the reference ranks a single gallery).  scores may be NULL: the score is

@@ -151,6 +151,14 @@ def _declare(lib: C.CDLL) -> None:
     lib.seam_rank_of_target_prepared.argtypes = [vp, vp, i32, vp, vp, vp, vp, i32, vp, vp, vp, vp, vp, sz, vp]
     lib.seam_rank_of_target_prepared_g16.restype = i32
     lib.seam_rank_of_target_prepared_g16.argtypes = [vp, vp, i32, vp, vp, vp, i32, vp, vp, vp, vp, vp, sz, vp]
+    lib.seam_shard_target_margin.restype = i32
+    lib.seam_shard_target_margin.argtypes = [vp, vp, i32, vp, i32, i32, vp, vp, vp]
+    lib.seam_shard_target_margin_g16.restype = i32
+    lib.seam_shard_target_margin_g16.argtypes = lib.seam_shard_target_margin.argtypes
+    lib.seam_shard_rank_count_prepared.restype = i32
+    lib.seam_shard_rank_count_prepared.argtypes = [vp, vp, i32, vp, vp, vp, vp, i32, i32, vp, vp, vp, vp, vp, sz, vp]
+    lib.seam_shard_rank_count_prepared_g16.restype = i32
+    lib.seam_shard_rank_count_prepared_g16.argtypes = [vp, vp, i32, vp, vp, vp, i32, i32, vp, vp, vp, vp, vp, sz, vp]
     xp = C.POINTER(SeamExchange)
     lib.seam_sharded_aggregate.restype = i32
     lib.seam_sharded_aggregate.argtypes = [vp, xp, vp, vp, vp, i32, i32, i64, i64, i32, i32, vp, vp]

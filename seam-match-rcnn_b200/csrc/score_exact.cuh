@@ -816,7 +816,9 @@ __global__ void __launch_bounds__(256) fused_dist_rank_kernel(const FusedDistPar
 // CTA per query: margin of the target, then count items ranking before it -- exhaustive, fp32 direct
 // form.  With a row list (count, rows) only those queries are processed (the rows the tensor-core
 // path below could not certify).
-template <typename Row>
+// EXT (one shard of a sharded gallery): the target's margin is ext_margin[qi] (the row may live on another GPU),
+// target[] holds global rows and row j of this shard is global row j + index_offset; out_rank is this shard's count.
+template <typename Row, bool EXT>
 __global__ void __launch_bounds__(256) rank_of_target_kernel(const float* __restrict__ q, int Q,
                                                              const Row* __restrict__ g, int G,
                                                              const int32_t* __restrict__ target,
@@ -824,7 +826,8 @@ __global__ void __launch_bounds__(256) rank_of_target_kernel(const float* __rest
                                                              const int32_t* __restrict__ count,
                                                              const int32_t* __restrict__ rows,
                                                              int32_t* __restrict__ out_rank,
-                                                             float* __restrict__ out_margin) {
+                                                             float* __restrict__ out_margin,
+                                                             const float* __restrict__ ext_margin, int index_offset) {
   __shared__ int cnt_s[8];
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const Slice w0 = load_slice(fold + Fold::LAST_W, lane);
@@ -834,10 +837,16 @@ __global__ void __launch_bounds__(256) rank_of_target_kernel(const float* __rest
   for (int e = blockIdx.x; e < nrows; e += gridDim.x) {
     const int qi = count ? rows[e] : e;
     const Slice qs = load_slice(q + (size_t)qi * 256, lane);
-    const int tj = target[qi];
+    // EXT: the target as a row of this shard (j + index_offset < target  <=>  j < target - index_offset)
+    const int tj = EXT ? target[qi] - index_offset : target[qi];
     float l0, l1;
-    pair_logits(qs, g + (size_t)tj * 256, w0, w1, b0, b1, lane, l0, l1);
-    const float dt = l1 - l0;
+    float dt;
+    if (EXT) {
+      dt = ext_margin[qi];
+    } else {
+      pair_logits(qs, g + (size_t)tj * 256, w0, w1, b0, b1, lane, l0, l1);
+      dt = l1 - l0;
+    }
     int cnt = 0;
     for (int j = warp; j < G; j += 8) {
       pair_logits(qs, g + (size_t)j * 256, w0, w1, b0, b1, lane, l0, l1);
@@ -855,6 +864,32 @@ __global__ void __launch_bounds__(256) rank_of_target_kernel(const float* __rest
   }
 }
 
+// warp per query: the target's margin l1 - l0 when global row target[qi] lies in this shard
+// [index_offset, index_offset + G), else -inf (so that a MAX over the shards is exact).  The same pair_logits call and
+// lane mapping as rank_prep_kernel: the bits are those of the unsharded path.
+template <typename Row>
+__global__ void __launch_bounds__(256) target_margin_kernel(const float* __restrict__ q, int Q,
+                                                            const Row* __restrict__ g, int G, int index_offset,
+                                                            const int32_t* __restrict__ target,
+                                                            const float* __restrict__ fold,
+                                                            float* __restrict__ out_margin) {
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  const int qi = blockIdx.x * 8 + warp;
+  if (qi >= Q) return;
+  const long long t = (long long)target[qi] - index_offset;
+  if (t < 0 || t >= G) {
+    if (lane == 0) out_margin[qi] = -INFINITY;
+    return;
+  }
+  const Slice w0 = load_slice(fold + Fold::LAST_W, lane);
+  const Slice w1 = load_slice(fold + Fold::LAST_W + 256, lane);
+  const float b0 = fold[Fold::CONSTS + 5], b1 = fold[Fold::CONSTS + 6];
+  const Slice qs = load_slice(q + (size_t)qi * 256, lane);
+  float l0, l1;
+  pair_logits(qs, g + (size_t)t * 256, w0, w1, b0, b1, lane, l0, l1);
+  if (lane == 0) out_margin[qi] = l1 - l0;
+}
+
 // ---------------------------------------------------------------- rank of a target item, tensor-core path
 // rank_i = #{ j : (d_ij, j) ranks before (d_it, t) } without visiting every pair in fp32: the tcgen05 pass
 // (score_tc.cuh, VAR_RANK) counts the elements whose value exceeds the target's by more than its error
@@ -864,24 +899,32 @@ __global__ void __launch_bounds__(256) rank_of_target_kernel(const float* __rest
 // warp per query: exact margin of the target, its image v* in the space of the tensor-core values
 // (v = d - rq - db), and the band v* +- E with E >= |w - v| for every element near the band:
 // EPS_COEFF ||a_i|| max_j ||g_j||  (fp16 operands)  +  TAG_REL_ERR (|v*| + that)  (column tag)  +  fp32 slack.
-template <typename Row>
+// EXT: the target's margin is ext_margin[qi] and no target row is read; the band is built from it in the same way,
+// with this shard's max_j ||g_j||, so it bounds the error of every row of this shard.
+template <typename Row, bool EXT>
 __global__ void __launch_bounds__(256) rank_prep_kernel(const float* __restrict__ q, int Q, const Row* __restrict__ g,
                                                         const int32_t* __restrict__ target,
                                                         const float* __restrict__ fold, const float* __restrict__ rq,
                                                         const float* __restrict__ anorm,
                                                         const float* __restrict__ gstat, float* __restrict__ lo,
                                                         float* __restrict__ hi, float* __restrict__ dtarget,
-                                                        int32_t* __restrict__ above, int nlists) {
+                                                        int32_t* __restrict__ above, int nlists,
+                                                        const float* __restrict__ ext_margin) {
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int qi = blockIdx.x * 8 + warp;
   if (qi >= Q) return;
-  const Slice w0 = load_slice(fold + Fold::LAST_W, lane);
-  const Slice w1 = load_slice(fold + Fold::LAST_W + 256, lane);
-  const float b0 = fold[Fold::CONSTS + 5], b1 = fold[Fold::CONSTS + 6];
-  const Slice qs = load_slice(q + (size_t)qi * 256, lane);
-  float l0, l1;
-  pair_logits(qs, g + (size_t)target[qi] * 256, w0, w1, b0, b1, lane, l0, l1);
-  const float dt = l1 - l0;
+  float dt;
+  if (EXT) {
+    dt = ext_margin[qi];
+  } else {
+    const Slice w0 = load_slice(fold + Fold::LAST_W, lane);
+    const Slice w1 = load_slice(fold + Fold::LAST_W + 256, lane);
+    const float b0 = fold[Fold::CONSTS + 5], b1 = fold[Fold::CONSTS + 6];
+    const Slice qs = load_slice(q + (size_t)qi * 256, lane);
+    float l0, l1;
+    pair_logits(qs, g + (size_t)target[qi] * 256, w0, w1, b0, b1, lane, l0, l1);
+    dt = l1 - l0;
+  }
   for (int l = lane; l < nlists; l += 32) above[(size_t)qi * nlists + l] = 0;
   if (lane == 0) {
     const float vstar = dt - rq[qi] - fold[Fold::CONSTS + 4];
@@ -913,13 +956,15 @@ struct RankResolveParams {
   float* out_margin;         // optional
   int32_t* counters;         // [0] rows for the exhaustive kernel, [1] query overflow flag
   int32_t* fallback_rows;
+  int index_offset;          // EXT: global row of this shard's row 0 (target[] holds global rows)
 };
 constexpr int RANK_CAND = 96;    // in-band candidates gathered before they are decided (+ 128 of headroom per round)
 
 // warp per query: certain count from the tensor-core pass + exact verdicts for the elements in the band
 // (a target in the bulk of the ranking has about 1 % of the gallery inside its band; one near the top,
 // the case the eval cares about, a handful)
-template <typename Row>
+// EXT: one shard of a sharded gallery -- ties with the target are broken by global row
+template <typename Row, bool EXT>
 __global__ void __launch_bounds__(256) rank_resolve_kernel(const RankResolveParams p) {
   __shared__ uint2 cand[8][RANK_CAND + 128];   // {approximate value, gallery row}
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -928,7 +973,7 @@ __global__ void __launch_bounds__(256) rank_resolve_kernel(const RankResolvePara
   const bool overflow = p.counters[1] != 0 || p.gstat[1] != 0.f;
   bool ok = !overflow && p.rowflag[qi] == 0;
   const float lo = p.lo[qi], hi = p.hi[qi], dt = p.dtarget[qi];
-  const int tj = p.target[qi];
+  const int tj = EXT ? p.target[qi] - p.index_offset : p.target[qi];   // EXT: as a row of this shard
   const int capq = p.CAP / 2;
   const uint4* rowq = reinterpret_cast<const uint4*>(p.rowbuf) + (size_t)qi * p.nlists * capq;
   uint2* cb = cand[warp];

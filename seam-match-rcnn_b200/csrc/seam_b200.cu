@@ -1137,9 +1137,8 @@ int seam_rank_of_target(seam_handle* h, const float* q, int Q, const float* g, i
   if (!q || !g || !target || !out_rank) return fail(h, SEAM_ERR_BAD_ARG, "seam_rank_of_target: null pointer");
   if (!aligned16(q) || !aligned16(g)) return fail(h, SEAM_ERR_UNSUPPORTED, "seam_rank_of_target: 16-byte alignment");
   DeviceGuard guard(h->device);
-  exact::rank_of_target_kernel<float><<<Q, 256, 0, static_cast<cudaStream_t>(stream_)>>>(q, Q, g, G, target, h->fold,
-                                                                                          nullptr, nullptr, out_rank,
-                                                                                          out_margin);
+  exact::rank_of_target_kernel<float, false><<<Q, 256, 0, static_cast<cudaStream_t>(stream_)>>>(
+      q, Q, g, G, target, h->fold, nullptr, nullptr, out_rank, out_margin, nullptr, 0);
   SEAM_LAUNCHED(h, "rank_of_target_kernel");
   return SEAM_OK;
 }
@@ -1152,41 +1151,27 @@ size_t seam_rank_workspace_bytes(const seam_handle* h, int Q, int G) {
 // Tensor-core path: prepare queries -> exact target margins + bands -> score_topk_kernel<VAR_RANK> (counts
 // what is certainly above, appends what is inside the band) -> rank_resolve_kernel -> exhaustive kernel for
 // the rows that could not be certified.  The workspace is laid out like seam_score_topk's (no sample tiles).
-// rows / rows_f16 as in score_topk_impl
-static int rank_prepared_impl(seam_handle* h, const float* q, int Q, const void* rows, bool rows_f16, const void* g16,
-                              const float* cg, const float* gstat, int G, const int32_t* target, int32_t* out_rank,
-                              float* out_margin, int32_t* stats, void* workspace, size_t workspace_bytes, void* stream_,
-                              const char* who) {
-  if (!h) return SEAM_ERR_BAD_ARG;
-  if (!h->have_scorer) return fail(h, SEAM_ERR_STATE, "%s: scorer weights not loaded", who);
-  if (Q < 0 || G <= 0) return fail(h, SEAM_ERR_BAD_ARG, "%s: bad size", who);
-  cudaStream_t stream = static_cast<cudaStream_t>(stream_);
-  DeviceGuard guard(h->device);
-  if (stats) SEAM_CUDA(h, cudaMemsetAsync(stats, 0, 16, stream));
-  if (Q == 0) return SEAM_OK;
-  if (!target || !out_rank) return fail(h, SEAM_ERR_BAD_ARG, "%s: null pointer", who);
-  ScoreWorkspace w;
-  int rc = carve_score_workspace(h, who, true, q, Q, rows, g16, cg, gstat, G, workspace, workspace_bytes, &w);
-  if (rc != SEAM_OK) return rc;
+// EXT: one shard of a sharded gallery -- the target margins are given (ext_margin), target[] holds global rows and
+// out_rank receives this shard's count of rows ranking before the target.
+extern "C++" {   // a template
+template <typename Row, bool EXT>
+static int rank_launch(seam_handle* h, const ScoreWorkspace& w, const float* q, int Q, const void* rows, const void* g16,
+                       const float* cg, const float* gstat, int G, int index_offset, const int32_t* target,
+                       const float* ext_margin, int32_t* out_rank, float* out_margin, cudaStream_t stream) {
   const int nlists = w.plan.P * score::NQ;
-
+  const Row* grows = static_cast<const Row*>(rows);
   xchg::Exchange no_x;
   memset(&no_x, 0, sizeof(no_x));
   exact::prep_queries_kernel<<<(Q + 7) / 8, 256, 0, stream>>>(q, Q, h->fold, w.a16, w.rq, w.anorm, w.thr, w.rowflag,
                                                               w.counters, nullptr, 0, no_x);
   SEAM_LAUNCHED(h, "prep_queries_kernel");
-  if (rows_f16)
-    exact::rank_prep_kernel<__half><<<(Q + 7) / 8, 256, 0, stream>>>(q, Q, static_cast<const __half*>(rows), target,
-                                                                     h->fold, w.rq, w.anorm, gstat, w.lo, w.hi,
-                                                                     w.dtarget, w.above, nlists);
-  else
-    exact::rank_prep_kernel<float><<<(Q + 7) / 8, 256, 0, stream>>>(q, Q, static_cast<const float*>(rows), target,
-                                                                    h->fold, w.rq, w.anorm, gstat, w.lo, w.hi,
-                                                                    w.dtarget, w.above, nlists);
+  exact::rank_prep_kernel<Row, EXT><<<(Q + 7) / 8, 256, 0, stream>>>(q, Q, grows, target, h->fold, w.rq, w.anorm, gstat,
+                                                                     w.lo, w.hi, w.dtarget, w.above, nlists, ext_margin);
   SEAM_LAUNCHED(h, "rank_prep_kernel");
 
   CUtensorMap tmA, tmB;
   score::Params sp;
+  int rc;
   if ((rc = score_kernel_args(h, w, Q, g16, cg, G, &tmA, &tmB, &sp)) != SEAM_OK) return rc;
   score::score_topk_kernel<score::VAR_RANK><<<w.plan.tiles.nb, score::THREADS, score::SMEM_BYTES, stream>>>(tmA, tmB, sp);
   SEAM_LAUNCHED(h, "score_topk_kernel<rank>");
@@ -1214,18 +1199,46 @@ static int rank_prepared_impl(seam_handle* h, const float* q, int Q, const void*
   rp.counters = w.counters;
   rp.fallback_rows = w.frows;
   rp.plan = w.plan.tiles;
-  if (rows_f16) exact::rank_resolve_kernel<__half><<<(Q + 7) / 8, 256, 0, stream>>>(rp);
-  else exact::rank_resolve_kernel<float><<<(Q + 7) / 8, 256, 0, stream>>>(rp);
+  rp.index_offset = index_offset;
+  exact::rank_resolve_kernel<Row, EXT><<<(Q + 7) / 8, 256, 0, stream>>>(rp);
   SEAM_LAUNCHED(h, "rank_resolve_kernel");
-  if (rows_f16)
-    exact::rank_of_target_kernel<__half><<<2 * h->num_sms, 256, 0, stream>>>(q, Q, static_cast<const __half*>(rows), G,
-                                                                              target, h->fold, w.counters, w.frows,
-                                                                              out_rank, out_margin);
-  else
-    exact::rank_of_target_kernel<float><<<2 * h->num_sms, 256, 0, stream>>>(q, Q, static_cast<const float*>(rows), G,
-                                                                             target, h->fold, w.counters, w.frows,
-                                                                             out_rank, out_margin);
+  exact::rank_of_target_kernel<Row, EXT><<<2 * h->num_sms, 256, 0, stream>>>(q, Q, grows, G, target, h->fold, w.counters,
+                                                                             w.frows, out_rank, out_margin, ext_margin,
+                                                                             index_offset);
   SEAM_LAUNCHED(h, "rank_of_target_kernel");
+  return SEAM_OK;
+}
+}  // extern "C++"
+
+// rows / rows_f16 as in score_topk_impl.  ext_margin null: the whole gallery (index_offset 0, out_margin optional);
+// else one shard of it, counting against the given target margins (out_margin null).
+static int rank_prepared_impl(seam_handle* h, const float* q, int Q, const void* rows, bool rows_f16, const void* g16,
+                              const float* cg, const float* gstat, int G, int index_offset, const int32_t* target,
+                              const float* ext_margin, int32_t* out_rank, float* out_margin, int32_t* stats,
+                              void* workspace, size_t workspace_bytes, void* stream_, const char* who) {
+  if (!h) return SEAM_ERR_BAD_ARG;
+  if (!h->have_scorer) return fail(h, SEAM_ERR_STATE, "%s: scorer weights not loaded", who);
+  if (Q < 0 || G <= 0) return fail(h, SEAM_ERR_BAD_ARG, "%s: bad size", who);
+  if (index_offset < 0) return fail(h, SEAM_ERR_BAD_ARG, "%s: negative index_offset %d", who, index_offset);
+  cudaStream_t stream = static_cast<cudaStream_t>(stream_);
+  DeviceGuard guard(h->device);
+  if (stats) SEAM_CUDA(h, cudaMemsetAsync(stats, 0, 16, stream));
+  if (Q == 0) return SEAM_OK;
+  if (!target || !out_rank) return fail(h, SEAM_ERR_BAD_ARG, "%s: null pointer", who);
+  ScoreWorkspace w;
+  int rc = carve_score_workspace(h, who, true, q, Q, rows, g16, cg, gstat, G, workspace, workspace_bytes, &w);
+  if (rc != SEAM_OK) return rc;
+  if (ext_margin)
+    rc = rows_f16 ? rank_launch<__half, true>(h, w, q, Q, rows, g16, cg, gstat, G, index_offset, target, ext_margin,
+                                              out_rank, nullptr, stream)
+                  : rank_launch<float, true>(h, w, q, Q, rows, g16, cg, gstat, G, index_offset, target, ext_margin,
+                                             out_rank, nullptr, stream);
+  else
+    rc = rows_f16 ? rank_launch<__half, false>(h, w, q, Q, rows, g16, cg, gstat, G, 0, target, nullptr, out_rank,
+                                               out_margin, stream)
+                  : rank_launch<float, false>(h, w, q, Q, rows, g16, cg, gstat, G, 0, target, nullptr, out_rank,
+                                              out_margin, stream);
+  if (rc != SEAM_OK) return rc;
   if (stats) SEAM_CUDA(h, cudaMemcpyAsync(stats, w.counters, 4, cudaMemcpyDeviceToDevice, stream));
   return SEAM_OK;
 }
@@ -1234,16 +1247,74 @@ int seam_rank_of_target_prepared(seam_handle* h, const float* q, int Q, const fl
                                  const float* cg, const float* gstat, int G, const int32_t* target, int32_t* out_rank,
                                  float* out_margin, int32_t* stats, void* workspace, size_t workspace_bytes,
                                  void* stream_) {
-  return rank_prepared_impl(h, q, Q, g, false, g16, cg, gstat, G, target, out_rank, out_margin, stats, workspace,
-                            workspace_bytes, stream_, "seam_rank_of_target_prepared");
+  return rank_prepared_impl(h, q, Q, g, false, g16, cg, gstat, G, 0, target, nullptr, out_rank, out_margin, stats,
+                            workspace, workspace_bytes, stream_, "seam_rank_of_target_prepared");
 }
 
 int seam_rank_of_target_prepared_g16(seam_handle* h, const float* q, int Q, const void* g16, const float* cg,
                                      const float* gstat, int G, const int32_t* target, int32_t* out_rank,
                                      float* out_margin, int32_t* stats, void* workspace, size_t workspace_bytes,
                                      void* stream_) {
-  return rank_prepared_impl(h, q, Q, g16, true, g16, cg, gstat, G, target, out_rank, out_margin, stats, workspace,
-                            workspace_bytes, stream_, "seam_rank_of_target_prepared_g16");
+  return rank_prepared_impl(h, q, Q, g16, true, g16, cg, gstat, G, 0, target, nullptr, out_rank, out_margin, stats,
+                            workspace, workspace_bytes, stream_, "seam_rank_of_target_prepared_g16");
+}
+
+// ------------------------------------------------------------------------------ rank over a sharded gallery
+// rank_i = sum over shards s of #{ j in s : (d_ij, j) ranks before (d_it, t) }: the owner of row t computes the
+// target's margin (-inf elsewhere, so a MAX all-reduce delivers it to every shard), every shard counts against it, and
+// the counts are summed.
+static int shard_target_margin_impl(seam_handle* h, const float* q, int Q, const void* rows, bool rows_f16, int G,
+                                    int index_offset, const int32_t* target, float* out_margin, void* stream_,
+                                    const char* who) {
+  if (!h) return SEAM_ERR_BAD_ARG;
+  if (!h->have_scorer) return fail(h, SEAM_ERR_STATE, "%s: scorer weights not loaded", who);
+  if (Q < 0 || G <= 0) return fail(h, SEAM_ERR_BAD_ARG, "%s: bad size", who);
+  if (index_offset < 0) return fail(h, SEAM_ERR_BAD_ARG, "%s: negative index_offset %d", who, index_offset);
+  if (Q == 0) return SEAM_OK;
+  if (!q || !rows || !target || !out_margin) return fail(h, SEAM_ERR_BAD_ARG, "%s: null pointer", who);
+  if (!aligned16(q) || !aligned16(rows)) return fail(h, SEAM_ERR_UNSUPPORTED, "%s: q/g need 16-byte alignment", who);
+  DeviceGuard guard(h->device);
+  cudaStream_t stream = static_cast<cudaStream_t>(stream_);
+  if (rows_f16)
+    exact::target_margin_kernel<__half><<<(Q + 7) / 8, 256, 0, stream>>>(q, Q, static_cast<const __half*>(rows), G,
+                                                                         index_offset, target, h->fold, out_margin);
+  else
+    exact::target_margin_kernel<float><<<(Q + 7) / 8, 256, 0, stream>>>(q, Q, static_cast<const float*>(rows), G,
+                                                                        index_offset, target, h->fold, out_margin);
+  SEAM_LAUNCHED(h, "target_margin_kernel");
+  return SEAM_OK;
+}
+
+int seam_shard_target_margin(seam_handle* h, const float* q, int Q, const float* g, int G, int index_offset,
+                             const int32_t* target, float* out_margin, void* stream_) {
+  return shard_target_margin_impl(h, q, Q, g, false, G, index_offset, target, out_margin, stream_,
+                                  "seam_shard_target_margin");
+}
+
+int seam_shard_target_margin_g16(seam_handle* h, const float* q, int Q, const void* g16, int G, int index_offset,
+                                 const int32_t* target, float* out_margin, void* stream_) {
+  return shard_target_margin_impl(h, q, Q, g16, true, G, index_offset, target, out_margin, stream_,
+                                  "seam_shard_target_margin_g16");
+}
+
+int seam_shard_rank_count_prepared(seam_handle* h, const float* q, int Q, const float* g, const void* g16,
+                                   const float* cg, const float* gstat, int G, int index_offset, const int32_t* target,
+                                   const float* target_margin, int32_t* out_count, int32_t* stats, void* workspace,
+                                   size_t workspace_bytes, void* stream_) {
+  if (h && Q > 0 && !target_margin)
+    return fail(h, SEAM_ERR_BAD_ARG, "seam_shard_rank_count_prepared: null target_margin");
+  return rank_prepared_impl(h, q, Q, g, false, g16, cg, gstat, G, index_offset, target, target_margin, out_count,
+                            nullptr, stats, workspace, workspace_bytes, stream_, "seam_shard_rank_count_prepared");
+}
+
+int seam_shard_rank_count_prepared_g16(seam_handle* h, const float* q, int Q, const void* g16, const float* cg,
+                                       const float* gstat, int G, int index_offset, const int32_t* target,
+                                       const float* target_margin, int32_t* out_count, int32_t* stats,
+                                       void* workspace, size_t workspace_bytes, void* stream_) {
+  if (h && Q > 0 && !target_margin)
+    return fail(h, SEAM_ERR_BAD_ARG, "seam_shard_rank_count_prepared_g16: null target_margin");
+  return rank_prepared_impl(h, q, Q, g16, true, g16, cg, gstat, G, index_offset, target, target_margin, out_count,
+                            nullptr, stats, workspace, workspace_bytes, stream_, "seam_shard_rank_count_prepared_g16");
 }
 
 // ------------------------------------------------------------------------------ backward (f4)

@@ -575,6 +575,53 @@ class SeamEngine:
             return rank, margin, stats
         return rank, margin
 
+    def _shard_targets(self, q: torch.Tensor, target: torch.Tensor) -> torch.Tensor:
+        t32 = target.to(device=self.device, dtype=torch.int32).contiguous()
+        if t32.shape != (q.shape[0],):
+            raise ValueError("target must have one gallery row per query")
+        return t32
+
+    def target_margin(self, q: torch.Tensor, gallery: PreparedGallery, target: torch.Tensor) -> torch.Tensor:
+        """Margin d = l1 - l0 of each query's target for one shard of a sharded gallery (``seam_shard_target_margin``).
+        ``target`` holds GLOBAL gallery rows; the shard covers ``[gallery.index_offset, gallery.index_offset + G)``.
+        Returns ``(Q,)`` fp32: the margin where the target lies in this shard (bit for bit the one ``rank_of_target``
+        reports), ``-inf`` elsewhere, so that a MAX all-reduce over the shards gives every shard every margin."""
+        q = self._f32(q, "queries")
+        gallery = self._fresh(gallery)
+        t32 = self._shard_targets(q, target)
+        Q = q.shape[0]
+        margin = torch.empty((Q,), dtype=torch.float32, device=self.device)
+        fn, rows = ((self._lib.seam_shard_target_margin_g16, gallery.g16) if gallery.rows_f16
+                    else (self._lib.seam_shard_target_margin, gallery.g))
+        self._check(fn(self._h, q.data_ptr() if Q else 0, Q, rows.data_ptr(), gallery.G, int(gallery.index_offset),
+                       t32.data_ptr() if Q else 0, margin.data_ptr() if Q else 0, self._stream()))
+        return margin
+
+    def rank_count(self, q: torch.Tensor, gallery: PreparedGallery, target: torch.Tensor, target_margin: torch.Tensor,
+                   return_stats: bool = False):
+        """This shard's count of the gallery rows ranking before each query's target, given every target's margin
+        (``target_margin``: the MAX over the shards of ``target_margin``): ``seam_shard_rank_count_prepared``, the
+        tensor-core path of ``rank_of_target``.  Ties with the target are broken by global row, so the SUM of the
+        shards' counts is the rank over the whole gallery.  Returns ``(Q,)`` int32 [, stats (4) int32: stats[0] is the
+        number of queries this shard counted exhaustively]."""
+        q = self._f32(q, "queries")
+        gallery = self._fresh(gallery)
+        t32 = self._shard_targets(q, target)
+        m = self._f32(target_margin, "target_margin")
+        Q, G = q.shape[0], gallery.G
+        if m.shape != (Q,):
+            raise ValueError("target_margin must have one margin per query")
+        count = torch.empty((Q,), dtype=torch.int32, device=self.device)
+        stats = torch.zeros((4,), dtype=torch.int32, device=self.device) if return_stats else None
+        if Q > 0:
+            ws = self._workspace("score", int(self._lib.seam_rank_workspace_bytes(self._h, Q, G)))
+            fn, rows = ((self._lib.seam_shard_rank_count_prepared_g16, ()) if gallery.rows_f16
+                        else (self._lib.seam_shard_rank_count_prepared, (gallery.g.data_ptr(),)))
+            self._check(fn(self._h, q.data_ptr(), Q, *rows, gallery.g16.data_ptr(), gallery.cg.data_ptr(),
+                           gallery.gstat.data_ptr(), G, int(gallery.index_offset), t32.data_ptr(), m.data_ptr(),
+                           count.data_ptr(), _ptr(stats), ws.data_ptr(), ws.numel(), self._stream()))
+        return (count, stats) if return_stats else count
+
     def upload_tracks(self, seq_host: torch.Tensor, lo: int, hi: int) -> torch.Tensor:
         """Tracks [lo, hi) of a HOST ``x3_1_seq (1+Tmax, Q, 256)`` -> device ``(1+Tmax, hi-lo, 256)`` on the
         current stream with one pitched copy of the frame rows (row 0, the dummy frame, stays untouched).  fp32 or fp16:

@@ -196,6 +196,9 @@ class ShardedRetriever:
         self.rank = rank if rank is not None else (dist.get_rank(group) if dist.is_initialized() else 0)
         self.gallery = (gallery_shard if isinstance(gallery_shard, PreparedGallery)
                         else ops.prepare_gallery(gallery_shard, index_offset=shard_offset))
+        self.shard_offset = shard_offset
+        self.shard_rows = gallery_shard.G if isinstance(gallery_shard, PreparedGallery) else gallery_shard.shape[0]
+        self._gallery_rows: Optional[int] = None     # rows of the whole gallery, found on first use
 
     @classmethod
     def from_full_gallery(cls, ops, gallery: torch.Tensor, group=None):
@@ -226,6 +229,52 @@ class ShardedRetriever:
 
     def search(self, seq: torch.Tensor, mask: Optional[torch.Tensor], k: int = 20):
         return self.search_descriptors(self.aggregate(seq, mask), k)
+
+    def gallery_rows(self, device) -> int:
+        """Rows of the whole gallery (the end of the last shard): one MAX all-reduce on first use."""
+        if self._gallery_rows is None:
+            end = self.shard_offset + self.shard_rows
+            if self.world > 1:
+                t = torch.tensor([end], dtype=torch.int64, device=device)
+                dist.all_reduce(t, op=dist.ReduceOp.MAX, group=self.group)
+                end = int(t)
+            self._gallery_rows = end
+        return self._gallery_rows
+
+    def rank_of_target(self, q: torch.Tensor, target: torch.Tensor) -> Tuple[torch.Tensor, torch.Tensor]:
+        """Rank (0 = best) of the global gallery row ``target[i]`` for every query over the whole sharded gallery,
+        and its margin: ``(rank int32 (Q,), margin fp32 (Q,))``, the same integers and bits as ``rank_of_target`` on
+        the unsharded gallery (evaluate_movingfashion.py:268-269).  The shard holding the target computes its margin
+        (``-inf`` on the others), a MAX all-reduce hands it to every shard, each counts the rows ranking before it
+        (ties by global row) and a SUM all-reduce adds the counts.  ``q`` holds every query on every rank."""
+        dev = self.gallery.g.device if isinstance(self.gallery, PreparedGallery) else q.device
+        G = self.gallery_rows(dev)
+        if q.shape[0] and (int(target.min()) < 0 or int(target.max()) >= G):
+            raise ValueError(f"target index out of range [0, {G})")
+        if self.world == 1:
+            return self.ops.rank_of_target(q, self.gallery, target)
+        Q = q.shape[0]
+        if self.shard_rows == 0:          # nothing to compute here; the library takes no empty shard
+            margin = torch.full((Q,), -float("inf"), dtype=torch.float32, device=dev)
+        else:
+            margin = self.ops.target_margin(q, self.gallery, target)
+        dist.all_reduce(margin, op=dist.ReduceOp.MAX, group=self.group)
+        if self.shard_rows == 0:
+            rank = torch.zeros((Q,), dtype=torch.int32, device=dev)
+        else:
+            rank = self.ops.rank_count(q, self.gallery, target, margin)
+        dist.all_reduce(rank, op=dist.ReduceOp.SUM, group=self.group)
+        return rank, margin
+
+    def evaluate_aggregated(self, seq, mask, target: torch.Tensor,
+                            k_thresholds: Sequence[int] = K_THRESHOLDS) -> "RetrievalReport":
+        """``evaluate_aggregated`` over the sharded gallery: the same ``RetrievalReport`` as the single-GPU function
+        on the whole gallery, from the sharded aggregation, search and rank.  ``seq`` / ``mask`` hold all tracks."""
+        q = self.aggregate(seq, mask)
+        kmax = min(max(k_thresholds), 32)
+        sc, _, ix = self.search_descriptors(q, kmax)
+        ranks, _ = self.rank_of_target(q, target)
+        return _report(ranks, k_thresholds, sc, ix)
 
     def search_peer(self, seq: torch.Tensor, mask: Optional[torch.Tensor], peer: "PeerExchange", lens=None):
         """Same result as ``search`` with the exchange done by the kernels themselves (``PeerExchange``): three
@@ -410,9 +459,13 @@ def evaluate_aggregated(engine: SeamEngine, seq, mask, gallery: torch.Tensor, ta
     kmax = min(max(k_thresholds), 32)
     sc, mg, ix = engine.score_topk(q, gal, kmax)
     ranks, _ = engine.rank_of_target(q, gal, target)
+    return _report(ranks, k_thresholds, sc, ix)
+
+
+def _report(ranks: torch.Tensor, k_thresholds: Sequence[int], sc: torch.Tensor, ix: torch.Tensor) -> RetrievalReport:
     r = ranks.cpu()
     hits = [int((r < k).sum()) for k in k_thresholds]
-    n = max(1, q.shape[0])
+    n = max(1, ranks.shape[0])
     return RetrievalReport(ranks=ranks, hits=hits, accuracies=[h / n for h in hits], topk_scores=sc, topk_idx=ix)
 
 
