@@ -235,6 +235,10 @@ int seam_score_prob(seam_handle* h, const float* q, int Q, const float* g, int G
  *   rank_avg / rank_max (P) int32; products without frames get G. */
 int seam_rank_fused_distances(seam_handle* h, const float* frames, const int32_t* start, int P, const float* g, int G,
                               const int32_t* target, int32_t* rank_avg, int32_t* rank_max, void* stream);
+/* seam_rank_fused_distances for an fp16 gallery g16 (G,256), 16-byte aligned (else SEAM_ERR_UNSUPPORTED): the same
+ * ranks as the fp32 entry on the widened gallery, bit for bit (frames stay fp32). */
+int seam_rank_fused_distances_g16(seam_handle* h, const float* frames, const int32_t* start, int P, const void* g16,
+                                  int G, const int32_t* target, int32_t* rank_avg, int32_t* rank_max, void* stream);
 
 /* Rank of one designated gallery item per query (0 = best), the quantity the eval script
  * reads out of its full argsort: evaluate_movingfashion.py:268-269.
@@ -287,6 +291,34 @@ int seam_shard_rank_count_prepared_g16(seam_handle* h, const float* q, int Q, co
                                        const float* gstat, int G, int index_offset, const int32_t* target,
                                        const float* target_margin, int32_t* out_count, int32_t* stats,
                                        void* workspace, size_t workspace_bytes, void* stream);
+
+/* The "AVG & MAX DISTANCE" fusions (seam_rank_fused_distances) over a gallery split into shards, exactly: for global
+ * target t of product p and either fusion f (average or maximum of the frames' class-1 probabilities),
+ *   rank_p = sum over shards s of #{ j in s : (f_pj, j) ranks before (f_pt, t) }   (ties by GLOBAL row).
+ * Only the shard holding row t can compute f_pt, so a sharded fusion rank is three steps per shard, every shard
+ * holding ALL the frames (same frames / start on every shard):
+ *   1. seam_shard_fused_target: out_avg / out_max (P) fp32 = the target's fused average / maximum where global row
+ *      target[p] lies in [index_offset, index_offset + G), else -inf (and -inf for a product without frames) --
+ *      bit for bit the values seam_rank_fused_distances compares against;
+ *   2. all-reduce MAX of both over the shards (every shard now holds every target value);
+ *   3. seam_shard_rank_fused_distances: rank_avg / rank_max (P) int32 = this shard's counts against target_avg /
+ *      target_max (zero-filled here; a product without frames gets this shard's G, so the sum is the whole G);
+ * then an all-reduce SUM of the counts gives the unsharded ranks, integer for integer.
+ *   target (P) int32 GLOBAL gallery rows; index_offset >= 0 (else SEAM_ERR_BAD_ARG); target_avg / target_max must not
+ *   be null (SEAM_ERR_BAD_ARG); P == 0 is a no-op.  The _g16 forms take an fp16 shard, 16-byte aligned (else
+ *   SEAM_ERR_UNSUPPORTED), and give the fp32 forms' results on the widened rows. */
+int seam_shard_fused_target(seam_handle* h, const float* frames, const int32_t* start, int P, const float* g, int G,
+                            int index_offset, const int32_t* target, float* out_avg, float* out_max, void* stream);
+int seam_shard_fused_target_g16(seam_handle* h, const float* frames, const int32_t* start, int P, const void* g16,
+                                int G, int index_offset, const int32_t* target, float* out_avg, float* out_max,
+                                void* stream);
+int seam_shard_rank_fused_distances(seam_handle* h, const float* frames, const int32_t* start, int P, const float* g,
+                                    int G, int index_offset, const int32_t* target, const float* target_avg,
+                                    const float* target_max, int32_t* rank_avg, int32_t* rank_max, void* stream);
+int seam_shard_rank_fused_distances_g16(seam_handle* h, const float* frames, const int32_t* start, int P,
+                                        const void* g16, int G, int index_offset, const int32_t* target,
+                                        const float* target_avg, const float* target_max, int32_t* rank_avg,
+                                        int32_t* rank_max, void* stream);
 
 /* Merge N per-shard top-k lists (after the all-gather) into one: lists are (N,Q,k)
  * contiguous; entries with idx < 0 are invalid.  Same ordering contract as seam_score_topk.

@@ -12,12 +12,12 @@ from ._build import build as build_library, LIB_PATH                          # 
 from .engine import SeamEngine, PreparedGallery, get_engine                   # noqa: F401
 from .modules import NONLocalBlock1D, MatchPredictor, TemporalAggregationNLB  # noqa: F401
 from .retrieval import (ShardedRetriever, RetrievalReport, ProductReport, evaluate_aggregated,   # noqa: F401
-                        evaluate_products, evaluate_distance_fusions, self_distances, search, PeerExchange,
+                        evaluate_products, evaluate_distance_fusions, product_means, self_distances, search, PeerExchange,
                         search_host, HostTrackStream, bind_to_gpu_numa_node, shard_bounds, all_gather_rows, exchange_layout, K_THRESHOLDS)
 
 __all__ = [
     "SeamError", "SeamEngine", "PreparedGallery", "get_engine", "NONLocalBlock1D", "MatchPredictor",
     "TemporalAggregationNLB", "ShardedRetriever", "RetrievalReport", "evaluate_aggregated", "search",
-    "search_host", "HostTrackStream", "ProductReport", "evaluate_products", "evaluate_distance_fusions", "self_distances", "PeerExchange",
+    "search_host", "HostTrackStream", "ProductReport", "evaluate_products", "evaluate_distance_fusions", "product_means", "self_distances", "PeerExchange",
     "shard_bounds", "all_gather_rows", "exchange_layout", "bind_to_gpu_numa_node", "build_library", "load_library", "declared_symbols", "K_THRESHOLDS",
 ]

@@ -143,6 +143,16 @@ def _declare(lib: C.CDLL) -> None:
     lib.seam_score_prob.argtypes = [vp, vp, i32, vp, i32, vp, vp]
     lib.seam_rank_fused_distances.restype = i32
     lib.seam_rank_fused_distances.argtypes = [vp, vp, vp, i32, vp, i32, vp, vp, vp, vp]
+    lib.seam_rank_fused_distances_g16.restype = i32
+    lib.seam_rank_fused_distances_g16.argtypes = lib.seam_rank_fused_distances.argtypes
+    lib.seam_shard_fused_target.restype = i32
+    lib.seam_shard_fused_target.argtypes = [vp, vp, vp, i32, vp, i32, i32, vp, vp, vp, vp]
+    lib.seam_shard_fused_target_g16.restype = i32
+    lib.seam_shard_fused_target_g16.argtypes = lib.seam_shard_fused_target.argtypes
+    lib.seam_shard_rank_fused_distances.restype = i32
+    lib.seam_shard_rank_fused_distances.argtypes = [vp, vp, vp, i32, vp, i32, i32, vp, vp, vp, vp, vp, vp]
+    lib.seam_shard_rank_fused_distances_g16.restype = i32
+    lib.seam_shard_rank_fused_distances_g16.argtypes = lib.seam_shard_rank_fused_distances.argtypes
     lib.seam_rank_of_target.restype = i32
     lib.seam_rank_of_target.argtypes = [vp, vp, i32, vp, i32, vp, vp, vp, vp]
     lib.seam_rank_workspace_bytes.restype = sz

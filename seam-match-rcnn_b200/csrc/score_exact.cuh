@@ -720,15 +720,58 @@ __global__ void __launch_bounds__(256) dense_logits_kernel(const float* __restri
 struct FusedDistParams {
   const float* frames;
   const int32_t* start;
-  const float* g;
+  const void* g;             // Row (float / __half) rows
   const int32_t* target;
   const float* fold;
   int P, G;
   int32_t* rank_avg;
   int32_t* rank_max;
+  // EXT (one shard of a sharded gallery): target[] holds global rows, row j of this shard is global row
+  // j + index_offset, and the target's fused values are given (its row may live on another GPU)
+  int index_offset;
+  const float* target_avg;
+  const float* target_max;
 };
 constexpr int FD_ROWS = 1024, FD_FRAMES = 16;
 
+// One gallery row (gs) against one chunk of a product's frames (f[0 .. nc), nc <= FD_FRAMES): sqdiff_dot2 over 4
+// frames per treduce<8>, the class-1 probabilities summed and maximised frame by frame, then folded into the row's
+// running sum / maximum (lane 0's).  Every kernel that needs a row's fused values calls this chunk by chunk in
+// ascending order, so a row's average acc_sum * (1/nf) and maximum have the same bits whichever kernel, CTA or
+// shard computes them.
+__device__ __forceinline__ void fused_row_chunk(const float (*f)[256], int nc, const Slice& gs, const Slice& w0,
+                                                const Slice& w1, float b0, float b1, int lane, float& acc_sum,
+                                                float& acc_max) {
+  float sum = 0.f, mx = -INFINITY;
+  for (int fb = 0; fb < nc; fb += 4) {
+    float part[8];
+#pragma unroll
+    for (int u = 0; u < 4; ++u) {
+      const Slice fr = load_slice(&f[min(fb + u, nc - 1)][0], lane);
+      sqdiff_dot2(fr, gs, w0, w1, part[2 * u], part[2 * u + 1]);
+    }
+    const float tot = ptx::treduce<8>(part, lane);   // lane l: total of part[l % 8]
+#pragma unroll
+    for (int u = 0; u < 4; ++u) {
+      const float l0 = __shfl_sync(ptx::FULL_MASK, tot, 2 * u) + b0;
+      const float l1 = __shfl_sync(ptx::FULL_MASK, tot, 2 * u + 1) + b1;
+      if (fb + u < nc) {
+        const float pr = softmax1(l0, l1);
+        sum += pr;
+        mx = fmaxf(mx, pr);
+      }
+    }
+  }
+  if (lane == 0) {
+    acc_sum += sum;
+    acc_max = fmaxf(acc_max, mx);
+  }
+}
+
+// EXT: this shard's count against target_avg[prod] / target_max[prod] (no target row is read); ties are decided
+// against the target as a row of this shard (j + index_offset < t  <=>  j < t - index_offset), so the SUM of the
+// shards' counts is the rank over the whole gallery.  A product without frames gets this shard's G.
+template <typename Row, bool EXT>
 __global__ void __launch_bounds__(256) fused_dist_rank_kernel(const FusedDistParams p) {
   __shared__ __align__(16) float fs[FD_FRAMES][256];
   __shared__ float acc_sum[FD_ROWS + 1], acc_max[FD_ROWS + 1];     // last slot: the target item
@@ -744,7 +787,8 @@ __global__ void __launch_bounds__(256) fused_dist_rank_kernel(const FusedDistPar
     return;
   }
   const int rows = min(FD_ROWS, p.G - j0);
-  const int tj = p.target[prod];
+  const int tj = EXT ? p.target[prod] - p.index_offset : p.target[prod];
+  const Row* g = static_cast<const Row*>(p.g);
   for (int i = threadIdx.x; i <= FD_ROWS; i += 256) {
     acc_sum[i] = 0.f;
     acc_max[i] = -INFINITY;
@@ -753,45 +797,31 @@ __global__ void __launch_bounds__(256) fused_dist_rank_kernel(const FusedDistPar
   const Slice w0 = load_slice(p.fold + Fold::LAST_W, lane);
   const Slice w1 = load_slice(p.fold + Fold::LAST_W + 256, lane);
   const float b0 = p.fold[Fold::CONSTS + 5], b1 = p.fold[Fold::CONSTS + 6];
+  const int last = EXT ? rows - 1 : rows;              // r == rows: the target item (not with EXT)
   for (int c0 = 0; c0 < nf; c0 += FD_FRAMES) {
     const int nc = min(FD_FRAMES, nf - c0);
     __syncthreads();                                   // previous chunk consumed (and the accumulators initialised)
     for (int e = threadIdx.x; e < nc * 64; e += 256)
       reinterpret_cast<float4*>(&fs[0][0])[e] = reinterpret_cast<const float4*>(p.frames + (size_t)(f0 + c0) * 256)[e];
     __syncthreads();
-    for (int r = warp; r <= rows; r += 8) {            // r == rows: the target item
+    for (int r = warp; r <= last; r += 8) {
       const int j = r < rows ? j0 + r : tj;
       const int slot = r < rows ? r : FD_ROWS;
-      const Slice gs = load_slice(p.g + (size_t)j * 256, lane);
-      float sum = 0.f, mx = -INFINITY;
-      for (int fb = 0; fb < nc; fb += 4) {
-        float part[8];
-#pragma unroll
-        for (int u = 0; u < 4; ++u) {
-          const Slice fr = load_slice(&fs[min(fb + u, nc - 1)][0], lane);
-          sqdiff_dot2(fr, gs, w0, w1, part[2 * u], part[2 * u + 1]);
-        }
-        const float tot = ptx::treduce<8>(part, lane);   // lane l: total of part[l % 8]
-#pragma unroll
-        for (int u = 0; u < 4; ++u) {
-          const float l0 = __shfl_sync(ptx::FULL_MASK, tot, 2 * u) + b0;
-          const float l1 = __shfl_sync(ptx::FULL_MASK, tot, 2 * u + 1) + b1;
-          if (fb + u < nc) {
-            const float pr = softmax1(l0, l1);
-            sum += pr;
-            mx = fmaxf(mx, pr);
-          }
-        }
-      }
-      if (lane == 0) {                                 // this warp owns the slot in this pass
-        acc_sum[slot] += sum;
-        acc_max[slot] = fmaxf(acc_max[slot], mx);
-      }
+      const Slice gs = load_slice(g + (size_t)j * 256, lane);
+      // this warp owns the slot in this pass
+      fused_row_chunk(fs, nc, gs, w0, w1, b0, b1, lane, acc_sum[slot], acc_max[slot]);
     }
   }
   __syncthreads();
   const float inv = 1.f / (float)nf;
-  const float tavg = acc_sum[FD_ROWS] * inv, tmax = acc_max[FD_ROWS];
+  float tavg, tmax;
+  if (EXT) {
+    tavg = p.target_avg[prod];
+    tmax = p.target_max[prod];
+  } else {
+    tavg = acc_sum[FD_ROWS] * inv;
+    tmax = acc_max[FD_ROWS];
+  }
   int ca = 0, cm = 0;
   for (int i = threadIdx.x; i < rows; i += 256) {
     const int j = j0 + i;
@@ -809,6 +839,40 @@ __global__ void __launch_bounds__(256) fused_dist_rank_kernel(const FusedDistPar
   if (threadIdx.x == 0) {
     atomicAdd(p.rank_avg + prod, cnt_s[0]);
     atomicAdd(p.rank_max + prod, cnt_s[1]);
+  }
+}
+
+// warp per product: the fused average / maximum of the target item when global row target[prod] lies in this shard
+// [index_offset, index_offset + G) -- fused_row_chunk over the product's frames, chunk by chunk as
+// fused_dist_rank_kernel does, so the bits are those the unsharded kernel compares against -- else, and for products
+// without frames, -inf (so that a MAX over the shards is exact).
+template <typename Row>
+__global__ void __launch_bounds__(256) fused_target_kernel(const FusedDistParams p, float* __restrict__ out_avg,
+                                                           float* __restrict__ out_max) {
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  const int prod = blockIdx.x * 8 + warp;
+  if (prod >= p.P) return;
+  const int f0 = p.start[prod], nf = p.start[prod + 1] - f0;
+  const long long t = (long long)p.target[prod] - p.index_offset;
+  if (nf <= 0 || t < 0 || t >= p.G) {
+    if (lane == 0) {
+      out_avg[prod] = -INFINITY;
+      out_max[prod] = -INFINITY;
+    }
+    return;
+  }
+  const Slice w0 = load_slice(p.fold + Fold::LAST_W, lane);
+  const Slice w1 = load_slice(p.fold + Fold::LAST_W + 256, lane);
+  const float b0 = p.fold[Fold::CONSTS + 5], b1 = p.fold[Fold::CONSTS + 6];
+  const Slice gs = load_slice(static_cast<const Row*>(p.g) + (size_t)t * 256, lane);
+  float acc_sum = 0.f, acc_max = -INFINITY;
+  for (int c0 = 0; c0 < nf; c0 += FD_FRAMES)
+    fused_row_chunk(reinterpret_cast<const float(*)[256]>(p.frames + (size_t)(f0 + c0) * 256), min(FD_FRAMES, nf - c0),
+                    gs, w0, w1, b0, b1, lane, acc_sum, acc_max);
+  if (lane == 0) {
+    const float inv = 1.f / (float)nf;
+    out_avg[prod] = acc_sum * inv;
+    out_max[prod] = acc_max;
   }
 }
 

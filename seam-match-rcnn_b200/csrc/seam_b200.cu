@@ -1097,18 +1097,21 @@ int seam_score_prob(seam_handle* h, const float* q, int Q, const float* g, int G
   return SEAM_OK;
 }
 
-int seam_rank_fused_distances(seam_handle* h, const float* frames, const int32_t* start, int P, const float* g, int G,
-                              const int32_t* target, int32_t* rank_avg, int32_t* rank_max, void* stream_) {
+// rows / rows_f16 as in score_topk_impl.  target_avg null: the whole gallery (index_offset 0); else one shard of it,
+// counting against the given target values (target[] holds global rows).
+static int fused_rank_impl(seam_handle* h, const float* frames, const int32_t* start, int P, const void* rows,
+                           bool rows_f16, int G, int index_offset, const int32_t* target, const float* target_avg,
+                           const float* target_max, int32_t* rank_avg, int32_t* rank_max, void* stream_,
+                           const char* who) {
   if (!h) return SEAM_ERR_BAD_ARG;
-  if (!h->have_scorer) return fail(h, SEAM_ERR_STATE, "seam_rank_fused_distances: scorer weights not loaded");
-  if (P < 0 || G <= 0) return fail(h, SEAM_ERR_BAD_ARG, "seam_rank_fused_distances: bad size");
+  if (!h->have_scorer) return fail(h, SEAM_ERR_STATE, "%s: scorer weights not loaded", who);
+  if (P < 0 || G <= 0) return fail(h, SEAM_ERR_BAD_ARG, "%s: bad size", who);
+  if (index_offset < 0) return fail(h, SEAM_ERR_BAD_ARG, "%s: negative index_offset %d", who, index_offset);
   if (P == 0) return SEAM_OK;
-  if (!start || !g || !target || !rank_avg || !rank_max)
-    return fail(h, SEAM_ERR_BAD_ARG, "seam_rank_fused_distances: null pointer");
-  if ((frames && !aligned16(frames)) || !aligned16(g))
-    return fail(h, SEAM_ERR_UNSUPPORTED, "seam_rank_fused_distances: 16-byte alignment");
+  if (!start || !rows || !target || !rank_avg || !rank_max) return fail(h, SEAM_ERR_BAD_ARG, "%s: null pointer", who);
+  if ((frames && !aligned16(frames)) || !aligned16(rows)) return fail(h, SEAM_ERR_UNSUPPORTED, "%s: 16-byte alignment", who);
   const int chunks = (G + exact::FD_ROWS - 1) / exact::FD_ROWS;
-  if (chunks > 65535) return fail(h, SEAM_ERR_UNSUPPORTED, "seam_rank_fused_distances: G too large");
+  if (chunks > 65535) return fail(h, SEAM_ERR_UNSUPPORTED, "%s: G too large", who);
   cudaStream_t stream = static_cast<cudaStream_t>(stream_);
   DeviceGuard guard(h->device);
   SEAM_CUDA(h, cudaMemsetAsync(rank_avg, 0, (size_t)P * 4, stream));
@@ -1116,16 +1119,102 @@ int seam_rank_fused_distances(seam_handle* h, const float* frames, const int32_t
   exact::FusedDistParams fp;
   fp.frames = frames;
   fp.start = start;
-  fp.g = g;
+  fp.g = rows;
   fp.target = target;
   fp.fold = h->fold;
   fp.P = P;
   fp.G = G;
   fp.rank_avg = rank_avg;
   fp.rank_max = rank_max;
-  exact::fused_dist_rank_kernel<<<dim3((unsigned)P, (unsigned)chunks), 256, 0, stream>>>(fp);
+  fp.index_offset = index_offset;
+  fp.target_avg = target_avg;
+  fp.target_max = target_max;
+  const dim3 grid((unsigned)P, (unsigned)chunks);
+  if (target_avg) {
+    if (rows_f16) exact::fused_dist_rank_kernel<__half, true><<<grid, 256, 0, stream>>>(fp);
+    else exact::fused_dist_rank_kernel<float, true><<<grid, 256, 0, stream>>>(fp);
+  } else {
+    if (rows_f16) exact::fused_dist_rank_kernel<__half, false><<<grid, 256, 0, stream>>>(fp);
+    else exact::fused_dist_rank_kernel<float, false><<<grid, 256, 0, stream>>>(fp);
+  }
   SEAM_LAUNCHED(h, "fused_dist_rank_kernel");
   return SEAM_OK;
+}
+
+int seam_rank_fused_distances(seam_handle* h, const float* frames, const int32_t* start, int P, const float* g, int G,
+                              const int32_t* target, int32_t* rank_avg, int32_t* rank_max, void* stream_) {
+  return fused_rank_impl(h, frames, start, P, g, false, G, 0, target, nullptr, nullptr, rank_avg, rank_max, stream_,
+                         "seam_rank_fused_distances");
+}
+
+int seam_rank_fused_distances_g16(seam_handle* h, const float* frames, const int32_t* start, int P, const void* g16,
+                                  int G, const int32_t* target, int32_t* rank_avg, int32_t* rank_max, void* stream_) {
+  return fused_rank_impl(h, frames, start, P, g16, true, G, 0, target, nullptr, nullptr, rank_avg, rank_max, stream_,
+                         "seam_rank_fused_distances_g16");
+}
+
+// ------------------------------------------------------------------------------ fusions over a sharded gallery
+// rank_p = sum over shards s of #{ j in s : (f_pj, j) ranks before (f_pt, t) } for either fusion f: the owner of row t
+// computes the target's fused values (-inf elsewhere, so a MAX all-reduce delivers them to every shard), every shard
+// counts against them, and the counts are summed.
+static int shard_fused_target_impl(seam_handle* h, const float* frames, const int32_t* start, int P, const void* rows,
+                                   bool rows_f16, int G, int index_offset, const int32_t* target, float* out_avg,
+                                   float* out_max, void* stream_, const char* who) {
+  if (!h) return SEAM_ERR_BAD_ARG;
+  if (!h->have_scorer) return fail(h, SEAM_ERR_STATE, "%s: scorer weights not loaded", who);
+  if (P < 0 || G <= 0) return fail(h, SEAM_ERR_BAD_ARG, "%s: bad size", who);
+  if (index_offset < 0) return fail(h, SEAM_ERR_BAD_ARG, "%s: negative index_offset %d", who, index_offset);
+  if (P == 0) return SEAM_OK;
+  if (!start || !rows || !target || !out_avg || !out_max) return fail(h, SEAM_ERR_BAD_ARG, "%s: null pointer", who);
+  if ((frames && !aligned16(frames)) || !aligned16(rows)) return fail(h, SEAM_ERR_UNSUPPORTED, "%s: 16-byte alignment", who);
+  cudaStream_t stream = static_cast<cudaStream_t>(stream_);
+  DeviceGuard guard(h->device);
+  exact::FusedDistParams fp;
+  memset(&fp, 0, sizeof(fp));
+  fp.frames = frames;
+  fp.start = start;
+  fp.g = rows;
+  fp.target = target;
+  fp.fold = h->fold;
+  fp.P = P;
+  fp.G = G;
+  fp.index_offset = index_offset;
+  if (rows_f16) exact::fused_target_kernel<__half><<<(P + 7) / 8, 256, 0, stream>>>(fp, out_avg, out_max);
+  else exact::fused_target_kernel<float><<<(P + 7) / 8, 256, 0, stream>>>(fp, out_avg, out_max);
+  SEAM_LAUNCHED(h, "fused_target_kernel");
+  return SEAM_OK;
+}
+
+int seam_shard_fused_target(seam_handle* h, const float* frames, const int32_t* start, int P, const float* g, int G,
+                            int index_offset, const int32_t* target, float* out_avg, float* out_max, void* stream_) {
+  return shard_fused_target_impl(h, frames, start, P, g, false, G, index_offset, target, out_avg, out_max, stream_,
+                                 "seam_shard_fused_target");
+}
+
+int seam_shard_fused_target_g16(seam_handle* h, const float* frames, const int32_t* start, int P, const void* g16,
+                                int G, int index_offset, const int32_t* target, float* out_avg, float* out_max,
+                                void* stream_) {
+  return shard_fused_target_impl(h, frames, start, P, g16, true, G, index_offset, target, out_avg, out_max, stream_,
+                                 "seam_shard_fused_target_g16");
+}
+
+int seam_shard_rank_fused_distances(seam_handle* h, const float* frames, const int32_t* start, int P, const float* g,
+                                    int G, int index_offset, const int32_t* target, const float* target_avg,
+                                    const float* target_max, int32_t* rank_avg, int32_t* rank_max, void* stream_) {
+  if (h && P > 0 && (!target_avg || !target_max))
+    return fail(h, SEAM_ERR_BAD_ARG, "seam_shard_rank_fused_distances: null target_avg / target_max");
+  return fused_rank_impl(h, frames, start, P, g, false, G, index_offset, target, target_avg, target_max, rank_avg,
+                         rank_max, stream_, "seam_shard_rank_fused_distances");
+}
+
+int seam_shard_rank_fused_distances_g16(seam_handle* h, const float* frames, const int32_t* start, int P,
+                                        const void* g16, int G, int index_offset, const int32_t* target,
+                                        const float* target_avg, const float* target_max, int32_t* rank_avg,
+                                        int32_t* rank_max, void* stream_) {
+  if (h && P > 0 && (!target_avg || !target_max))
+    return fail(h, SEAM_ERR_BAD_ARG, "seam_shard_rank_fused_distances_g16: null target_avg / target_max");
+  return fused_rank_impl(h, frames, start, P, g16, true, G, index_offset, target, target_avg, target_max, rank_avg,
+                         rank_max, stream_, "seam_shard_rank_fused_distances_g16");
 }
 
 int seam_rank_of_target(seam_handle* h, const float* q, int Q, const float* g, int G, const int32_t* target,

@@ -522,22 +522,77 @@ class SeamEngine:
                                               out.data_ptr(), self._stream()))
         return out
 
-    def rank_fused_distances(self, frames: torch.Tensor, start: torch.Tensor, g: torch.Tensor, target: torch.Tensor):
-        """Ranks of the true shop items under the per-product average / maximum of the frames' class-1
-        probabilities (evaluate_movingfashion.py:294-316).  ``frames (N,256)`` sorted by product, ``start (P+1)``
-        CSR offsets, ``target (P)``.  Returns ``(rank_avg, rank_max)`` int32 ``(P,)``; no host synchronisation."""
-        frames, g = self._f32(frames, "frames"), self._f32(g, "gallery")
+    def _rows(self, g: torch.Tensor) -> torch.Tensor:
+        """Gallery rows for the direct-form kernels: an fp16 ``g`` stays fp16 (used in place when it is on this device,
+        contiguous and 16-byte aligned, else copied once, as ``prepare_gallery`` does); other dtypes become fp32."""
+        if g.dim() != 2 or g.shape[1] != D_MODEL:
+            raise ValueError(f"gallery must be (G,256), got {tuple(g.shape)}")
+        if g.dtype == torch.float16:
+            g = g.to(self.device)
+            if not g.is_contiguous() or g.data_ptr() % 16:
+                g = g.clone(memory_format=torch.contiguous_format)
+            return g
+        return self._f32(g, "gallery")
+
+    def _fused_args(self, frames: torch.Tensor, start: torch.Tensor, g: torch.Tensor, target: torch.Tensor):
+        frames, g = self._f32(frames, "frames"), self._rows(g)
         s32 = start.to(device=self.device, dtype=torch.int32).contiguous()
         t32 = target.to(device=self.device, dtype=torch.int32).contiguous()
         P = int(t32.shape[0])
         if s32.shape != (P + 1,):
             raise ValueError("start must hold P+1 offsets")
+        return frames, s32, g, t32, P
+
+    def rank_fused_distances(self, frames: torch.Tensor, start: torch.Tensor, g: torch.Tensor, target: torch.Tensor):
+        """Ranks of the true shop items under the per-product average / maximum of the frames' class-1
+        probabilities (evaluate_movingfashion.py:294-316).  ``frames (N,256)`` sorted by product, ``start (P+1)``
+        CSR offsets, ``target (P)``.  An fp16 gallery ``g`` is read as fp16 (``seam_rank_fused_distances_g16``: the
+        ranks of ``g.float()``, no fp32 copy).  Returns ``(rank_avg, rank_max)`` int32 ``(P,)``; no host
+        synchronisation."""
+        frames, s32, g, t32, P = self._fused_args(frames, start, g, target)
         ra = torch.empty((P,), dtype=torch.int32, device=self.device)
         rm = torch.empty((P,), dtype=torch.int32, device=self.device)
-        self._check(self._lib.seam_rank_fused_distances(self._h, frames.data_ptr() if frames.numel() else 0,
-                                                        s32.data_ptr(), P, g.data_ptr(), g.shape[0], t32.data_ptr(),
-                                                        ra.data_ptr(), rm.data_ptr(), self._stream()))
+        fn = self._lib.seam_rank_fused_distances_g16 if g.dtype == torch.float16 else self._lib.seam_rank_fused_distances
+        self._check(fn(self._h, frames.data_ptr() if frames.numel() else 0, s32.data_ptr(), P, g.data_ptr(), g.shape[0],
+                       t32.data_ptr(), ra.data_ptr(), rm.data_ptr(), self._stream()))
         return ra, rm
+
+    def fused_target(self, frames: torch.Tensor, start: torch.Tensor, g: torch.Tensor, index_offset: int,
+                     target: torch.Tensor) -> Tuple[torch.Tensor, torch.Tensor]:
+        """The target item's fused average / maximum for one shard ``g`` (global rows ``[index_offset,
+        index_offset + G)``) of a sharded gallery (``seam_shard_fused_target``); ``target`` holds GLOBAL rows.
+        Returns ``(avg, max)`` fp32 ``(P,)``: the values ``rank_fused_distances`` compares against, bit for bit, where
+        the target lies in this shard and the product has frames, ``-inf`` elsewhere, so that a MAX all-reduce over
+        the shards gives every shard every target value."""
+        frames, s32, g, t32, P = self._fused_args(frames, start, g, target)
+        avg = torch.empty((P,), dtype=torch.float32, device=self.device)
+        mx = torch.empty((P,), dtype=torch.float32, device=self.device)
+        fn = self._lib.seam_shard_fused_target_g16 if g.dtype == torch.float16 else self._lib.seam_shard_fused_target
+        self._check(fn(self._h, frames.data_ptr() if frames.numel() else 0, s32.data_ptr(), P, g.data_ptr(), g.shape[0],
+                       int(index_offset), t32.data_ptr(), avg.data_ptr() if P else 0, mx.data_ptr() if P else 0,
+                       self._stream()))
+        return avg, mx
+
+    def fused_rank_count(self, frames: torch.Tensor, start: torch.Tensor, g: torch.Tensor, index_offset: int,
+                         target: torch.Tensor, target_avg: torch.Tensor,
+                         target_max: torch.Tensor) -> Tuple[torch.Tensor, torch.Tensor]:
+        """This shard's counts of the rows ranking before each product's target under the two fusions, given every
+        target's values (the MAX over the shards of ``fused_target``): ``seam_shard_rank_fused_distances``.  Ties
+        with the target are broken by global row and a product without frames counts this shard's G, so the SUM of
+        the shards' counts is ``rank_fused_distances`` on the whole gallery.  Returns ``(count_avg, count_max)``
+        int32 ``(P,)``."""
+        frames, s32, g, t32, P = self._fused_args(frames, start, g, target)
+        ta, tm = self._f32(target_avg, "target_avg"), self._f32(target_max, "target_max")
+        if ta.shape != (P,) or tm.shape != (P,):
+            raise ValueError("target_avg / target_max must hold one value per product")
+        ca = torch.empty((P,), dtype=torch.int32, device=self.device)
+        cm = torch.empty((P,), dtype=torch.int32, device=self.device)
+        fn = (self._lib.seam_shard_rank_fused_distances_g16 if g.dtype == torch.float16
+              else self._lib.seam_shard_rank_fused_distances)
+        self._check(fn(self._h, frames.data_ptr() if frames.numel() else 0, s32.data_ptr(), P, g.data_ptr(), g.shape[0],
+                       int(index_offset), t32.data_ptr(), ta.data_ptr() if P else 0, tm.data_ptr() if P else 0,
+                       ca.data_ptr() if P else 0, cm.data_ptr() if P else 0, self._stream()))
+        return ca, cm
 
     def rank_of_target(self, q: torch.Tensor, g, target: torch.Tensor, return_stats: bool = False):
         """Rank (0 = best) of gallery row target[i] for query i: evaluate_movingfashion.py:268-269.

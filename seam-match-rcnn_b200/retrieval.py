@@ -247,24 +247,98 @@ class ShardedRetriever:
         the unsharded gallery (evaluate_movingfashion.py:268-269).  The shard holding the target computes its margin
         (``-inf`` on the others), a MAX all-reduce hands it to every shard, each counts the rows ranking before it
         (ties by global row) and a SUM all-reduce adds the counts.  ``q`` holds every query on every rank."""
-        dev = self.gallery.g.device if isinstance(self.gallery, PreparedGallery) else q.device
+        return self._rank_over_shards(q, self.gallery, target)
+
+    def _rank_over_shards(self, q: torch.Tensor, shard, target: torch.Tensor) -> Tuple[torch.Tensor, torch.Tensor]:
+        """``rank_of_target``'s protocol on any prepared shard covering this rank's global rows (``shard`` may be None
+        for a rank without rows): target margin, MAX all-reduce, count, SUM all-reduce."""
+        dev = shard.g.device if isinstance(shard, PreparedGallery) else q.device
         G = self.gallery_rows(dev)
         if q.shape[0] and (int(target.min()) < 0 or int(target.max()) >= G):
             raise ValueError(f"target index out of range [0, {G})")
         if self.world == 1:
-            return self.ops.rank_of_target(q, self.gallery, target)
+            return self.ops.rank_of_target(q, shard, target)
         Q = q.shape[0]
         if self.shard_rows == 0:          # nothing to compute here; the library takes no empty shard
             margin = torch.full((Q,), -float("inf"), dtype=torch.float32, device=dev)
         else:
-            margin = self.ops.target_margin(q, self.gallery, target)
+            margin = self.ops.target_margin(q, shard, target)
         dist.all_reduce(margin, op=dist.ReduceOp.MAX, group=self.group)
         if self.shard_rows == 0:
             rank = torch.zeros((Q,), dtype=torch.int32, device=dev)
         else:
-            rank = self.ops.rank_count(q, self.gallery, target, margin)
+            rank = self.ops.rank_count(q, shard, target, margin)
         dist.all_reduce(rank, op=dist.ReduceOp.SUM, group=self.group)
         return rank, margin
+
+    def _check_shop_shard(self, shop_desc_shard: torch.Tensor) -> None:
+        if shop_desc_shard.dim() != 2 or shop_desc_shard.shape[0] != self.shard_rows:
+            raise ValueError(f"shop_desc_shard must hold this rank's {self.shard_rows} gallery rows "
+                             f"[{self.shard_offset}, {self.shard_offset + self.shard_rows}), "
+                             f"got {tuple(shop_desc_shard.shape)}")
+
+    def evaluate_products(self, frame_desc: torch.Tensor, frame_product: torch.Tensor, shop_desc_shard: torch.Tensor,
+                          target: torch.Tensor, frame_last: Tuple[torch.Tensor, torch.Tensor], seq: torch.Tensor,
+                          mask: Optional[torch.Tensor], aggr_last: Tuple[torch.Tensor, torch.Tensor],
+                          k_thresholds: Sequence[int] = K_THRESHOLDS) -> "ProductReport":
+        """``evaluate_products`` over the sharded gallery: the same ``ProductReport`` as the single-GPU function on the
+        whole gallery.  ``shop_desc_shard`` is this rank's rows of the frame scorer's gallery (the same global rows as
+        ``self.gallery``, which is the aggregated-descriptor gallery); every rank passes all frames, products, targets
+        and tracks.  Rows 0 and 2 are ranked with ``rank_of_target``'s protocol on ``shop_desc_shard`` under
+        ``frame_last``, row 1 is derived from row 0, row 3 is ``evaluate_aggregated``.  The average descriptors of
+        row 2 are summed frame by frame in a fixed order, so every rank scores the same bits."""
+        self._check_shop_shard(shop_desc_shard)
+        dev = self.ops.device
+        frame_desc = frame_desc.to(dev, torch.float32)
+        fp = frame_product.to(dev, torch.int64)
+        target = target.to(dev, torch.int64)
+        P = int(target.shape[0])
+        ks = list(k_thresholds)
+        big = torch.iinfo(torch.int32).max
+        with self.ops.scorer(*frame_last):                  # the caller's scorer is put back on exit
+            shop = (self.ops.prepare_gallery(shop_desc_shard, index_offset=self.shard_offset)
+                    if self.shard_rows > 0 else None)
+            fr, _ = self._rank_over_shards(frame_desc, shop, target[fp])
+            best = torch.full((P,), big, dtype=torch.int32, device=dev).scatter_reduce(0, fp, fr, "amin")
+            avg, has = product_means(frame_desc, fp, P)
+            ar, _ = self._rank_over_shards(avg, shop, target)
+            ar = torch.where(has, ar, torch.full_like(ar, big))
+        with self.ops.scorer(*aggr_last):
+            rep = self.evaluate_aggregated(seq, mask, target, ks)
+        return _product_report(fr, best, ar, rep.ranks, P, ks, dev)
+
+    def evaluate_distance_fusions(self, frame_desc: torch.Tensor, frame_product: torch.Tensor,
+                                  shop_desc_shard: torch.Tensor, target: torch.Tensor,
+                                  frame_last: Tuple[torch.Tensor, torch.Tensor],
+                                  k_thresholds: Sequence[int] = K_THRESHOLDS):
+        """``evaluate_distance_fusions`` over the sharded gallery: the same ``(ranks (2,P) int64, hits)``.
+        ``shop_desc_shard`` is this rank's rows of the frame scorer's gallery (fp32 or fp16, the same global rows as
+        ``self.gallery``); every rank passes all frames, products and targets.  The shard holding each product's target
+        computes its fused average / maximum (``-inf`` on the others), a MAX all-reduce hands them to every shard, each
+        counts its rows ranking before them (ties by global row) and a SUM all-reduce adds the counts."""
+        self._check_shop_shard(shop_desc_shard)
+        if self.world == 1:
+            return evaluate_distance_fusions(self.ops, frame_desc, frame_product, shop_desc_shard, target, frame_last,
+                                             k_thresholds)
+        dev = self.ops.device
+        P = int(target.shape[0])
+        G = self.gallery_rows(dev)
+        if P and (int(target.min()) < 0 or int(target.max()) >= G):
+            raise ValueError(f"target index out of range [0, {G})")
+        frames, start = _group_frames(frame_desc, frame_product, P, dev)
+        with self.ops.scorer(*frame_last):                  # the caller's scorer is put back on exit
+            if self.shard_rows == 0:      # nothing to compute here; the library takes no empty shard
+                tv = torch.full((2, P), -float("inf"), dtype=torch.float32, device=dev)
+            else:
+                tv = torch.stack(self.ops.fused_target(frames, start, shop_desc_shard, self.shard_offset, target))
+            dist.all_reduce(tv, op=dist.ReduceOp.MAX, group=self.group)
+            if self.shard_rows == 0:
+                counts = torch.zeros((2, P), dtype=torch.int32, device=dev)
+            else:
+                counts = torch.stack(self.ops.fused_rank_count(frames, start, shop_desc_shard, self.shard_offset,
+                                                               target, tv[0], tv[1]))
+            dist.all_reduce(counts, op=dist.ReduceOp.SUM, group=self.group)
+        return _fusion_hits(counts.to(torch.int64), k_thresholds, dev)
 
     def evaluate_aggregated(self, seq, mask, target: torch.Tensor,
                             k_thresholds: Sequence[int] = K_THRESHOLDS) -> "RetrievalReport":
@@ -526,17 +600,38 @@ def evaluate_products(engine: SeamEngine, frame_desc: torch.Tensor, frame_produc
 
     with engine.scorer(*aggr_last):
         rep = evaluate_aggregated(engine, seq, mask, shop_aggr, target, ks)
+    return _product_report(fr, best, ar, rep.ranks, P, ks, dev)
 
+
+def _product_report(fr: torch.Tensor, best: torch.Tensor, ar: torch.Tensor, aggr_ranks: torch.Tensor, P: int,
+                    ks: Sequence[int], dev) -> ProductReport:
     def row(r, n):
         return [float((r < k).sum()) / max(1, n) for k in ks]
 
     n_frames = int(fr.shape[0])
-    perf = torch.tensor([row(fr, n_frames), row(best, P), row(ar, P), row(rep.ranks, P)], dtype=torch.float32) * 100.0
+    perf = torch.tensor([row(fr, n_frames), row(best, P), row(ar, P), row(aggr_ranks, P)], dtype=torch.float32) * 100.0
     frf = fr.float()
     qs = torch.quantile(frf, torch.tensor([0.25, 0.5, 0.75], device=dev)) if n_frames else torch.zeros(3)
     return ProductReport(perf=perf, ret=(perf[0, 0].item() / 100.0, perf[2, 0].item() / 100.0, perf[3, 0].item() / 100.0),
-                         frame_ranks=fr, product_ranks=torch.stack([best, ar, rep.ranks.to(torch.int32)]),
+                         frame_ranks=fr, product_ranks=torch.stack([best, ar, aggr_ranks.to(torch.int32)]),
                          rank_median=float(qs[1]), rank_q1=float(qs[0]), rank_q3=float(qs[2]))
+
+
+def product_means(frame_desc: torch.Tensor, frame_product: torch.Tensor, P: int) -> Tuple[torch.Tensor, torch.Tensor]:
+    """Average descriptor of each product's frames (evaluate_movingfashion.py:279-292) with a fixed summation order:
+    the frames are grouped by product (stable), and the k-th frame of every product is added in step k, so the bits
+    depend on the inputs only (``index_add_`` adds with atomics in an unspecified order).  The sharded report needs
+    that: every rank must score the same average descriptors.  Returns ``(avg (P,256) fp32, has (P,) bool)``; a
+    product without frames gets zeros and ``has = False``."""
+    frames, start = _group_frames(frame_desc, frame_product, P, frame_desc.device)
+    counts = start[1:] - start[:-1]
+    acc = torch.zeros((P, frames.shape[1]), dtype=torch.float32, device=frames.device)
+    lmax = int(counts.max()) if P else 0
+    for k in range(lmax):
+        more = counts > k
+        rows = frames.index_select(0, torch.where(more, start[:-1] + k, 0))
+        acc += torch.where(more[:, None], rows, 0.0)
+    return acc / counts.clamp(min=1).to(torch.float32)[:, None], counts > 0
 
 
 def evaluate_distance_fusions(engine: SeamEngine, frame_desc: torch.Tensor, frame_product: torch.Tensor,
@@ -549,22 +644,30 @@ def evaluate_distance_fusions(engine: SeamEngine, frame_desc: torch.Tensor, fram
 
     One fused kernel for all products (``seam_rank_fused_distances``): the (frames x gallery) matrix is never
     materialised, nothing synchronises with the host (the frames are grouped by product with a device sort, the
-    hit counts are device reductions).  Returns ``(ranks (2,P) int64 [avg, max], hits (2, len(k_thresholds))
-    int64)``; products without frames get rank G; ties rank by lower index first, like ``seam_rank_of_target``.
-    ``max_pairs`` is accepted for compatibility and ignored."""
+    hit counts are device reductions).  An fp16 ``shop_desc`` is read as fp16 (the ranks of ``shop_desc.float()``).
+    Returns ``(ranks (2,P) int64 [avg, max], hits (2, len(k_thresholds)) int64)``; products without frames get
+    rank G; ties rank by lower index first, like ``seam_rank_of_target``.  ``max_pairs`` is accepted for
+    compatibility and ignored."""
     dev = engine.device
+    P = int(target.shape[0])
+    frames, start = _group_frames(frame_desc, frame_product, P, dev)
+    with engine.scorer(*frame_last):                         # the caller's scorer is put back on exit
+        ra, rm = engine.rank_fused_distances(frames, start, shop_desc, target)
+    return _fusion_hits(torch.stack([ra, rm]).to(torch.int64), k_thresholds, dev)
+
+
+def _group_frames(frame_desc: torch.Tensor, frame_product: torch.Tensor, P: int, dev):
+    """frames fp32 sorted by product (stable: each product's frames keep their order), start (P+1) int64 offsets"""
     frame_desc = frame_desc.to(dev, torch.float32)
     fp = frame_product.to(dev, torch.int64)
-    shop = shop_desc.to(dev, torch.float32).contiguous()
-    P = int(target.shape[0])
     order = torch.argsort(fp, stable=True)
     counts = torch.bincount(fp, minlength=P)[:P]
     start = torch.zeros(P + 1, dtype=torch.int64, device=dev)
     start[1:] = torch.cumsum(counts, 0)
-    frames = frame_desc.index_select(0, order).contiguous()
-    with engine.scorer(*frame_last):                         # the caller's scorer is put back on exit
-        ra, rm = engine.rank_fused_distances(frames, start, shop, target)
-    ranks = torch.stack([ra, rm]).to(torch.int64)
+    return frame_desc.index_select(0, order).contiguous(), start
+
+
+def _fusion_hits(ranks: torch.Tensor, k_thresholds: Sequence[int], dev):
     ks = torch.tensor(list(k_thresholds), device=dev)
     hits = (ranks[:, :, None] < ks[None, None, :]).sum(1)
     return ranks, hits
