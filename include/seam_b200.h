@@ -397,13 +397,15 @@ int seam_sharded_merge(seam_handle* h, const seam_exchange* x, float* out_score,
  * The reference trains through the aggregator with autograd: its losses consume x5 of TemporalAggregationNLB's
  * x-branch (models/match_head.py:339, 429; stuffs/engine.py:158-185).  These entries give the vector-Jacobian
  * products the forward entries need to sit inside an autograd graph (the Python host wraps them in
- * torch.autograd.Function).  The forward kernels run on folded weights; the backward recomputes each track in the
- * reference's un-folded formulation (models/nlb.py:66-101, match_head.py:144-151) and differentiates that.
+ * torch.autograd.Function).  The backward of the block (models/nlb.py:66-101, match_head.py:144-151) collapses the
+ * way its forward does: it is computed from the weights folded from `w` (not from the handle's loaded weights) with
+ * O(T*256 + T^2) work per track.
  *
  * seam_aggregate_backward: dout (Q,256) = d loss / d x3_1b  ->  dseq (1+Tmax,Q,256) contiguous fp32 = d loss / d
  * x3_1_seq (the caller zero-fills it: row 0 and padded frames stay zero) and the parameter gradients, ACCUMULATED
- * into the buffers of `grads` (same shapes as the weights; the caller zero-fills them).  Tracks of at most 16
- * frames (training uses about 10: train_movingfashion.py:165).  `w` holds the un-folded parameters (last_* unused). */
+ * into the buffers of `grads` (same shapes as the weights; the caller zero-fills them).  Tracks of at most
+ * SEAM_MAX_T frames, as in the forward.  dseq does not depend on the launch (no atomics); the parameter gradients
+ * are summed with atomics and are not bit-reproducible.  `w` holds the un-folded parameters (last_* unused). */
 typedef struct seam_weight_grads {
   float* theta_w; float* theta_b;
   float* phi_w;   float* phi_b;

@@ -286,8 +286,8 @@ int seam_create(seam_handle** out, int device) {
                        (int)score::SMEM_BYTES);
   opt_in_aggregate_smem<float>();
   opt_in_aggregate_smem<__half>();
-  cudaFuncSetAttribute(bwd::agg_backward_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                       (int)bwd::agg_bwd_smem_bytes(bwd::BWD_MAX_T));
+  cudaFuncSetAttribute(bwd::agg_backward_folded_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                       (int)bwd::agg_bwd_smem_bytes(SEAM_MAX_T));
   cudaFuncSetAttribute(tower::conv3x3_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tower::SMEM_BYTES);
   cudaFuncSetAttribute(nlbgemm::nlb_full_front_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
                        (int)((SEAM_MAX_T * 257 + 2 * SEAM_MAX_T) * sizeof(float)));
@@ -1414,9 +1414,8 @@ int seam_aggregate_backward(seam_handle* h, const seam_weights* w, const float* 
   if (!w || !grads) return fail(h, SEAM_ERR_BAD_ARG, "seam_aggregate_backward: weights / grads struct is null");
   if (Q < 0 || Tmax < 0) return fail(h, SEAM_ERR_BAD_ARG, "seam_aggregate_backward: negative size");
   if (Q == 0 || Tmax == 0) return SEAM_OK;
-  if (Tmax > bwd::BWD_MAX_T)
-    return fail(h, SEAM_ERR_UNSUPPORTED, "seam_aggregate_backward: Tmax=%d exceeds the %d frames per track the training path supports",
-                Tmax, bwd::BWD_MAX_T);
+  if (Tmax > SEAM_MAX_T)
+    return fail(h, SEAM_ERR_UNSUPPORTED, "seam_aggregate_backward: Tmax=%d exceeds %d", Tmax, SEAM_MAX_T);
   if (!seq || !dout || !dseq) return fail(h, SEAM_ERR_BAD_ARG, "seam_aggregate_backward: null pointer");
   const float* const* wp = reinterpret_cast<const float* const*>(w);
   float* const* gp = reinterpret_cast<float* const*>(grads);
@@ -1436,8 +1435,15 @@ int seam_aggregate_backward(seam_handle* h, const seam_weights* w, const float* 
   p.w = {w->theta_w, w->theta_b, w->phi_w, w->phi_b, w->g_w, w->g_b, w->W_w, w->W_b, w->concat_w, w->att_w, w->att_b};
   p.g = {grads->theta_w, grads->theta_b, grads->phi_w, grads->phi_b, grads->g_w, grads->g_b,
          grads->W_w,     grads->W_b,     grads->concat_w, grads->att_w, grads->att_b};
-  bwd::agg_backward_kernel<<<Q, 256, bwd::agg_bwd_smem_bytes(Tmax), static_cast<cudaStream_t>(stream_)>>>(p);
-  SEAM_LAUNCHED(h, "agg_backward_kernel");
+  // persistent CTAs: each folds the weights once, so no more of them than can be resident at once
+  const size_t smem = bwd::agg_bwd_smem_bytes(Tmax);
+  int per_sm = 0;
+  if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, bwd::agg_backward_folded_kernel, 256, smem) != cudaSuccess ||
+      per_sm < 1)
+    return fail(h, SEAM_ERR_CUDA, "seam_aggregate_backward: occupancy query failed: %s", cudaGetErrorString(cudaGetLastError()));
+  const int grid = Q < per_sm * h->num_sms ? Q : per_sm * h->num_sms;
+  bwd::agg_backward_folded_kernel<<<grid, 256, smem, static_cast<cudaStream_t>(stream_)>>>(p);
+  SEAM_LAUNCHED(h, "agg_backward_folded_kernel");
   return SEAM_OK;
 }
 

@@ -25,7 +25,7 @@ _AGG_FIELDS = ("theta_w", "theta_b", "phi_w", "phi_b", "g_w", "g_b", "W_w", "W_b
 
 class _AggregateFn(torch.autograd.Function):
     """x3_1b = aggregate(x3_1_seq) inside an autograd graph: forward = the fused aggregation kernel (folded
-    weights), backward = seam_aggregate_backward (the un-folded block re-derived per track)."""
+    weights), backward = seam_aggregate_backward (the same folded algebra, differentiated; tracks of up to 64 frames)."""
 
     @staticmethod
     def forward(ctx, eng, seq, mask, *params):
@@ -283,7 +283,8 @@ class TemporalAggregationNLB(MatchPredictor):
         """Same signature and return tuple as models/match_head.py:90-169.  Limits (errors, not fallbacks):
         tracks of at most 64 frames (``SEAM_MAX_T``), x5 for at most 64M pairs (``DENSE_PAIR_LIMIT``; use
         ``score_topk`` beyond).  The conv tower of the x-branch runs under autograd (``x3_2`` keeps its graph);
-        aggregation and scorer outputs are detached (inference kernels)."""
+        aggregation and scorer outputs are detached (inference kernels).  In training mode with grad enabled (and
+        ``getatt=False``) aggregation and scorer are differentiable, for the same tracks and both values of ``nlb``."""
         x3_1 = x3_1_ids = None
         if x3_1_seq is None and self._tower_ready(x):          # x-branch, eval: the tower writes the track layout itself
             with torch.no_grad():
@@ -326,9 +327,10 @@ class TemporalAggregationNLB(MatchPredictor):
     def _forward_train(self, x3_1, x3_1_ids, x3_1_seq, x3_1_mask, x3_2):
         """Training (models/match_head.py:339, 429 call this forward under autograd): the same kernels forward,
         ``seam_aggregate_backward`` / ``seam_score_dense_backward`` behind them, the grouping of ROI embeddings into
-        tracks as differentiable index operations.  x5 carries the graph the losses differentiate."""
-        if not self.nlb:
-            raise NotImplementedError("training with nlb=False is not supported by the CUDA path")
+        tracks as differentiable index operations.  x5 carries the graph the losses differentiate.  Tracks of up to
+        64 frames (``SEAM_MAX_T``), as in eval mode.  With ``nlb=False`` the block is not in the graph, as in the
+        reference: the forward runs with a zero ``W`` (the eval upload), the backward gets a zero ``W`` too, and the
+        ``newnlb.*`` parameters are passed detached, so their ``.grad`` stays ``None``."""
         if x3_1_seq is None:
             if x3_1_ids.numel() == 0:
                 return None, x3_2, None, None, None, x3_1_ids
@@ -337,7 +339,11 @@ class TemporalAggregationNLB(MatchPredictor):
             x3_1_ids = torch.zeros((1, 2))
         eng = self._engine_for(x3_1_seq.device)
         self._sync_weights(eng)
-        x3_1b = _AggregateFn.apply(eng, x3_1_seq, x3_1_mask, *self._agg_params())
+        params = self._agg_params()
+        if not self.nlb:
+            params = tuple(t.detach() for t in params[:6]) + (torch.zeros_like(params[6]), torch.zeros_like(params[7]),
+                                                              params[8].detach()) + params[9:]
+        x3_1b = _AggregateFn.apply(eng, x3_1_seq, x3_1_mask, *params)
         g = x3_2.to(x3_1b.device).reshape(-1, D_MODEL)
         if x3_1b.shape[0] * g.shape[0] > DENSE_PAIR_LIMIT:
             raise SeamError(2, "x5 too large for the training path")
