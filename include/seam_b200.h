@@ -130,6 +130,12 @@ int seam_aggregate(seam_handle* h, const float* seq, const uint8_t* mask, const 
 int seam_aggregate_f16(seam_handle* h, const void* seq, const uint8_t* mask, const int32_t* lens, int Tmax, int Q,
                        int64_t frame_stride, int64_t track_stride, float* out, float* att, void* workspace,
                        size_t workspace_bytes, void* stream);
+/* seam_aggregate for bf16 tracks (the dtype of torch.autocast(dtype=torch.bfloat16)): seq holds bf16 bit patterns;
+ * strides, alignment and SEAM_ERR_UNSUPPORTED as seam_aggregate_f16.  Widening bf16 to fp32 is exact (a 16-bit
+ * shift), so out / att are bit-identical to seam_aggregate on the widened tracks, for half the bytes read. */
+int seam_aggregate_bf16(seam_handle* h, const void* seq, const uint8_t* mask, const int32_t* lens, int Tmax, int Q,
+                        int64_t frame_stride, int64_t track_stride, float* out, float* att, void* workspace,
+                        size_t workspace_bytes, void* stream);
 
 /* Full non-local block output (not pooled): NONLocalBlock1D.forward, models/nlb.py:66-101.
  *   x, z  (B, 256, T) fp32 channel-major as in the reference; T <= 64.
@@ -208,7 +214,14 @@ int seam_search_f16(seam_handle* h, const void* seq, const uint8_t* mask, const 
                     const float* cg, const float* gstat, int G, int index_offset, int k, float* out_score,
                     float* out_margin, int32_t* out_idx, int32_t* stats, void* workspace, size_t workspace_bytes,
                     void* stream);
-/* seam_search / seam_search_f16 (fp32 / fp16 tracks) for an fp16 gallery (see seam_score_topk_g16). */
+/* seam_search for bf16 tracks (seq, strides and alignment as seam_aggregate_bf16); the rest as seam_search_f16. */
+int seam_search_bf16(seam_handle* h, const void* seq, const uint8_t* mask, const int32_t* lens, int Tmax, int Q,
+                     int64_t frame_stride, int64_t track_stride, float* q_out, const float* g, const void* g16,
+                     const float* cg, const float* gstat, int G, int index_offset, int k, float* out_score,
+                     float* out_margin, int32_t* out_idx, int32_t* stats, void* workspace, size_t workspace_bytes,
+                     void* stream);
+/* seam_search / seam_search_f16 / seam_search_bf16 (fp32 / fp16 / bf16 tracks) for an fp16 gallery (see
+ * seam_score_topk_g16). */
 int seam_search_g16(seam_handle* h, const float* seq, const uint8_t* mask, const int32_t* lens, int Tmax, int Q,
                     int64_t frame_stride, int64_t track_stride, float* q_out, const void* g16, const float* cg,
                     const float* gstat, int G, int index_offset, int k, float* out_score, float* out_margin,
@@ -217,6 +230,10 @@ int seam_search_f16_g16(seam_handle* h, const void* seq, const uint8_t* mask, co
                         int64_t frame_stride, int64_t track_stride, float* q_out, const void* g16, const float* cg,
                         const float* gstat, int G, int index_offset, int k, float* out_score, float* out_margin,
                         int32_t* out_idx, int32_t* stats, void* workspace, size_t workspace_bytes, void* stream);
+int seam_search_bf16_g16(seam_handle* h, const void* seq, const uint8_t* mask, const int32_t* lens, int Tmax, int Q,
+                         int64_t frame_stride, int64_t track_stride, float* q_out, const void* g16, const float* cg,
+                         const float* gstat, int G, int index_offset, int k, float* out_score, float* out_margin,
+                         int32_t* out_idx, int32_t* stats, void* workspace, size_t workspace_bytes, void* stream);
 
 /* Dense logits (parity / small problems): x5 (Q,G,2) fp32 = last((q-g)^2).
  * models/match_head.py:160-162 and MatchPredictor.forward :70-74. */
@@ -378,6 +395,10 @@ int seam_sharded_aggregate(seam_handle* h, const seam_exchange* x, const float* 
 int seam_sharded_aggregate_f16(seam_handle* h, const seam_exchange* x, const void* seq, const uint8_t* mask,
                                const int32_t* lens, int Tmax, int Qlocal, int64_t frame_stride, int64_t track_stride,
                                int row0, int last, float* att, void* stream);
+/* seam_sharded_aggregate for bf16 tracks (seq, strides and alignment as seam_aggregate_bf16). */
+int seam_sharded_aggregate_bf16(seam_handle* h, const seam_exchange* x, const void* seq, const uint8_t* mask,
+                                const int32_t* lens, int Tmax, int Qlocal, int64_t frame_stride, int64_t track_stride,
+                                int row0, int last, float* att, void* stream);
 /* seam_score_topk of all Q queries (this rank's q_all, once every rank's descriptors have landed) against the
  * rank's prepared gallery shard; the top-k rows go to the queries' owners.  Workspace as seam_score_topk. */
 int seam_sharded_score_topk(seam_handle* h, const seam_exchange* x, const float* g, const void* g16, const float* cg,
@@ -450,8 +471,9 @@ int seam_tower_forward(seam_handle* h, const float* x, int K, float* out, const 
  * models/match_head.py:101-111) is neither read nor written.  Pinned host memory makes it asynchronous. */
 int seam_upload_tracks(seam_handle* h, const float* seq_host, int Tmax, int Q, int lo, int hi, float* seq_dev,
                        void* stream);
-/* seam_upload_tracks for an fp16 host x3_1_seq: the same single pitched copy with 512-byte rows into an fp16
- * device tensor (1+Tmax, hi-lo, 256) -- half the PCIe bytes; feed the result to the _f16 entry points. */
+/* seam_upload_tracks for a host x3_1_seq of any 2-byte element type (fp16 or bf16): the same single pitched copy
+ * with 512-byte rows into a device tensor (1+Tmax, hi-lo, 256) of that type -- half the PCIe bytes; feed the result
+ * to the _f16 or _bf16 entry points. */
 int seam_upload_tracks_f16(seam_handle* h, const void* seq_host, int Tmax, int Q, int lo, int hi, void* seq_dev,
                            void* stream);
 

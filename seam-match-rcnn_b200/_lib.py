@@ -111,6 +111,8 @@ def _declare(lib: C.CDLL) -> None:
     lib.seam_aggregate.argtypes = [vp, vp, vp, vp, i32, i32, i64, i64, vp, vp, vp, sz, vp]
     lib.seam_aggregate_f16.restype = i32
     lib.seam_aggregate_f16.argtypes = lib.seam_aggregate.argtypes
+    lib.seam_aggregate_bf16.restype = i32
+    lib.seam_aggregate_bf16.argtypes = lib.seam_aggregate.argtypes
     lib.seam_nlb_workspace_bytes.restype = sz
     lib.seam_nlb_workspace_bytes.argtypes = [i32, i32]
     lib.seam_nlb_forward.restype = i32
@@ -133,10 +135,14 @@ def _declare(lib: C.CDLL) -> None:
     lib.seam_search.argtypes = [vp, vp, vp, vp, i32, i32, i64, i64, vp, vp, vp, vp, vp, i32, i32, i32, vp, vp, vp, vp, vp, sz, vp]
     lib.seam_search_f16.restype = i32
     lib.seam_search_f16.argtypes = lib.seam_search.argtypes
+    lib.seam_search_bf16.restype = i32
+    lib.seam_search_bf16.argtypes = lib.seam_search.argtypes
     lib.seam_search_g16.restype = i32
     lib.seam_search_g16.argtypes = [vp, vp, vp, vp, i32, i32, i64, i64, vp, vp, vp, vp, i32, i32, i32, vp, vp, vp, vp, vp, sz, vp]
     lib.seam_search_f16_g16.restype = i32
     lib.seam_search_f16_g16.argtypes = lib.seam_search_g16.argtypes
+    lib.seam_search_bf16_g16.restype = i32
+    lib.seam_search_bf16_g16.argtypes = lib.seam_search_g16.argtypes
     lib.seam_score_dense.restype = i32
     lib.seam_score_dense.argtypes = [vp, vp, i32, vp, i32, vp, vp]
     lib.seam_score_prob.restype = i32
@@ -174,6 +180,8 @@ def _declare(lib: C.CDLL) -> None:
     lib.seam_sharded_aggregate.argtypes = [vp, xp, vp, vp, vp, i32, i32, i64, i64, i32, i32, vp, vp]
     lib.seam_sharded_aggregate_f16.restype = i32
     lib.seam_sharded_aggregate_f16.argtypes = lib.seam_sharded_aggregate.argtypes
+    lib.seam_sharded_aggregate_bf16.restype = i32
+    lib.seam_sharded_aggregate_bf16.argtypes = lib.seam_sharded_aggregate.argtypes
     lib.seam_sharded_score_topk.restype = i32
     lib.seam_sharded_score_topk.argtypes = [vp, xp, vp, vp, vp, vp, i32, i32, vp, vp, sz, vp]
     lib.seam_sharded_score_topk_g16.restype = i32

@@ -23,9 +23,9 @@
 // Results do not depend on how tracks are grouped into batches (a column of D depends on its own track
 // only; the accumulation order over k is fixed), nor on which slot a track lands in.
 //
-// Tracks are fp32 or fp16 (template parameter In): only the track buffers and the copies into them follow the element
-// size; load_frame widens an fp16 frame to fp32 as it leaves shared memory (exact), so the fp16 instantiations give
-// bit for bit what the fp32 ones give on the widened tracks.
+// Tracks are fp32, fp16 or bf16 (template parameter In): only the track buffers and the copies into them follow the
+// element size; load_frame widens a 16-bit frame to fp32 as it leaves shared memory (exact), so the fp16 and bf16
+// instantiations give bit for bit what the fp32 ones give on the widened tracks.
 //
 // A producer's iteration is a LATENCY CHAIN (2-3 producer warps per scheduler: shuffle rounds, named barriers,
 // shared-memory atomics, mbarrier polls and the hand-over of a copy to the copy engine all sit on one warp's
@@ -36,6 +36,7 @@
 #include <cstdint>
 #include <type_traits>
 #include <cuda.h>
+#include <cuda_bf16.h>
 #include <cuda_fp16.h>
 #include "exchange.cuh"
 #include "fold.cuh"
@@ -80,7 +81,7 @@ __host__ __device__ constexpr uint32_t fused_bytes() {
 }
 
 struct Params {
-  const void* seq;         // float or __half: the kernels' In
+  const void* seq;         // float, __half or __nv_bfloat16: the kernels' In
   const uint8_t* mask;     // (Q, 1+Tmax) or null
   const int32_t* lens;     // (Q) or null
   int Tmax, Q;
@@ -134,21 +135,28 @@ __device__ __forceinline__ Vec8 load_vec8(const float* row, int lane) {
   const ulonglong2 hi = *reinterpret_cast<const ulonglong2*>(row + 128 + 4 * lane);
   return Vec8{lo.x, lo.y, hi.x, hi.y};
 }
-// a frame of the track buffer (In = float or __half) -> registers, with the lane -> channel mapping of load_vec8.
-// fp16 frames are widened here (exact), so every instruction after this load is the fp32 path's.
-__device__ __forceinline__ u64 widen2(uint32_t h2) {
-  const float2 f = __half22float2(*reinterpret_cast<const __half2*>(&h2));
-  return pk(f.x, f.y);
+// a frame of the track buffer (In = float, __half or __nv_bfloat16) -> registers, with the lane -> channel mapping of
+// load_vec8.  16-bit frames are widened here (exact), so every instruction after this load is the fp32 path's.
+template <typename In>
+__device__ __forceinline__ u64 widen2(uint32_t v) {
+  if constexpr (std::is_same<In, __half>::value) {
+    const float2 f = __half22float2(*reinterpret_cast<const __half2*>(&v));
+    return pk(f.x, f.y);
+  } else {   // a bf16 value is the upper half of the fp32 with the same value
+    return pk(__uint_as_float(v << 16), __uint_as_float(v & 0xffff0000u));
+  }
 }
 template <typename In>
 __device__ __forceinline__ Vec8 load_frame(const In* row, int lane) {
+  static_assert(std::is_same<In, float>::value || std::is_same<In, __half>::value ||
+                    std::is_same<In, __nv_bfloat16>::value,
+                "frames are float, __half or __nv_bfloat16");
   if constexpr (std::is_same<In, float>::value) {
     return load_vec8(row, lane);
   } else {
-    static_assert(std::is_same<In, __half>::value, "frames are float or __half");
     const uint2 lo = *reinterpret_cast<const uint2*>(row + 4 * lane);
     const uint2 hi = *reinterpret_cast<const uint2*>(row + 128 + 4 * lane);
-    return Vec8{widen2(lo.x), widen2(lo.y), widen2(hi.x), widen2(hi.y)};
+    return Vec8{widen2<In>(lo.x), widen2<In>(lo.y), widen2<In>(hi.x), widen2<In>(hi.y)};
   }
 }
 __device__ __forceinline__ Vec8 zero_vec8() { return Vec8{0ull, 0ull, 0ull, 0ull}; }
@@ -484,7 +492,8 @@ struct Cfg<10> { static constexpr int NW = 11, SLOTS = 1, LOADER = 1, REGS_P = 1
 template <>
 struct Cfg<16> { static constexpr int NW = 8, SLOTS = 1, LOADER = 0, REGS_P = 224, REGS_H = 56; };
 
-// In: the element type of the tracks (float or __half); only the track buffers and the copies into them depend on it
+// In: the element type of the tracks (float, __half or __nv_bfloat16); only the track buffers and the copies into them
+// depend on it
 template <int TR, typename In>
 constexpr size_t warp_smem_bytes() {
   return 1024 + fused_bytes<true>() + (size_t)Cfg<TR>::NW * Cfg<TR>::SLOTS * TR * D * sizeof(In)   // track buffers
@@ -857,7 +866,7 @@ struct alignas(16) GroupSmem {
 };
 template <int GW, typename In>
 struct GSmem {
-  In x[GWARPS][FB][D];                 // 8 x 16 KB (fp32) / 8 x 8 KB (fp16)
+  In x[GWARPS][FB][D];                 // 8 x 16 KB (fp32) / 8 x 8 KB (fp16, bf16)
   GroupSmem<GW> g[GWARPS / GW];
   uint64_t bar[GWARPS];
 };

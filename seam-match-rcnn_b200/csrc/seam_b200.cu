@@ -10,6 +10,7 @@
 #include <vector>
 
 #include <cuda.h>
+#include <cuda_bf16.h>
 #include <cuda_fp16.h>
 #include <cuda_runtime.h>
 
@@ -119,7 +120,8 @@ static inline size_t align_up(size_t x, size_t a) { return (x + a - 1) / a * a; 
 static inline bool aligned16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15u) == 0; }
 
 // Full tracks / full frame blocks are fetched with one 3-D tensor-map copy: box {256, 1 track, frames} over seq viewed as
-// (1+Tmax, Q, 256) with the caller's strides (elements of In: float or __half).  Returns whether the map is usable.
+// (1+Tmax, Q, 256) with the caller's strides (elements of In: float, __half or __nv_bfloat16).  Returns whether the map
+// is usable.
 template <typename In>
 static int encode_seq_map(seam_handle* h, const aggf::Params& p, int box_frames, CUtensorMap* tm) {
   constexpr long long ES = sizeof(In);
@@ -131,7 +133,9 @@ static int encode_seq_map(seam_handle* h, const aggf::Params& p, int box_frames,
   const cuuint64_t strides[2] = {(cuuint64_t)(p.track_stride * ES), (cuuint64_t)(p.frame_stride * ES)};
   const cuuint32_t box[3] = {256, 1, (cuuint32_t)box_frames};
   const cuuint32_t estr[3] = {1, 1, 1};
-  const CUtensorMapDataType dt = ES == 2 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT16 : CU_TENSOR_MAP_DATA_TYPE_FLOAT32;
+  const CUtensorMapDataType dt = std::is_same<In, __half>::value          ? CU_TENSOR_MAP_DATA_TYPE_FLOAT16
+                                 : std::is_same<In, __nv_bfloat16>::value ? CU_TENSOR_MAP_DATA_TYPE_BFLOAT16
+                                                                          : CU_TENSOR_MAP_DATA_TYPE_FLOAT32;
   return h->encode(tm, dt, 3, const_cast<void*>(p.seq), dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
                    CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
                    CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
@@ -286,6 +290,7 @@ int seam_create(seam_handle** out, int device) {
                        (int)score::SMEM_BYTES);
   opt_in_aggregate_smem<float>();
   opt_in_aggregate_smem<__half>();
+  opt_in_aggregate_smem<__nv_bfloat16>();
   cudaFuncSetAttribute(bwd::agg_backward_folded_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
                        (int)bwd::agg_bwd_smem_bytes(SEAM_MAX_T));
   cudaFuncSetAttribute(tower::conv3x3_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tower::SMEM_BYTES);
@@ -398,8 +403,11 @@ size_t seam_aggregate_workspace_bytes(int Q) {
   return 256;   // the fused kernel keeps every intermediate on the SM
 }
 
-// seq holds fp32 values, or fp16 bit patterns when f16 is set (strides in elements either way)
-static int aggregate_impl(seam_handle* h, const xchg::Exchange* x, int row0, int last, const void* seq, bool f16,
+// the element type of a track tensor x3_1_seq, as the entry point that received it says
+enum class TrackType { F32, F16, BF16 };
+
+// seq holds values of type tt (strides in elements)
+static int aggregate_impl(seam_handle* h, const xchg::Exchange* x, int row0, int last, const void* seq, TrackType tt,
                           const uint8_t* mask, const int32_t* lens, int Tmax, int Q, int64_t frame_stride,
                           int64_t track_stride, float* out, float* att, cudaStream_t stream, const char* who) {
   if (!h->have_aggregator) return fail(h, SEAM_ERR_STATE, "%s: weights not loaded", who);
@@ -414,10 +422,10 @@ static int aggregate_impl(seam_handle* h, const xchg::Exchange* x, int row0, int
   }
   if (Q > 0 && Tmax > 0 && !seq) return fail(h, SEAM_ERR_BAD_ARG, "%s: null pointer", who);
   // the bulk copies and the tensor map move whole frames: 16-byte aligned rows
-  const int64_t stride_mask = f16 ? 7 : 3;
+  const int64_t stride_mask = tt == TrackType::F32 ? 3 : 7;
   if (!aligned16(seq) || (out && !aligned16(out)) || (frame_stride & stride_mask) || (track_stride & stride_mask))
     return fail(h, SEAM_ERR_UNSUPPORTED, "%s: seq/out must be 16-byte aligned, strides multiples of %s", who,
-                f16 ? "8 fp16 elements" : "4");
+                tt == TrackType::F32 ? "4" : tt == TrackType::F16 ? "8 fp16 elements" : "8 bf16 elements");
   ProfileScope prof(h, SEAM_KERNEL_AGGREGATE, stream);
   aggf::Params p;
   memset(&p, 0, sizeof(p));
@@ -449,7 +457,8 @@ static int aggregate_impl(seam_handle* h, const xchg::Exchange* x, int row0, int
     }
     return SEAM_OK;
   }
-  if (f16) launch_aggregate<__half>(h, p, stream);
+  if (tt == TrackType::F16) launch_aggregate<__half>(h, p, stream);
+  else if (tt == TrackType::BF16) launch_aggregate<__nv_bfloat16>(h, p, stream);
   else launch_aggregate<float>(h, p, stream);
   SEAM_LAUNCHED(h, "aggregate kernel");
   return SEAM_OK;
@@ -461,8 +470,8 @@ int seam_aggregate(seam_handle* h, const float* seq, const uint8_t* mask, const 
   (void)workspace;
   (void)workspace_bytes;
   if (!h) return SEAM_ERR_BAD_ARG;
-  return aggregate_impl(h, nullptr, 0, 0, seq, false, mask, lens, Tmax, Q, frame_stride, track_stride, out, att,
-                        static_cast<cudaStream_t>(stream_), "seam_aggregate");
+  return aggregate_impl(h, nullptr, 0, 0, seq, TrackType::F32, mask, lens, Tmax, Q, frame_stride, track_stride, out,
+                        att, static_cast<cudaStream_t>(stream_), "seam_aggregate");
 }
 
 int seam_aggregate_f16(seam_handle* h, const void* seq, const uint8_t* mask, const int32_t* lens, int Tmax, int Q,
@@ -471,35 +480,52 @@ int seam_aggregate_f16(seam_handle* h, const void* seq, const uint8_t* mask, con
   (void)workspace;
   (void)workspace_bytes;
   if (!h) return SEAM_ERR_BAD_ARG;
-  return aggregate_impl(h, nullptr, 0, 0, seq, true, mask, lens, Tmax, Q, frame_stride, track_stride, out, att,
-                        static_cast<cudaStream_t>(stream_), "seam_aggregate_f16");
+  return aggregate_impl(h, nullptr, 0, 0, seq, TrackType::F16, mask, lens, Tmax, Q, frame_stride, track_stride, out,
+                        att, static_cast<cudaStream_t>(stream_), "seam_aggregate_f16");
 }
 
-static int sharded_aggregate_impl(seam_handle* h, const seam_exchange* x, const void* seq, bool f16, const uint8_t* mask,
-                                  const int32_t* lens, int Tmax, int Qlocal, int64_t frame_stride, int64_t track_stride,
-                                  int row0, int last, float* att, void* stream_, const char* who) {
+int seam_aggregate_bf16(seam_handle* h, const void* seq, const uint8_t* mask, const int32_t* lens, int Tmax, int Q,
+                        int64_t frame_stride, int64_t track_stride, float* out, float* att, void* workspace,
+                        size_t workspace_bytes, void* stream_) {
+  (void)workspace;
+  (void)workspace_bytes;
+  if (!h) return SEAM_ERR_BAD_ARG;
+  return aggregate_impl(h, nullptr, 0, 0, seq, TrackType::BF16, mask, lens, Tmax, Q, frame_stride, track_stride, out,
+                        att, static_cast<cudaStream_t>(stream_), "seam_aggregate_bf16");
+}
+
+static int sharded_aggregate_impl(seam_handle* h, const seam_exchange* x, const void* seq, TrackType tt,
+                                  const uint8_t* mask, const int32_t* lens, int Tmax, int Qlocal, int64_t frame_stride,
+                                  int64_t track_stride, int row0, int last, float* att, void* stream_, const char* who) {
   if (!h) return SEAM_ERR_BAD_ARG;
   xchg::Exchange e;
   int rc = import_exchange(h, x, &e, who);
   if (rc != SEAM_OK) return rc;
   if (row0 < 0 || Qlocal < 0 || row0 + Qlocal > x->Q)
     return fail(h, SEAM_ERR_BAD_ARG, "%s: rows [%d,%d) outside the %d queries", who, row0, row0 + Qlocal, x->Q);
-  return aggregate_impl(h, &e, row0, last ? 1 : 0, seq, f16, mask, lens, Tmax, Qlocal, frame_stride, track_stride, nullptr,
-                        att, static_cast<cudaStream_t>(stream_), who);
+  return aggregate_impl(h, &e, row0, last ? 1 : 0, seq, tt, mask, lens, Tmax, Qlocal, frame_stride, track_stride,
+                        nullptr, att, static_cast<cudaStream_t>(stream_), who);
 }
 
 int seam_sharded_aggregate(seam_handle* h, const seam_exchange* x, const float* seq, const uint8_t* mask,
                            const int32_t* lens, int Tmax, int Qlocal, int64_t frame_stride, int64_t track_stride,
                            int row0, int last, float* att, void* stream_) {
-  return sharded_aggregate_impl(h, x, seq, false, mask, lens, Tmax, Qlocal, frame_stride, track_stride, row0, last, att,
-                                stream_, "seam_sharded_aggregate");
+  return sharded_aggregate_impl(h, x, seq, TrackType::F32, mask, lens, Tmax, Qlocal, frame_stride, track_stride, row0,
+                                last, att, stream_, "seam_sharded_aggregate");
 }
 
 int seam_sharded_aggregate_f16(seam_handle* h, const seam_exchange* x, const void* seq, const uint8_t* mask,
                                const int32_t* lens, int Tmax, int Qlocal, int64_t frame_stride, int64_t track_stride,
                                int row0, int last, float* att, void* stream_) {
-  return sharded_aggregate_impl(h, x, seq, true, mask, lens, Tmax, Qlocal, frame_stride, track_stride, row0, last, att,
-                                stream_, "seam_sharded_aggregate_f16");
+  return sharded_aggregate_impl(h, x, seq, TrackType::F16, mask, lens, Tmax, Qlocal, frame_stride, track_stride, row0,
+                                last, att, stream_, "seam_sharded_aggregate_f16");
+}
+
+int seam_sharded_aggregate_bf16(seam_handle* h, const seam_exchange* x, const void* seq, const uint8_t* mask,
+                                const int32_t* lens, int Tmax, int Qlocal, int64_t frame_stride, int64_t track_stride,
+                                int row0, int last, float* att, void* stream_) {
+  return sharded_aggregate_impl(h, x, seq, TrackType::BF16, mask, lens, Tmax, Qlocal, frame_stride, track_stride, row0,
+                                last, att, stream_, "seam_sharded_aggregate_bf16");
 }
 
 size_t seam_nlb_workspace_bytes(int B, int T) {
@@ -973,15 +999,15 @@ int seam_score_topk_g16(seam_handle* h, const float* q, int Q, const void* g16, 
                          stats, workspace, workspace_bytes, stream_, "seam_score_topk_g16", "seam_score_topk_g16");
 }
 
-// f16: fp16 tracks; rows / rows_f16: the gallery rows as in score_topk_impl.  Scorer errors name score_who.
-static int search_impl(seam_handle* h, const void* seq, bool f16, const uint8_t* mask, const int32_t* lens, int Tmax,
-                       int Q, int64_t frame_stride, int64_t track_stride, float* q_out, const void* rows, bool rows_f16,
-                       const void* g16, const float* cg, const float* gstat, int G, int index_offset, int k,
+// tt: the tracks' element type; rows / rows_f16: the gallery rows as in score_topk_impl.  Scorer errors name score_who.
+static int search_impl(seam_handle* h, const void* seq, TrackType tt, const uint8_t* mask, const int32_t* lens,
+                       int Tmax, int Q, int64_t frame_stride, int64_t track_stride, float* q_out, const void* rows,
+                       bool rows_f16, const void* g16, const float* cg, const float* gstat, int G, int index_offset, int k,
                        float* out_score, float* out_margin, int32_t* out_idx, int32_t* stats, void* workspace,
                        size_t workspace_bytes, void* stream_, const char* who, const char* score_who) {
   if (!h) return SEAM_ERR_BAD_ARG;
   if (!q_out && Q > 0) return fail(h, SEAM_ERR_BAD_ARG, "%s: q_out is null", who);
-  int rc = aggregate_impl(h, nullptr, 0, 0, seq, f16, mask, lens, Tmax, Q, frame_stride, track_stride, q_out, nullptr,
+  int rc = aggregate_impl(h, nullptr, 0, 0, seq, tt, mask, lens, Tmax, Q, frame_stride, track_stride, q_out, nullptr,
                           static_cast<cudaStream_t>(stream_), who);
   if (rc != SEAM_OK) return rc;
   return score_topk_impl(h, nullptr, q_out, Q, rows, rows_f16, g16, cg, gstat, G, index_offset, k, out_score, out_margin,
@@ -992,9 +1018,9 @@ int seam_search(seam_handle* h, const float* seq, const uint8_t* mask, const int
                 int64_t frame_stride, int64_t track_stride, float* q_out, const float* g, const void* g16, const float* cg,
                 const float* gstat, int G, int index_offset, int k, float* out_score, float* out_margin, int32_t* out_idx,
                 int32_t* stats, void* workspace, size_t workspace_bytes, void* stream_) {
-  return search_impl(h, seq, false, mask, lens, Tmax, Q, frame_stride, track_stride, q_out, g, false, g16, cg, gstat, G,
-                     index_offset, k, out_score, out_margin, out_idx, stats, workspace, workspace_bytes, stream_,
-                     "seam_search", "seam_score_topk");
+  return search_impl(h, seq, TrackType::F32, mask, lens, Tmax, Q, frame_stride, track_stride, q_out, g, false, g16, cg,
+                     gstat, G, index_offset, k, out_score, out_margin, out_idx, stats, workspace, workspace_bytes,
+                     stream_, "seam_search", "seam_score_topk");
 }
 
 int seam_search_f16(seam_handle* h, const void* seq, const uint8_t* mask, const int32_t* lens, int Tmax, int Q,
@@ -1002,27 +1028,46 @@ int seam_search_f16(seam_handle* h, const void* seq, const uint8_t* mask, const 
                     const float* cg, const float* gstat, int G, int index_offset, int k, float* out_score,
                     float* out_margin, int32_t* out_idx, int32_t* stats, void* workspace, size_t workspace_bytes,
                     void* stream_) {
-  return search_impl(h, seq, true, mask, lens, Tmax, Q, frame_stride, track_stride, q_out, g, false, g16, cg, gstat, G,
-                     index_offset, k, out_score, out_margin, out_idx, stats, workspace, workspace_bytes, stream_,
-                     "seam_search_f16", "seam_score_topk");
+  return search_impl(h, seq, TrackType::F16, mask, lens, Tmax, Q, frame_stride, track_stride, q_out, g, false, g16, cg,
+                     gstat, G, index_offset, k, out_score, out_margin, out_idx, stats, workspace, workspace_bytes,
+                     stream_, "seam_search_f16", "seam_score_topk");
+}
+
+int seam_search_bf16(seam_handle* h, const void* seq, const uint8_t* mask, const int32_t* lens, int Tmax, int Q,
+                     int64_t frame_stride, int64_t track_stride, float* q_out, const float* g, const void* g16,
+                     const float* cg, const float* gstat, int G, int index_offset, int k, float* out_score,
+                     float* out_margin, int32_t* out_idx, int32_t* stats, void* workspace, size_t workspace_bytes,
+                     void* stream_) {
+  return search_impl(h, seq, TrackType::BF16, mask, lens, Tmax, Q, frame_stride, track_stride, q_out, g, false, g16, cg,
+                     gstat, G, index_offset, k, out_score, out_margin, out_idx, stats, workspace, workspace_bytes,
+                     stream_, "seam_search_bf16", "seam_score_topk");
 }
 
 int seam_search_g16(seam_handle* h, const float* seq, const uint8_t* mask, const int32_t* lens, int Tmax, int Q,
                     int64_t frame_stride, int64_t track_stride, float* q_out, const void* g16, const float* cg,
                     const float* gstat, int G, int index_offset, int k, float* out_score, float* out_margin,
                     int32_t* out_idx, int32_t* stats, void* workspace, size_t workspace_bytes, void* stream_) {
-  return search_impl(h, seq, false, mask, lens, Tmax, Q, frame_stride, track_stride, q_out, g16, true, g16, cg, gstat, G,
-                     index_offset, k, out_score, out_margin, out_idx, stats, workspace, workspace_bytes, stream_,
-                     "seam_search_g16", "seam_search_g16");
+  return search_impl(h, seq, TrackType::F32, mask, lens, Tmax, Q, frame_stride, track_stride, q_out, g16, true, g16, cg,
+                     gstat, G, index_offset, k, out_score, out_margin, out_idx, stats, workspace, workspace_bytes,
+                     stream_, "seam_search_g16", "seam_search_g16");
 }
 
 int seam_search_f16_g16(seam_handle* h, const void* seq, const uint8_t* mask, const int32_t* lens, int Tmax, int Q,
                         int64_t frame_stride, int64_t track_stride, float* q_out, const void* g16, const float* cg,
                         const float* gstat, int G, int index_offset, int k, float* out_score, float* out_margin,
                         int32_t* out_idx, int32_t* stats, void* workspace, size_t workspace_bytes, void* stream_) {
-  return search_impl(h, seq, true, mask, lens, Tmax, Q, frame_stride, track_stride, q_out, g16, true, g16, cg, gstat, G,
-                     index_offset, k, out_score, out_margin, out_idx, stats, workspace, workspace_bytes, stream_,
-                     "seam_search_f16_g16", "seam_search_f16_g16");
+  return search_impl(h, seq, TrackType::F16, mask, lens, Tmax, Q, frame_stride, track_stride, q_out, g16, true, g16, cg,
+                     gstat, G, index_offset, k, out_score, out_margin, out_idx, stats, workspace, workspace_bytes,
+                     stream_, "seam_search_f16_g16", "seam_search_f16_g16");
+}
+
+int seam_search_bf16_g16(seam_handle* h, const void* seq, const uint8_t* mask, const int32_t* lens, int Tmax, int Q,
+                         int64_t frame_stride, int64_t track_stride, float* q_out, const void* g16, const float* cg,
+                         const float* gstat, int G, int index_offset, int k, float* out_score, float* out_margin,
+                         int32_t* out_idx, int32_t* stats, void* workspace, size_t workspace_bytes, void* stream_) {
+  return search_impl(h, seq, TrackType::BF16, mask, lens, Tmax, Q, frame_stride, track_stride, q_out, g16, true, g16,
+                     cg, gstat, G, index_offset, k, out_score, out_margin, out_idx, stats, workspace, workspace_bytes,
+                     stream_, "seam_search_bf16_g16", "seam_search_bf16_g16");
 }
 
 static int sharded_score_topk_impl(seam_handle* h, const seam_exchange* x, const void* rows, bool rows_f16,
@@ -1582,7 +1627,7 @@ int seam_tower_forward(seam_handle* h, const float* x, int K, float* out, const 
   return SEAM_OK;
 }
 
-// es: bytes per element (4: fp32, 2: fp16); a frame row of one track is 256 * es bytes
+// es: bytes per element (4: fp32, 2: fp16 or bf16); a frame row of one track is 256 * es bytes
 static int upload_tracks_impl(seam_handle* h, const void* seq_host, size_t es, int Tmax, int Q, int lo, int hi,
                               void* seq_dev, void* stream_, const char* who) {
   if (!h) return SEAM_ERR_BAD_ARG;

@@ -197,7 +197,7 @@ class SeamEngine:
     def aggregate_backward(self, seq: torch.Tensor, mask, lens, params: Mapping[str, torch.Tensor], dout: torch.Tensor):
         """Vector-Jacobian product of ``aggregate``: ``dout (Q,256)`` -> ``(dseq (1+Tmax,Q,256), {field: grad})`` for
         the 11 aggregator parameters (fields of ``struct seam_weights``, un-folded fp32 tensors in ``params``)."""
-        seq, m8, l32, Tmax, Q = self._tracks(seq, mask, lens, keep_f16=False)     # the backward kernel reads fp32
+        seq, m8, l32, Tmax, Q = self._tracks(seq, mask, lens, keep_16bit=False)   # the backward kernel reads fp32
         dout = self._f32(dout, "dout")
         tensors = {f: self._f32(params[f].detach(), f) for f in SeamWeightGrads.FIELDS}
         w = SeamWeights(**{f: (tensors[f].data_ptr() if f in tensors else 0) for f in SeamWeights.FIELDS})
@@ -290,30 +290,30 @@ class SeamEngine:
 
         seq (1+Tmax, Q, 256) fp32 with dummy row 0, mask (Q, 1+Tmax) bool (True = padding):
         the arguments ``x3_1_seq`` / ``x3_1_mask`` of models/match_head.py:90, :133-154.
-        An fp16 ``seq`` on this device is read as fp16 (``seam_aggregate_f16``: no conversion pass, same results as
-        on ``seq.float()``); other dtypes are converted to fp32.
+        An fp16 or bf16 ``seq`` on this device is read as it is (``seam_aggregate_f16`` / ``seam_aggregate_bf16``: no
+        conversion pass, same results as on ``seq.float()``); other dtypes are converted to fp32.
         """
         seq, m8, l32, Tmax, Q = self._tracks(seq, mask, lens)
         out = self._out(out, (Q, D_MODEL), torch.float32, "aggregate")
         att = torch.empty((Q, Tmax), dtype=torch.float32, device=self.device) if getatt else None
         nbytes = int(self._lib.seam_aggregate_workspace_bytes(Q))
         ws = self._workspace("agg", nbytes)
-        fn = self._lib.seam_aggregate_f16 if seq.dtype == torch.float16 else self._lib.seam_aggregate
+        fn = self._track_entry("aggregate", seq)
         self._check(fn(self._h, seq.data_ptr(), _ptr(m8), _ptr(l32), Tmax, Q, seq.stride(0), seq.stride(1),
                        out.data_ptr(), _ptr(att), ws.data_ptr(), ws.numel(), self._stream()))
         return (out, att) if getatt else out
 
     # ------------------------------------------------------------------ gallery-sharded search (exchange in the kernels)
-    def _tracks(self, seq, mask, lens, keep_f16: bool = True):
+    def _tracks(self, seq, mask, lens, keep_16bit: bool = True):
         """Argument normalisation shared by aggregate / search / sharded_aggregate / aggregate_backward.  ``seq`` comes
-        back fp32, or fp16 when it is fp16 on this device and ``keep_f16`` (the ``_f16`` entry points read it as it
-        is), with 16-byte strides: copied only when its own strides do not allow that."""
+        back fp32, or fp16 / bf16 when it has that dtype on this device and ``keep_16bit`` (the ``_f16`` / ``_bf16``
+        entry points read it as it is), with 16-byte strides: copied only when its own strides do not allow that."""
         if seq.dim() != 3 or seq.shape[2] != D_MODEL:
             raise ValueError(f"x3_1_seq must be (1+Tmax, Q, 256), got {tuple(seq.shape)}")
-        if not (keep_f16 and seq.dtype == torch.float16 and seq.device == self.device) and (
+        if not (keep_16bit and seq.dtype in (torch.float16, torch.bfloat16) and seq.device == self.device) and (
                 seq.device != self.device or seq.dtype != torch.float32):
             seq = seq.to(device=self.device, dtype=torch.float32)
-        per16 = 16 // seq.element_size()                 # elements per 16 bytes: 4 (fp32) / 8 (fp16)
+        per16 = 16 // seq.element_size()                 # elements per 16 bytes: 4 (fp32) / 8 (fp16, bf16)
         if seq.stride(2) != 1 or seq.stride(0) % per16 or seq.stride(1) % per16:
             seq = seq.contiguous()
         Tmax, Q = seq.shape[0] - 1, seq.shape[1]
@@ -327,6 +327,14 @@ class SeamEngine:
         l32 = lens.to(device=self.device, dtype=torch.int32).contiguous() if lens is not None else None
         return seq, m8, l32, Tmax, Q
 
+    _TRACK_SUFFIX = {torch.float32: "", torch.float16: "_f16", torch.bfloat16: "_bf16"}
+
+    def _track_entry(self, op: str, seq: torch.Tensor, rows_f16: bool = False):
+        """The C entry point of ``op`` (``aggregate``, ``search`` or ``sharded_aggregate``) for tracks of ``seq``'s
+        dtype (as ``_tracks`` returns them), and for ``search`` against an fp16 gallery's rows when ``rows_f16``:
+        e.g. ``seam_search_bf16_g16``."""
+        return getattr(self._lib, f"seam_{op}{self._TRACK_SUFFIX[seq.dtype]}{'_g16' if rows_f16 else ''}")
+
     def sharded_aggregate(self, x, seq: torch.Tensor, mask=None, lens=None, row0: Optional[int] = None,
                           last: bool = True, getatt: bool = False):
         """This rank's tracks (queries ``row0 .. row0+Qlocal`` of the step, default: the rows it owns) -> their
@@ -335,7 +343,7 @@ class SeamEngine:
         seq, m8, l32, Tmax, Q = self._tracks(seq, mask, lens)
         row0 = x.q_lo[x.rank] if row0 is None else int(row0)
         att = torch.empty((Q, Tmax), dtype=torch.float32, device=self.device) if getatt else None
-        fn = self._lib.seam_sharded_aggregate_f16 if seq.dtype == torch.float16 else self._lib.seam_sharded_aggregate
+        fn = self._track_entry("sharded_aggregate", seq)
         self._check(fn(self._h, C.byref(x.struct), seq.data_ptr() if Q else 0, _ptr(m8), _ptr(l32), Tmax, Q,
                        seq.stride(0), seq.stride(1), row0, 1 if last else 0, _ptr(att), self._stream()))
         return att
@@ -486,11 +494,9 @@ class SeamEngine:
         ix = torch.empty((Q, k), dtype=torch.int32, device=self.device)
         stats = torch.zeros((4,), dtype=torch.int32, device=self.device) if return_stats else None
         ws = self._workspace("score", nbytes)
-        f16 = seq.dtype == torch.float16
-        if gallery.rows_f16:
-            fn, rows = (self._lib.seam_search_f16_g16 if f16 else self._lib.seam_search_g16), ()
-        else:
-            fn, rows = (self._lib.seam_search_f16 if f16 else self._lib.seam_search), (gallery.g.data_ptr(),)
+        # an fp16 gallery has no separate rows: the _g16 entry reads g16 for both the operand and the direct form
+        fn = self._track_entry("search", seq, gallery.rows_f16)
+        rows = () if gallery.rows_f16 else (gallery.g.data_ptr(),)
         self._check(fn(self._h, seq.data_ptr() if Q else 0, _ptr(m8), _ptr(l32), Tmax, Q, seq.stride(0), seq.stride(1),
                        q.data_ptr(), *rows, gallery.g16.data_ptr(), gallery.cg.data_ptr(),
                        gallery.gstat.data_ptr(), G, int(gallery.index_offset), k, sc.data_ptr(), mg.data_ptr(),
@@ -679,17 +685,18 @@ class SeamEngine:
 
     def upload_tracks(self, seq_host: torch.Tensor, lo: int, hi: int) -> torch.Tensor:
         """Tracks [lo, hi) of a HOST ``x3_1_seq (1+Tmax, Q, 256)`` -> device ``(1+Tmax, hi-lo, 256)`` on the
-        current stream with one pitched copy of the frame rows (row 0, the dummy frame, stays untouched).  fp32 or fp16:
-        the device tensor has the host tensor's dtype (fp16 tracks cross the bus at half the bytes and are aggregated
-        as fp16)."""
-        if (seq_host.device.type != "cpu" or seq_host.dtype not in (torch.float32, torch.float16)
+        current stream with one pitched copy of the frame rows (row 0, the dummy frame, stays untouched).  fp32, fp16
+        or bf16: the device tensor has the host tensor's dtype (16-bit tracks cross the bus at half the bytes and are
+        aggregated as they are)."""
+        if (seq_host.device.type != "cpu" or seq_host.dtype not in self._TRACK_SUFFIX
                 or not seq_host.is_contiguous()):
-            raise SeamError(2, "upload_tracks: seq_host must be a contiguous fp32 or fp16 host tensor")
+            raise SeamError(2, "upload_tracks: seq_host must be a contiguous fp32, fp16 or bf16 host tensor")
         T1, Q, D = seq_host.shape
         if D != D_MODEL:
             raise SeamError(3, f"upload_tracks: feature size {D} != {D_MODEL}")
         out = torch.empty((T1, hi - lo, D), dtype=seq_host.dtype, device=self.device)
-        fn = self._lib.seam_upload_tracks_f16 if seq_host.dtype == torch.float16 else self._lib.seam_upload_tracks
+        # the _f16 entry copies any 2-byte element type
+        fn = self._lib.seam_upload_tracks if seq_host.element_size() == 4 else self._lib.seam_upload_tracks_f16
         self._check(fn(self._h, seq_host.data_ptr(), T1 - 1, Q, lo, hi, out.data_ptr(), self._stream()))
         return out
 
