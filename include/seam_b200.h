@@ -156,6 +156,14 @@ int seam_prepare_gallery(seam_handle* h, const float* g, int G, void* g16, float
  * gstat, bit-identical to seam_prepare_gallery of the widened rows (overflow flag included).  A gallery prepared this
  * way is scored through the _g16 entry points below. */
 int seam_prepare_gallery_f16(seam_handle* h, const void* g16, int G, float* cg, float* gstat, void* stream);
+/* Preparation of a bf16 gallery (the dtype torch.autocast(dtype=torch.bfloat16) produces): g (G,256) bf16, 256 contiguous
+ * bf16 values per row, 16-byte aligned (otherwise SEAM_ERR_UNSUPPORTED), is read only; g16 (G,256) fp16 is written as
+ * seam_prepare_gallery writes it.  A bf16 value need not be an fp16 one (above 65,504 it overflows, below 6.1e-5 it loses
+ * bits), so the bf16 rows cannot serve as the tensor-core operand themselves: the prepared gallery is g, g16 and cg,
+ * 1,028 instead of 1,540 bytes per row.  Widening bf16 to fp32 is exact, so g16, cg and gstat (overflow flag included)
+ * are bit-identical to seam_prepare_gallery of the widened rows.  A gallery prepared this way is scored through the
+ * _gbf16 entry points below.  Same parameters as seam_prepare_gallery. */
+int seam_prepare_gallery_bf16(seam_handle* h, const void* g, int G, void* g16, float* cg, float* gstat, void* stream);
 
 /* Fused scorer + top-k.  Replaces, for all queries at once, the per-query loop body
  * evaluate_movingfashion.py:263-269 (evaluate_multiDF2.py:220-226):
@@ -197,6 +205,15 @@ int seam_score_topk(seam_handle* h, const float* q, int Q, const float* g, const
 int seam_score_topk_g16(seam_handle* h, const float* q, int Q, const void* g16, const float* cg, const float* gstat,
                         int G, int index_offset, int k, float* out_score, float* out_margin, int32_t* out_idx,
                         int32_t* stats, void* workspace, size_t workspace_bytes, void* stream);
+/* The _gbf16 entry points take a bf16 gallery prepared by seam_prepare_gallery_bf16: each has exactly the parameter list
+ * of its fp32 twin, with the rows g typed const void* and holding (G,256) bf16, 16-byte aligned (otherwise
+ * SEAM_ERR_UNSUPPORTED).  g16 is the fp16 image that preparation wrote.  The direct form reads g widened exactly, the
+ * tensor-core pass reads g16, so every score, margin, index, rank, count and stats counter is bit-identical to the fp32
+ * entry on the widened gallery g.float(); everything else as the fp32 twin.
+ * seam_score_topk for a bf16 gallery: */
+int seam_score_topk_gbf16(seam_handle* h, const float* q, int Q, const void* g, const void* g16, const float* cg,
+                          const float* gstat, int G, int index_offset, int k, float* out_score, float* out_margin,
+                          int32_t* out_idx, int32_t* stats, void* workspace, size_t workspace_bytes, void* stream);
 
 /* seam_aggregate + seam_score_topk in one call: tracks in, descriptors (q_out (Q,256) = x3_1b) and per-query top-k
  * out -- the whole per-product loop body evaluate_movingfashion.py:252-277 for all products at once; same results as
@@ -234,6 +251,23 @@ int seam_search_bf16_g16(seam_handle* h, const void* seq, const uint8_t* mask, c
                          int64_t frame_stride, int64_t track_stride, float* q_out, const void* g16, const float* cg,
                          const float* gstat, int G, int index_offset, int k, float* out_score, float* out_margin,
                          int32_t* out_idx, int32_t* stats, void* workspace, size_t workspace_bytes, void* stream);
+/* seam_search / seam_search_f16 / seam_search_bf16 (fp32 / fp16 / bf16 tracks) for a bf16 gallery (see
+ * seam_score_topk_gbf16). */
+int seam_search_gbf16(seam_handle* h, const float* seq, const uint8_t* mask, const int32_t* lens, int Tmax, int Q,
+                      int64_t frame_stride, int64_t track_stride, float* q_out, const void* g, const void* g16,
+                      const float* cg, const float* gstat, int G, int index_offset, int k, float* out_score,
+                      float* out_margin, int32_t* out_idx, int32_t* stats, void* workspace, size_t workspace_bytes,
+                      void* stream);
+int seam_search_f16_gbf16(seam_handle* h, const void* seq, const uint8_t* mask, const int32_t* lens, int Tmax, int Q,
+                          int64_t frame_stride, int64_t track_stride, float* q_out, const void* g, const void* g16,
+                          const float* cg, const float* gstat, int G, int index_offset, int k, float* out_score,
+                          float* out_margin, int32_t* out_idx, int32_t* stats, void* workspace, size_t workspace_bytes,
+                          void* stream);
+int seam_search_bf16_gbf16(seam_handle* h, const void* seq, const uint8_t* mask, const int32_t* lens, int Tmax, int Q,
+                           int64_t frame_stride, int64_t track_stride, float* q_out, const void* g, const void* g16,
+                           const float* cg, const float* gstat, int G, int index_offset, int k, float* out_score,
+                           float* out_margin, int32_t* out_idx, int32_t* stats, void* workspace, size_t workspace_bytes,
+                           void* stream);
 
 /* Dense logits (parity / small problems): x5 (Q,G,2) fp32 = last((q-g)^2).
  * models/match_head.py:160-162 and MatchPredictor.forward :70-74. */
@@ -256,6 +290,10 @@ int seam_rank_fused_distances(seam_handle* h, const float* frames, const int32_t
  * ranks as the fp32 entry on the widened gallery, bit for bit (frames stay fp32). */
 int seam_rank_fused_distances_g16(seam_handle* h, const float* frames, const int32_t* start, int P, const void* g16,
                                   int G, const int32_t* target, int32_t* rank_avg, int32_t* rank_max, void* stream);
+/* seam_rank_fused_distances for a bf16 gallery g (G,256), 16-byte aligned (else SEAM_ERR_UNSUPPORTED): the same ranks as
+ * the fp32 entry on the widened gallery, bit for bit.  Reads the rows only, so g need not be prepared. */
+int seam_rank_fused_distances_gbf16(seam_handle* h, const float* frames, const int32_t* start, int P, const void* g,
+                                    int G, const int32_t* target, int32_t* rank_avg, int32_t* rank_max, void* stream);
 
 /* Rank of one designated gallery item per query (0 = best), the quantity the eval script
  * reads out of its full argsort: evaluate_movingfashion.py:268-269.
@@ -281,6 +319,11 @@ int seam_rank_of_target_prepared_g16(seam_handle* h, const float* q, int Q, cons
                                      const float* gstat, int G, const int32_t* target, int32_t* out_rank,
                                      float* out_margin, int32_t* stats, void* workspace, size_t workspace_bytes,
                                      void* stream);
+/* seam_rank_of_target_prepared for a bf16 gallery (see seam_score_topk_gbf16), its exhaustive fallback included. */
+int seam_rank_of_target_prepared_gbf16(seam_handle* h, const float* q, int Q, const void* g, const void* g16,
+                                       const float* cg, const float* gstat, int G, const int32_t* target,
+                                       int32_t* out_rank, float* out_margin, int32_t* stats, void* workspace,
+                                       size_t workspace_bytes, void* stream);
 
 /* Rank of the target over a gallery split into shards (one per GPU), exactly: for global target t,
  *   rank_i = sum over shards s of #{ j in s : (d_ij, j) ranks before (d_it, t) }   (ties by GLOBAL row).
@@ -294,12 +337,15 @@ int seam_rank_of_target_prepared_g16(seam_handle* h, const float* q, int Q, cons
  *      (their number in stats[0]);
  * then an all-reduce SUM of the counts gives the unsharded rank, integer for integer.
  *   target (Q) int32 GLOBAL gallery rows; index_offset >= 0 (else SEAM_ERR_BAD_ARG); target_margin must not be null
- *   (SEAM_ERR_BAD_ARG); Q == 0 is a no-op.  The _g16 forms take an fp16 shard (see seam_score_topk_g16), 16-byte
- *   aligned (else SEAM_ERR_UNSUPPORTED), and give the fp32 forms' results on the widened rows. */
+ *   (SEAM_ERR_BAD_ARG); Q == 0 is a no-op.  The _g16 forms take an fp16 shard (see seam_score_topk_g16), the _gbf16
+ *   forms a bf16 shard (see seam_score_topk_gbf16), 16-byte aligned (else SEAM_ERR_UNSUPPORTED), and give the fp32
+ *   forms' results on the widened rows. */
 int seam_shard_target_margin(seam_handle* h, const float* q, int Q, const float* g, int G, int index_offset,
                              const int32_t* target, float* out_margin, void* stream);
 int seam_shard_target_margin_g16(seam_handle* h, const float* q, int Q, const void* g16, int G, int index_offset,
                                  const int32_t* target, float* out_margin, void* stream);
+int seam_shard_target_margin_gbf16(seam_handle* h, const float* q, int Q, const void* g, int G, int index_offset,
+                                   const int32_t* target, float* out_margin, void* stream);
 int seam_shard_rank_count_prepared(seam_handle* h, const float* q, int Q, const float* g, const void* g16,
                                    const float* cg, const float* gstat, int G, int index_offset, const int32_t* target,
                                    const float* target_margin, int32_t* out_count, int32_t* stats, void* workspace,
@@ -308,6 +354,10 @@ int seam_shard_rank_count_prepared_g16(seam_handle* h, const float* q, int Q, co
                                        const float* gstat, int G, int index_offset, const int32_t* target,
                                        const float* target_margin, int32_t* out_count, int32_t* stats,
                                        void* workspace, size_t workspace_bytes, void* stream);
+int seam_shard_rank_count_prepared_gbf16(seam_handle* h, const float* q, int Q, const void* g, const void* g16,
+                                         const float* cg, const float* gstat, int G, int index_offset,
+                                         const int32_t* target, const float* target_margin, int32_t* out_count,
+                                         int32_t* stats, void* workspace, size_t workspace_bytes, void* stream);
 
 /* The "AVG & MAX DISTANCE" fusions (seam_rank_fused_distances) over a gallery split into shards, exactly: for global
  * target t of product p and either fusion f (average or maximum of the frames' class-1 probabilities),
@@ -322,13 +372,16 @@ int seam_shard_rank_count_prepared_g16(seam_handle* h, const float* q, int Q, co
  *      target_max (zero-filled here; a product without frames gets this shard's G, so the sum is the whole G);
  * then an all-reduce SUM of the counts gives the unsharded ranks, integer for integer.
  *   target (P) int32 GLOBAL gallery rows; index_offset >= 0 (else SEAM_ERR_BAD_ARG); target_avg / target_max must not
- *   be null (SEAM_ERR_BAD_ARG); P == 0 is a no-op.  The _g16 forms take an fp16 shard, 16-byte aligned (else
- *   SEAM_ERR_UNSUPPORTED), and give the fp32 forms' results on the widened rows. */
+ *   be null (SEAM_ERR_BAD_ARG); P == 0 is a no-op.  The _g16 forms take an fp16 shard, the _gbf16 forms a bf16 shard,
+ *   16-byte aligned (else SEAM_ERR_UNSUPPORTED), and give the fp32 forms' results on the widened rows. */
 int seam_shard_fused_target(seam_handle* h, const float* frames, const int32_t* start, int P, const float* g, int G,
                             int index_offset, const int32_t* target, float* out_avg, float* out_max, void* stream);
 int seam_shard_fused_target_g16(seam_handle* h, const float* frames, const int32_t* start, int P, const void* g16,
                                 int G, int index_offset, const int32_t* target, float* out_avg, float* out_max,
                                 void* stream);
+int seam_shard_fused_target_gbf16(seam_handle* h, const float* frames, const int32_t* start, int P, const void* g, int G,
+                                  int index_offset, const int32_t* target, float* out_avg, float* out_max,
+                                  void* stream);
 int seam_shard_rank_fused_distances(seam_handle* h, const float* frames, const int32_t* start, int P, const float* g,
                                     int G, int index_offset, const int32_t* target, const float* target_avg,
                                     const float* target_max, int32_t* rank_avg, int32_t* rank_max, void* stream);
@@ -336,6 +389,10 @@ int seam_shard_rank_fused_distances_g16(seam_handle* h, const float* frames, con
                                         const void* g16, int G, int index_offset, const int32_t* target,
                                         const float* target_avg, const float* target_max, int32_t* rank_avg,
                                         int32_t* rank_max, void* stream);
+int seam_shard_rank_fused_distances_gbf16(seam_handle* h, const float* frames, const int32_t* start, int P,
+                                          const void* g, int G, int index_offset, const int32_t* target,
+                                          const float* target_avg, const float* target_max, int32_t* rank_avg,
+                                          int32_t* rank_max, void* stream);
 
 /* Merge N per-shard top-k lists (after the all-gather) into one: lists are (N,Q,k)
  * contiguous; entries with idx < 0 are invalid.  Same ordering contract as seam_score_topk.
@@ -408,6 +465,10 @@ int seam_sharded_score_topk(seam_handle* h, const seam_exchange* x, const float*
 int seam_sharded_score_topk_g16(seam_handle* h, const seam_exchange* x, const void* g16, const float* cg,
                                 const float* gstat, int G, int index_offset, int32_t* stats, void* workspace,
                                 size_t workspace_bytes, void* stream);
+/* seam_sharded_score_topk for a bf16 gallery shard (see seam_score_topk_gbf16). */
+int seam_sharded_score_topk_gbf16(seam_handle* h, const seam_exchange* x, const void* g, const void* g16,
+                                  const float* cg, const float* gstat, int G, int index_offset, int32_t* stats,
+                                  void* workspace, size_t workspace_bytes, void* stream);
 /* Merges the world lists of the queries this rank owns and ends the step.  With final buffers in the exchange every
  * rank holds the complete (Q,k) result when its stream reaches the end of this call; without, out_* (own,k) receive
  * the owner's rows. */

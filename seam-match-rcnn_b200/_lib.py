@@ -121,6 +121,8 @@ def _declare(lib: C.CDLL) -> None:
     lib.seam_prepare_gallery.argtypes = [vp, vp, i32, vp, vp, vp, vp]
     lib.seam_prepare_gallery_f16.restype = i32
     lib.seam_prepare_gallery_f16.argtypes = [vp, vp, i32, vp, vp, vp]
+    lib.seam_prepare_gallery_bf16.restype = i32
+    lib.seam_prepare_gallery_bf16.argtypes = lib.seam_prepare_gallery.argtypes
     lib.seam_score_workspace_bytes.restype = sz
     lib.seam_score_workspace_bytes.argtypes = [vp, i32, i32, i32]
     lib.seam_score_partition.restype = i32
@@ -131,6 +133,8 @@ def _declare(lib: C.CDLL) -> None:
     lib.seam_score_topk.argtypes = [vp, vp, i32, vp, vp, vp, vp, i32, i32, i32, vp, vp, vp, vp, vp, sz, vp]
     lib.seam_score_topk_g16.restype = i32
     lib.seam_score_topk_g16.argtypes = [vp, vp, i32, vp, vp, vp, i32, i32, i32, vp, vp, vp, vp, vp, sz, vp]
+    lib.seam_score_topk_gbf16.restype = i32
+    lib.seam_score_topk_gbf16.argtypes = lib.seam_score_topk.argtypes
     lib.seam_search.restype = i32
     lib.seam_search.argtypes = [vp, vp, vp, vp, i32, i32, i64, i64, vp, vp, vp, vp, vp, i32, i32, i32, vp, vp, vp, vp, vp, sz, vp]
     lib.seam_search_f16.restype = i32
@@ -143,6 +147,12 @@ def _declare(lib: C.CDLL) -> None:
     lib.seam_search_f16_g16.argtypes = lib.seam_search_g16.argtypes
     lib.seam_search_bf16_g16.restype = i32
     lib.seam_search_bf16_g16.argtypes = lib.seam_search_g16.argtypes
+    lib.seam_search_gbf16.restype = i32
+    lib.seam_search_gbf16.argtypes = lib.seam_search.argtypes
+    lib.seam_search_f16_gbf16.restype = i32
+    lib.seam_search_f16_gbf16.argtypes = lib.seam_search.argtypes
+    lib.seam_search_bf16_gbf16.restype = i32
+    lib.seam_search_bf16_gbf16.argtypes = lib.seam_search.argtypes
     lib.seam_score_dense.restype = i32
     lib.seam_score_dense.argtypes = [vp, vp, i32, vp, i32, vp, vp]
     lib.seam_score_prob.restype = i32
@@ -151,14 +161,20 @@ def _declare(lib: C.CDLL) -> None:
     lib.seam_rank_fused_distances.argtypes = [vp, vp, vp, i32, vp, i32, vp, vp, vp, vp]
     lib.seam_rank_fused_distances_g16.restype = i32
     lib.seam_rank_fused_distances_g16.argtypes = lib.seam_rank_fused_distances.argtypes
+    lib.seam_rank_fused_distances_gbf16.restype = i32
+    lib.seam_rank_fused_distances_gbf16.argtypes = lib.seam_rank_fused_distances.argtypes
     lib.seam_shard_fused_target.restype = i32
     lib.seam_shard_fused_target.argtypes = [vp, vp, vp, i32, vp, i32, i32, vp, vp, vp, vp]
     lib.seam_shard_fused_target_g16.restype = i32
     lib.seam_shard_fused_target_g16.argtypes = lib.seam_shard_fused_target.argtypes
+    lib.seam_shard_fused_target_gbf16.restype = i32
+    lib.seam_shard_fused_target_gbf16.argtypes = lib.seam_shard_fused_target.argtypes
     lib.seam_shard_rank_fused_distances.restype = i32
     lib.seam_shard_rank_fused_distances.argtypes = [vp, vp, vp, i32, vp, i32, i32, vp, vp, vp, vp, vp, vp]
     lib.seam_shard_rank_fused_distances_g16.restype = i32
     lib.seam_shard_rank_fused_distances_g16.argtypes = lib.seam_shard_rank_fused_distances.argtypes
+    lib.seam_shard_rank_fused_distances_gbf16.restype = i32
+    lib.seam_shard_rank_fused_distances_gbf16.argtypes = lib.seam_shard_rank_fused_distances.argtypes
     lib.seam_rank_of_target.restype = i32
     lib.seam_rank_of_target.argtypes = [vp, vp, i32, vp, i32, vp, vp, vp, vp]
     lib.seam_rank_workspace_bytes.restype = sz
@@ -167,14 +183,20 @@ def _declare(lib: C.CDLL) -> None:
     lib.seam_rank_of_target_prepared.argtypes = [vp, vp, i32, vp, vp, vp, vp, i32, vp, vp, vp, vp, vp, sz, vp]
     lib.seam_rank_of_target_prepared_g16.restype = i32
     lib.seam_rank_of_target_prepared_g16.argtypes = [vp, vp, i32, vp, vp, vp, i32, vp, vp, vp, vp, vp, sz, vp]
+    lib.seam_rank_of_target_prepared_gbf16.restype = i32
+    lib.seam_rank_of_target_prepared_gbf16.argtypes = lib.seam_rank_of_target_prepared.argtypes
     lib.seam_shard_target_margin.restype = i32
     lib.seam_shard_target_margin.argtypes = [vp, vp, i32, vp, i32, i32, vp, vp, vp]
     lib.seam_shard_target_margin_g16.restype = i32
     lib.seam_shard_target_margin_g16.argtypes = lib.seam_shard_target_margin.argtypes
+    lib.seam_shard_target_margin_gbf16.restype = i32
+    lib.seam_shard_target_margin_gbf16.argtypes = lib.seam_shard_target_margin.argtypes
     lib.seam_shard_rank_count_prepared.restype = i32
     lib.seam_shard_rank_count_prepared.argtypes = [vp, vp, i32, vp, vp, vp, vp, i32, i32, vp, vp, vp, vp, vp, sz, vp]
     lib.seam_shard_rank_count_prepared_g16.restype = i32
     lib.seam_shard_rank_count_prepared_g16.argtypes = [vp, vp, i32, vp, vp, vp, i32, i32, vp, vp, vp, vp, vp, sz, vp]
+    lib.seam_shard_rank_count_prepared_gbf16.restype = i32
+    lib.seam_shard_rank_count_prepared_gbf16.argtypes = lib.seam_shard_rank_count_prepared.argtypes
     xp = C.POINTER(SeamExchange)
     lib.seam_sharded_aggregate.restype = i32
     lib.seam_sharded_aggregate.argtypes = [vp, xp, vp, vp, vp, i32, i32, i64, i64, i32, i32, vp, vp]
@@ -186,6 +208,8 @@ def _declare(lib: C.CDLL) -> None:
     lib.seam_sharded_score_topk.argtypes = [vp, xp, vp, vp, vp, vp, i32, i32, vp, vp, sz, vp]
     lib.seam_sharded_score_topk_g16.restype = i32
     lib.seam_sharded_score_topk_g16.argtypes = [vp, xp, vp, vp, vp, i32, i32, vp, vp, sz, vp]
+    lib.seam_sharded_score_topk_gbf16.restype = i32
+    lib.seam_sharded_score_topk_gbf16.argtypes = lib.seam_sharded_score_topk.argtypes
     lib.seam_sharded_merge.restype = i32
     lib.seam_sharded_merge.argtypes = [vp, xp, vp, vp, vp, vp]
     lib.seam_aggregate_backward.restype = i32

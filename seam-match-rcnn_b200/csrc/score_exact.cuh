@@ -9,6 +9,7 @@
 #include <type_traits>
 #include <climits>
 #include <cstdint>
+#include <cuda_bf16.h>
 #include <cuda_fp16.h>
 #include "exchange.cuh"
 #include "fold.cuh"
@@ -53,6 +54,17 @@ __device__ __forceinline__ Slice load_slice(const __half* row, int lane) {
   s.hi = widen4(*reinterpret_cast<const uint2*>(row + 128 + 4 * lane));
   return s;
 }
+// ... and of a bf16 row: a bf16 value is the high half of its fp32 value, so widening is a shift / a mask (exact)
+__device__ __forceinline__ float4 widen4_bf16(uint2 v) {
+  return make_float4(__uint_as_float(v.x << 16), __uint_as_float(v.x & 0xffff0000u), __uint_as_float(v.y << 16),
+                     __uint_as_float(v.y & 0xffff0000u));
+}
+__device__ __forceinline__ Slice load_slice(const __nv_bfloat16* row, int lane) {
+  Slice s;
+  s.lo = widen4_bf16(*reinterpret_cast<const uint2*>(row + 4 * lane));
+  s.hi = widen4_bf16(*reinterpret_cast<const uint2*>(row + 128 + 4 * lane));
+  return s;
+}
 // Packed fp32 pairs (sub/mul/fma .f32x2 = one issue slot for two IEEE fp32 operations: every kernel
 // here is bound by instruction issue).  Each lane forms two partial sums per logit (even / odd
 // channels of its slice) and adds them at the end.
@@ -85,7 +97,7 @@ __device__ __forceinline__ void sqdiff_dot2(const Slice& q, const Slice& g, cons
   p0 = sum2(a0);
   p1 = sum2(a1);
 }
-// both logits of one pair, all lanes get the result; Row: float or __half gallery rows
+// both logits of one pair, all lanes get the result; Row: float, __half or __nv_bfloat16 gallery rows
 template <typename Row>
 __device__ __forceinline__ void pair_logits(const Slice& q, const Row* grow, const Slice& w0, const Slice& w1,
                                             float b0, float b1, int lane, float& l0, float& l1) {
@@ -98,7 +110,9 @@ __device__ __forceinline__ void pair_logits(const Slice& q, const Row* grow, con
 
 // ---------------------------------------------------------------- gallery preparation
 // warp per gallery row: fp16 copy, cg_j = dw . g_j^2, max_j ||g_j|| (gstat[0]), overflow flag (gstat[1]).
-// Row = __half: the caller's rows are the fp16 operand already -- cg and gstat only (g16 is not written).
+// Row = __half: the caller's rows are the fp16 operand already -- cg and gstat only (g16 is not written).  Row =
+// __nv_bfloat16 writes g16 as fp32 does: a bf16 value need not be an fp16 one (range, subnormals), and __float2half_rn
+// of the exactly widened value is the fp32 path's g16 bit for bit.
 template <typename Row>
 __global__ void __launch_bounds__(256) prep_gallery_kernel(const Row* __restrict__ g, int G,
                                                            const float* __restrict__ fold, __half* __restrict__ g16,
@@ -119,7 +133,7 @@ __global__ void __launch_bounds__(256) prep_gallery_kernel(const Row* __restrict
     amax = fmaxf(amax, fabsf(xs[e]));
     h[e] = __float2half_rn(xs[e]);
   }
-  if constexpr (std::is_same<Row, float>::value) {
+  if constexpr (!std::is_same<Row, __half>::value) {
     __half* dst = g16 + (size_t)j * 256;
     *reinterpret_cast<uint2*>(dst + 4 * lane) = *reinterpret_cast<const uint2*>(&h[0]);
     *reinterpret_cast<uint2*>(dst + 128 + 4 * lane) = *reinterpret_cast<const uint2*>(&h[4]);
@@ -189,7 +203,7 @@ __global__ void __launch_bounds__(256) prep_queries_kernel(const float* q, int Q
 // ---------------------------------------------------------------- re-score + certify
 struct RescoreParams {
   const float* q;        // (Q,256)
-  const void* g;         // (G,256) rows of the kernel's Row type (float or __half)
+  const void* g;         // (G,256) rows of the kernel's Row type (float, __half or __nv_bfloat16)
   const float* fold;
   const uint2* rowbuf;         // (Q,nlists,CAP x 8 bytes): CAP/2 quad records {w0,w1,w2,w3} per sub-list
   const uint32_t* rowcnt;      // (Q,nlists) quad records in each sub-list
@@ -720,7 +734,7 @@ __global__ void __launch_bounds__(256) dense_logits_kernel(const float* __restri
 struct FusedDistParams {
   const float* frames;
   const int32_t* start;
-  const void* g;             // Row (float / __half) rows
+  const void* g;             // Row (float / __half / __nv_bfloat16) rows
   const int32_t* target;
   const float* fold;
   int P, G;

@@ -572,9 +572,12 @@ int seam_nlb_forward(seam_handle* h, const float* x, int B, int T, float* z, voi
 }
 
 // ------------------------------------------------------------------------------ scorer
-// rows: the gallery's (G,256) rows, fp32 or (rows_f16) fp16.  An fp16 gallery is its own tensor-core operand: g16 is
-// then the same pointer and is not written.
-static int prepare_gallery_impl(seam_handle* h, const void* rows, bool rows_f16, void* g16, int G, float* cg,
+// the element type of a gallery's (G,256) rows, as the entry point that received them says.  An fp16 gallery is its own
+// tensor-core operand (g16 is the same pointer as the rows); fp32 and bf16 rows have a separate fp16 image g16.
+enum class RowType { F32, F16, BF16 };
+
+// rows: the gallery's (G,256) rows of type rt.  For an fp16 gallery g16 is the same pointer and is not written.
+static int prepare_gallery_impl(seam_handle* h, const void* rows, RowType rt, void* g16, int G, float* cg,
                                 float* gstat, void* stream_, const char* who) {
   if (!h) return SEAM_ERR_BAD_ARG;
   if (!h->have_scorer) return fail(h, SEAM_ERR_STATE, "%s: scorer weights not loaded", who);
@@ -588,9 +591,12 @@ static int prepare_gallery_impl(seam_handle* h, const void* rows, bool rows_f16,
   if (!aligned16(rows) || !aligned16(g16)) return fail(h, SEAM_ERR_UNSUPPORTED, "%s: 16-byte alignment", who);
   {
     ProfileScope prof(h, SEAM_KERNEL_PREP_GALLERY, stream);
-    if (rows_f16)
+    if (rt == RowType::F16)
       exact::prep_gallery_kernel<__half><<<(G + 7) / 8, 256, 0, stream>>>(static_cast<const __half*>(rows), G, h->fold,
                                                                           nullptr, cg, gstat);
+    else if (rt == RowType::BF16)
+      exact::prep_gallery_kernel<__nv_bfloat16><<<(G + 7) / 8, 256, 0, stream>>>(
+          static_cast<const __nv_bfloat16*>(rows), G, h->fold, static_cast<__half*>(g16), cg, gstat);
     else
       exact::prep_gallery_kernel<float><<<(G + 7) / 8, 256, 0, stream>>>(static_cast<const float*>(rows), G, h->fold,
                                                                          static_cast<__half*>(g16), cg, gstat);
@@ -600,11 +606,16 @@ static int prepare_gallery_impl(seam_handle* h, const void* rows, bool rows_f16,
 }
 
 int seam_prepare_gallery(seam_handle* h, const float* g, int G, void* g16, float* cg, float* gstat, void* stream_) {
-  return prepare_gallery_impl(h, g, false, g16, G, cg, gstat, stream_, "seam_prepare_gallery");
+  return prepare_gallery_impl(h, g, RowType::F32, g16, G, cg, gstat, stream_, "seam_prepare_gallery");
 }
 
 int seam_prepare_gallery_f16(seam_handle* h, const void* g16, int G, float* cg, float* gstat, void* stream_) {
-  return prepare_gallery_impl(h, g16, true, const_cast<void*>(g16), G, cg, gstat, stream_, "seam_prepare_gallery_f16");
+  return prepare_gallery_impl(h, g16, RowType::F16, const_cast<void*>(g16), G, cg, gstat, stream_,
+                              "seam_prepare_gallery_f16");
+}
+
+int seam_prepare_gallery_bf16(seam_handle* h, const void* g, int G, void* g16, float* cg, float* gstat, void* stream_) {
+  return prepare_gallery_impl(h, g, RowType::BF16, g16, G, cg, gstat, stream_, "seam_prepare_gallery_bf16");
 }
 
 struct ScorePlan {
@@ -875,10 +886,10 @@ static int score_kernel_args(seam_handle* h, const ScoreWorkspace& w, int Q, con
   return SEAM_OK;
 }
 
-// rows: the gallery rows of the direct form, fp32 or (rows_f16) fp16 -- then the same pointer as g16.  who names the
-// entry point in errors, xwho the sharded entry in the check only a sharded call can fail.
+// rows: the gallery rows of the direct form, of type rt (for fp16 the same pointer as g16).  who names the entry point
+// in errors, xwho the sharded entry in the check only a sharded call can fail.
 static int score_topk_impl(seam_handle* h, const xchg::Exchange* x, const float* q, int Q, const void* rows,
-                           bool rows_f16, const void* g16, const float* cg, const float* gstat, int G, int index_offset,
+                           RowType rt, const void* g16, const float* cg, const float* gstat, int G, int index_offset,
                            int k, float* out_score, float* out_margin, int32_t* out_idx, int32_t* stats, void* workspace,
                            size_t workspace_bytes, void* stream_, const char* who, const char* xwho) {
   if (!h->have_scorer) return fail(h, SEAM_ERR_STATE, "%s: scorer weights not loaded", who);
@@ -950,7 +961,8 @@ static int score_topk_impl(seam_handle* h, const xchg::Exchange* x, const float*
   rp.plan = w.plan.tiles;
   {
     ProfileScope prof(h, SEAM_KERNEL_RESCORE, stream);
-    if (rows_f16) exact::rescore_kernel<__half><<<(Q + 7) / 8, 256, 0, stream>>>(rp);
+    if (rt == RowType::F16) exact::rescore_kernel<__half><<<(Q + 7) / 8, 256, 0, stream>>>(rp);
+    else if (rt == RowType::BF16) exact::rescore_kernel<__nv_bfloat16><<<(Q + 7) / 8, 256, 0, stream>>>(rp);
     else exact::rescore_kernel<float><<<(Q + 7) / 8, 256, 0, stream>>>(rp);
     SEAM_LAUNCHED(h, "rescore_kernel");
   }
@@ -975,7 +987,8 @@ static int score_topk_impl(seam_handle* h, const xchg::Exchange* x, const float*
   ep.x = xe;
   {
     ProfileScope prof(h, SEAM_KERNEL_EXACT, stream);
-    if (rows_f16) exact::exact_topk_kernel<__half><<<2 * h->num_sms, 256, 0, stream>>>(ep);
+    if (rt == RowType::F16) exact::exact_topk_kernel<__half><<<2 * h->num_sms, 256, 0, stream>>>(ep);
+    else if (rt == RowType::BF16) exact::exact_topk_kernel<__nv_bfloat16><<<2 * h->num_sms, 256, 0, stream>>>(ep);
     else exact::exact_topk_kernel<float><<<2 * h->num_sms, 256, 0, stream>>>(ep);
     SEAM_LAUNCHED(h, "exact_topk_kernel");
   }
@@ -987,22 +1000,31 @@ int seam_score_topk(seam_handle* h, const float* q, int Q, const float* g, const
                     const float* gstat, int G, int index_offset, int k, float* out_score, float* out_margin,
                     int32_t* out_idx, int32_t* stats, void* workspace, size_t workspace_bytes, void* stream_) {
   if (!h) return SEAM_ERR_BAD_ARG;
-  return score_topk_impl(h, nullptr, q, Q, g, false, g16, cg, gstat, G, index_offset, k, out_score, out_margin, out_idx,
-                         stats, workspace, workspace_bytes, stream_, "seam_score_topk", "seam_score_topk");
+  return score_topk_impl(h, nullptr, q, Q, g, RowType::F32, g16, cg, gstat, G, index_offset, k, out_score, out_margin,
+                         out_idx, stats, workspace, workspace_bytes, stream_, "seam_score_topk", "seam_score_topk");
 }
 
 int seam_score_topk_g16(seam_handle* h, const float* q, int Q, const void* g16, const float* cg, const float* gstat,
                         int G, int index_offset, int k, float* out_score, float* out_margin, int32_t* out_idx,
                         int32_t* stats, void* workspace, size_t workspace_bytes, void* stream_) {
   if (!h) return SEAM_ERR_BAD_ARG;
-  return score_topk_impl(h, nullptr, q, Q, g16, true, g16, cg, gstat, G, index_offset, k, out_score, out_margin, out_idx,
-                         stats, workspace, workspace_bytes, stream_, "seam_score_topk_g16", "seam_score_topk_g16");
+  return score_topk_impl(h, nullptr, q, Q, g16, RowType::F16, g16, cg, gstat, G, index_offset, k, out_score, out_margin,
+                         out_idx, stats, workspace, workspace_bytes, stream_, "seam_score_topk_g16", "seam_score_topk_g16");
 }
 
-// tt: the tracks' element type; rows / rows_f16: the gallery rows as in score_topk_impl.  Scorer errors name score_who.
+int seam_score_topk_gbf16(seam_handle* h, const float* q, int Q, const void* g, const void* g16, const float* cg,
+                          const float* gstat, int G, int index_offset, int k, float* out_score, float* out_margin,
+                          int32_t* out_idx, int32_t* stats, void* workspace, size_t workspace_bytes, void* stream_) {
+  if (!h) return SEAM_ERR_BAD_ARG;
+  return score_topk_impl(h, nullptr, q, Q, g, RowType::BF16, g16, cg, gstat, G, index_offset, k, out_score, out_margin,
+                         out_idx, stats, workspace, workspace_bytes, stream_, "seam_score_topk_gbf16",
+                         "seam_score_topk_gbf16");
+}
+
+// tt: the tracks' element type; rows / rt: the gallery rows as in score_topk_impl.  Scorer errors name score_who.
 static int search_impl(seam_handle* h, const void* seq, TrackType tt, const uint8_t* mask, const int32_t* lens,
                        int Tmax, int Q, int64_t frame_stride, int64_t track_stride, float* q_out, const void* rows,
-                       bool rows_f16, const void* g16, const float* cg, const float* gstat, int G, int index_offset, int k,
+                       RowType rt, const void* g16, const float* cg, const float* gstat, int G, int index_offset, int k,
                        float* out_score, float* out_margin, int32_t* out_idx, int32_t* stats, void* workspace,
                        size_t workspace_bytes, void* stream_, const char* who, const char* score_who) {
   if (!h) return SEAM_ERR_BAD_ARG;
@@ -1010,7 +1032,7 @@ static int search_impl(seam_handle* h, const void* seq, TrackType tt, const uint
   int rc = aggregate_impl(h, nullptr, 0, 0, seq, tt, mask, lens, Tmax, Q, frame_stride, track_stride, q_out, nullptr,
                           static_cast<cudaStream_t>(stream_), who);
   if (rc != SEAM_OK) return rc;
-  return score_topk_impl(h, nullptr, q_out, Q, rows, rows_f16, g16, cg, gstat, G, index_offset, k, out_score, out_margin,
+  return score_topk_impl(h, nullptr, q_out, Q, rows, rt, g16, cg, gstat, G, index_offset, k, out_score, out_margin,
                          out_idx, stats, workspace, workspace_bytes, stream_, score_who, score_who);
 }
 
@@ -1018,8 +1040,8 @@ int seam_search(seam_handle* h, const float* seq, const uint8_t* mask, const int
                 int64_t frame_stride, int64_t track_stride, float* q_out, const float* g, const void* g16, const float* cg,
                 const float* gstat, int G, int index_offset, int k, float* out_score, float* out_margin, int32_t* out_idx,
                 int32_t* stats, void* workspace, size_t workspace_bytes, void* stream_) {
-  return search_impl(h, seq, TrackType::F32, mask, lens, Tmax, Q, frame_stride, track_stride, q_out, g, false, g16, cg,
-                     gstat, G, index_offset, k, out_score, out_margin, out_idx, stats, workspace, workspace_bytes,
+  return search_impl(h, seq, TrackType::F32, mask, lens, Tmax, Q, frame_stride, track_stride, q_out, g, RowType::F32,
+                     g16, cg, gstat, G, index_offset, k, out_score, out_margin, out_idx, stats, workspace, workspace_bytes,
                      stream_, "seam_search", "seam_score_topk");
 }
 
@@ -1028,8 +1050,8 @@ int seam_search_f16(seam_handle* h, const void* seq, const uint8_t* mask, const 
                     const float* cg, const float* gstat, int G, int index_offset, int k, float* out_score,
                     float* out_margin, int32_t* out_idx, int32_t* stats, void* workspace, size_t workspace_bytes,
                     void* stream_) {
-  return search_impl(h, seq, TrackType::F16, mask, lens, Tmax, Q, frame_stride, track_stride, q_out, g, false, g16, cg,
-                     gstat, G, index_offset, k, out_score, out_margin, out_idx, stats, workspace, workspace_bytes,
+  return search_impl(h, seq, TrackType::F16, mask, lens, Tmax, Q, frame_stride, track_stride, q_out, g, RowType::F32,
+                     g16, cg, gstat, G, index_offset, k, out_score, out_margin, out_idx, stats, workspace, workspace_bytes,
                      stream_, "seam_search_f16", "seam_score_topk");
 }
 
@@ -1038,8 +1060,8 @@ int seam_search_bf16(seam_handle* h, const void* seq, const uint8_t* mask, const
                      const float* cg, const float* gstat, int G, int index_offset, int k, float* out_score,
                      float* out_margin, int32_t* out_idx, int32_t* stats, void* workspace, size_t workspace_bytes,
                      void* stream_) {
-  return search_impl(h, seq, TrackType::BF16, mask, lens, Tmax, Q, frame_stride, track_stride, q_out, g, false, g16, cg,
-                     gstat, G, index_offset, k, out_score, out_margin, out_idx, stats, workspace, workspace_bytes,
+  return search_impl(h, seq, TrackType::BF16, mask, lens, Tmax, Q, frame_stride, track_stride, q_out, g, RowType::F32,
+                     g16, cg, gstat, G, index_offset, k, out_score, out_margin, out_idx, stats, workspace, workspace_bytes,
                      stream_, "seam_search_bf16", "seam_score_topk");
 }
 
@@ -1047,8 +1069,8 @@ int seam_search_g16(seam_handle* h, const float* seq, const uint8_t* mask, const
                     int64_t frame_stride, int64_t track_stride, float* q_out, const void* g16, const float* cg,
                     const float* gstat, int G, int index_offset, int k, float* out_score, float* out_margin,
                     int32_t* out_idx, int32_t* stats, void* workspace, size_t workspace_bytes, void* stream_) {
-  return search_impl(h, seq, TrackType::F32, mask, lens, Tmax, Q, frame_stride, track_stride, q_out, g16, true, g16, cg,
-                     gstat, G, index_offset, k, out_score, out_margin, out_idx, stats, workspace, workspace_bytes,
+  return search_impl(h, seq, TrackType::F32, mask, lens, Tmax, Q, frame_stride, track_stride, q_out, g16, RowType::F16,
+                     g16, cg, gstat, G, index_offset, k, out_score, out_margin, out_idx, stats, workspace, workspace_bytes,
                      stream_, "seam_search_g16", "seam_search_g16");
 }
 
@@ -1056,8 +1078,8 @@ int seam_search_f16_g16(seam_handle* h, const void* seq, const uint8_t* mask, co
                         int64_t frame_stride, int64_t track_stride, float* q_out, const void* g16, const float* cg,
                         const float* gstat, int G, int index_offset, int k, float* out_score, float* out_margin,
                         int32_t* out_idx, int32_t* stats, void* workspace, size_t workspace_bytes, void* stream_) {
-  return search_impl(h, seq, TrackType::F16, mask, lens, Tmax, Q, frame_stride, track_stride, q_out, g16, true, g16, cg,
-                     gstat, G, index_offset, k, out_score, out_margin, out_idx, stats, workspace, workspace_bytes,
+  return search_impl(h, seq, TrackType::F16, mask, lens, Tmax, Q, frame_stride, track_stride, q_out, g16, RowType::F16,
+                     g16, cg, gstat, G, index_offset, k, out_score, out_margin, out_idx, stats, workspace, workspace_bytes,
                      stream_, "seam_search_f16_g16", "seam_search_f16_g16");
 }
 
@@ -1065,12 +1087,42 @@ int seam_search_bf16_g16(seam_handle* h, const void* seq, const uint8_t* mask, c
                          int64_t frame_stride, int64_t track_stride, float* q_out, const void* g16, const float* cg,
                          const float* gstat, int G, int index_offset, int k, float* out_score, float* out_margin,
                          int32_t* out_idx, int32_t* stats, void* workspace, size_t workspace_bytes, void* stream_) {
-  return search_impl(h, seq, TrackType::BF16, mask, lens, Tmax, Q, frame_stride, track_stride, q_out, g16, true, g16,
-                     cg, gstat, G, index_offset, k, out_score, out_margin, out_idx, stats, workspace, workspace_bytes,
+  return search_impl(h, seq, TrackType::BF16, mask, lens, Tmax, Q, frame_stride, track_stride, q_out, g16, RowType::F16,
+                     g16, cg, gstat, G, index_offset, k, out_score, out_margin, out_idx, stats, workspace, workspace_bytes,
                      stream_, "seam_search_bf16_g16", "seam_search_bf16_g16");
 }
 
-static int sharded_score_topk_impl(seam_handle* h, const seam_exchange* x, const void* rows, bool rows_f16,
+int seam_search_gbf16(seam_handle* h, const float* seq, const uint8_t* mask, const int32_t* lens, int Tmax, int Q,
+                      int64_t frame_stride, int64_t track_stride, float* q_out, const void* g, const void* g16,
+                      const float* cg, const float* gstat, int G, int index_offset, int k, float* out_score,
+                      float* out_margin, int32_t* out_idx, int32_t* stats, void* workspace, size_t workspace_bytes,
+                      void* stream_) {
+  return search_impl(h, seq, TrackType::F32, mask, lens, Tmax, Q, frame_stride, track_stride, q_out, g, RowType::BF16,
+                     g16, cg, gstat, G, index_offset, k, out_score, out_margin, out_idx, stats, workspace, workspace_bytes,
+                     stream_, "seam_search_gbf16", "seam_search_gbf16");
+}
+
+int seam_search_f16_gbf16(seam_handle* h, const void* seq, const uint8_t* mask, const int32_t* lens, int Tmax, int Q,
+                          int64_t frame_stride, int64_t track_stride, float* q_out, const void* g, const void* g16,
+                          const float* cg, const float* gstat, int G, int index_offset, int k, float* out_score,
+                          float* out_margin, int32_t* out_idx, int32_t* stats, void* workspace, size_t workspace_bytes,
+                          void* stream_) {
+  return search_impl(h, seq, TrackType::F16, mask, lens, Tmax, Q, frame_stride, track_stride, q_out, g, RowType::BF16,
+                     g16, cg, gstat, G, index_offset, k, out_score, out_margin, out_idx, stats, workspace, workspace_bytes,
+                     stream_, "seam_search_f16_gbf16", "seam_search_f16_gbf16");
+}
+
+int seam_search_bf16_gbf16(seam_handle* h, const void* seq, const uint8_t* mask, const int32_t* lens, int Tmax, int Q,
+                           int64_t frame_stride, int64_t track_stride, float* q_out, const void* g, const void* g16,
+                           const float* cg, const float* gstat, int G, int index_offset, int k, float* out_score,
+                           float* out_margin, int32_t* out_idx, int32_t* stats, void* workspace, size_t workspace_bytes,
+                           void* stream_) {
+  return search_impl(h, seq, TrackType::BF16, mask, lens, Tmax, Q, frame_stride, track_stride, q_out, g, RowType::BF16,
+                     g16, cg, gstat, G, index_offset, k, out_score, out_margin, out_idx, stats, workspace, workspace_bytes,
+                     stream_, "seam_search_bf16_gbf16", "seam_search_bf16_gbf16");
+}
+
+static int sharded_score_topk_impl(seam_handle* h, const seam_exchange* x, const void* rows, RowType rt,
                                    const void* g16, const float* cg, const float* gstat, int G, int index_offset,
                                    int32_t* stats, void* workspace, size_t workspace_bytes, void* stream_,
                                    const char* who, const char* score_who) {
@@ -1078,22 +1130,30 @@ static int sharded_score_topk_impl(seam_handle* h, const seam_exchange* x, const
   xchg::Exchange e;
   int rc = import_exchange(h, x, &e, who);
   if (rc != SEAM_OK) return rc;
-  return score_topk_impl(h, &e, nullptr, x->Q, rows, rows_f16, g16, cg, gstat, G, index_offset, x->k, nullptr, nullptr,
+  return score_topk_impl(h, &e, nullptr, x->Q, rows, rt, g16, cg, gstat, G, index_offset, x->k, nullptr, nullptr,
                          nullptr, stats, workspace, workspace_bytes, stream_, score_who, who);
 }
 
 int seam_sharded_score_topk(seam_handle* h, const seam_exchange* x, const float* g, const void* g16, const float* cg,
                             const float* gstat, int G, int index_offset, int32_t* stats, void* workspace,
                             size_t workspace_bytes, void* stream_) {
-  return sharded_score_topk_impl(h, x, g, false, g16, cg, gstat, G, index_offset, stats, workspace, workspace_bytes,
+  return sharded_score_topk_impl(h, x, g, RowType::F32, g16, cg, gstat, G, index_offset, stats, workspace, workspace_bytes,
                                  stream_, "seam_sharded_score_topk", "seam_score_topk");
 }
 
 int seam_sharded_score_topk_g16(seam_handle* h, const seam_exchange* x, const void* g16, const float* cg,
                                 const float* gstat, int G, int index_offset, int32_t* stats, void* workspace,
                                 size_t workspace_bytes, void* stream_) {
-  return sharded_score_topk_impl(h, x, g16, true, g16, cg, gstat, G, index_offset, stats, workspace, workspace_bytes,
-                                 stream_, "seam_sharded_score_topk_g16", "seam_sharded_score_topk_g16");
+  return sharded_score_topk_impl(h, x, g16, RowType::F16, g16, cg, gstat, G, index_offset, stats, workspace,
+                                 workspace_bytes, stream_, "seam_sharded_score_topk_g16", "seam_sharded_score_topk_g16");
+}
+
+int seam_sharded_score_topk_gbf16(seam_handle* h, const seam_exchange* x, const void* g, const void* g16,
+                                  const float* cg, const float* gstat, int G, int index_offset, int32_t* stats,
+                                  void* workspace, size_t workspace_bytes, void* stream_) {
+  return sharded_score_topk_impl(h, x, g, RowType::BF16, g16, cg, gstat, G, index_offset, stats, workspace,
+                                 workspace_bytes, stream_, "seam_sharded_score_topk_gbf16",
+                                 "seam_sharded_score_topk_gbf16");
 }
 
 int seam_sharded_merge(seam_handle* h, const seam_exchange* x, float* out_score, float* out_margin, int32_t* out_idx,
@@ -1142,10 +1202,10 @@ int seam_score_prob(seam_handle* h, const float* q, int Q, const float* g, int G
   return SEAM_OK;
 }
 
-// rows / rows_f16 as in score_topk_impl.  target_avg null: the whole gallery (index_offset 0); else one shard of it,
+// rows / rt as in score_topk_impl.  target_avg null: the whole gallery (index_offset 0); else one shard of it,
 // counting against the given target values (target[] holds global rows).
 static int fused_rank_impl(seam_handle* h, const float* frames, const int32_t* start, int P, const void* rows,
-                           bool rows_f16, int G, int index_offset, const int32_t* target, const float* target_avg,
+                           RowType rt, int G, int index_offset, const int32_t* target, const float* target_avg,
                            const float* target_max, int32_t* rank_avg, int32_t* rank_max, void* stream_,
                            const char* who) {
   if (!h) return SEAM_ERR_BAD_ARG;
@@ -1176,10 +1236,12 @@ static int fused_rank_impl(seam_handle* h, const float* frames, const int32_t* s
   fp.target_max = target_max;
   const dim3 grid((unsigned)P, (unsigned)chunks);
   if (target_avg) {
-    if (rows_f16) exact::fused_dist_rank_kernel<__half, true><<<grid, 256, 0, stream>>>(fp);
+    if (rt == RowType::F16) exact::fused_dist_rank_kernel<__half, true><<<grid, 256, 0, stream>>>(fp);
+    else if (rt == RowType::BF16) exact::fused_dist_rank_kernel<__nv_bfloat16, true><<<grid, 256, 0, stream>>>(fp);
     else exact::fused_dist_rank_kernel<float, true><<<grid, 256, 0, stream>>>(fp);
   } else {
-    if (rows_f16) exact::fused_dist_rank_kernel<__half, false><<<grid, 256, 0, stream>>>(fp);
+    if (rt == RowType::F16) exact::fused_dist_rank_kernel<__half, false><<<grid, 256, 0, stream>>>(fp);
+    else if (rt == RowType::BF16) exact::fused_dist_rank_kernel<__nv_bfloat16, false><<<grid, 256, 0, stream>>>(fp);
     else exact::fused_dist_rank_kernel<float, false><<<grid, 256, 0, stream>>>(fp);
   }
   SEAM_LAUNCHED(h, "fused_dist_rank_kernel");
@@ -1188,14 +1250,20 @@ static int fused_rank_impl(seam_handle* h, const float* frames, const int32_t* s
 
 int seam_rank_fused_distances(seam_handle* h, const float* frames, const int32_t* start, int P, const float* g, int G,
                               const int32_t* target, int32_t* rank_avg, int32_t* rank_max, void* stream_) {
-  return fused_rank_impl(h, frames, start, P, g, false, G, 0, target, nullptr, nullptr, rank_avg, rank_max, stream_,
+  return fused_rank_impl(h, frames, start, P, g, RowType::F32, G, 0, target, nullptr, nullptr, rank_avg, rank_max, stream_,
                          "seam_rank_fused_distances");
 }
 
 int seam_rank_fused_distances_g16(seam_handle* h, const float* frames, const int32_t* start, int P, const void* g16,
                                   int G, const int32_t* target, int32_t* rank_avg, int32_t* rank_max, void* stream_) {
-  return fused_rank_impl(h, frames, start, P, g16, true, G, 0, target, nullptr, nullptr, rank_avg, rank_max, stream_,
-                         "seam_rank_fused_distances_g16");
+  return fused_rank_impl(h, frames, start, P, g16, RowType::F16, G, 0, target, nullptr, nullptr, rank_avg, rank_max,
+                         stream_, "seam_rank_fused_distances_g16");
+}
+
+int seam_rank_fused_distances_gbf16(seam_handle* h, const float* frames, const int32_t* start, int P, const void* g,
+                                    int G, const int32_t* target, int32_t* rank_avg, int32_t* rank_max, void* stream_) {
+  return fused_rank_impl(h, frames, start, P, g, RowType::BF16, G, 0, target, nullptr, nullptr, rank_avg, rank_max,
+                         stream_, "seam_rank_fused_distances_gbf16");
 }
 
 // ------------------------------------------------------------------------------ fusions over a sharded gallery
@@ -1203,7 +1271,7 @@ int seam_rank_fused_distances_g16(seam_handle* h, const float* frames, const int
 // computes the target's fused values (-inf elsewhere, so a MAX all-reduce delivers them to every shard), every shard
 // counts against them, and the counts are summed.
 static int shard_fused_target_impl(seam_handle* h, const float* frames, const int32_t* start, int P, const void* rows,
-                                   bool rows_f16, int G, int index_offset, const int32_t* target, float* out_avg,
+                                   RowType rt, int G, int index_offset, const int32_t* target, float* out_avg,
                                    float* out_max, void* stream_, const char* who) {
   if (!h) return SEAM_ERR_BAD_ARG;
   if (!h->have_scorer) return fail(h, SEAM_ERR_STATE, "%s: scorer weights not loaded", who);
@@ -1224,7 +1292,9 @@ static int shard_fused_target_impl(seam_handle* h, const float* frames, const in
   fp.P = P;
   fp.G = G;
   fp.index_offset = index_offset;
-  if (rows_f16) exact::fused_target_kernel<__half><<<(P + 7) / 8, 256, 0, stream>>>(fp, out_avg, out_max);
+  if (rt == RowType::F16) exact::fused_target_kernel<__half><<<(P + 7) / 8, 256, 0, stream>>>(fp, out_avg, out_max);
+  else if (rt == RowType::BF16)
+    exact::fused_target_kernel<__nv_bfloat16><<<(P + 7) / 8, 256, 0, stream>>>(fp, out_avg, out_max);
   else exact::fused_target_kernel<float><<<(P + 7) / 8, 256, 0, stream>>>(fp, out_avg, out_max);
   SEAM_LAUNCHED(h, "fused_target_kernel");
   return SEAM_OK;
@@ -1232,15 +1302,22 @@ static int shard_fused_target_impl(seam_handle* h, const float* frames, const in
 
 int seam_shard_fused_target(seam_handle* h, const float* frames, const int32_t* start, int P, const float* g, int G,
                             int index_offset, const int32_t* target, float* out_avg, float* out_max, void* stream_) {
-  return shard_fused_target_impl(h, frames, start, P, g, false, G, index_offset, target, out_avg, out_max, stream_,
+  return shard_fused_target_impl(h, frames, start, P, g, RowType::F32, G, index_offset, target, out_avg, out_max, stream_,
                                  "seam_shard_fused_target");
 }
 
 int seam_shard_fused_target_g16(seam_handle* h, const float* frames, const int32_t* start, int P, const void* g16,
                                 int G, int index_offset, const int32_t* target, float* out_avg, float* out_max,
                                 void* stream_) {
-  return shard_fused_target_impl(h, frames, start, P, g16, true, G, index_offset, target, out_avg, out_max, stream_,
-                                 "seam_shard_fused_target_g16");
+  return shard_fused_target_impl(h, frames, start, P, g16, RowType::F16, G, index_offset, target, out_avg, out_max,
+                                 stream_, "seam_shard_fused_target_g16");
+}
+
+int seam_shard_fused_target_gbf16(seam_handle* h, const float* frames, const int32_t* start, int P, const void* g, int G,
+                                  int index_offset, const int32_t* target, float* out_avg, float* out_max,
+                                  void* stream_) {
+  return shard_fused_target_impl(h, frames, start, P, g, RowType::BF16, G, index_offset, target, out_avg, out_max,
+                                 stream_, "seam_shard_fused_target_gbf16");
 }
 
 int seam_shard_rank_fused_distances(seam_handle* h, const float* frames, const int32_t* start, int P, const float* g,
@@ -1248,7 +1325,7 @@ int seam_shard_rank_fused_distances(seam_handle* h, const float* frames, const i
                                     const float* target_max, int32_t* rank_avg, int32_t* rank_max, void* stream_) {
   if (h && P > 0 && (!target_avg || !target_max))
     return fail(h, SEAM_ERR_BAD_ARG, "seam_shard_rank_fused_distances: null target_avg / target_max");
-  return fused_rank_impl(h, frames, start, P, g, false, G, index_offset, target, target_avg, target_max, rank_avg,
+  return fused_rank_impl(h, frames, start, P, g, RowType::F32, G, index_offset, target, target_avg, target_max, rank_avg,
                          rank_max, stream_, "seam_shard_rank_fused_distances");
 }
 
@@ -1258,8 +1335,18 @@ int seam_shard_rank_fused_distances_g16(seam_handle* h, const float* frames, con
                                         int32_t* rank_max, void* stream_) {
   if (h && P > 0 && (!target_avg || !target_max))
     return fail(h, SEAM_ERR_BAD_ARG, "seam_shard_rank_fused_distances_g16: null target_avg / target_max");
-  return fused_rank_impl(h, frames, start, P, g16, true, G, index_offset, target, target_avg, target_max, rank_avg,
-                         rank_max, stream_, "seam_shard_rank_fused_distances_g16");
+  return fused_rank_impl(h, frames, start, P, g16, RowType::F16, G, index_offset, target, target_avg, target_max,
+                         rank_avg, rank_max, stream_, "seam_shard_rank_fused_distances_g16");
+}
+
+int seam_shard_rank_fused_distances_gbf16(seam_handle* h, const float* frames, const int32_t* start, int P,
+                                          const void* g, int G, int index_offset, const int32_t* target,
+                                          const float* target_avg, const float* target_max, int32_t* rank_avg,
+                                          int32_t* rank_max, void* stream_) {
+  if (h && P > 0 && (!target_avg || !target_max))
+    return fail(h, SEAM_ERR_BAD_ARG, "seam_shard_rank_fused_distances_gbf16: null target_avg / target_max");
+  return fused_rank_impl(h, frames, start, P, g, RowType::BF16, G, index_offset, target, target_avg, target_max,
+                         rank_avg, rank_max, stream_, "seam_shard_rank_fused_distances_gbf16");
 }
 
 int seam_rank_of_target(seam_handle* h, const float* q, int Q, const float* g, int G, const int32_t* target,
@@ -1344,9 +1431,9 @@ static int rank_launch(seam_handle* h, const ScoreWorkspace& w, const float* q, 
 }
 }  // extern "C++"
 
-// rows / rows_f16 as in score_topk_impl.  ext_margin null: the whole gallery (index_offset 0, out_margin optional);
+// rows / rt as in score_topk_impl.  ext_margin null: the whole gallery (index_offset 0, out_margin optional);
 // else one shard of it, counting against the given target margins (out_margin null).
-static int rank_prepared_impl(seam_handle* h, const float* q, int Q, const void* rows, bool rows_f16, const void* g16,
+static int rank_prepared_impl(seam_handle* h, const float* q, int Q, const void* rows, RowType rt, const void* g16,
                               const float* cg, const float* gstat, int G, int index_offset, const int32_t* target,
                               const float* ext_margin, int32_t* out_rank, float* out_margin, int32_t* stats,
                               void* workspace, size_t workspace_bytes, void* stream_, const char* who) {
@@ -1362,16 +1449,27 @@ static int rank_prepared_impl(seam_handle* h, const float* q, int Q, const void*
   ScoreWorkspace w;
   int rc = carve_score_workspace(h, who, true, q, Q, rows, g16, cg, gstat, G, workspace, workspace_bytes, &w);
   if (rc != SEAM_OK) return rc;
-  if (ext_margin)
-    rc = rows_f16 ? rank_launch<__half, true>(h, w, q, Q, rows, g16, cg, gstat, G, index_offset, target, ext_margin,
-                                              out_rank, nullptr, stream)
-                  : rank_launch<float, true>(h, w, q, Q, rows, g16, cg, gstat, G, index_offset, target, ext_margin,
-                                             out_rank, nullptr, stream);
-  else
-    rc = rows_f16 ? rank_launch<__half, false>(h, w, q, Q, rows, g16, cg, gstat, G, 0, target, nullptr, out_rank,
-                                               out_margin, stream)
-                  : rank_launch<float, false>(h, w, q, Q, rows, g16, cg, gstat, G, 0, target, nullptr, out_rank,
-                                              out_margin, stream);
+  if (ext_margin) {
+    if (rt == RowType::F16)
+      rc = rank_launch<__half, true>(h, w, q, Q, rows, g16, cg, gstat, G, index_offset, target, ext_margin, out_rank,
+                                     nullptr, stream);
+    else if (rt == RowType::BF16)
+      rc = rank_launch<__nv_bfloat16, true>(h, w, q, Q, rows, g16, cg, gstat, G, index_offset, target, ext_margin,
+                                            out_rank, nullptr, stream);
+    else
+      rc = rank_launch<float, true>(h, w, q, Q, rows, g16, cg, gstat, G, index_offset, target, ext_margin, out_rank,
+                                    nullptr, stream);
+  } else {
+    if (rt == RowType::F16)
+      rc = rank_launch<__half, false>(h, w, q, Q, rows, g16, cg, gstat, G, 0, target, nullptr, out_rank, out_margin,
+                                      stream);
+    else if (rt == RowType::BF16)
+      rc = rank_launch<__nv_bfloat16, false>(h, w, q, Q, rows, g16, cg, gstat, G, 0, target, nullptr, out_rank,
+                                             out_margin, stream);
+    else
+      rc = rank_launch<float, false>(h, w, q, Q, rows, g16, cg, gstat, G, 0, target, nullptr, out_rank, out_margin,
+                                     stream);
+  }
   if (rc != SEAM_OK) return rc;
   if (stats) SEAM_CUDA(h, cudaMemcpyAsync(stats, w.counters, 4, cudaMemcpyDeviceToDevice, stream));
   return SEAM_OK;
@@ -1381,7 +1479,7 @@ int seam_rank_of_target_prepared(seam_handle* h, const float* q, int Q, const fl
                                  const float* cg, const float* gstat, int G, const int32_t* target, int32_t* out_rank,
                                  float* out_margin, int32_t* stats, void* workspace, size_t workspace_bytes,
                                  void* stream_) {
-  return rank_prepared_impl(h, q, Q, g, false, g16, cg, gstat, G, 0, target, nullptr, out_rank, out_margin, stats,
+  return rank_prepared_impl(h, q, Q, g, RowType::F32, g16, cg, gstat, G, 0, target, nullptr, out_rank, out_margin, stats,
                             workspace, workspace_bytes, stream_, "seam_rank_of_target_prepared");
 }
 
@@ -1389,15 +1487,23 @@ int seam_rank_of_target_prepared_g16(seam_handle* h, const float* q, int Q, cons
                                      const float* gstat, int G, const int32_t* target, int32_t* out_rank,
                                      float* out_margin, int32_t* stats, void* workspace, size_t workspace_bytes,
                                      void* stream_) {
-  return rank_prepared_impl(h, q, Q, g16, true, g16, cg, gstat, G, 0, target, nullptr, out_rank, out_margin, stats,
-                            workspace, workspace_bytes, stream_, "seam_rank_of_target_prepared_g16");
+  return rank_prepared_impl(h, q, Q, g16, RowType::F16, g16, cg, gstat, G, 0, target, nullptr, out_rank, out_margin,
+                            stats, workspace, workspace_bytes, stream_, "seam_rank_of_target_prepared_g16");
+}
+
+int seam_rank_of_target_prepared_gbf16(seam_handle* h, const float* q, int Q, const void* g, const void* g16,
+                                       const float* cg, const float* gstat, int G, const int32_t* target,
+                                       int32_t* out_rank, float* out_margin, int32_t* stats, void* workspace,
+                                       size_t workspace_bytes, void* stream_) {
+  return rank_prepared_impl(h, q, Q, g, RowType::BF16, g16, cg, gstat, G, 0, target, nullptr, out_rank, out_margin,
+                            stats, workspace, workspace_bytes, stream_, "seam_rank_of_target_prepared_gbf16");
 }
 
 // ------------------------------------------------------------------------------ rank over a sharded gallery
 // rank_i = sum over shards s of #{ j in s : (d_ij, j) ranks before (d_it, t) }: the owner of row t computes the
 // target's margin (-inf elsewhere, so a MAX all-reduce delivers it to every shard), every shard counts against it, and
 // the counts are summed.
-static int shard_target_margin_impl(seam_handle* h, const float* q, int Q, const void* rows, bool rows_f16, int G,
+static int shard_target_margin_impl(seam_handle* h, const float* q, int Q, const void* rows, RowType rt, int G,
                                     int index_offset, const int32_t* target, float* out_margin, void* stream_,
                                     const char* who) {
   if (!h) return SEAM_ERR_BAD_ARG;
@@ -1409,9 +1515,12 @@ static int shard_target_margin_impl(seam_handle* h, const float* q, int Q, const
   if (!aligned16(q) || !aligned16(rows)) return fail(h, SEAM_ERR_UNSUPPORTED, "%s: q/g need 16-byte alignment", who);
   DeviceGuard guard(h->device);
   cudaStream_t stream = static_cast<cudaStream_t>(stream_);
-  if (rows_f16)
+  if (rt == RowType::F16)
     exact::target_margin_kernel<__half><<<(Q + 7) / 8, 256, 0, stream>>>(q, Q, static_cast<const __half*>(rows), G,
                                                                          index_offset, target, h->fold, out_margin);
+  else if (rt == RowType::BF16)
+    exact::target_margin_kernel<__nv_bfloat16><<<(Q + 7) / 8, 256, 0, stream>>>(
+        q, Q, static_cast<const __nv_bfloat16*>(rows), G, index_offset, target, h->fold, out_margin);
   else
     exact::target_margin_kernel<float><<<(Q + 7) / 8, 256, 0, stream>>>(q, Q, static_cast<const float*>(rows), G,
                                                                         index_offset, target, h->fold, out_margin);
@@ -1421,14 +1530,20 @@ static int shard_target_margin_impl(seam_handle* h, const float* q, int Q, const
 
 int seam_shard_target_margin(seam_handle* h, const float* q, int Q, const float* g, int G, int index_offset,
                              const int32_t* target, float* out_margin, void* stream_) {
-  return shard_target_margin_impl(h, q, Q, g, false, G, index_offset, target, out_margin, stream_,
+  return shard_target_margin_impl(h, q, Q, g, RowType::F32, G, index_offset, target, out_margin, stream_,
                                   "seam_shard_target_margin");
 }
 
 int seam_shard_target_margin_g16(seam_handle* h, const float* q, int Q, const void* g16, int G, int index_offset,
                                  const int32_t* target, float* out_margin, void* stream_) {
-  return shard_target_margin_impl(h, q, Q, g16, true, G, index_offset, target, out_margin, stream_,
+  return shard_target_margin_impl(h, q, Q, g16, RowType::F16, G, index_offset, target, out_margin, stream_,
                                   "seam_shard_target_margin_g16");
+}
+
+int seam_shard_target_margin_gbf16(seam_handle* h, const float* q, int Q, const void* g, int G, int index_offset,
+                                   const int32_t* target, float* out_margin, void* stream_) {
+  return shard_target_margin_impl(h, q, Q, g, RowType::BF16, G, index_offset, target, out_margin, stream_,
+                                  "seam_shard_target_margin_gbf16");
 }
 
 int seam_shard_rank_count_prepared(seam_handle* h, const float* q, int Q, const float* g, const void* g16,
@@ -1437,7 +1552,7 @@ int seam_shard_rank_count_prepared(seam_handle* h, const float* q, int Q, const 
                                    size_t workspace_bytes, void* stream_) {
   if (h && Q > 0 && !target_margin)
     return fail(h, SEAM_ERR_BAD_ARG, "seam_shard_rank_count_prepared: null target_margin");
-  return rank_prepared_impl(h, q, Q, g, false, g16, cg, gstat, G, index_offset, target, target_margin, out_count,
+  return rank_prepared_impl(h, q, Q, g, RowType::F32, g16, cg, gstat, G, index_offset, target, target_margin, out_count,
                             nullptr, stats, workspace, workspace_bytes, stream_, "seam_shard_rank_count_prepared");
 }
 
@@ -1447,8 +1562,20 @@ int seam_shard_rank_count_prepared_g16(seam_handle* h, const float* q, int Q, co
                                        void* workspace, size_t workspace_bytes, void* stream_) {
   if (h && Q > 0 && !target_margin)
     return fail(h, SEAM_ERR_BAD_ARG, "seam_shard_rank_count_prepared_g16: null target_margin");
-  return rank_prepared_impl(h, q, Q, g16, true, g16, cg, gstat, G, index_offset, target, target_margin, out_count,
-                            nullptr, stats, workspace, workspace_bytes, stream_, "seam_shard_rank_count_prepared_g16");
+  return rank_prepared_impl(h, q, Q, g16, RowType::F16, g16, cg, gstat, G, index_offset, target, target_margin,
+                            out_count, nullptr, stats, workspace, workspace_bytes, stream_,
+                            "seam_shard_rank_count_prepared_g16");
+}
+
+int seam_shard_rank_count_prepared_gbf16(seam_handle* h, const float* q, int Q, const void* g, const void* g16,
+                                         const float* cg, const float* gstat, int G, int index_offset,
+                                         const int32_t* target, const float* target_margin, int32_t* out_count,
+                                         int32_t* stats, void* workspace, size_t workspace_bytes, void* stream_) {
+  if (h && Q > 0 && !target_margin)
+    return fail(h, SEAM_ERR_BAD_ARG, "seam_shard_rank_count_prepared_gbf16: null target_margin");
+  return rank_prepared_impl(h, q, Q, g, RowType::BF16, g16, cg, gstat, G, index_offset, target, target_margin,
+                            out_count, nullptr, stats, workspace, workspace_bytes, stream_,
+                            "seam_shard_rank_count_prepared_gbf16");
 }
 
 // ------------------------------------------------------------------------------ backward (f4)

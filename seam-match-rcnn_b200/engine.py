@@ -23,6 +23,9 @@ WEIGHT_SHAPES = {
     "concat_w": (1, 256, 1, 1), "att_w": (1, 256), "att_b": (1,), "last_w": (2, 256), "last_b": (2,),
 }
 SCORE_WS_LIMIT = 2 << 30      # bytes of scorer workspace above which score_topk works through the queries in slabs
+# gallery row dtype -> suffix of the C entry points that read such rows (fp16 rows are g16 itself; bf16 rows have an
+# fp16 image g16 beside them and take the fp32 entries' parameters)
+ROW_SUFFIX = {torch.float32: "", torch.float16: "_g16", torch.bfloat16: "_gbf16"}
 
 
 def _ptr(t: Optional[torch.Tensor]) -> Optional[int]:
@@ -33,14 +36,15 @@ def _ptr(t: Optional[torch.Tensor]) -> Optional[int]:
 class PreparedGallery:
     """A gallery shard resident on the device with its tensor-core operands.
 
-    g    (G,256) fp32   the shop descriptors (x3_2 of models/match_head.py:131/156), or fp16 when the caller's
-                        gallery is fp16: then it is the caller's tensor (or one contiguous copy of it) and
+    g    (G,256) fp32   the shop descriptors (x3_2 of models/match_head.py:131/156), or fp16 / bf16 when the
+                        caller's gallery has that dtype: then it is the caller's tensor (or one contiguous copy of it)
     g16  (G,256) fp16   operand of the tcgen05 pass -- the same tensor as ``g`` for an fp16 gallery
     cg   (G)     fp32   dw . g_j^2
     gstat (4)    fp32   [max_j ||g_j||, fp16-overflow flag, -, -]
 
-    An fp32 gallery holds 1,540 bytes per row (g, g16, cg), an fp16 one 516 (g16, cg); both score the same: the fp16
-    rows are widened exactly wherever the fp32 direct form reads them.
+    Bytes per row: fp32 1,540 (g, g16, cg), fp16 516 (g16, cg), bf16 1,028 (g, g16, cg).  All three score the same:
+    16-bit rows are widened exactly wherever the fp32 direct form reads them, and a bf16 gallery's g16 is the one its
+    fp32 widening would get (a bf16 value need not be an fp16 one, so bf16 rows cannot be the operand themselves).
     """
     g: torch.Tensor
     g16: torch.Tensor
@@ -57,6 +61,16 @@ class PreparedGallery:
     def rows_f16(self) -> bool:
         """The gallery rows are fp16 (``g is g16``): scored through the ``_g16`` entry points."""
         return self.g.dtype == torch.float16
+
+    @property
+    def rows_bf16(self) -> bool:
+        """The gallery rows are bf16 (with a separate fp16 ``g16``): scored through the ``_gbf16`` entry points."""
+        return self.g.dtype == torch.bfloat16
+
+    @property
+    def row_suffix(self) -> str:
+        """Suffix of the C entry points that score this gallery: ``""``, ``"_g16"`` or ``"_gbf16"``."""
+        return ROW_SUFFIX[self.g.dtype]
 
 
 class SeamEngine:
@@ -329,11 +343,14 @@ class SeamEngine:
 
     _TRACK_SUFFIX = {torch.float32: "", torch.float16: "_f16", torch.bfloat16: "_bf16"}
 
-    def _track_entry(self, op: str, seq: torch.Tensor, rows_f16: bool = False):
-        """The C entry point of ``op`` (``aggregate``, ``search`` or ``sharded_aggregate``) for tracks of ``seq``'s
-        dtype (as ``_tracks`` returns them), and for ``search`` against an fp16 gallery's rows when ``rows_f16``:
-        e.g. ``seam_search_bf16_g16``."""
-        return getattr(self._lib, f"seam_{op}{self._TRACK_SUFFIX[seq.dtype]}{'_g16' if rows_f16 else ''}")
+    def _track_entry(self, op: str, seq: Optional[torch.Tensor], rows=""):
+        """The C entry point of ``op`` for tracks of ``seq``'s dtype (as ``_tracks`` returns them; None for an op that
+        takes no tracks) against gallery rows of the type ``rows`` names: a ``PreparedGallery.row_suffix`` (``""``,
+        ``"_g16"``, ``"_gbf16"``), or a bool that says whether the rows are fp16.  E.g. ``seam_search_bf16_gbf16``,
+        ``seam_score_topk_g16``, ``seam_aggregate_f16``."""
+        if isinstance(rows, bool):
+            rows = "_g16" if rows else ""
+        return getattr(self._lib, f"seam_{op}{'' if seq is None else self._TRACK_SUFFIX[seq.dtype]}{rows}")
 
     def sharded_aggregate(self, x, seq: torch.Tensor, mask=None, lens=None, row0: Optional[int] = None,
                           last: bool = True, getatt: bool = False):
@@ -356,16 +373,12 @@ class SeamEngine:
         stats = torch.zeros((4,), dtype=torch.int32, device=self.device) if return_stats else None
         nbytes = int(self._lib.seam_score_workspace_bytes(self._h, x.Q, gallery.G, x.k))
         ws = self._workspace("score", nbytes)
-        if gallery.rows_f16:
-            self._check(self._lib.seam_sharded_score_topk_g16(self._h, C.byref(x.struct), gallery.g16.data_ptr(),
-                                                              gallery.cg.data_ptr(), gallery.gstat.data_ptr(), gallery.G,
-                                                              int(gallery.index_offset), _ptr(stats), ws.data_ptr(),
-                                                              ws.numel(), self._stream()))
-        else:
-            self._check(self._lib.seam_sharded_score_topk(self._h, C.byref(x.struct), gallery.g.data_ptr(),
-                                                          gallery.g16.data_ptr(), gallery.cg.data_ptr(),
-                                                          gallery.gstat.data_ptr(), gallery.G, int(gallery.index_offset),
-                                                          _ptr(stats), ws.data_ptr(), ws.numel(), self._stream()))
+        # an fp16 gallery has no separate rows: the _g16 entry reads g16 for both the operand and the direct form
+        fn = self._track_entry("sharded_score_topk", None, gallery.row_suffix)
+        rows = () if gallery.rows_f16 else (gallery.g.data_ptr(),)
+        self._check(fn(self._h, C.byref(x.struct), *rows, gallery.g16.data_ptr(), gallery.cg.data_ptr(),
+                       gallery.gstat.data_ptr(), gallery.G, int(gallery.index_offset), _ptr(stats), ws.data_ptr(),
+                       ws.numel(), self._stream()))
         return stats
 
     def sharded_merge(self, x):
@@ -400,19 +413,14 @@ class SeamEngine:
 
     # ------------------------------------------------------------------ (b)+(c) scorer
     def prepare_gallery(self, g: torch.Tensor, index_offset: int = 0) -> PreparedGallery:
-        """Device-resident gallery with its tensor-core operands.  An fp16 ``g`` stays fp16: used in place when it is
-        on this device, contiguous and 16-byte aligned (``seam_prepare_gallery_f16``: no fp32 copy, no second fp16
-        copy), else copied once to a contiguous fp16 tensor here.  Other dtypes are converted to fp32."""
-        if g.dim() != 2 or g.shape[1] != D_MODEL:
-            raise ValueError(f"gallery must be (G,256), got {tuple(g.shape)}")
-        if g.dtype == torch.float16:
-            g = g.to(self.device)
-            if not g.is_contiguous() or g.data_ptr() % 16:
-                g = g.clone(memory_format=torch.contiguous_format)
-            g16 = g
-        else:
-            g = self._f32(g, "gallery")
-            g16 = torch.empty((g.shape[0], D_MODEL), dtype=torch.float16, device=self.device)
+        """Device-resident gallery with its tensor-core operands.  An fp16 or bf16 ``g`` keeps its dtype: used in place
+        when it is on this device, contiguous and 16-byte aligned, else copied once to a contiguous tensor here.  fp16
+        rows are the tensor-core operand themselves (``seam_prepare_gallery_f16``: no fp32 copy, no second fp16
+        copy); bf16 rows get an fp16 image beside them (``seam_prepare_gallery_bf16``: no fp32 copy).  Other dtypes are
+        converted to fp32."""
+        g = self._rows(g)
+        g16 = g if g.dtype == torch.float16 else torch.empty((g.shape[0], D_MODEL), dtype=torch.float16,
+                                                             device=self.device)
         G = g.shape[0]
         cg = torch.empty((max(G, 1),), dtype=torch.float32, device=self.device)
         gstat = torch.empty((4,), dtype=torch.float32, device=self.device)
@@ -426,9 +434,10 @@ class SeamEngine:
             self._check(self._lib.seam_prepare_gallery_f16(self._h, gallery.g16.data_ptr(), gallery.G,
                                                            gallery.cg.data_ptr(), gallery.gstat.data_ptr(),
                                                            self._stream()))
-        else:
-            self._check(self._lib.seam_prepare_gallery(self._h, gallery.g.data_ptr(), gallery.G, gallery.g16.data_ptr(),
-                                                       gallery.cg.data_ptr(), gallery.gstat.data_ptr(), self._stream()))
+        else:       # fp32 or bf16 rows: both write g16
+            fn = self._lib.seam_prepare_gallery_bf16 if gallery.rows_bf16 else self._lib.seam_prepare_gallery
+            self._check(fn(self._h, gallery.g.data_ptr(), gallery.G, gallery.g16.data_ptr(), gallery.cg.data_ptr(),
+                           gallery.gstat.data_ptr(), self._stream()))
 
     def _fresh(self, gallery: PreparedGallery) -> PreparedGallery:
         """A gallery prepared under another scorer (its cg = dw . g^2 and overflow statistics are stale after
@@ -466,8 +475,8 @@ class SeamEngine:
             ws = self._workspace("score", nbytes)
             st = stats if (slab == Q or stats is None) else torch.zeros((4,), dtype=torch.int32, device=self.device)
             # an fp16 gallery has no separate rows: the _g16 entry reads g16 for both the operand and the direct form
-            fn, rows = ((self._lib.seam_score_topk_g16, ()) if gallery.rows_f16
-                        else (self._lib.seam_score_topk, (gallery.g.data_ptr(),)))
+            fn = self._track_entry("score_topk", None, gallery.row_suffix)
+            rows = () if gallery.rows_f16 else (gallery.g.data_ptr(),)
             self._check(fn(self._h, q[lo:hi].data_ptr() if n else 0, n, *rows, gallery.g16.data_ptr(),
                            gallery.cg.data_ptr(), gallery.gstat.data_ptr(), G, int(gallery.index_offset), k,
                            sc[lo:hi].data_ptr() if n else 0, mg[lo:hi].data_ptr() if n else 0,
@@ -495,7 +504,7 @@ class SeamEngine:
         stats = torch.zeros((4,), dtype=torch.int32, device=self.device) if return_stats else None
         ws = self._workspace("score", nbytes)
         # an fp16 gallery has no separate rows: the _g16 entry reads g16 for both the operand and the direct form
-        fn = self._track_entry("search", seq, gallery.rows_f16)
+        fn = self._track_entry("search", seq, gallery.row_suffix)
         rows = () if gallery.rows_f16 else (gallery.g.data_ptr(),)
         self._check(fn(self._h, seq.data_ptr() if Q else 0, _ptr(m8), _ptr(l32), Tmax, Q, seq.stride(0), seq.stride(1),
                        q.data_ptr(), *rows, gallery.g16.data_ptr(), gallery.cg.data_ptr(),
@@ -529,11 +538,11 @@ class SeamEngine:
         return out
 
     def _rows(self, g: torch.Tensor) -> torch.Tensor:
-        """Gallery rows for the direct-form kernels: an fp16 ``g`` stays fp16 (used in place when it is on this device,
-        contiguous and 16-byte aligned, else copied once, as ``prepare_gallery`` does); other dtypes become fp32."""
+        """Gallery rows for the direct-form kernels: an fp16 or bf16 ``g`` keeps its dtype (used in place when it is on
+        this device, contiguous and 16-byte aligned, else copied once); other dtypes become fp32."""
         if g.dim() != 2 or g.shape[1] != D_MODEL:
             raise ValueError(f"gallery must be (G,256), got {tuple(g.shape)}")
-        if g.dtype == torch.float16:
+        if g.dtype in (torch.float16, torch.bfloat16):
             g = g.to(self.device)
             if not g.is_contiguous() or g.data_ptr() % 16:
                 g = g.clone(memory_format=torch.contiguous_format)
@@ -552,13 +561,13 @@ class SeamEngine:
     def rank_fused_distances(self, frames: torch.Tensor, start: torch.Tensor, g: torch.Tensor, target: torch.Tensor):
         """Ranks of the true shop items under the per-product average / maximum of the frames' class-1
         probabilities (evaluate_movingfashion.py:294-316).  ``frames (N,256)`` sorted by product, ``start (P+1)``
-        CSR offsets, ``target (P)``.  An fp16 gallery ``g`` is read as fp16 (``seam_rank_fused_distances_g16``: the
-        ranks of ``g.float()``, no fp32 copy).  Returns ``(rank_avg, rank_max)`` int32 ``(P,)``; no host
-        synchronisation."""
+        CSR offsets, ``target (P)``.  An fp16 or bf16 gallery ``g`` is read as it is (``seam_rank_fused_distances_g16``
+        / ``_gbf16``: the ranks of ``g.float()``, no fp32 copy).  Returns ``(rank_avg, rank_max)`` int32 ``(P,)``; no
+        host synchronisation."""
         frames, s32, g, t32, P = self._fused_args(frames, start, g, target)
         ra = torch.empty((P,), dtype=torch.int32, device=self.device)
         rm = torch.empty((P,), dtype=torch.int32, device=self.device)
-        fn = self._lib.seam_rank_fused_distances_g16 if g.dtype == torch.float16 else self._lib.seam_rank_fused_distances
+        fn = self._track_entry("rank_fused_distances", None, ROW_SUFFIX[g.dtype])
         self._check(fn(self._h, frames.data_ptr() if frames.numel() else 0, s32.data_ptr(), P, g.data_ptr(), g.shape[0],
                        t32.data_ptr(), ra.data_ptr(), rm.data_ptr(), self._stream()))
         return ra, rm
@@ -573,7 +582,7 @@ class SeamEngine:
         frames, s32, g, t32, P = self._fused_args(frames, start, g, target)
         avg = torch.empty((P,), dtype=torch.float32, device=self.device)
         mx = torch.empty((P,), dtype=torch.float32, device=self.device)
-        fn = self._lib.seam_shard_fused_target_g16 if g.dtype == torch.float16 else self._lib.seam_shard_fused_target
+        fn = self._track_entry("shard_fused_target", None, ROW_SUFFIX[g.dtype])
         self._check(fn(self._h, frames.data_ptr() if frames.numel() else 0, s32.data_ptr(), P, g.data_ptr(), g.shape[0],
                        int(index_offset), t32.data_ptr(), avg.data_ptr() if P else 0, mx.data_ptr() if P else 0,
                        self._stream()))
@@ -593,8 +602,7 @@ class SeamEngine:
             raise ValueError("target_avg / target_max must hold one value per product")
         ca = torch.empty((P,), dtype=torch.int32, device=self.device)
         cm = torch.empty((P,), dtype=torch.int32, device=self.device)
-        fn = (self._lib.seam_shard_rank_fused_distances_g16 if g.dtype == torch.float16
-              else self._lib.seam_shard_rank_fused_distances)
+        fn = self._track_entry("shard_rank_fused_distances", None, ROW_SUFFIX[g.dtype])
         self._check(fn(self._h, frames.data_ptr() if frames.numel() else 0, s32.data_ptr(), P, g.data_ptr(), g.shape[0],
                        int(index_offset), t32.data_ptr(), ta.data_ptr() if P else 0, tm.data_ptr() if P else 0,
                        ca.data_ptr() if P else 0, cm.data_ptr() if P else 0, self._stream()))
@@ -623,8 +631,8 @@ class SeamEngine:
         if prepared and Q > 0:
             nbytes = int(self._lib.seam_rank_workspace_bytes(self._h, Q, G))
             ws = self._workspace("score", nbytes)
-            fn, rows = ((self._lib.seam_rank_of_target_prepared_g16, ()) if g.rows_f16
-                        else (self._lib.seam_rank_of_target_prepared, (gm.data_ptr(),)))
+            fn = self._track_entry("rank_of_target_prepared", None, g.row_suffix)
+            rows = () if g.rows_f16 else (gm.data_ptr(),)
             self._check(fn(self._h, q.data_ptr(), Q, *rows, g.g16.data_ptr(), g.cg.data_ptr(), g.gstat.data_ptr(), G,
                            t32.data_ptr(), rank.data_ptr(), margin.data_ptr(), stats.data_ptr(), ws.data_ptr(), ws.numel(),
                            self._stream()))
@@ -652,9 +660,8 @@ class SeamEngine:
         t32 = self._shard_targets(q, target)
         Q = q.shape[0]
         margin = torch.empty((Q,), dtype=torch.float32, device=self.device)
-        fn, rows = ((self._lib.seam_shard_target_margin_g16, gallery.g16) if gallery.rows_f16
-                    else (self._lib.seam_shard_target_margin, gallery.g))
-        self._check(fn(self._h, q.data_ptr() if Q else 0, Q, rows.data_ptr(), gallery.G, int(gallery.index_offset),
+        fn = self._track_entry("shard_target_margin", None, gallery.row_suffix)
+        self._check(fn(self._h, q.data_ptr() if Q else 0, Q, gallery.g.data_ptr(), gallery.G, int(gallery.index_offset),
                        t32.data_ptr() if Q else 0, margin.data_ptr() if Q else 0, self._stream()))
         return margin
 
@@ -676,8 +683,8 @@ class SeamEngine:
         stats = torch.zeros((4,), dtype=torch.int32, device=self.device) if return_stats else None
         if Q > 0:
             ws = self._workspace("score", int(self._lib.seam_rank_workspace_bytes(self._h, Q, G)))
-            fn, rows = ((self._lib.seam_shard_rank_count_prepared_g16, ()) if gallery.rows_f16
-                        else (self._lib.seam_shard_rank_count_prepared, (gallery.g.data_ptr(),)))
+            fn = self._track_entry("shard_rank_count_prepared", None, gallery.row_suffix)
+            rows = () if gallery.rows_f16 else (gallery.g.data_ptr(),)
             self._check(fn(self._h, q.data_ptr(), Q, *rows, gallery.g16.data_ptr(), gallery.cg.data_ptr(),
                            gallery.gstat.data_ptr(), G, int(gallery.index_offset), t32.data_ptr(), m.data_ptr(),
                            count.data_ptr(), _ptr(stats), ws.data_ptr(), ws.numel(), self._stream()))

@@ -155,7 +155,8 @@ def search_host(engine: SeamEngine, seq_h: torch.Tensor, mask_h: Optional[torch.
     """Host tensors in, host tensors out: gallery upload + preparation, chunked track upload overlapped
     with aggregation and scoring, results copied back per chunk into ``out`` (three (Q,k) host tensors:
     scores fp32, margins fp32, idx int32; allocated pinned when not given).  Returns ``out``; the caller
-    synchronises the current stream before reading it."""
+    synchronises the current stream before reading it.  An fp16 or bf16 ``gallery_h`` crosses the bus and is
+    prepared in its own dtype (half the bytes of fp32, the results of ``gallery_h.float()``)."""
     dev = engine.device
     stream = stream or HostTrackStream(engine)
     Q = seq_h.shape[1]
@@ -312,10 +313,10 @@ class ShardedRetriever:
                                   frame_last: Tuple[torch.Tensor, torch.Tensor],
                                   k_thresholds: Sequence[int] = K_THRESHOLDS):
         """``evaluate_distance_fusions`` over the sharded gallery: the same ``(ranks (2,P) int64, hits)``.
-        ``shop_desc_shard`` is this rank's rows of the frame scorer's gallery (fp32 or fp16, the same global rows as
-        ``self.gallery``); every rank passes all frames, products and targets.  The shard holding each product's target
-        computes its fused average / maximum (``-inf`` on the others), a MAX all-reduce hands them to every shard, each
-        counts its rows ranking before them (ties by global row) and a SUM all-reduce adds the counts."""
+        ``shop_desc_shard`` is this rank's rows of the frame scorer's gallery (fp32, fp16 or bf16, the same global rows
+        as ``self.gallery``); every rank passes all frames, products and targets.  The shard holding each product's
+        target computes its fused average / maximum (``-inf`` on the others), a MAX all-reduce hands them to every
+        shard, each counts its rows ranking before them (ties by global row) and a SUM all-reduce adds the counts."""
         self._check_shop_shard(shop_desc_shard)
         if self.world == 1:
             return evaluate_distance_fusions(self.ops, frame_desc, frame_product, shop_desc_shard, target, frame_last,
@@ -573,8 +574,9 @@ def evaluate_products(engine: SeamEngine, frame_desc: torch.Tensor, frame_produc
 
     ``frame_desc (N,256)`` are the match features of the tracked boxes, ``frame_product (N,)`` the product
     (0..P-1) each belongs to, ``shop_desc (G,256)`` / ``shop_aggr (G,256)`` the shop boxes' match features
-    and aggregator descriptors, ``target (P,)`` each product's shop row; ``seq`` / ``mask`` the aggregator
-    input of the P tracks.  Ranks come from ``seam_rank_of_target_prepared`` (tensor-core count + fp32 verdicts near the target), i.e.
+    and aggregator descriptors (fp32, fp16 or bf16: 16-bit ones are read as they are and rank as their fp32
+    widening), ``target (P,)`` each product's shop row; ``seq`` / ``mask`` the aggregator input of the P tracks.
+    Ranks come from ``seam_rank_of_target_prepared`` (tensor-core count + fp32 verdicts near the target), i.e.
     the position the reference reads out of its full argsort, without sorting.  The reference runs rows 0-2 in
     numpy fp16 (:82-100); these are the fp32 values of the same formulas (SURVEY.md section 0, fact 5).
     The average / maximum *distance* fusions (:294-316) reduce a (frames x gallery) score matrix per product
@@ -644,7 +646,8 @@ def evaluate_distance_fusions(engine: SeamEngine, frame_desc: torch.Tensor, fram
 
     One fused kernel for all products (``seam_rank_fused_distances``): the (frames x gallery) matrix is never
     materialised, nothing synchronises with the host (the frames are grouped by product with a device sort, the
-    hit counts are device reductions).  An fp16 ``shop_desc`` is read as fp16 (the ranks of ``shop_desc.float()``).
+    hit counts are device reductions).  An fp16 or bf16 ``shop_desc`` is read as it is (the ranks of
+    ``shop_desc.float()``).
     Returns ``(ranks (2,P) int64 [avg, max], hits (2, len(k_thresholds)) int64)``; products without frames get
     rank G; ties rank by lower index first, like ``seam_rank_of_target``.  ``max_pairs`` is accepted for
     compatibility and ignored."""
