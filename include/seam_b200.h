@@ -147,7 +147,9 @@ int seam_nlb_forward(seam_handle* h, const float* x, int B, int T, float* z, voi
 /* ---- (b)+(c) pair scorer and per-query top-k ----------------------------------------
  * Gallery preparation (once per gallery shard): fp16 copy for the tensor-core pass, the
  * per-item term cg_j = sum_k dw_k g_jk^2 (dw = last.weight[1]-last.weight[0]) and
- * gstat[0] = max_j ||g_j||_2.  g (G,256) fp32 -> g16 (G,256) fp16, cg (G) fp32, gstat (4) fp32. */
+ * gstat[0] = max_j ||g_j||_2, gstat[1] = fp16 overflow flag, gstat[2] = max_j sum_k |dw_k| g_jk^2 and
+ * gstat[3] = max_j sum_k (|W0_k| + |W1_k|) g_jk^2 (the certification bound's terms for the fp32 rounding of cg and of
+ * the direct form).  g (G,256) fp32 -> g16 (G,256) fp16, cg (G) fp32, gstat (4) fp32. */
 int seam_prepare_gallery(seam_handle* h, const float* g, int G, void* g16, float* cg, float* gstat, void* stream);
 /* Preparation of an fp16 gallery (the dtype the reference's shop-descriptor store, evaluate_movingfashion.py:82-92, and
  * torch.autocast produce): g16 (G,256) fp16, 256 contiguous halves per row, 16-byte aligned (otherwise

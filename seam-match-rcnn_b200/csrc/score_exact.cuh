@@ -21,10 +21,40 @@ namespace seam {
 namespace exact {
 
 constexpr float FP16_MAX = 65504.f;
-// bound on |fp16 tensor-core value - exact value| relative to ||a_i|| * max_j ||g_j||:
-// two operand roundings (2^-11 each) + fp32 accumulation slack.
+// Bound on |fp16 tensor-core value - exact value| (operand_err_bound), every constant of it here:
+//  - normal fp16 operands round with a RELATIVE error of 2^-11 each: EPS_COEFF ||a_i|| max_j ||g_j||;
+//  - fp16 subnormals (|x| < 2^-14) round with an ABSOLUTE error of up to 2^-25 per element, which the relative term
+//    does not see (a_i can round to zero while a_i . g_j does not vanish): 2^-25 (||g_j||_1 + ||a_i||_1)
+//    <= 2^-21 (max_j ||g_j|| + ||a_i||), as ||x||_1 <= 16 ||x|| in 256 dimensions; SUB_COEFF = 2^-20 (2x slack);
+//  - cg_j = dw . g_j^2 is summed in fp32 (a product, 8 fmas, a 5-step butterfly: 14 roundings), an error of up to
+//    14 * 2^-24 sum_k |dw_k| g_jk^2, which cancellation in dw can make large against |cg_j|: CG_COEFF = 2^-20 times
+//    max_j sum_k |dw_k| g_jk^2 (gstat[2], prep_gallery_kernel);
+//  - EPS_ABS: fp32 accumulation of values near zero.
+// The certificate also needs the fp32 direct form, which orders the re-scored items, to be within the bound of the exact
+// margin (direct_err_bound): 14 roundings along each logit's path and one for l1 - l0 give
+// |d~ - d| <= 15 * 2^-24 (sum_c sum_k |W_ck| (q_k - g_jk)^2 + |b0| + |b1|), and (q - g)^2 <= 2 q^2 + 2 g^2 bounds the sum
+// by 2 qw_i + 2 max_j gw_j with qw_i = sum_k (|W_0k| + |W_1k|) q_ik^2 (weighted_sq_norm, formed where the query's slice
+// and W are in registers already) and gw_j the same of g_j (gstat[3], prep_gallery_kernel); DIRECT_COEFF = 2^-20.  The rank band adds DIRECT_COEFF qw_i for the fp32
+// rounding of rq_i = dw . q_i^2 (14 roundings of a sum bounded by qw_i), which its target image v* = d_t - rq_i - db
+// carries.
 constexpr float EPS_COEFF = 9.9e-4f;   // 2^-10 = 9.77e-4, plus accumulation slack
+constexpr float SUB_COEFF = 9.5367431640625e-7f;   // 2^-20
+constexpr float CG_COEFF = 9.5367431640625e-7f;    // 2^-20 > 14 * 2^-24
+constexpr float DIRECT_COEFF = 9.5367431640625e-7f;  // 2^-20 > 15 * 2^-24
+constexpr float EPS_ABS = 1e-5f;
 constexpr float TAG_REL_ERR = 8e-6f;   // > 2^-17 = 7.63e-6: 6 mantissa bits replaced by a column tag
+constexpr float RANK_SLACK = 4e-6f;    // rank band: fp32 rounding of the target's margin and of its image v*
+
+// gstat: [0] max_j ||g_j||, [1] fp16 overflow flag, [2] max_j sum_k |dw_k| g_jk^2, [3] max_j gw_j (prep_gallery_kernel)
+__device__ __forceinline__ float operand_err_bound(float anorm, const float* gstat) {
+  return EPS_COEFF * anorm * gstat[0] + SUB_COEFF * (anorm + gstat[0]) + CG_COEFF * gstat[2] + EPS_ABS;
+}
+__device__ __forceinline__ float direct_err_bound(float qw, const float* gstat, float b0, float b1) {
+  return DIRECT_COEFF * (2.f * qw + 2.f * gstat[3] + fabsf(b0) + fabsf(b1));
+}
+__device__ __forceinline__ float cert_err_bound(float anorm, float qw, const float* gstat, float b0, float b1) {
+  return operand_err_bound(anorm, gstat) + direct_err_bound(qw, gstat, b0, b1);
+}
 
 __device__ __forceinline__ float softmax1(float l0, float l1) {
   const float m = fmaxf(l0, l1);
@@ -97,6 +127,16 @@ __device__ __forceinline__ void sqdiff_dot2(const Slice& q, const Slice& g, cons
   p0 = sum2(a0);
   p1 = sum2(a1);
 }
+// qw = sum_k (|W_0k| + |W_1k|) x_k^2 of a lane-sliced row, all lanes get it (the direct form's error bound)
+__device__ __forceinline__ float weighted_sq_norm(const Slice& x, const Slice& w0, const Slice& w1) {
+  const float xs[8] = {x.lo.x, x.lo.y, x.lo.z, x.lo.w, x.hi.x, x.hi.y, x.hi.z, x.hi.w};
+  const float was[8] = {w0.lo.x, w0.lo.y, w0.lo.z, w0.lo.w, w0.hi.x, w0.hi.y, w0.hi.z, w0.hi.w};
+  const float wbs[8] = {w1.lo.x, w1.lo.y, w1.lo.z, w1.lo.w, w1.hi.x, w1.hi.y, w1.hi.z, w1.hi.w};
+  float s = 0.f;
+#pragma unroll
+  for (int e = 0; e < 8; ++e) s = fmaf(fabsf(was[e]) + fabsf(wbs[e]), xs[e] * xs[e], s);
+  return ptx::warp_sum(s);
+}
 // both logits of one pair, all lanes get the result; Row: float, __half or __nv_bfloat16 gallery rows
 template <typename Row>
 __device__ __forceinline__ void pair_logits(const Slice& q, const Row* grow, const Slice& w0, const Slice& w1,
@@ -109,7 +149,8 @@ __device__ __forceinline__ void pair_logits(const Slice& q, const Row* grow, con
 }
 
 // ---------------------------------------------------------------- gallery preparation
-// warp per gallery row: fp16 copy, cg_j = dw . g_j^2, max_j ||g_j|| (gstat[0]), overflow flag (gstat[1]).
+// warp per gallery row: fp16 copy, cg_j = dw . g_j^2, max_j ||g_j|| (gstat[0]), overflow flag (gstat[1]), the bounds'
+// terms max_j sum_k |dw_k| g_jk^2 (gstat[2]) and max_j gw_j (gstat[3]).
 // Row = __half: the caller's rows are the fp16 operand already -- cg and gstat only (g16 is not written).  Row =
 // __nv_bfloat16 writes g16 as fp32 does: a bf16 value need not be an fp16 one (range, subnormals), and __float2half_rn
 // of the exactly widened value is the fp32 path's g16 bit for bit.
@@ -122,13 +163,18 @@ __global__ void __launch_bounds__(256) prep_gallery_kernel(const Row* __restrict
   if (j >= G) return;
   const Slice x = load_slice(g + (size_t)j * 256, lane);
   const Slice dw = load_slice(fold + Fold::DW, lane);
+  const Slice wa = load_slice(fold + Fold::LAST_W, lane), wb = load_slice(fold + Fold::LAST_W + 256, lane);
   const float xs[8] = {x.lo.x, x.lo.y, x.lo.z, x.lo.w, x.hi.x, x.hi.y, x.hi.z, x.hi.w};
   const float ds[8] = {dw.lo.x, dw.lo.y, dw.lo.z, dw.lo.w, dw.hi.x, dw.hi.y, dw.hi.z, dw.hi.w};
-  float c = 0.f, n2 = 0.f, amax = 0.f;
+  const float was[8] = {wa.lo.x, wa.lo.y, wa.lo.z, wa.lo.w, wa.hi.x, wa.hi.y, wa.hi.z, wa.hi.w};
+  const float wbs[8] = {wb.lo.x, wb.lo.y, wb.lo.z, wb.lo.w, wb.hi.x, wb.hi.y, wb.hi.z, wb.hi.w};
+  float c = 0.f, cabs = 0.f, gw = 0.f, n2 = 0.f, amax = 0.f;
   __half h[8];
 #pragma unroll
   for (int e = 0; e < 8; ++e) {
     c = fmaf(ds[e], xs[e] * xs[e], c);
+    cabs = fmaf(fabsf(ds[e]), xs[e] * xs[e], cabs);
+    gw = fmaf(fabsf(was[e]) + fabsf(wbs[e]), xs[e] * xs[e], gw);
     n2 = fmaf(xs[e], xs[e], n2);
     amax = fmaxf(amax, fabsf(xs[e]));
     h[e] = __float2half_rn(xs[e]);
@@ -139,11 +185,15 @@ __global__ void __launch_bounds__(256) prep_gallery_kernel(const Row* __restrict
     *reinterpret_cast<uint2*>(dst + 128 + 4 * lane) = *reinterpret_cast<const uint2*>(&h[4]);
   }
   c = ptx::warp_sum(c);
+  cabs = ptx::warp_sum(cabs);
+  gw = ptx::warp_sum(gw);
   n2 = ptx::warp_sum(n2);
   amax = ptx::warp_max(amax);
   if (lane == 0) {
     cg[j] = c;
     atomicMax(reinterpret_cast<unsigned int*>(gstat), __float_as_uint(sqrtf(n2)));   // non-negative floats
+    atomicMax(reinterpret_cast<unsigned int*>(gstat + 2), __float_as_uint(cabs));    // bound on cg's rounding
+    atomicMax(reinterpret_cast<unsigned int*>(gstat + 3), __float_as_uint(gw));      // bound on the direct form's
     if (!(amax < FP16_MAX)) atomicMax(reinterpret_cast<unsigned int*>(gstat + 1), __float_as_uint(1.f));
   }
 }
@@ -457,17 +507,17 @@ __global__ void __launch_bounds__(256) rescore_kernel(const RescoreParams p) {
   // the tensor-core pass tags the 6 low mantissa bits of a value with its column (score_tc.cuh):
   // |tagged - untagged| <= 2^-17 |value|, bounded here by the largest magnitude in the window
   const float amax = ptx::warp_max(valid ? fabsf(cv) : 0.f);
-  const float eps = EPS_COEFF * p.anorm[qi] * p.gstat[0] + 1e-5f + TAG_REL_ERR * amax;
+  const Slice qs = load_slice(qbase + (size_t)qi * 256, lane);
+  const Slice w0 = load_slice(p.fold + Fold::LAST_W, lane);
+  const Slice w1 = load_slice(p.fold + Fold::LAST_W + 256, lane);
+  const float b0 = p.fold[Fold::CONSTS + 5], b1 = p.fold[Fold::CONSTS + 6];
+  const float eps = cert_err_bound(p.anorm[qi], weighted_sq_norm(qs, w0, w1), p.gstat, b0, b1) + TAG_REL_ERR * amax;
   const float cutoff = a_k - 2.f * eps;                   // a_k = -inf when fewer than k candidates
   const bool in_S = valid && cv >= cutoff;
   const uint32_t smask = __ballot_sync(ptx::FULL_MASK, in_S);
   if (p.G > 32 && (smask >> 31)) certified = false;       // S fills the window
   const int ns = __popc(smask);                           // S is a prefix of the sorted lanes
 
-  const Slice qs = load_slice(qbase + (size_t)qi * 256, lane);
-  const Slice w0 = load_slice(p.fold + Fold::LAST_W, lane);
-  const Slice w1 = load_slice(p.fold + Fold::LAST_W + 256, lane);
-  const float b0 = p.fold[Fold::CONSTS + 5], b1 = p.fold[Fold::CONSTS + 6];
   float my_l0 = 0.f, my_l1 = 0.f;
   if (certified) {
     // four candidates per step: their 1 KB gallery rows are fetched together
@@ -976,7 +1026,7 @@ __global__ void __launch_bounds__(256) target_margin_kernel(const float* __restr
 //
 // warp per query: exact margin of the target, its image v* in the space of the tensor-core values
 // (v = d - rq - db), and the band v* +- E with E >= |w - v| for every element near the band:
-// EPS_COEFF ||a_i|| max_j ||g_j||  (fp16 operands)  +  TAG_REL_ERR (|v*| + that)  (column tag)  +  fp32 slack.
+// cert_err_bound (fp16 operands, subnormals included, the direct form) + rq's rounding  +  TAG_REL_ERR (|v*| + that)  (column tag)  +  fp32 slack.
 // EXT: the target's margin is ext_margin[qi] and no target row is read; the band is built from it in the same way,
 // with this shard's max_j ||g_j||, so it bounds the error of every row of this shard.
 template <typename Row, bool EXT>
@@ -991,14 +1041,15 @@ __global__ void __launch_bounds__(256) rank_prep_kernel(const float* __restrict_
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int qi = blockIdx.x * 8 + warp;
   if (qi >= Q) return;
+  const Slice w0 = load_slice(fold + Fold::LAST_W, lane);
+  const Slice w1 = load_slice(fold + Fold::LAST_W + 256, lane);
+  const float b0 = fold[Fold::CONSTS + 5], b1 = fold[Fold::CONSTS + 6];
+  const Slice qs = load_slice(q + (size_t)qi * 256, lane);
+  const float qw = weighted_sq_norm(qs, w0, w1);
   float dt;
   if (EXT) {
     dt = ext_margin[qi];
   } else {
-    const Slice w0 = load_slice(fold + Fold::LAST_W, lane);
-    const Slice w1 = load_slice(fold + Fold::LAST_W + 256, lane);
-    const float b0 = fold[Fold::CONSTS + 5], b1 = fold[Fold::CONSTS + 6];
-    const Slice qs = load_slice(q + (size_t)qi * 256, lane);
     float l0, l1;
     pair_logits(qs, g + (size_t)target[qi] * 256, w0, w1, b0, b1, lane, l0, l1);
     dt = l1 - l0;
@@ -1006,8 +1057,8 @@ __global__ void __launch_bounds__(256) rank_prep_kernel(const float* __restrict_
   for (int l = lane; l < nlists; l += 32) above[(size_t)qi * nlists + l] = 0;
   if (lane == 0) {
     const float vstar = dt - rq[qi] - fold[Fold::CONSTS + 4];
-    const float e0 = EPS_COEFF * anorm[qi] * gstat[0] + 1e-5f;
-    const float E = e0 + TAG_REL_ERR * (fabsf(vstar) + e0) + 4e-6f * (1.f + fabsf(dt) + fabsf(vstar));
+    const float e0 = cert_err_bound(anorm[qi], qw, gstat, b0, b1) + DIRECT_COEFF * qw;   // + rq's rounding, carried by v*
+    const float E = e0 + TAG_REL_ERR * (fabsf(vstar) + e0) + RANK_SLACK * (1.f + fabsf(dt) + fabsf(vstar));
     lo[qi] = vstar - E;
     hi[qi] = vstar + E;
     dtarget[qi] = dt;

@@ -40,7 +40,8 @@ class PreparedGallery:
                         caller's gallery has that dtype: then it is the caller's tensor (or one contiguous copy of it)
     g16  (G,256) fp16   operand of the tcgen05 pass -- the same tensor as ``g`` for an fp16 gallery
     cg   (G)     fp32   dw . g_j^2
-    gstat (4)    fp32   [max_j ||g_j||, fp16-overflow flag, -, -]
+    gstat (4)    fp32   [max_j ||g_j||, fp16-overflow flag, max_j |dw| . g_j^2, max_j (|W0| + |W1|) . g_j^2]: the last
+                        two bound the fp32 rounding of cg and of the direct form in the certificate
 
     Bytes per row: fp32 1,540 (g, g16, cg), fp16 516 (g16, cg), bf16 1,028 (g, g16, cg).  All three score the same:
     16-bit rows are widened exactly wherever the fp32 direct form reads them, and a bf16 gallery's g16 is the one its
